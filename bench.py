@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          (N > 1: launched under torch.distributed.run)
     python bench.py --impl reference ...                    (the CPU arm: the oracle port on all host cores)
+    python bench.py ... --dump-outputs DIR                  (also writes the last timed step's outputs as DIR/<name>.npy)
 
 Workload (BASELINE.json configs[2], the configuration the metric is quoted on): shems_LU1 random-action
 rollout, 2^20 instances per GPU x 8760 hourly steps on a synthetic ChargerID98-shaped 8761-row year series,
@@ -62,7 +63,13 @@ def parse():
     ap.add_argument("--cpu-sample-envs", type=int, default=0, help="0: auto-size the CPU sample to ~15 s")
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--skip-ddpg", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
+    return args
 
 
 # ------------------------------------------------------------------------------ CPU arm (oracle port)
@@ -454,6 +461,25 @@ def ddpg_dp_updates_per_s(sb, torch, dist, rank, ser_train, n_updates=300):
     return out
 
 
+DUMP_SAMPLE = 1 << 18   # instances and replay rows --dump-outputs writes at most: ~41 MB in all
+
+
+def dump_outputs(dirname, env, mem, out):
+    """--dump-outputs: what the last timed step left its caller, as float32 / float64 DIR/<name>.npy — episode return, state and row
+    index of a fixed seeded sample of the instances, and the transitions at a fixed seeded sample of the replay ring's logical
+    indices (0 = oldest).  The same arguments give the same inputs, so two builds can be compared array by array."""
+    os.makedirs(dirname, exist_ok=True)
+    rng = np.random.default_rng(0)
+    envs = np.sort(rng.choice(env.n_envs, min(env.n_envs, DUMP_SAMPLE), replace=False))
+    rows = np.sort(rng.choice(len(mem), min(len(mem), DUMP_SAMPLE), replace=False)).astype(np.int32)
+    s, a, r, s2, done = (x.cpu().numpy() for x in mem.sample(len(rows), idx=rows))
+    arrays = dict(env_ids=envs.astype(np.float64), ep_return=out["ep_return"].cpu().numpy()[envs], state=env.state[:, envs],
+                  state_idx=env.idx[envs].astype(np.float64), replay_rows=rows.astype(np.float64), replay_s=s, replay_a=a, replay_r=r,
+                  replay_s2=s2, replay_done=done)
+    for name, x in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), x)
+
+
 def main():
     args = parse()
     _quiet_stdout()
@@ -523,11 +549,13 @@ def main():
     launches0 = int(sb._lib.lib().shems_env_kernel_launches())
     ev[0].record()
     for k in range(args.steps):
-        device_step(1000 + k, True)
+        out = device_step(1000 + k, True)
     ev[1].record()
     launches_timed = int(sb._lib.lib().shems_env_kernel_launches()) - launches0   # counted by the library at its launch sites
     barrier()
     ms = ev[0].elapsed_time(ev[1])
+    if args.dump_outputs and rank == 0:        # before the e2e steps below overwrite the environment and the ring
+        dump_outputs(args.dump_outputs, env, mem, out)
     # ---- end-to-end through the public API with host buffers (`e2e`) ----
     for w in range(max(1, args.warmup // 2)):
         e2e_step(200 + w)

@@ -24,7 +24,7 @@ def dev(x):
     return torch.as_tensor(np.ascontiguousarray(x), device="cuda")
 
 
-def test_reference_driver_call_sequence(sb, O, train_series, charger98_test_series):
+def test_reference_driver_call_sequence(sb, O, train_series, charger98_test_series, tmp_path):
     T, B, MEM, NUM_EP, TEST_EVERY, TEST_RUNS = 72, 120, 72 * 12, 3, 2, 3
     rng = np.random.default_rng(7)
     P = O.params_for_charger(98)
@@ -125,7 +125,7 @@ def test_reference_driver_call_sequence(sb, O, train_series, charger98_test_seri
         r_ref, _, _ = ref_eval.step(osc)
         score_ref += float(r_ref[0])
     assert float(out["ep_return"][0]) == pytest.approx(score_ref, rel=1e-3)
-    summary = sb.tracker.write_results_csv("/tmp/_walk_results.csv", out["trace"])     # write_to_results_file
+    summary = sb.tracker.write_results_csv(str(tmp_path / "results.csv"), out["trace"])     # write_to_results_file
     assert summary["rewards"] == pytest.approx(float(out["ep_return"][0]), rel=1e-12)
     # --- inference(track < 0): the rule-based benchmark on the same data (driver :105)
     env_eval.reset(rng=-1)
