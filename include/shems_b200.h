@@ -222,6 +222,9 @@ SHEMS_API int32_t replay_destroy(ShemsReplay* rp);
 SHEMS_API int32_t replay_set_stream(ShemsReplay* rp, void* cuda_stream);
 SHEMS_API int64_t replay_length(const ShemsReplay* rp);
 SHEMS_API int64_t replay_capacity(const ShemsReplay* rp);
+/* number of env series the ring holds copies of: a rollout from a series-consistent env stores 32-byte compact records that
+ * name a row of such a copy instead of the 88-byte transition (SHEMS_RING_COMPACT=0 forces full records) */
+SHEMS_API int32_t replay_series_count(const ShemsReplay* rp);
 /* remember(s, a, r, s', done) for n transitions (memory_plotting_saving.jl:46-47);
  * a is the UNSCALED action in [-1,1] (DDPG.jl:229). done_dev may be NULL (finished == false). */
 SHEMS_API int32_t replay_push(ShemsReplay* rp, const float* s_dev /*[9][n]*/, const float* a_dev /*[2][n]*/,

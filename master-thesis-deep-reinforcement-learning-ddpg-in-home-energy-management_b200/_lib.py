@@ -92,6 +92,7 @@ SIGNATURES = {
     "replay_set_stream": (I32, [VP, VP]),
     "replay_length": (I64, [VP]),
     "replay_capacity": (I64, [VP]),
+    "replay_series_count": (I32, [VP]),
     "replay_push": (I32, [VP, VP, VP, VP, VP, VP, I64]),
     "replay_push_groups": (I32, [C.POINTER(VP), I32, VP, VP, VP, VP, VP, I64]),
     "replay_sample": (I32, [VP, I32, PI, U64, VP, VP, VP, VP, VP]),

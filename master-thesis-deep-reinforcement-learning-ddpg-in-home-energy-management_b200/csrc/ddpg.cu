@@ -859,8 +859,14 @@ ddpg_gather_kernel(const float* const* __restrict__ rings, const float* __restri
     long long slot = head - len + li;
     if (slot < 0) slot += cap;
     const float* q = ring + ring_base(slot);
-    sv = q[(RING_S + k) * 32]; s2v = q[(RING_S2 + k) * 32];
-    if (k == 0) { a0 = q[(RING_A + 0) * 32]; a1 = q[(RING_A + 1) * 32]; rv = q[RING_R * 32]; dv = q[RING_DONE * 32]; }
+    const uint32_t tag = __float_as_uint(q[RING_SRC * 32]);
+    if (tag && k >= 2) {  // compact record: s[k] / s'[k] are column k - 1 of series rows row / row + 1
+      const float* row = ring_src_row(ring, tag);
+      sv = row[k - 1]; s2v = row[8 + k - 1];
+    } else {
+      sv = q[(RING_S + k) * 32]; s2v = q[(RING_S2 + k) * 32];
+    }
+    if (k == 0) { a0 = q[(RING_A + 0) * 32]; a1 = q[(RING_A + 1) * 32]; rv = q[RING_R * 32]; dv = tag ? 0.0f : q[RING_DONE * 32]; }
   } else {
     sv = rs[k * ld + j]; s2v = rs2[k * ld + j];
     if (k == 0) { a0 = ra[j]; a1 = ra[ld + j]; rv = rr[j]; dv = rd ? rd[j] : 0.0f; }
@@ -2200,6 +2206,7 @@ ddpg_episode_post_step_kernel(float* __restrict__ ring, long long cap, long long
 #pragma unroll
   for (int k = 0; k < 9; ++k) q[(RING_S2 + k) * 32] = s2[k * n + i];
   q[RING_DONE * 32] = 0.0f;
+  q[RING_SRC * 32] = 0.0f;
   if (ep_ret) ep_ret[i] = (first ? 0.0 : ep_ret[i]) + r64[i];
 }
 

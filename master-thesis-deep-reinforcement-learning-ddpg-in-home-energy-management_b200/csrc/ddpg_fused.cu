@@ -38,6 +38,7 @@ STAMP(0, 0);
   if (tid < 8) {
     const int j = g.row0 + tid;
     unsigned long long where = (unsigned long long)j;
+    const float* ser = nullptr;
     if (ring) {
       const long long len = a.ctrl->len, head = a.ctrl->head, cap = a.ctrl->cap;
       long long li;
@@ -51,8 +52,11 @@ STAMP(0, 0);
       long long slot = head - len + li;
       if (slot < 0) slot += cap;
       where = (unsigned long long)ring_base(slot);
+      const uint32_t tag = __float_as_uint(ring[where + RING_SRC * 32]);
+      ser = tag ? ring_src_row(ring, tag) : nullptr;
     }
     S->src_row[tid] = where;
+    S->src_ser[tid] = ser;
   }
   stage_w2(S->W[0], a.actor_t + a.ao.w2, l1, l2, g.n0, g.nv, vec16, tid);   // slot 0: actor_target W2
   STAMP(0, 17);
@@ -69,11 +73,15 @@ STAMP(0, 0);
   const float b3at = __ldg(a.actor_t + a.ao.b3 + (tid & 1)), b3c = __ldg(a.critic + a.co.b3), b3ct = __ldg(a.critic_t + a.co.b3);
   STAMP(0, 19);
   __syncthreads();   // src_row
-  if (tid < 8 * RING_FIELDS) {  // thread = (row, field): the ring's field order s[9] a[2] r s'[9] done
-    const int r = tid / RING_FIELDS, f = tid - r * RING_FIELDS;
+  if (tid < 8 * RING_TRANSITION_FIELDS) {  // thread = (row, field): the ring's field order s[9] a[2] r s'[9] done
+    const int r = tid / RING_TRANSITION_FIELDS, f = tid - r * RING_TRANSITION_FIELDS;
     const unsigned long long where = S->src_row[r];
+    const float* ser = S->src_ser[r];
     float v;
-    if (ring) v = ring[where + (unsigned long long)f * 32];
+    if (ser && f >= RING_S + 2 && f < RING_A) v = ser[f - RING_S - 1];                  // compact record: s[2..8] = series row
+    else if (ser && f >= RING_S2 + 2 && f < RING_DONE) v = ser[8 + f - RING_S2 - 1];  // s'[2..8] = the next row
+    else if (ser && f == RING_DONE) v = 0.0f;
+    else if (ring) v = ring[where + (unsigned long long)f * 32];
     else if (f < RING_A) v = a.src_s[(long long)f * a.src_ld + where];
     else if (f < RING_R) v = a.src_a[(long long)(f - RING_A) * a.src_ld + where];
     else if (f == RING_R) v = a.src_r[where];

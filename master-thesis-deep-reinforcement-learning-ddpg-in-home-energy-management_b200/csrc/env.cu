@@ -318,6 +318,7 @@ struct RolloutSinks {
   float* reward_traj;  // [T][N]
   float* ring;         // replay ring (tiled SoA, common.h ring_off), capacity cap, first slot `head`
   long long cap, head;
+  uint32_t src_entry;  // COMPACT: the ring's series-table entry of this group's series, pre-shifted (ring_tag(entry, 0))
 };
 
 // Occupancy matters more than anything else here (measured, profiles/r1_rollout_sweep.md): 128 threads x >= 6 blocks/SM
@@ -332,7 +333,9 @@ struct RolloutSinks {
 // MINB = resident CTAs per SM the register budget is cut for (6: 80 registers, 7: 72, 8: 64).  6 is the fastest per wave; 7 or 8 are
 // chosen when they save a mostly empty last wave (e.g. 2^20 instances over 8 GPUs = 1024 CTAs per GPU: 1.15 waves of 148 x 6 CTAs,
 // but ONE wave of 148 x 7) — see rollout_min_blocks().
-template <int POLICY, bool WANT_TRACE, int MINB, bool FAST>
+// COMPACT: the ring sink stores 8 words per transition (Soc_b, Soc_ev, a, r, Soc_b', Soc_ev', series tag; common.h) instead of 23 —
+// only when s[2..8] is series row idx, i.e. the env is consistent.
+template <int POLICY, bool WANT_TRACE, int MINB, bool FAST, bool COMPACT>
 __global__ void __launch_bounds__(ROLLOUT_THREADS, MINB)
 shems_rollout_kernel(DevParams P, const float4* __restrict__ series, long long N, float* __restrict__ obs,
                      int32_t* __restrict__ idx_arr, int T, int step0, unsigned long long seed, long long env_id_base,
@@ -386,16 +389,23 @@ shems_rollout_kernel(DevParams P, const float4* __restrict__ series, long long N
     const Row8 nx = load_row(series, idx + 1);
     float Soc_ev_new = o.Soc_ev;
     if (nx.cd >= 0.0f && cd_here == -1.0f) Soc_ev_new = nx.soc_ev;
-    if (S.ring) {  // remember(s, a, r, s', finished) — memory_plotting_saving.jl:46-47; 22 stores at fixed 128-byte strides
+    if (S.ring) {  // remember(s, a, r, s', finished) — memory_plotting_saving.jl:46-47; stores at fixed 128-byte strides
       float* q = S.ring + ring_base(slot);
-#pragma unroll
-      for (int k = 0; k < 9; ++k) q[(RING_S + k) * 32] = st[k];
+      q[(RING_S + 0) * 32] = st[0]; q[(RING_S + 1) * 32] = st[1];
       q[(RING_A + 0) * 32] = a_raw0; q[(RING_A + 1) * 32] = a_raw1;
       q[RING_R * 32] = (float)o.reward;
-      q[(RING_S2 + 0) * 32] = o.Soc_b; q[(RING_S2 + 1) * 32] = Soc_ev_new; q[(RING_S2 + 2) * 32] = nx.cd;
-      q[(RING_S2 + 3) * 32] = nx.d_e; q[(RING_S2 + 4) * 32] = nx.g_e; q[(RING_S2 + 5) * 32] = nx.p_buy;
-      q[(RING_S2 + 6) * 32] = nx.h_cos; q[(RING_S2 + 7) * 32] = nx.h_sin; q[(RING_S2 + 8) * 32] = nx.season;
-      q[RING_DONE * 32] = 0.0f;  // finished() is always false (shems_LU1.jl:487-502)
+      q[(RING_S2 + 0) * 32] = o.Soc_b; q[(RING_S2 + 1) * 32] = Soc_ev_new;
+      if (COMPACT) {  // s[2..8] = series row idx, s'[2..8] = row idx + 1, done = 0: the tag names them
+        q[RING_SRC * 32] = __uint_as_float(S.src_entry | (uint32_t)idx);
+      } else {
+#pragma unroll
+        for (int k = 2; k < 9; ++k) q[(RING_S + k) * 32] = st[k];
+        q[(RING_S2 + 2) * 32] = nx.cd;
+        q[(RING_S2 + 3) * 32] = nx.d_e; q[(RING_S2 + 4) * 32] = nx.g_e; q[(RING_S2 + 5) * 32] = nx.p_buy;
+        q[(RING_S2 + 6) * 32] = nx.h_cos; q[(RING_S2 + 7) * 32] = nx.h_sin; q[(RING_S2 + 8) * 32] = nx.season;
+        q[RING_DONE * 32] = 0.0f;  // finished() is always false (shems_LU1.jl:487-502)
+        q[RING_SRC * 32] = 0.0f;
+      }
       slot += N;
       if (slot >= S.cap) slot -= S.cap;
     }
@@ -432,11 +442,15 @@ static inline unsigned grid_for(long long n, int block) { return (unsigned)((n +
 // Resident CTAs per SM for a rollout over n instances.  A wave of 148 x b CTAs takes about the same time for b = 6, 7, 8 per CTA slot
 // (measured: 6 is 1-3 % faster per instance, profiles/r1_rollout_sweep.md), but a sparsely filled LAST wave runs its few warps at a
 // fraction of the issue rate: cost model = full waves + the last wave's fill, floored at 0.45 (a lone warp per scheduler is latency
-// bound), times the per-instance penalty of the tighter register budget.  SHEMS_ROLLOUT_MIN_BLOCKS=6|7|8 overrides.
-static int rollout_min_blocks(int device, long long n) {
+// bound), times the per-instance penalty of the tighter register budget.  That model was measured on the store-bound kernel that
+// writes full ring records.  With compact records the kernel is issue bound and its MINB = 6 build needs only 66 registers (7 CTAs
+// per SM anyway); it was the fastest of 6 / 7 / 8 at 2^20 and at 2^17 instances (profiles/r3_ring_compact.md), so compact launches
+// take 6.  SHEMS_ROLLOUT_MIN_BLOCKS=6|7|8 overrides.
+static int rollout_min_blocks(int device, long long n, bool compact) {
   static int forced = -1;
   if (forced < 0) { const char* ev = getenv("SHEMS_ROLLOUT_MIN_BLOCKS"); forced = ev ? atoi(ev) : 0; }
   if (forced == 6 || forced == 7 || forced == 8) return forced;
+  if (compact) return 6;
   static int sms[64];
   if (device >= 0 && device < 64 && sms[device] == 0) {
     int v = 0;
@@ -455,6 +469,12 @@ static int rollout_min_blocks(int device, long long n) {
     if (cost < best_cost - 1e-9) { best_cost = cost; best = b; }
   }
   return best;
+}
+
+// Compact ring records (see common.h) unless SHEMS_RING_COMPACT=0 forces full ones (read at every rollout: the A/B switch).
+static bool ring_compact_enabled() {
+  const char* ev = getenv("SHEMS_RING_COMPACT");
+  return !(ev && atoi(ev) == 0);
 }
 
 // Shems(maxsteps, path) for G groups of instances (group g: group_sizes[g] consecutive instances with params[g] and, when
@@ -479,6 +499,8 @@ extern "C" int32_t shems_create_groups(const ShemsParams* params, int32_t n_grou
   e->device = device; e->stream = 0; e->params = params[0]; e->dp = make_dev_params(params[0]);
   e->nrows = nrows; e->maxsteps = maxsteps; e->n = n_envs; e->max_idx = 1; e->consistent = true;
   e->n_groups = n_groups;
+  static unsigned long long next_serial = 0;
+  e->serial = __atomic_add_fetch(&next_serial, 1, __ATOMIC_RELAXED);
   const int n_series = series_per_group ? n_groups : 1;
   // interleave the 8 columns into 32-byte rows
   std::vector<float> rows((size_t)n_series * nrows * 8);
@@ -718,11 +740,13 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
     REQUIRE(e->n <= rp->capacity, SHEMS_ERR_INVALID, "shems_rollout: replay capacity %lld < n_envs %lld", (long long)rp->capacity, (long long)e->n);
     S.ring = rp->ring; S.cap = rp->capacity; S.head = rp->head;
   }
-#define LAUNCH_RO_F(POL, TR, MB, FA)                                                                                                \
-  shems_rollout_kernel<POL, TR, MB, FA><<<grid_for(n1 - n0, ROLLOUT_THREADS), ROLLOUT_THREADS, 0, e->stream>>>(                          \
+#define LAUNCH_RO_F(POL, TR, MB, FA, CO)                                                                                            \
+  shems_rollout_kernel<POL, TR, MB, FA, CO><<<grid_for(n1 - n0, ROLLOUT_THREADS), ROLLOUT_THREADS, 0, e->stream>>>(                      \
       e->gdp[g], e->gseries[g], e->n, e->obs, e->idx, a->n_steps, e->step, a->seed, a->env_id_base, a->tape_dev, a->tape_unscaled, S, n0, n1)
+#define LAUNCH_RO_C(POL, TR, MB, FA)                                                                                                \
+  do { if (compact) LAUNCH_RO_F(POL, TR, MB, FA, true); else LAUNCH_RO_F(POL, TR, MB, FA, false); } while (0)
 #define LAUNCH_RO(POL, TR, MB)                                                                                                      \
-  do { if (!TR && e->gdp[g].fast_all) LAUNCH_RO_F(POL, false, MB, true); else LAUNCH_RO_F(POL, TR, MB, false); } while (0)
+  do { if (!TR && e->gdp[g].fast_all) LAUNCH_RO_C(POL, false, MB, true); else LAUNCH_RO_C(POL, TR, MB, false); } while (0)
 #define LAUNCH_RO_MB(POL)                                                                                                           \
   do {                                                                                                                              \
     if (tr) LAUNCH_RO(POL, true, ROLLOUT_MIN_BLOCKS);                                                                               \
@@ -731,9 +755,20 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
     else LAUNCH_RO(POL, false, ROLLOUT_MIN_BLOCKS);                                                                                 \
   } while (0)
   const bool tr = a->trace_dev != nullptr;
+  // compact records need s[2..8] == series row idx (consistent), a row that fits the tag and a series-table entry in the ring
+  const bool may_compact = a->replay && e->consistent && e->nrows <= (int32_t)RING_TAG_ROW_MASK && ring_compact_enabled();
   for (int g = 0; g < e->n_groups; ++g) {
     const long long n0 = e->gstart[g], n1 = e->gstart[g + 1];
-    const int mb = rollout_min_blocks(e->device, n1 - n0);
+    bool compact = false;
+    if (may_compact) {
+      int entry;
+      const int series = (int)((e->gseries[g] - e->series) / (2 * (size_t)e->nrows));
+      const int st = replay_series_entry(a->replay, e->serial, series, e->gseries[g], e->nrows, e->stream, &entry);
+      if (st) return st;
+      compact = entry >= 0;
+      S.src_entry = compact ? ring_tag(entry, 0) : 0u;
+    }
+    const int mb = rollout_min_blocks(e->device, n1 - n0, compact);
     COUNT_LAUNCH();
     switch (a->policy) {
       case SHEMS_POLICY_RULE: LAUNCH_RO_MB(SHEMS_POLICY_RULE); break;
@@ -743,6 +778,7 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
   }
 #undef LAUNCH_RO_MB
 #undef LAUNCH_RO
+#undef LAUNCH_RO_C
 #undef LAUNCH_RO_F
   CUDA_TRY(cudaGetLastError());
   e->max_idx += a->n_steps;

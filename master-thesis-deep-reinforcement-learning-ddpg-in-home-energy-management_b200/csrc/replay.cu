@@ -2,8 +2,9 @@
 // [s, a, r, s', done] (RL-SHEMS/input.jl:140; src/memory_plotting_saving.jl:31-57) as a
 // structure-of-arrays ring in HBM with on-device sampling.
 //
-// Layout: 22 float32 fields per transition (s 9, a 2, r 1, s' 9, done 1 = 88 B) in 32-slot tiles, see
-// ring_off() in common.h.  Logical index i (0 = oldest) lives in physical slot (head - length + i) mod cap.
+// Layout: 23 float32 fields per slot in 32-slot tiles, see ring_off() in common.h: a full record (s 9, a 2, r 1, s' 9, done 1 = 88 B,
+// RING_SRC = 0) or a compact one (Soc_b, Soc_ev, a 2, r, Soc_b', Soc_ev', RING_SRC = series tag: 32 B) whose other fields are rows
+// of the ring's copy of an env series.  Logical index i (0 = oldest) lives in physical slot (head - length + i) mod cap.
 #include <new>
 #include <vector>
 #include <string.h>
@@ -19,22 +20,24 @@ extern "C" int32_t replay_create(int64_t capacity, int32_t device, ShemsReplay**
   REQUIRE(rp, SHEMS_ERR_INVALID, "replay_create: out of host memory");
   memset(rp, 0, sizeof(*rp));
   rp->device = device; rp->capacity = capacity;
-  const size_t tiles = ((size_t)capacity + 31) / 32;
+  const size_t floats = RING_HEADER_FLOATS + RING_FIELDS * 32 * (((size_t)capacity + 31) / 32);
   cudaError_t st;
-  if ((st = cudaMalloc(&rp->ring, sizeof(float) * RING_FIELDS * 32 * tiles)) != cudaSuccess ||
-      (st = cudaMemset(rp->ring, 0, sizeof(float) * RING_FIELDS * 32 * tiles)) != cudaSuccess ||
+  if ((st = cudaMalloc(&rp->alloc, sizeof(float) * floats)) != cudaSuccess ||
+      (st = cudaMemset(rp->alloc, 0, sizeof(float) * floats)) != cudaSuccess ||
       (st = cudaMalloc(&rp->minmax_scratch, sizeof(float) * 18)) != cudaSuccess) {
     shems_set_error("replay_create: %s", cudaGetErrorString(st));
     replay_destroy(rp);
     return SHEMS_ERR_CUDA;
   }
+  rp->ring = rp->alloc + RING_HEADER_FLOATS;
   *out = rp;
   return SHEMS_OK;
 }
 extern "C" int32_t replay_destroy(ShemsReplay* rp) {
   if (!rp) return SHEMS_OK;
   GUARD(rp->device);
-  cudaFree(rp->ring); cudaFree(rp->idx_scratch); cudaFree(rp->minmax_scratch); cudaFree(rp->group_refs);
+  for (int i = 0; i < rp->n_src; ++i) cudaFree(rp->src[i].rows);
+  cudaFree(rp->alloc); cudaFree(rp->idx_scratch); cudaFree(rp->minmax_scratch); cudaFree(rp->group_refs);
   delete rp;
   return SHEMS_OK;
 }
@@ -45,10 +48,37 @@ extern "C" int32_t replay_set_stream(ShemsReplay* rp, void* s) {
 }
 extern "C" int64_t replay_length(const ShemsReplay* rp) { return rp ? rp->length : 0; }
 extern "C" int64_t replay_capacity(const ShemsReplay* rp) { return rp ? rp->capacity : 0; }
+extern "C" int32_t replay_series_count(const ShemsReplay* rp) { return rp ? rp->n_src : 0; }
 
 int replay_after_rollout(ShemsReplay* rp, int64_t n_written) {
   rp->head = (rp->head + n_written) % rp->capacity;
   rp->length = rp->length + n_written > rp->capacity ? rp->capacity : rp->length + n_written;
+  return SHEMS_OK;
+}
+
+int replay_series_entry(ShemsReplay* rp, unsigned long long serial, int series, const float4* rows_dev, int nrows, cudaStream_t user,
+                        int* entry) {
+  for (int i = 0; i < rp->n_src; ++i)
+    if (rp->src[i].env_serial == serial && rp->src[i].series == series) { *entry = i; return SHEMS_OK; }
+  *entry = -1;
+  if (rp->n_src == SHEMS_MAX_GROUPS) return SHEMS_OK;
+  const int i = rp->n_src;
+  float* rows = nullptr;
+  CUDA_TRY(cudaMalloc(&rows, sizeof(float) * 8 * (size_t)nrows));
+  rp->src[i].env_serial = serial; rp->src[i].series = series; rp->src[i].nrows = nrows; rp->src[i].rows = rows;
+  rp->src_ptrs[i] = rows;
+  rp->n_src = i + 1;
+  CUDA_TRY(cudaMemcpyAsync(rows, rows_dev, sizeof(float) * 8 * (size_t)nrows, cudaMemcpyDeviceToDevice, rp->stream));
+  CUDA_TRY(cudaMemcpyAsync(rp->alloc + 2 * i, &rp->src_ptrs[i], sizeof(float*), cudaMemcpyHostToDevice, rp->stream));
+  if (user != rp->stream) {  // the records that will point at the copy are written on `user`: order them after it
+    cudaEvent_t ev;
+    CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+    cudaError_t st = cudaEventRecord(ev, rp->stream);
+    if (st == cudaSuccess) st = cudaStreamWaitEvent(user, ev, 0);
+    cudaEventDestroy(ev);
+    CUDA_TRY(st);
+  }
+  *entry = i;
   return SHEMS_OK;
 }
 
@@ -69,6 +99,7 @@ replay_push_kernel(float* __restrict__ ring, long long cap, long long head, cons
 #pragma unroll
   for (int k = 0; k < 9; ++k) q[(RING_S2 + k) * 32] = s2[k * n + i];
   q[RING_DONE * 32] = done ? done[i] : 0.0f;
+  q[RING_SRC * 32] = 0.0f;
 }
 
 extern "C" int32_t replay_push(ShemsReplay* rp, const float* s_dev, const float* a_dev, const float* r_dev, const float* s2_dev,
@@ -107,6 +138,7 @@ replay_push_groups_kernel(const RingRef* __restrict__ refs, const float* __restr
 #pragma unroll
   for (int k = 0; k < 9; ++k) q[(RING_S2 + k) * 32] = s2[k * N + g];
   q[RING_DONE * 32] = done ? done[g] : 0.0f;
+  q[RING_SRC * 32] = 0.0f;
 }
 
 extern "C" int32_t replay_push_groups(ShemsReplay* const* rps, int32_t n_groups, const float* s_dev, const float* a_dev, const float* r_dev,
@@ -161,14 +193,22 @@ replay_sample_kernel(const float* __restrict__ ring, long long cap, long long he
     if (li >= len) li = len - 1;
   }
   const float* q = ring + ring_base(replay_slot(li, head, len, cap));
-#pragma unroll
-  for (int k = 0; k < 9; ++k) s[k * B + j] = q[(RING_S + k) * 32];
+  const uint32_t tag = __float_as_uint(q[RING_SRC * 32]);
+  s[j] = q[RING_S * 32]; s[B + j] = q[(RING_S + 1) * 32];
+  s2[j] = q[RING_S2 * 32]; s2[B + j] = q[(RING_S2 + 1) * 32];
   a[j] = q[(RING_A + 0) * 32];
   a[B + j] = q[(RING_A + 1) * 32];
   r[j] = q[RING_R * 32];
+  if (tag) {  // compact record: s[2..8] / s'[2..8] are series rows row / row + 1, done = 0
+    const float* row = ring_src_row(ring, tag);
 #pragma unroll
-  for (int k = 0; k < 9; ++k) s2[k * B + j] = q[(RING_S2 + k) * 32];
-  done[j] = q[RING_DONE * 32];
+    for (int k = 2; k < 9; ++k) { s[k * B + j] = row[k - 1]; s2[k * B + j] = row[8 + k - 1]; }
+    done[j] = 0.0f;
+  } else {
+#pragma unroll
+    for (int k = 2; k < 9; ++k) { s[k * B + j] = q[(RING_S + k) * 32]; s2[k * B + j] = q[(RING_S2 + k) * 32]; }
+    done[j] = q[RING_DONE * 32];
+  }
 }
 
 static int ensure_idx_scratch(ShemsReplay* rp, int64_t n) {
@@ -229,8 +269,19 @@ replay_minmax_kernel(const float* __restrict__ ring, long long cap, long long he
       if (li >= len) li = len - 1;
     }
     const float* q = ring + ring_base(replay_slot(li, head, len, cap));
+    const uint32_t tag = __float_as_uint(q[RING_SRC * 32]);
+    float v[9];
+    v[0] = q[RING_S * 32]; v[1] = q[(RING_S + 1) * 32];
+    if (tag) {  // compact record: s[2..8] is the series row
+      const float* row = ring_src_row(ring, tag);
 #pragma unroll
-    for (int k = 0; k < 9; ++k) { const float v = q[(RING_S + k) * 32]; mn[k] = fminf(mn[k], v); mx[k] = fmaxf(mx[k], v); }
+      for (int k = 2; k < 9; ++k) v[k] = row[k - 1];
+    } else {
+#pragma unroll
+      for (int k = 2; k < 9; ++k) v[k] = q[(RING_S + k) * 32];
+    }
+#pragma unroll
+    for (int k = 0; k < 9; ++k) { mn[k] = fminf(mn[k], v[k]); mx[k] = fmaxf(mx[k], v[k]); }
   }
 #pragma unroll
   for (int k = 0; k < 9; ++k) {
@@ -281,17 +332,25 @@ extern "C" int32_t replay_get(ShemsReplay* rp, float* s_host, float* a_host, flo
   const size_t tiles = ((size_t)cap + 31) / 32;
   std::vector<float> host(RING_FIELDS * 32 * tiles);
   CUDA_TRY(cudaMemcpy(host.data(), rp->ring, sizeof(float) * host.size(), cudaMemcpyDeviceToHost));
+  std::vector<std::vector<float>> rows((size_t)rp->n_src);  // the series table of the compact records
+  for (int e = 0; e < rp->n_src; ++e) {
+    rows[e].resize((size_t)8 * rp->src[e].nrows);
+    CUDA_TRY(cudaMemcpy(rows[e].data(), rp->src[e].rows, sizeof(float) * rows[e].size(), cudaMemcpyDeviceToHost));
+  }
   for (int64_t i = 0; i < len; ++i) {  // logical order, oldest first
     int64_t slot = rp->head - len + i;
     if (slot < 0) slot += cap;
     const float* q = host.data() + ring_base(slot);
+    uint32_t tag;
+    memcpy(&tag, q + RING_SRC * 32, sizeof(tag));
+    const float* row = tag ? rows[tag >> RING_TAG_ROW_BITS].data() + 8 * (size_t)((tag & RING_TAG_ROW_MASK) - 1u) : nullptr;
     for (int k = 0; k < 9; ++k) {
-      if (s_host) s_host[(size_t)k * len + i] = q[(RING_S + k) * 32];
-      if (s2_host) s2_host[(size_t)k * len + i] = q[(RING_S2 + k) * 32];
+      if (s_host) s_host[(size_t)k * len + i] = (row && k >= 2) ? row[k - 1] : q[(RING_S + k) * 32];
+      if (s2_host) s2_host[(size_t)k * len + i] = (row && k >= 2) ? row[8 + k - 1] : q[(RING_S2 + k) * 32];
     }
     if (a_host) { a_host[i] = q[(RING_A + 0) * 32]; a_host[(size_t)len + i] = q[(RING_A + 1) * 32]; }
     if (r_host) r_host[i] = q[RING_R * 32];
-    if (done_host) done_host[i] = q[RING_DONE * 32];
+    if (done_host) done_host[i] = row ? 0.0f : q[RING_DONE * 32];
   }
   return SHEMS_OK;
 }

@@ -59,6 +59,11 @@ class Replay:
     def capacity(self):
         return int(self.lib.replay_capacity(self._h))
 
+    @property
+    def series_copies(self):
+        """env series the ring holds copies of (rollouts store compact records that point into them)"""
+        return int(self.lib.replay_series_count(self._h))
+
     def push(self, s, a, r, s2, done=None):
         """remember(): s, s2 [9][n]; a [2][n] (UNSCALED action, DDPG.jl:229); r [n]; device float32 tensors."""
         n = r.numel()
