@@ -5,6 +5,7 @@
 #include <stdio.h>
 #include <stdarg.h>
 #include "../../include/shems_b200.h"
+#include "ring.cuh"  // the replay ring's record format and sampling rule
 
 // thread-local last-error string (shems_last_error)
 void shems_set_error(const char* fmt, ...);
@@ -67,42 +68,7 @@ struct DevParams {
                                 // FAST instantiation (no flag tests, no guarded division sequences) — same results
 };
 
-// ---- replay ring layout: 23 fields per slot, tiled so that one slot's fields sit at fixed 128-byte strides:
-// element (slot, k) lives at ((slot >> 5) * 23 + k) * 32 + (slot & 31).
-// A warp writing 32 consecutive slots stores one full 128-byte line per field, with the field offset an
-// immediate (no per-field address arithmetic in the rollout kernel).
-//
-// A slot holds one of two record forms, told apart by field RING_SRC:
-//   RING_SRC == 0 (all bits): a FULL record, fields 0..21 = s[9] a[2] r s'[9] done.  cudaMemset at creation makes every slot full.
-//   RING_SRC != 0: a COMPACT record written by a rollout whose state rows come from an env series: only s[0..1] (Soc_b, Soc_ev),
-//     a[0..1], r and s'[0..1] are stored; s[2..8] is series row `row` (1-based) and s'[2..8] row `row + 1` of the ring's copy of
-//     that series (entry `entry` of the ring's series table), done = 0.  RING_SRC holds the bits of ring_tag(entry, row).
-// The series table is reachable from the ring pointer alone: RING_HEADER_FLOATS floats in front of slot 0 hold SHEMS_MAX_GROUPS
-// device pointers to the ring's copies of the series (32-byte rows, as ShemsEnv::series).
-#define RING_FIELDS 23
-#define RING_S 0      // s[0..8]
-#define RING_A 9      // a[0..1]
-#define RING_R 11     // r
-#define RING_S2 12    // s'[0..8]
-#define RING_DONE 21  // done
-#define RING_SRC 22   // 0: full record; else the bits of ring_tag(entry, row) of a compact record
-#define RING_TRANSITION_FIELDS 22  // the logical transition s a r s' done
-__host__ __device__ __forceinline__ size_t ring_base(long long slot) { return ((size_t)(slot >> 5) * RING_FIELDS) * 32 + (size_t)(slot & 31); }
-__host__ __device__ __forceinline__ size_t ring_off(long long slot, int k) { return ring_base(slot) + (size_t)k * 32; }
-
 #define SHEMS_MAX_GROUPS 16
-#define RING_HEADER_FLOATS 32   // 128 bytes: SHEMS_MAX_GROUPS pointers; keeps slot 0 on a 128-byte line
-#define RING_TAG_ROW_BITS 24    // row < 2^24, entry < SHEMS_MAX_GROUPS; the row is >= 1, so a tag is never 0
-#define RING_TAG_ROW_MASK ((1u << RING_TAG_ROW_BITS) - 1u)
-__host__ __device__ __forceinline__ uint32_t ring_tag(int entry, int row1) { return ((uint32_t)entry << RING_TAG_ROW_BITS) | (uint32_t)row1; }
-#ifdef __CUDACC__
-// the 8 floats of series row `row` of a compact record's tag, (soc_ev, h_countdown, electkwh, PV_generation | p_buy, hour_cos,
-// hour_sin, season): state field k = 2..8 is column k - 1; row + 1 (s') follows at +8
-__device__ __forceinline__ const float* ring_src_row(const float* ring, uint32_t tag) {
-  const float* const* table = reinterpret_cast<const float* const*>(ring - RING_HEADER_FLOATS);
-  return table[tag >> RING_TAG_ROW_BITS] + 8 * (size_t)((tag & RING_TAG_ROW_MASK) - 1u);
-}
-#endif
 
 struct RingSeries {                // the ring's copy of one env series
   unsigned long long env_serial;   // ShemsEnv::serial of the env it was copied from (never a pointer: those get reused after free)
@@ -115,14 +81,14 @@ struct ShemsReplay {
   int device;
   cudaStream_t stream;
   int64_t capacity, length, head;  // head = physical slot of the next push
-  float* alloc;  // RING_HEADER_FLOATS header + the ring
-  float* ring;   // alloc + RING_HEADER_FLOATS: tiled SoA, see ring_off(): ceil(cap/32) tiles x 23 fields x 32 slots
+  float* alloc;  // the series-table header + the ring (ring_alloc_floats)
+  float* ring;   // ring_in_alloc(alloc): tiled SoA, see ring.cuh: ceil(cap/32) tiles x 23 fields x 32 slots
   int32_t* idx_scratch;  // device scratch for sampled indices
   int64_t idx_scratch_n;
   float* minmax_scratch; // [18]
   void* group_refs; int group_refs_n;  // device scratch of replay_push_groups (ring / capacity / head of every learner's memory)
-  RingSeries src[SHEMS_MAX_GROUPS];    // series table of the compact records (entry i <-> header pointer i)
-  const float* src_ptrs[SHEMS_MAX_GROUPS];
+  RingSeries src[RING_MAX_SERIES];     // series table of the compact records (entry i <-> header pointer i)
+  const float* src_ptrs[RING_MAX_SERIES];
   int n_src;
 };
 

@@ -836,8 +836,8 @@ ddpg_gather_kernel(const float* const* __restrict__ rings, const float* __restri
                    const int32_t* __restrict__ idx, long long idx_stride, const float* __restrict__ norm, int B, float* __restrict__ xs,
                    float* __restrict__ xs2, float* __restrict__ xspi, float* __restrict__ r, float* __restrict__ done, long long pop_stride) {
   asm volatile("griddepcontrol.launch_dependents;\n" ::: "memory");   // the forward-chain launch after it stages its weights under this kernel
-  const int g = blockIdx.x * blockDim.x + threadIdx.x;
-  const int j = g / 9, k = g - j * 9;
+  const unsigned g = blockIdx.x * blockDim.x + threadIdx.x;
+  const int j = g / 9, k = g % 9;  // unsigned: k is known to be < 9, which folds ring_field's field-range tests
   if (j >= B) return;
   {  // blockIdx.y = learner of a population: own ring, control block, indices and slab
     const long long lo = (long long)blockIdx.y * pop_stride;
@@ -848,25 +848,13 @@ ddpg_gather_kernel(const float* const* __restrict__ rings, const float* __restri
   float sv, s2v, a0 = 0.f, a1 = 0.f, rv = 0.f, dv = 0.f;
   if (ring) {
     const long long len = ctrl->len, head = ctrl->head, cap = ctrl->cap;
-    long long li;
-    if (ctrl->use_idx) li = idx[(long long)ctrl->idx_cursor * B + j];
-    else {
-      uint32_t w[4];
-      philox4x32_10(ctrl->seed, (uint64_t)j, ctrl->update, STREAM_SAMPLE, w);
-      li = (long long)(u53(w[0], w[1]) * (double)len);
-      if (li >= len) li = len - 1;
+    const long long li = ctrl->use_idx ? idx[(long long)ctrl->idx_cursor * B + j] : ring_draw(ctrl->seed, j, ctrl->update, len);
+    const float* q = ring + ring_base(ring_slot(li, head, len, cap));
+    const float* row = ring_row(ring_table(ring), q);
+    sv = ring_field(q, row, RING_S + k); s2v = ring_field(q, row, RING_S2 + k);
+    if (k == 0) {
+      a0 = ring_field(q, row, RING_A); a1 = ring_field(q, row, RING_A + 1); rv = ring_field(q, row, RING_R); dv = ring_field(q, row, RING_DONE);
     }
-    long long slot = head - len + li;
-    if (slot < 0) slot += cap;
-    const float* q = ring + ring_base(slot);
-    const uint32_t tag = __float_as_uint(q[RING_SRC * 32]);
-    if (tag && k >= 2) {  // compact record: s[k] / s'[k] are column k - 1 of series rows row / row + 1
-      const float* row = ring_src_row(ring, tag);
-      sv = row[k - 1]; s2v = row[8 + k - 1];
-    } else {
-      sv = q[(RING_S + k) * 32]; s2v = q[(RING_S2 + k) * 32];
-    }
-    if (k == 0) { a0 = q[(RING_A + 0) * 32]; a1 = q[(RING_A + 1) * 32]; rv = q[RING_R * 32]; dv = tag ? 0.0f : q[RING_DONE * 32]; }
   } else {
     sv = rs[k * ld + j]; s2v = rs2[k * ld + j];
     if (k == 0) { a0 = ra[j]; a1 = ra[ld + j]; rv = rr[j]; dv = rd ? rd[j] : 0.0f; }
@@ -2194,19 +2182,11 @@ ddpg_episode_post_step_kernel(float* __restrict__ ring, long long cap, long long
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i == 0 && ctrl) { *reinterpret_cast<CtrlHostPart*>(ctrl) = hp; rings_dev[0] = ring; }
   if (i >= n) return;
-  long long slot = head + i;
-  slot -= (slot / cap) * cap;
-  float* q = ring + ring_base(slot);
+  float* q = ring + ring_base(ring_push_slot(head, i, cap));
+  float si[9], s2i[9];
 #pragma unroll
-  for (int k = 0; k < 9; ++k) q[(RING_S + k) * 32] = s[k * n + i];
-  q[(RING_A + 0) * 32] = a[i];
-  q[(RING_A + 1) * 32] = a[n + i];
-  const float ri = r[i];
-  q[RING_R * 32] = ri;
-#pragma unroll
-  for (int k = 0; k < 9; ++k) q[(RING_S2 + k) * 32] = s2[k * n + i];
-  q[RING_DONE * 32] = 0.0f;
-  q[RING_SRC * 32] = 0.0f;
+  for (int k = 0; k < 9; ++k) { si[k] = s[k * n + i]; s2i[k] = s2[k * n + i]; }
+  ring_store_full(q, si, a[i], a[n + i], r[i], s2i, 0.0f);
   if (ep_ret) ep_ret[i] = (first ? 0.0 : ep_ret[i]) + r64[i];
 }
 

@@ -32,8 +32,8 @@ ddpg_fused_critic_kernel(const FusedArgs a) {
 STAMP(0, 0);
     cluster_arrive();  // "this CTA runs": waited for before the first write into a peer's shared memory
   STAMP(0, 16);
-  // the cluster's 8 transitions: Philox (or host-supplied) indices into the replay ring, as ddpg_gather_kernel draws them (replay.cu
-  // sample spec: counter = (row, update number), stream SAMPLE), or the rows of a caller-supplied minibatch
+  // the cluster's 8 transitions: ring_draw (or host-supplied) indices into the replay ring, as ddpg_gather_kernel draws them, or the
+  // rows of a caller-supplied minibatch
   const float* ring = a.rings ? a.rings[0] : nullptr;
   if (tid < 8) {
     const int j = g.row0 + tid;
@@ -41,19 +41,9 @@ STAMP(0, 0);
     const float* ser = nullptr;
     if (ring) {
       const long long len = a.ctrl->len, head = a.ctrl->head, cap = a.ctrl->cap;
-      long long li;
-      if (a.ctrl->use_idx) li = a.idx[(long long)a.ctrl->idx_cursor * a.B + j];
-      else {
-        uint32_t w[4];
-        philox4x32_10(a.ctrl->seed, (uint64_t)j, a.ctrl->update, STREAM_SAMPLE, w);
-        li = (long long)(u53(w[0], w[1]) * (double)len);
-        if (li >= len) li = len - 1;
-      }
-      long long slot = head - len + li;
-      if (slot < 0) slot += cap;
-      where = (unsigned long long)ring_base(slot);
-      const uint32_t tag = __float_as_uint(ring[where + RING_SRC * 32]);
-      ser = tag ? ring_src_row(ring, tag) : nullptr;
+      const long long li = a.ctrl->use_idx ? a.idx[(long long)a.ctrl->idx_cursor * a.B + j] : ring_draw(a.ctrl->seed, j, a.ctrl->update, len);
+      where = (unsigned long long)ring_base(ring_slot(li, head, len, cap));
+      ser = ring_row(ring_table(ring), ring + where);
     }
     S->src_row[tid] = where;
     S->src_ser[tid] = ser;
@@ -76,12 +66,8 @@ STAMP(0, 0);
   if (tid < 8 * RING_TRANSITION_FIELDS) {  // thread = (row, field): the ring's field order s[9] a[2] r s'[9] done
     const int r = tid / RING_TRANSITION_FIELDS, f = tid - r * RING_TRANSITION_FIELDS;
     const unsigned long long where = S->src_row[r];
-    const float* ser = S->src_ser[r];
     float v;
-    if (ser && f >= RING_S + 2 && f < RING_A) v = ser[f - RING_S - 1];                  // compact record: s[2..8] = series row
-    else if (ser && f >= RING_S2 + 2 && f < RING_DONE) v = ser[8 + f - RING_S2 - 1];  // s'[2..8] = the next row
-    else if (ser && f == RING_DONE) v = 0.0f;
-    else if (ring) v = ring[where + (unsigned long long)f * 32];
+    if (ring) v = ring_field(ring + where, S->src_ser[r], f);
     else if (f < RING_A) v = a.src_s[(long long)f * a.src_ld + where];
     else if (f < RING_R) v = a.src_a[(long long)(f - RING_A) * a.src_ld + where];
     else if (f == RING_R) v = a.src_r[where];

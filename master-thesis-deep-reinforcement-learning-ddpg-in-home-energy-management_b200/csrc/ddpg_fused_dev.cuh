@@ -36,7 +36,7 @@ struct FusedSmem {
   float dout[8 * 2];               // gradient at the net's output [row][j]
   float qv[8], rr[8], dd[8];
   unsigned long long src_row[8];   // where the cluster's 8 sampled transitions live (ring offset or column of the caller's arrays)
-  const float* src_ser[8];         // a compact ring record's series row (common.h ring_src_row), else NULL
+  const float* src_ser[8];         // a compact ring record's series row (ring.cuh ring_row), else NULL
 };
 
 __device__ __forceinline__ void cp_async4z(float* smem_dst, const float* gsrc, bool valid) {

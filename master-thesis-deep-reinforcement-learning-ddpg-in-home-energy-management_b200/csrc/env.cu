@@ -316,7 +316,7 @@ struct RolloutSinks {
   double* trace;       // [T][23][N]
   float* obs_traj;     // [T][9][N]
   float* reward_traj;  // [T][N]
-  float* ring;         // replay ring (tiled SoA, common.h ring_off), capacity cap, first slot `head`
+  float* ring;         // replay ring (tiled SoA, ring.cuh), capacity cap, first slot `head`
   long long cap, head;
   uint32_t src_entry;  // COMPACT: the ring's series-table entry of this group's series, pre-shifted (ring_tag(entry, 0))
 };
@@ -333,7 +333,7 @@ struct RolloutSinks {
 // MINB = resident CTAs per SM the register budget is cut for (6: 80 registers, 7: 72, 8: 64).  6 is the fastest per wave; 7 or 8 are
 // chosen when they save a mostly empty last wave (e.g. 2^20 instances over 8 GPUs = 1024 CTAs per GPU: 1.15 waves of 148 x 6 CTAs,
 // but ONE wave of 148 x 7) — see rollout_min_blocks().
-// COMPACT: the ring sink stores 8 words per transition (Soc_b, Soc_ev, a, r, Soc_b', Soc_ev', series tag; common.h) instead of 23 —
+// COMPACT: the ring sink stores 8 words per transition (Soc_b, Soc_ev, a, r, Soc_b', Soc_ev', series tag; ring.cuh) instead of 23 —
 // only when s[2..8] is series row idx, i.e. the env is consistent.
 template <int POLICY, bool WANT_TRACE, int MINB, bool FAST, bool COMPACT>
 __global__ void __launch_bounds__(ROLLOUT_THREADS, MINB)
@@ -391,20 +391,13 @@ shems_rollout_kernel(DevParams P, const float4* __restrict__ series, long long N
     if (nx.cd >= 0.0f && cd_here == -1.0f) Soc_ev_new = nx.soc_ev;
     if (S.ring) {  // remember(s, a, r, s', finished) — memory_plotting_saving.jl:46-47; stores at fixed 128-byte strides
       float* q = S.ring + ring_base(slot);
-      q[(RING_S + 0) * 32] = st[0]; q[(RING_S + 1) * 32] = st[1];
-      q[(RING_A + 0) * 32] = a_raw0; q[(RING_A + 1) * 32] = a_raw1;
-      q[RING_R * 32] = (float)o.reward;
-      q[(RING_S2 + 0) * 32] = o.Soc_b; q[(RING_S2 + 1) * 32] = Soc_ev_new;
       if (COMPACT) {  // s[2..8] = series row idx, s'[2..8] = row idx + 1, done = 0: the tag names them
-        q[RING_SRC * 32] = __uint_as_float(S.src_entry | (uint32_t)idx);
+        ring_store_compact(q, st[0], st[1], a_raw0, a_raw1, (float)o.reward, o.Soc_b, Soc_ev_new, S.src_entry, idx);
       } else {
-#pragma unroll
-        for (int k = 2; k < 9; ++k) q[(RING_S + k) * 32] = st[k];
-        q[(RING_S2 + 2) * 32] = nx.cd;
-        q[(RING_S2 + 3) * 32] = nx.d_e; q[(RING_S2 + 4) * 32] = nx.g_e; q[(RING_S2 + 5) * 32] = nx.p_buy;
-        q[(RING_S2 + 6) * 32] = nx.h_cos; q[(RING_S2 + 7) * 32] = nx.h_sin; q[(RING_S2 + 8) * 32] = nx.season;
-        q[RING_DONE * 32] = 0.0f;  // finished() is always false (shems_LU1.jl:487-502)
-        q[RING_SRC * 32] = 0.0f;
+        // sv copies st: passing st itself takes its address, and the kernel then compiles to a different register allocation
+        const float sv[9] = {st[0], st[1], st[2], st[3], st[4], st[5], st[6], st[7], st[8]};
+        const float s2v[9] = {o.Soc_b, Soc_ev_new, nx.cd, nx.d_e, nx.g_e, nx.p_buy, nx.h_cos, nx.h_sin, nx.season};
+        ring_store_full(q, sv, a_raw0, a_raw1, (float)o.reward, s2v, 0.0f);  // finished() is always false (shems_LU1.jl:487-502)
       }
       slot += N;
       if (slot >= S.cap) slot -= S.cap;
@@ -471,7 +464,7 @@ static int rollout_min_blocks(int device, long long n, bool compact) {
   return best;
 }
 
-// Compact ring records (see common.h) unless SHEMS_RING_COMPACT=0 forces full ones (read at every rollout: the A/B switch).
+// Compact ring records (see ring.cuh) unless SHEMS_RING_COMPACT=0 forces full ones (read at every rollout: the A/B switch).
 static bool ring_compact_enabled() {
   const char* ev = getenv("SHEMS_RING_COMPACT");
   return !(ev && atoi(ev) == 0);
@@ -756,7 +749,7 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
   } while (0)
   const bool tr = a->trace_dev != nullptr;
   // compact records need s[2..8] == series row idx (consistent), a row that fits the tag and a series-table entry in the ring
-  const bool may_compact = a->replay && e->consistent && e->nrows <= (int32_t)RING_TAG_ROW_MASK && ring_compact_enabled();
+  const bool may_compact = a->replay && e->consistent && e->nrows <= RING_TAG_MAX_ROW && ring_compact_enabled();
   for (int g = 0; g < e->n_groups; ++g) {
     const long long n0 = e->gstart[g], n1 = e->gstart[g + 1];
     bool compact = false;

@@ -2,15 +2,13 @@
 // [s, a, r, s', done] (RL-SHEMS/input.jl:140; src/memory_plotting_saving.jl:31-57) as a
 // structure-of-arrays ring in HBM with on-device sampling.
 //
-// Layout: 23 float32 fields per slot in 32-slot tiles, see ring_off() in common.h: a full record (s 9, a 2, r 1, s' 9, done 1 = 88 B,
-// RING_SRC = 0) or a compact one (Soc_b, Soc_ev, a 2, r, Soc_b', Soc_ev', RING_SRC = series tag: 32 B) whose other fields are rows
-// of the ring's copy of an env series.  Logical index i (0 = oldest) lives in physical slot (head - length + i) mod cap.
+// Layout: 23 float32 fields per slot in 32-slot tiles, see ring.cuh: a full record (s 9, a 2, r 1, s' 9, done 1 = 88 B) or a compact
+// one (Soc_b, Soc_ev, a 2, r, Soc_b', Soc_ev', series tag: 32 B) whose other fields are rows of the ring's copy of an env series.
 #include <new>
 #include <vector>
 #include <string.h>
 
 #include "common.h"
-#include "philox.cuh"
 
 extern "C" int32_t replay_create(int64_t capacity, int32_t device, ShemsReplay** out) {
   REQUIRE(out && capacity >= 1, SHEMS_ERR_INVALID, "replay_create: capacity=%lld", (long long)capacity);
@@ -20,7 +18,7 @@ extern "C" int32_t replay_create(int64_t capacity, int32_t device, ShemsReplay**
   REQUIRE(rp, SHEMS_ERR_INVALID, "replay_create: out of host memory");
   memset(rp, 0, sizeof(*rp));
   rp->device = device; rp->capacity = capacity;
-  const size_t floats = RING_HEADER_FLOATS + RING_FIELDS * 32 * (((size_t)capacity + 31) / 32);
+  const size_t floats = ring_alloc_floats(capacity);
   cudaError_t st;
   if ((st = cudaMalloc(&rp->alloc, sizeof(float) * floats)) != cudaSuccess ||
       (st = cudaMemset(rp->alloc, 0, sizeof(float) * floats)) != cudaSuccess ||
@@ -29,7 +27,7 @@ extern "C" int32_t replay_create(int64_t capacity, int32_t device, ShemsReplay**
     replay_destroy(rp);
     return SHEMS_ERR_CUDA;
   }
-  rp->ring = rp->alloc + RING_HEADER_FLOATS;
+  rp->ring = ring_in_alloc(rp->alloc);
   *out = rp;
   return SHEMS_OK;
 }
@@ -61,7 +59,7 @@ int replay_series_entry(ShemsReplay* rp, unsigned long long serial, int series, 
   for (int i = 0; i < rp->n_src; ++i)
     if (rp->src[i].env_serial == serial && rp->src[i].series == series) { *entry = i; return SHEMS_OK; }
   *entry = -1;
-  if (rp->n_src == SHEMS_MAX_GROUPS) return SHEMS_OK;
+  if (rp->n_src == RING_MAX_SERIES) return SHEMS_OK;
   const int i = rp->n_src;
   float* rows = nullptr;
   CUDA_TRY(cudaMalloc(&rows, sizeof(float) * 8 * (size_t)nrows));
@@ -69,7 +67,7 @@ int replay_series_entry(ShemsReplay* rp, unsigned long long serial, int series, 
   rp->src_ptrs[i] = rows;
   rp->n_src = i + 1;
   CUDA_TRY(cudaMemcpyAsync(rows, rows_dev, sizeof(float) * 8 * (size_t)nrows, cudaMemcpyDeviceToDevice, rp->stream));
-  CUDA_TRY(cudaMemcpyAsync(rp->alloc + 2 * i, &rp->src_ptrs[i], sizeof(float*), cudaMemcpyHostToDevice, rp->stream));
+  CUDA_TRY(cudaMemcpyAsync((void*)(ring_table(rp->ring) + i), &rp->src_ptrs[i], sizeof(float*), cudaMemcpyHostToDevice, rp->stream));
   if (user != rp->stream) {  // the records that will point at the copy are written on `user`: order them after it
     cudaEvent_t ev;
     CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
@@ -88,18 +86,11 @@ replay_push_kernel(float* __restrict__ ring, long long cap, long long head, cons
                    const float* __restrict__ r, const float* __restrict__ s2, const float* __restrict__ done, long long n, long long first) {
   const long long i = first + (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  long long slot = head + i;
-  slot -= (slot / cap) * cap;
-  float* q = ring + ring_base(slot);
+  float* q = ring + ring_base(ring_push_slot(head, i, cap));
+  float si[9], s2i[9];
 #pragma unroll
-  for (int k = 0; k < 9; ++k) q[(RING_S + k) * 32] = s[k * n + i];
-  q[(RING_A + 0) * 32] = a[i];
-  q[(RING_A + 1) * 32] = a[n + i];
-  q[RING_R * 32] = r[i];
-#pragma unroll
-  for (int k = 0; k < 9; ++k) q[(RING_S2 + k) * 32] = s2[k * n + i];
-  q[RING_DONE * 32] = done ? done[i] : 0.0f;
-  q[RING_SRC * 32] = 0.0f;
+  for (int k = 0; k < 9; ++k) { si[k] = s[k * n + i]; s2i[k] = s2[k * n + i]; }
+  ring_store_full(q, si, a[i], a[n + i], r[i], s2i, done ? done[i] : 0.0f);
 }
 
 extern "C" int32_t replay_push(ShemsReplay* rp, const float* s_dev, const float* a_dev, const float* r_dev, const float* s2_dev,
@@ -127,18 +118,11 @@ replay_push_groups_kernel(const RingRef* __restrict__ refs, const float* __restr
   if (i >= n_per) return;
   const RingRef ref = refs[blockIdx.y];
   const long long g = (long long)blockIdx.y * n_per + i;  // global instance
-  long long slot = ref.head + i;
-  slot -= (slot / ref.cap) * ref.cap;
-  float* q = ref.ring + ring_base(slot);
+  float* q = ref.ring + ring_base(ring_push_slot(ref.head, i, ref.cap));
+  float sg[9], s2g[9];
 #pragma unroll
-  for (int k = 0; k < 9; ++k) q[(RING_S + k) * 32] = s[k * N + g];
-  q[(RING_A + 0) * 32] = a[g];
-  q[(RING_A + 1) * 32] = a[N + g];
-  q[RING_R * 32] = r[g];
-#pragma unroll
-  for (int k = 0; k < 9; ++k) q[(RING_S2 + k) * 32] = s2[k * N + g];
-  q[RING_DONE * 32] = done ? done[g] : 0.0f;
-  q[RING_SRC * 32] = 0.0f;
+  for (int k = 0; k < 9; ++k) { sg[k] = s[k * N + g]; s2g[k] = s2[k * N + g]; }
+  ring_store_full(q, sg, a[g], a[N + g], r[g], s2g, done ? done[g] : 0.0f);
 }
 
 extern "C" int32_t replay_push_groups(ShemsReplay* const* rps, int32_t n_groups, const float* s_dev, const float* a_dev, const float* r_dev,
@@ -172,43 +156,22 @@ extern "C" int32_t replay_push_groups(ShemsReplay* const* rps, int32_t n_groups,
 }
 
 // getData(): gather B sampled transitions into SoA minibatch arrays [k][B].
-// idx != NULL: logical indices; else Philox(seed, id = draw j, ctr = update) -> floor(u * len).
-__device__ __forceinline__ long long replay_slot(long long logical, long long head, long long len, long long cap) {
-  long long slot = head - len + logical;
-  if (slot < 0) slot += cap;
-  return slot;
-}
+// idx != NULL: logical indices; else ring_draw(seed, j, update).
 __global__ void __launch_bounds__(128)
 replay_sample_kernel(const float* __restrict__ ring, long long cap, long long head, long long len, const int32_t* __restrict__ idx,
                      unsigned long long seed, unsigned update, int B, float* __restrict__ s, float* __restrict__ a, float* __restrict__ r,
                      float* __restrict__ s2, float* __restrict__ done) {
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= B) return;
-  long long li;
-  if (idx) li = idx[j];
-  else {
-    uint32_t w[4];
-    philox4x32_10(seed, (uint64_t)j, update, STREAM_SAMPLE, w);
-    li = (long long)(u53(w[0], w[1]) * (double)len);
-    if (li >= len) li = len - 1;
-  }
-  const float* q = ring + ring_base(replay_slot(li, head, len, cap));
-  const uint32_t tag = __float_as_uint(q[RING_SRC * 32]);
-  s[j] = q[RING_S * 32]; s[B + j] = q[(RING_S + 1) * 32];
-  s2[j] = q[RING_S2 * 32]; s2[B + j] = q[(RING_S2 + 1) * 32];
-  a[j] = q[(RING_A + 0) * 32];
-  a[B + j] = q[(RING_A + 1) * 32];
-  r[j] = q[RING_R * 32];
-  if (tag) {  // compact record: s[2..8] / s'[2..8] are series rows row / row + 1, done = 0
-    const float* row = ring_src_row(ring, tag);
+  const long long li = idx ? idx[j] : ring_draw(seed, j, update, len);
+  const float* q = ring + ring_base(ring_slot(li, head, len, cap));
+  const float* row = ring_row(ring_table(ring), q);
 #pragma unroll
-    for (int k = 2; k < 9; ++k) { s[k * B + j] = row[k - 1]; s2[k * B + j] = row[8 + k - 1]; }
-    done[j] = 0.0f;
-  } else {
-#pragma unroll
-    for (int k = 2; k < 9; ++k) { s[k * B + j] = q[(RING_S + k) * 32]; s2[k * B + j] = q[(RING_S2 + k) * 32]; }
-    done[j] = q[RING_DONE * 32];
-  }
+  for (int k = 0; k < 9; ++k) { s[k * B + j] = ring_field(q, row, RING_S + k); s2[k * B + j] = ring_field(q, row, RING_S2 + k); }
+  a[j] = ring_field(q, row, RING_A);
+  a[B + j] = ring_field(q, row, RING_A + 1);
+  r[j] = ring_field(q, row, RING_R);
+  done[j] = ring_field(q, row, RING_DONE);
 }
 
 static int ensure_idx_scratch(ShemsReplay* rp, int64_t n) {
@@ -260,28 +223,14 @@ replay_minmax_kernel(const float* __restrict__ ring, long long cap, long long he
 #pragma unroll
   for (int k = 0; k < 9; ++k) { mn[k] = INFINITY; mx[k] = -INFINITY; }
   for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (long long)gridDim.x * blockDim.x) {
-    long long li;
-    if (idx) li = idx[j];
-    else {
-      uint32_t w[4];
-      philox4x32_10(seed, (uint64_t)j, 0u, STREAM_SAMPLE, w);
-      li = (long long)(u53(w[0], w[1]) * (double)len);
-      if (li >= len) li = len - 1;
+    const long long li = idx ? idx[j] : ring_draw(seed, j, 0u, len);
+    const float* q = ring + ring_base(ring_slot(li, head, len, cap));
+    const float* row = ring_row(ring_table(ring), q);
+#pragma unroll
+    for (int k = 0; k < 9; ++k) {
+      const float v = ring_field(q, row, RING_S + k);
+      mn[k] = fminf(mn[k], v); mx[k] = fmaxf(mx[k], v);
     }
-    const float* q = ring + ring_base(replay_slot(li, head, len, cap));
-    const uint32_t tag = __float_as_uint(q[RING_SRC * 32]);
-    float v[9];
-    v[0] = q[RING_S * 32]; v[1] = q[(RING_S + 1) * 32];
-    if (tag) {  // compact record: s[2..8] is the series row
-      const float* row = ring_src_row(ring, tag);
-#pragma unroll
-      for (int k = 2; k < 9; ++k) v[k] = row[k - 1];
-    } else {
-#pragma unroll
-      for (int k = 2; k < 9; ++k) v[k] = q[(RING_S + k) * 32];
-    }
-#pragma unroll
-    for (int k = 0; k < 9; ++k) { mn[k] = fminf(mn[k], v[k]); mx[k] = fmaxf(mx[k], v[k]); }
   }
 #pragma unroll
   for (int k = 0; k < 9; ++k) {
@@ -329,28 +278,26 @@ extern "C" int32_t replay_get(ShemsReplay* rp, float* s_host, float* a_host, flo
   const int64_t len = rp->length, cap = rp->capacity;
   if (len == 0) return SHEMS_OK;
   CUDA_TRY(cudaStreamSynchronize(rp->stream));
-  const size_t tiles = ((size_t)cap + 31) / 32;
-  std::vector<float> host(RING_FIELDS * 32 * tiles);
-  CUDA_TRY(cudaMemcpy(host.data(), rp->ring, sizeof(float) * host.size(), cudaMemcpyDeviceToHost));
-  std::vector<std::vector<float>> rows((size_t)rp->n_src);  // the series table of the compact records
+  std::vector<float> host(ring_alloc_floats(cap));
+  CUDA_TRY(cudaMemcpy(host.data(), rp->alloc, sizeof(float) * host.size(), cudaMemcpyDeviceToHost));
+  const float* ring = ring_in_alloc(host.data());
+  std::vector<std::vector<float>> rows((size_t)rp->n_src);  // host copies of the series table of the compact records
+  std::vector<const float*> table((size_t)rp->n_src);
   for (int e = 0; e < rp->n_src; ++e) {
     rows[e].resize((size_t)8 * rp->src[e].nrows);
     CUDA_TRY(cudaMemcpy(rows[e].data(), rp->src[e].rows, sizeof(float) * rows[e].size(), cudaMemcpyDeviceToHost));
+    table[e] = rows[e].data();
   }
   for (int64_t i = 0; i < len; ++i) {  // logical order, oldest first
-    int64_t slot = rp->head - len + i;
-    if (slot < 0) slot += cap;
-    const float* q = host.data() + ring_base(slot);
-    uint32_t tag;
-    memcpy(&tag, q + RING_SRC * 32, sizeof(tag));
-    const float* row = tag ? rows[tag >> RING_TAG_ROW_BITS].data() + 8 * (size_t)((tag & RING_TAG_ROW_MASK) - 1u) : nullptr;
+    const float* q = ring + ring_base(ring_slot(i, rp->head, len, cap));
+    const float* row = ring_row(table.data(), q);
     for (int k = 0; k < 9; ++k) {
-      if (s_host) s_host[(size_t)k * len + i] = (row && k >= 2) ? row[k - 1] : q[(RING_S + k) * 32];
-      if (s2_host) s2_host[(size_t)k * len + i] = (row && k >= 2) ? row[8 + k - 1] : q[(RING_S2 + k) * 32];
+      if (s_host) s_host[(size_t)k * len + i] = ring_field(q, row, RING_S + k);
+      if (s2_host) s2_host[(size_t)k * len + i] = ring_field(q, row, RING_S2 + k);
     }
-    if (a_host) { a_host[i] = q[(RING_A + 0) * 32]; a_host[(size_t)len + i] = q[(RING_A + 1) * 32]; }
-    if (r_host) r_host[i] = q[RING_R * 32];
-    if (done_host) done_host[i] = row ? 0.0f : q[RING_DONE * 32];
+    if (a_host) { a_host[i] = ring_field(q, row, RING_A); a_host[(size_t)len + i] = ring_field(q, row, RING_A + 1); }
+    if (r_host) r_host[i] = ring_field(q, row, RING_R);
+    if (done_host) done_host[i] = ring_field(q, row, RING_DONE);
   }
   return SHEMS_OK;
 }

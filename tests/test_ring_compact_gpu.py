@@ -1,4 +1,4 @@
-"""Compact replay records (csrc/common.h): a rollout from a series-consistent env stores 8 words per transition and names the
+"""Compact replay records (csrc/ring.cuh): a rollout from a series-consistent env stores 8 words per transition and names the
 series rows that hold the other 14 fields.  Every reader must hand back exactly the bits a full 22-field record gives.
 
 Each case fills two rings the same way, one with SHEMS_RING_COMPACT=0 (full records only) and one with compact records allowed,
