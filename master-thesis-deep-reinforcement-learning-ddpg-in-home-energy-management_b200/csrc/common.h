@@ -52,7 +52,9 @@ struct DevParams {
   float one_m_l_e;   // Float32(Float32(1 - b.loss) - 1f-7)
   float C;           // ev.soc_max - ev.soc_min
   float span;        // b.soc_max - b.soc_min
-  float R_f;         // Float32(b.rate_max) (only where the Float64 min is provably equivalent)
+  float R_f;         // Float32(b.rate_max) = RN32(R)
+  float R_dn, R_up;  // RD32(R), RU32(R): Float32 comparisons with R (FAST: charge_request_f / discharge_request_f)
+  float smax95_up;   // RU32(smax95)
   double R, sell, dw, pot;
   double pw_d;               // Float64 penalty weight of the sibling envs (pen_f64 != 0)
   int pen_f64, reward_form;

@@ -127,6 +127,17 @@ static int verify_fdiv_const(float d) {
   return ok;
 }
 
+// RD32(c) / RU32(c): the Float32 neighbours of a Float64 c (c itself when it is Float32-valued); for Float32 x,
+// x > c <=> x > RD32(c) and x < c <=> x < RU32(c)
+static float f32_round_down(double c) {
+  const float f = (float)c;
+  return ((double)f > c) ? nextafterf(f, -INFINITY) : f;
+}
+static float f32_round_up(double c) {
+  const float f = (float)c;
+  return ((double)f < c) ? nextafterf(f, INFINITY) : f;
+}
+
 static DevParams make_dev_params(const ShemsParams& p) {
   DevParams d;
   d.pv_eta = p.pv_eta; d.b_eta = p.b_eta; d.smin = p.b_soc_min; d.smax = p.b_soc_max; d.loss = p.b_loss;
@@ -149,6 +160,7 @@ static DevParams make_dev_params(const ShemsParams& p) {
   // eta_d and C_d are converted Float32 values by construction (<= 24 significant bits): see ddiv_const
   d.fast_d = ((double)(float)d.eta_d == d.eta_d) && ((double)(float)d.C_d == d.C_d) && d.eta_d != 0.0 && d.C_d != 0.0;
   d.span_d = (double)d.span; d.r_span_d = 1.0 / d.span_d;
+  d.R_dn = f32_round_down(d.R); d.R_up = f32_round_up(d.R); d.smax95_up = f32_round_up(d.smax95);
   d.fast_all = d.fast_d && d.span_d != 0.0 && d.span == d.span && fabs(d.span_d) < 1e30 && !d.pen_f64 && d.reward_mode == 0;
   return d;
 }
@@ -302,7 +314,7 @@ shems_action_kernel(DevParams P, long long N, const float* __restrict__ obs, con
   const long long n = n0 + (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (n >= n1) return;
   float B, EV;
-  if (RULE) shems_action_rule(P, obs[0 * N + n], obs[1 * N + n], obs[3 * N + n], obs[4 * N + n], B, EV);
+  if (RULE) shems_action_rule<false>(P, obs[0 * N + n], obs[1 * N + n], obs[3 * N + n], obs[4 * N + n], B, EV);
   else shems_action_drl<false>(P, obs[0 * N + n], obs[1 * N + n], obs[2 * N + n], obs[3 * N + n], obs[4 * N + n], target[n], target[N + n], B, EV);
   bev[n] = B;
   bev[N + n] = EV;
@@ -357,17 +369,16 @@ shems_rollout_kernel(DevParams P, const float4* __restrict__ series, long long N
     float B, EV, Bt, EVt, a_raw0, a_raw1;
     bool track_neg = false;
     if (POLICY == SHEMS_POLICY_RULE) {  // DDPG.jl:209-212
-      shems_action_rule(P, s.Soc_b, s.Soc_ev, s.d_e, s.g_e, B, EV);
+      shems_action_rule<FAST>(P, s.Soc_b, s.Soc_ev, s.d_e, s.g_e, B, EV);
       Bt = 0.0f; EVt = 0.0f; a_raw0 = B; a_raw1 = EV; track_neg = true;
     } else {
       if (POLICY == SHEMS_POLICY_RANDOM) {  // memory_plotting_saving.jl:14-19
-        // one Philox block per two steps; u = w * 2^-32; a = Float32(2u - 1).  1 + u is assembled in the
-        // significand of a double in [1, 2): 2 (1 + u) - 3 == 2u - 1 exactly.
+        // one Philox block per two steps; u = w * 2^-32; a = Float32(2u - 1) (action_from_word, philox.cuh)
         const unsigned st_abs = (unsigned)(step0 + t);
         if (t == 0 || (st_abs & 1u) == 0u) philox4x32_10(seed, (uint64_t)(env_id_base + n), st_abs >> 1, STREAM_ACTION, rw);
         const uint32_t w0 = (st_abs & 1u) ? rw[2] : rw[0], w1 = (st_abs & 1u) ? rw[3] : rw[1];
-        a_raw0 = (float)fma(__hiloint2double((int)(0x3ff00000u | (w0 >> 12)), (int)(w0 << 20)), 2.0, -3.0);
-        a_raw1 = (float)fma(__hiloint2double((int)(0x3ff00000u | (w1 >> 12)), (int)(w1 << 20)), 2.0, -3.0);
+        a_raw0 = action_from_word(w0);
+        a_raw1 = action_from_word(w1);
         // scale_action with bounds (0,0)/(1,1) (DDPG.jl:178-184, input.jl:182-183): Float32((Float64(a) + 1.0) * 0.5).
         // a is a multiple of 2^-31, so a + 1.0 and the halving are exact in Float64 and the single final rounding
         // equals the Float32 add followed by the exact halving.

@@ -61,7 +61,18 @@ __device__ __forceinline__ double ddiv_const(double x, double d, double r, int o
 
 // FAST (template parameter of everything below) = the constants are in their usual state — P.fast_all: Float32-valued divisors,
 // Float32 penalty weight, shems_LU1's reward form — so the flag tests, the fall-back branches and the guarded Float32 division
-// sequences are compiled out (the Float32 quotients go through fdiv_const_wide).  Both instantiations give the same bits.
+// sequences are compiled out (the Float32 quotients go through fdiv_const_wide), and Float32 decisions against Float64 constants are
+// taken in FP32 against thresholds the host rounded (x > c <=> x > RD32(c), x < c <=> x < RU32(c) for Float32 x; the Float32 value
+// of c where a branch yields it is RN32(c)).  Both instantiations give the same bits.
+
+// Float32(clamp(Float64(pv), 0.0, min(R, Float64(h)))) for Float32 pv, h (charge request, :307-308 / :331-332): h < R <=> h < RU32(R),
+// pv > R <=> pv > RD32(R), and the Float64 result is h, R, 0 or pv, so its Float32 value is h, RN32(R), 0 or pv
+__device__ __forceinline__ float charge_request_f(const DevParams& P, float pv, float h) {
+  const bool h_lo = h < P.R_up;
+  return (pv > (h_lo ? h : P.R_dn)) ? (h_lo ? h : P.R_f) : ((pv < 0.0f) ? 0.0f : pv);
+}
+// Float32(-min(R, Float64(x))) for Float32 x (discharge request, :310 / :334): x < R <=> x < RU32(R); -RN32(R) = RN32(-R)
+__device__ __forceinline__ float discharge_request_f(const DevParams& P, float x) { return -((x < P.R_up) ? x : P.R_f); }
 
 // action(env, a::ShemsAction) :283-316 -> Float32.([B, EV])
 template <bool FAST>
@@ -73,17 +84,30 @@ __device__ __forceinline__ void shems_action_drl(const DevParams& P, float Soc_b
   const float pv = (g_e - d_e) - EV;                                                      // :301
   // :304-313 evaluated branch-free: charge request / discharge request / nothing
   const float Btv = Bt * P.span + P.smin;                                                 // :306 (two roundings, fmad off)
-  const double hi = jl_mind(P.R, (double)((Btv - Soc_b) + P.loss));                       // :307
-  const float Bc = (float)jl_clampd((double)pv, 0.0, hi);
-  const float Bd = (float)(-jl_mind(P.R, (double)(P.one_m_l * Soc_b)));                   // :310
+  float Bc, Bd;
+  if (FAST) {
+    Bc = charge_request_f(P, pv, (Btv - Soc_b) + P.loss);
+    Bd = discharge_request_f(P, P.one_m_l * Soc_b);
+  } else {
+    const double hi = jl_mind(P.R, (double)((Btv - Soc_b) + P.loss));                     // :307
+    Bc = (float)jl_clampd((double)pv, 0.0, hi);
+    Bd = (float)(-jl_mind(P.R, (double)(P.one_m_l * Soc_b)));                             // :310
+  }
   B = (pv > 0.0f && perc < Bt) ? Bc : ((Soc_b > 1e-3f) ? Bd : 0.0f);
 }
 
 // action(env, track) rule-based controller :318-340 -> Float32.([B, EV])
+template <bool FAST>
 __device__ __forceinline__ void shems_action_rule(const DevParams& P, float Soc_b, float Soc_ev, float d_e, float g_e,
                                                   float& B, float& EV) {
   EV = jl_minf(P.evR, (1.0f - Soc_ev) * P.C);                                     // :323
   const float pv = (g_e - d_e) - EV;                                              // :327
+  if (FAST) {
+    const float Bc = charge_request_f(P, pv, (P.smax - Soc_b) + P.loss);
+    const float Bd = discharge_request_f(P, P.one_m_l * Soc_b);
+    B = (pv > 0.0f && Soc_b < P.smax95_up) ? Bc : ((Soc_b > 1e-3f) ? Bd : 0.0f);   // Soc_b < 0.95 smax <=> Soc_b < RU32(0.95 smax)
+    return;
+  }
   const double hi = jl_mind(P.R, (double)((P.smax - Soc_b) + P.loss));            // :331
   const float Bc = (float)jl_clampd((double)pv, 0.0, hi);
   const float Bd = (float)(-jl_mind(P.R, (double)(P.one_m_l * Soc_b)));           // :334
