@@ -357,6 +357,14 @@ SHEMS_API int32_t ddpg_update_phase(Ddpg* h, ShemsReplay* rp, int32_t phase, con
 SHEMS_API int32_t ddpg_select_learner(Ddpg* h, int32_t learner);
 SHEMS_API int32_t ddpg_population(const Ddpg* h);
 SHEMS_API int32_t ddpg_update_population(Ddpg* h, ShemsReplay* const* rps, int32_t n_updates, const int32_t* idx_host, const uint64_t* seeds);
+/* Per-learner hyper-parameters of the learner chosen by ddpg_select_learner (valid for P == 1 too): the ADAM learning rates η_act,
+ * η_crit, the discount γ, the Polyak rate τ and an exploration-noise scale.  ddpg_create gives every learner the DdpgParams values
+ * and noise_scale = 1.  Wherever the library draws noise (ddpg_act*, ddpg_act_ou, ddpg_episode, ddpg_rollout) it uses
+ * σ_eff = RN32(sigma × noise_scale) with the sigma of the call; caller-supplied noise_dev is added as is.  The write is ordered on
+ * the handle's stream, so it applies to the next launch.  Values must be finite, lr_* >= 0, noise_scale >= 0 and gamma, tau in
+ * [0, 1]; anything else returns SHEMS_ERR_INVALID and changes nothing.  Data-parallel ranks must all make the same call. */
+SHEMS_API int32_t ddpg_set_hparams(Ddpg* h, float lr_actor, float lr_critic, float gamma, float tau, float noise_scale);
+SHEMS_API int32_t ddpg_get_hparams(Ddpg* h, float* lr_actor, float* lr_critic, float* gamma, float* tau, float* noise_scale);
 /* Data-parallel learner with the gradient all-reduce fused into the optimiser kernels over NVLink peer memory (one process per
  * GPU).  Each rank exports DDPG_DP_HANDLE_BYTES (the CUDA IPC handle of its exchange box: per-block flags and one inbound row of
  * gradient sums per peer, which the peers write), the caller gathers the

@@ -127,6 +127,8 @@ SIGNATURES = {
     "ddpg_select_learner": (I32, [VP, I32]),
     "ddpg_population": (I32, [VP]),
     "ddpg_update_population": (I32, [VP, C.POINTER(VP), I32, PI, C.POINTER(U64)]),
+    "ddpg_set_hparams": (I32, [VP, F32, F32, F32, F32, F32]),
+    "ddpg_get_hparams": (I32, [VP, PF, PF, PF, PF, PF]),
     "shems_tc_gemm": (I32, [VP, I64, I32, VP, I64, I32, VP, I64, I32, I32, I32, I32, VP, VP, I64, I32, VP, VP]),
     "ddpg_grad_buffer": (I32, [VP, C.POINTER(VP), C.POINTER(I64)]),
     "ddpg_rollout": (I32, [VP, VP, I32, F32, U64, I64, VP, VP, VP]),

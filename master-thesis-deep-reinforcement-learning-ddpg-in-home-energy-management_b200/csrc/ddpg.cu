@@ -46,7 +46,8 @@ struct GemmProblem {
   const float* aux3;   // TD_TARGET: q[m] (critic output on (s,a))
   float* out2;         // TD_TARGET: dq[m] = 2 (q - y) / B
   float* dbias;        // column sums of B(k,n) over k (bias gradient), written by the m-tile 0 CTAs
-  float alpha;         // TD_TARGET: gamma; SCALE_MASK: scale
+  float alpha;         // SCALE_MASK: scale
+  const DdpgCtrl* ctrl;  // TD_TARGET: learner 0's control block; γ = ctrl[learner].hp.gamma
   float inv_batch;     // TD_TARGET: 1/B
 };
 struct GemmBatch {
@@ -58,8 +59,9 @@ struct GemmBatch {
   // (B, bias) ls_w floats and everything else (A, C, aux*, out2, dbias) ls_x floats behind learner 0's pointers
   int pop; long long ls_w, ls_x;
 };
-__device__ __forceinline__ void gemm_shift(GemmProblem& p, long long ow, long long ox) {
+__device__ __forceinline__ void gemm_shift(GemmProblem& p, int learner, long long ow, long long ox) {
   p.A += ox; p.B += ow; p.C += ox;
+  if (p.ctrl) p.ctrl += learner;
   if (p.bias) p.bias += ow;
   if (p.aux) p.aux += ox;
   if (p.aux2) p.aux2 += ox;
@@ -94,7 +96,7 @@ __device__ __forceinline__ float gemm_epilogue(const GemmProblem& p, int m, int 
     case EPI_TANH_GRAD: { const float y = p.aux[m * p.auxld + n]; v = v * (1.0f - y * y); } break;
     case EPI_TD_TARGET: {  // y = r + γ(1-done) q'   (DDPG.jl:133);  dq = 2 (q - y) / B  (d mse / d q)
       const float q2 = v + p.bias[n];
-      const float y = p.aux[m] + (p.alpha * (1.0f - p.aux2[m])) * q2;
+      const float y = p.aux[m] + (p.ctrl->hp.gamma * (1.0f - p.aux2[m])) * q2;
       v = y;
       p.out2[m] = 2.0f * (p.aux3[m] - y) * p.inv_batch;
     } break;
@@ -119,7 +121,7 @@ gemm_batch_kernel(const GemmBatch gb) {
   const bool splitk = gb.ksplit > 1;
   const int learner = splitk ? 0 : blockIdx.z / gb.count;
   GemmProblem p = gb.p[splitk ? 0 : blockIdx.z - learner * gb.count];
-  if (learner) gemm_shift(p, learner * gb.ls_w, learner * gb.ls_x);
+  if (learner) gemm_shift(p, learner, learner * gb.ls_w, learner * gb.ls_x);
   const int split = splitk ? blockIdx.z : 0;
   const int m0 = blockIdx.x * TBM, n0 = blockIdx.y * TBN;  // M tiles on grid.x (no 65535 limit for large batches)
   if (m0 >= p.M || n0 >= p.N) return;
@@ -230,7 +232,7 @@ gemm_batch_kernel(const GemmBatch gb) {
 __global__ void __launch_bounds__(256)
 gemm_skinny_kernel(const GemmBatch gb) {
   GemmProblem p = gb.p[blockIdx.y];
-  if (blockIdx.z) gemm_shift(p, blockIdx.z * gb.ls_w, blockIdx.z * gb.ls_x);
+  if (blockIdx.z) gemm_shift(p, blockIdx.z, blockIdx.z * gb.ls_w, blockIdx.z * gb.ls_x);
   // the one or two weight columns are shared by the block's 8 rows: staged once in shared memory (K <= SKINNY_MAX_K)
   constexpr int SKINNY_MAX_K = 1024;
   __shared__ float bsm[2][SKINNY_MAX_K];
@@ -541,6 +543,7 @@ struct Ddpg {
   bool fused; float* parts[2];
   bool rollout_ok;   // ddpg_rollout may run as the persistent cluster kernel (one learner, widths within the shared-memory plan)
   int noise_kind; float ou_theta, ou_mu, ou_dt;   // ddpg_set_noise
+  DdpgHparams* hp;   // [pop] host copy of every learner's ctrl->hp (ddpg_get_hparams; σ_eff of the one-learner cluster kernels)
   float* ou_x; long long ou_cap;                   // OUNoise.X of every instance of ddpg_episode's environment ([2][N])
 };
 static inline int round_ld(int x) { return (x + 31) & ~31; }  // activation rows start on 128-byte lines: one L2 request per TMA box row
@@ -659,6 +662,8 @@ extern "C" int32_t ddpg_create(const DdpgParams* p, int32_t device, Ddpg** out) 
   }
   DMALLOC(h->ctrl, pop);
   DMALLOC(h->rings_dev, pop);
+  h->hp = (DdpgHparams*)malloc(sizeof(DdpgHparams) * (size_t)pop);
+  if (!h->hp) { shems_set_error("ddpg_create: out of host memory"); ddpg_destroy(h); return SHEMS_ERR_INVALID; }
   {
     std::vector<float> c((size_t)B, -1.0f / (float)B);
     float nm[18];
@@ -672,6 +677,8 @@ extern "C" int32_t ddpg_create(const DdpgParams* p, int32_t device, Ddpg** out) 
         ctl[l].bp[n][0] = p->adam_beta1; ctl[l].bp[n][1] = p->adam_beta2;
         ctl[l].rc[n][0] = 1.0 / (1.0 - p->adam_beta1); ctl[l].rc[n][1] = 1.0 / (1.0 - p->adam_beta2);
       }
+      h->hp[l] = DdpgHparams{{p->lr_critic, p->lr_actor}, p->gamma, p->tau, 1.0f};
+      ctl[l].hp = h->hp[l];
     }
     cudaMemcpy(h->ctrl, ctl.data(), sizeof(DdpgCtrl) * (size_t)pop, cudaMemcpyHostToDevice);
   }
@@ -699,6 +706,7 @@ extern "C" int32_t ddpg_destroy(Ddpg* h) {
   if (h->ev_mid) cudaEventDestroy(h->ev_mid);
   if (h->ev_join) cudaEventDestroy(h->ev_join);
   if (h->side) cudaStreamDestroy(h->side);
+  free(h->hp);
   delete h;
   return SHEMS_OK;
 }
@@ -711,6 +719,32 @@ extern "C" int32_t ddpg_select_learner(Ddpg* h, int32_t learner) {
 }
 extern "C" int32_t ddpg_population(const Ddpg* h) { return h ? h->pop : 0; }
 static inline long long sel_off(const Ddpg* h) { return (long long)h->sel * h->pop_stride; }
+
+// η_actor, η_critic, γ, τ and the exploration-noise scale of the selected learner.  The write is enqueued on the handle's stream:
+// updates and act() calls enqueued before it use the old values, everything enqueued after it the new ones.  Captured update graphs
+// read the values from the control block, so nothing is re-captured.
+extern "C" int32_t ddpg_set_hparams(Ddpg* h, float lr_actor, float lr_critic, float gamma, float tau, float noise_scale) {
+  REQUIRE(h, SHEMS_ERR_INVALID, "ddpg_set_hparams: NULL handle");
+  REQUIRE(isfinite(lr_actor) && isfinite(lr_critic) && isfinite(gamma) && isfinite(tau) && isfinite(noise_scale), SHEMS_ERR_INVALID,
+          "ddpg_set_hparams: values must be finite (lr_actor=%g lr_critic=%g gamma=%g tau=%g noise_scale=%g)", (double)lr_actor, (double)lr_critic,
+          (double)gamma, (double)tau, (double)noise_scale);
+  REQUIRE(lr_actor >= 0.0f && lr_critic >= 0.0f && noise_scale >= 0.0f, SHEMS_ERR_INVALID,
+          "ddpg_set_hparams: lr_actor=%g lr_critic=%g noise_scale=%g must be >= 0", (double)lr_actor, (double)lr_critic, (double)noise_scale);
+  REQUIRE(gamma >= 0.0f && gamma <= 1.0f && tau >= 0.0f && tau <= 1.0f, SHEMS_ERR_INVALID, "ddpg_set_hparams: gamma=%g tau=%g outside [0, 1]",
+          (double)gamma, (double)tau);
+  GUARD(h->device);
+  const DdpgHparams v{{lr_critic, lr_actor}, gamma, tau, noise_scale};
+  // pageable source: the runtime stages the copy before returning (no synchronisation, which a data-parallel peer could be waiting on)
+  CUDA_TRY(cudaMemcpyAsync((char*)(h->ctrl + h->sel) + offsetof(DdpgCtrl, hp), &v, sizeof(v), cudaMemcpyHostToDevice, h->stream));
+  h->hp[h->sel] = v;
+  return SHEMS_OK;
+}
+extern "C" int32_t ddpg_get_hparams(Ddpg* h, float* lr_actor, float* lr_critic, float* gamma, float* tau, float* noise_scale) {
+  REQUIRE(h && lr_actor && lr_critic && gamma && tau && noise_scale, SHEMS_ERR_INVALID, "ddpg_get_hparams: NULL argument");
+  const DdpgHparams& v = h->hp[h->sel];
+  *lr_actor = v.eta[1]; *lr_critic = v.eta[0]; *gamma = v.gamma; *tau = v.tau; *noise_scale = v.noise_scale;
+  return SHEMS_OK;
+}
 
 extern "C" int32_t ddpg_set_stream(Ddpg* h, void* s) {
   REQUIRE(h, SHEMS_ERR_INVALID, "ddpg_set_stream: NULL handle");
@@ -910,7 +944,7 @@ __device__ __forceinline__ void adam_advance(DdpgCtrl* ctrl, double b1, double b
 template <bool FAST>
 __global__ void __launch_bounds__(256)
 adam_polyak_kernel(float* __restrict__ x, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, long long n, double b1,
-                   double b2, double eps, float eta, DdpgCtrl* __restrict__ ctrl, int opt, float* __restrict__ target, float tau,
+                   double b2, double eps, DdpgCtrl* __restrict__ ctrl, int opt, float* __restrict__ target,
                    float* __restrict__ target2, const float* __restrict__ model2, long long n2, int advance, float gscale, long long pop_stride) {
   {  // blockIdx.y = learner of a population
     const long long lo = (long long)blockIdx.y * pop_stride;
@@ -922,7 +956,9 @@ adam_polyak_kernel(float* __restrict__ x, const float* __restrict__ g, float* __
   // q = a*r; e = fma(-q, c, a); q' = fma(e, r, q) is the correctly rounded quotient (Markstein), at 3 DFMA instead of a DDIV
   const double c1 = 1.0 - ctrl->bp[opt][0], c2 = 1.0 - ctrl->bp[opt][1];
   const double r1 = ctrl->rc[opt][0], r2 = ctrl->rc[opt][1];
-  const float omt = __fsub_rn(1.0f, tau);
+  // this learner's η of optimiser `opt` and τ (ddpg_set_hparams) are read inside every loop, after the element's own loads: read once
+  // up front, they are moved to uniform registers before the first element load is issued, and each thread waits for them first
+#define ETA_TAU const float eta = ctrl->hp.eta[opt], tau = ctrl->hp.tau, omt = __fsub_rn(1.0f, tau); (void)eta
   const long long stride = (long long)gridDim.x * blockDim.x;
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long j0 = 0, k0 = 0;  // scalar loops start here (FAST: after the float4 body)
@@ -931,6 +967,7 @@ adam_polyak_kernel(float* __restrict__ x, const float* __restrict__ g, float* __
     for (long long q = tid; q < n4; q += stride) {
       float4 xv = reinterpret_cast<float4*>(x)[q], mv = reinterpret_cast<float4*>(m)[q], vv = reinterpret_cast<float4*>(v)[q];
       const float4 gv = reinterpret_cast<const float4*>(g)[q];
+      ETA_TAU;
       float xs[4] = {xv.x, xv.y, xv.z, xv.w}, ms[4] = {mv.x, mv.y, mv.z, mv.w}, vs[4] = {vv.x, vv.y, vv.z, vv.w};
       const float gs[4] = {gv.x, gv.y, gv.z, gv.w};
 #pragma unroll
@@ -951,6 +988,7 @@ adam_polyak_kernel(float* __restrict__ x, const float* __restrict__ g, float* __
     for (long long q = tid; q < m4; q += stride) {
       float4 t = reinterpret_cast<float4*>(target2)[q];
       const float4 w = reinterpret_cast<const float4*>(model2)[q];
+      ETA_TAU;
       t.x = __fadd_rn(__fmul_rn(omt, t.x), __fmul_rn(tau, w.x)); t.y = __fadd_rn(__fmul_rn(omt, t.y), __fmul_rn(tau, w.y));
       t.z = __fadd_rn(__fmul_rn(omt, t.z), __fmul_rn(tau, w.z)); t.w = __fadd_rn(__fmul_rn(omt, t.w), __fmul_rn(tau, w.w));
       reinterpret_cast<float4*>(target2)[q] = t;
@@ -959,13 +997,17 @@ adam_polyak_kernel(float* __restrict__ x, const float* __restrict__ g, float* __
   }
   for (long long j = j0 + tid; j < n; j += stride) {
     const float gj = (gscale == 1.0f) ? g[j] : __fmul_rn(g[j], gscale);  // data-parallel: mean of the ranks' summed gradients
+    ETA_TAU;
     const float xn = adam_element<FAST>(x[j], gj, m + j, v + j, b1, b2, eps, eta, c1, c2, r1, r2);
     x[j] = xn;
     if (target) target[j] = __fadd_rn(__fmul_rn(omt, target[j]), __fmul_rn(tau, xn));
   }
   // second Polyak pair: the critic target moves together with the actor step (DDPG.jl:142-143)
-  for (long long j = k0 + tid; j < n2; j += stride)
+  for (long long j = k0 + tid; j < n2; j += stride) {
+    ETA_TAU;
     target2[j] = __fadd_rn(__fmul_rn(omt, target2[j]), __fmul_rn(tau, model2[j]));
+  }
+#undef ETA_TAU
   if (advance) adam_advance(ctrl, b1, b2);
 }
 
@@ -974,14 +1016,13 @@ adam_polyak_kernel(float* __restrict__ x, const float* __restrict__ g, float* __
 // above.  The summed gradient is also stored to g_out (ddpg_get_grad).
 __global__ void __launch_bounds__(256)
 adam_polyak_parts_kernel(float* __restrict__ x, const float* __restrict__ parts, int nparts, long long part_stride, float* __restrict__ g_out,
-                         float* __restrict__ m, float* __restrict__ v, long long n, double b1, double b2, double eps, float eta,
-                         DdpgCtrl* __restrict__ ctrl, int opt, float* __restrict__ target, float tau, float* __restrict__ target2,
+                         float* __restrict__ m, float* __restrict__ v, long long n, double b1, double b2, double eps,
+                         DdpgCtrl* __restrict__ ctrl, int opt, float* __restrict__ target, float* __restrict__ target2,
                          const float* __restrict__ model2, long long n2, int advance) {
   // the fused actor pass is a programmatic dependent of ADAM(critic): its actor forward pass may run beside this kernel
   asm volatile("griddepcontrol.launch_dependents;\n" ::: "memory");
   const double c1 = 1.0 - ctrl->bp[opt][0], c2 = 1.0 - ctrl->bp[opt][1];
   const double r1 = ctrl->rc[opt][0], r2 = ctrl->rc[opt][1];
-  const float omt = __fsub_rn(1.0f, tau);
   const long long stride = (long long)gridDim.x * blockDim.x;
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   // one element per thread at the reference's sizes: every load of the element (partials, parameter, moments, both Polyak
@@ -991,6 +1032,8 @@ adam_polyak_parts_kernel(float* __restrict__ x, const float* __restrict__ parts,
     float t2 = 0.0f, w2 = 0.0f, xj = 0.0f, tj = 0.0f;
     if (in2) { t2 = target2[j]; w2 = model2[j]; }
     if (in1) { xj = x[j]; if (target) tj = target[j]; }
+    // η and τ are read here rather than before the loop: live across it they cost an 8-byte spill at this kernel's 48 registers
+    const float eta = ctrl->hp.eta[opt], tau = ctrl->hp.tau, omt = __fsub_rn(1.0f, tau);
     if (in1) {
       float gj = 0.0f;
       for (int c0 = 0; c0 < nparts; c0 += 8) {
@@ -1073,7 +1116,7 @@ template <int W>
 __global__ void __launch_bounds__(256)
 adam_polyak_dp_kernel(const DpPeers peers, long long seg_off, const float* __restrict__ parts, int nparts, long long part_stride,
                       float* __restrict__ g_own, float* __restrict__ x, float* __restrict__ m, float* __restrict__ v, long long n, double b1,
-                      double b2, double eps, float eta, DdpgCtrl* __restrict__ ctrl, int opt, float* __restrict__ target, float tau,
+                      double b2, double eps, DdpgCtrl* __restrict__ ctrl, int opt, float* __restrict__ target,
                       float* __restrict__ target2, const float* __restrict__ model2, long long n2, int advance) {
   __shared__ int ok_s, last_s;
   // the fused actor pass is a programmatic dependent of the critic exchange: its actor forward pass (which does not read the critic)
@@ -1157,6 +1200,7 @@ adam_polyak_dp_kernel(const DpPeers peers, long long seg_off, const float* __res
   const bool ok = ok_s && ld_volatile_u32(&ctrl->dp_abort) != epoch;
   const double c1 = 1.0 - ctrl->bp[opt][0], c2 = 1.0 - ctrl->bp[opt][1];
   const double r1 = ctrl->rc[opt][0], r2 = ctrl->rc[opt][1];
+  const float eta = ctrl->hp.eta[opt], tau = ctrl->hp.tau;
   const float omt = __fsub_rn(1.0f, tau), inv_w = 1.0f / (float)W;
   if (ok) {
     const float* in = reinterpret_cast<const float*>(peers.box[rank] + DP_BOX_FLAG_WORDS) + seg_off;
@@ -1194,8 +1238,8 @@ adam_polyak_dp_kernel(const DpPeers peers, long long seg_off, const float* __res
 // of blocks that are co-resident (the blocks wait for one another in step 1)
 static int dp_grid_cap = 0;
 static int launch_adam_dp(cudaStream_t st, const DpPeers& peers, long long seg_off, const float* parts, int nparts, long long part_stride, float* g_own,
-                          float* x, float* m, float* v, long long n, double b1, double b2, double eps, float eta, DdpgCtrl* ctrl, int opt,
-                          float* target, float tau, float* target2, const float* model2, long long n2, int advance) {
+                          float* x, float* m, float* v, long long n, double b1, double b2, double eps, DdpgCtrl* ctrl, int opt,
+                          float* target, float* target2, const float* model2, long long n2, int advance) {
 #define DP_CASE(WW)                                                                                                                          \
   case WW: {                                                                                                                                 \
     if (!dp_grid_cap) {                                                                                                                      \
@@ -1207,8 +1251,8 @@ static int launch_adam_dp(cudaStream_t st, const DpPeers& peers, long long seg_o
     }                                                                                                                                        \
     const long long want = ((n > n2 ? n : n2) + 255) / 256;                                                                                  \
     const unsigned grid = (unsigned)(want < dp_grid_cap ? want : dp_grid_cap);                                                               \
-    adam_polyak_dp_kernel<WW><<<grid, 256, 0, st>>>(peers, seg_off, parts, nparts, part_stride, g_own, x, m, v, n, b1, b2, eps, eta, ctrl, opt, \
-                                                    target, tau, target2, model2, n2, advance);                                              \
+    adam_polyak_dp_kernel<WW><<<grid, 256, 0, st>>>(peers, seg_off, parts, nparts, part_stride, g_own, x, m, v, n, b1, b2, eps, ctrl, opt, target, \
+                                                    target2, model2, n2, advance);                                                    \
   } break;
   switch (peers.world) {
     DP_CASE(1) DP_CASE(2) DP_CASE(3) DP_CASE(4) DP_CASE(5) DP_CASE(6) DP_CASE(7) DP_CASE(8) DP_CASE(16)
@@ -1425,7 +1469,8 @@ static int enqueue_phase0(Ddpg* h, cudaStream_t st) {
     // q' = critic_target(vcat(s'_n, a'));  y = r + gamma (1 - done) q';  dq = 2 (q - y) / B     (:132-133)
     TcFwdChainArgs t = chain_args(h, 1);
     chain_set(t, 0, h->xs2, critic_t, dc, nullptr, nullptr, TC_OUT_TD, h->y, 1);
-    t.td_r = h->r; t.td_done = h->done; t.td_q = h->q; t.td_dq = h->dq; t.gamma = p.gamma; t.inv_batch = 1.0f / (float)B;
+    t.td_r = h->r; t.td_done = h->done; t.td_q = h->q; t.td_dq = h->dq; t.inv_batch = 1.0f / (float)B;
+    t.td_gamma = &h->ctrl->hp.gamma; t.td_gamma_stride = sizeof(DdpgCtrl) / sizeof(float);
     t.pdl = 1; t.early_weights = 1;   // after the three-net launch: a' and q are its output, critic_target's weights are not
     TRY(tc_fwd_chain(st, t));
   } else {
@@ -1471,7 +1516,7 @@ static int enqueue_phase0(Ddpg* h, cudaStream_t st) {
     TRY(launch_gemms(st, g, 1, h->pop, h->pop_stride, h->pop_stride));
   }
   g[0] = gp_fwd(h->tc_h2, l2, B, critic_t, dc.l[2], h->y, 1, EPI_TD_TARGET);
-  g[0].aux = h->r; g[0].aux2 = h->done; g[0].aux3 = h->q; g[0].out2 = h->dq; g[0].alpha = p.gamma; g[0].inv_batch = 1.0f / (float)B;
+  g[0].aux = h->r; g[0].aux2 = h->done; g[0].aux3 = h->q; g[0].out2 = h->dq; g[0].ctrl = h->ctrl; g[0].inv_batch = 1.0f / (float)B;
   TRY(launch_gemms(st, g, 1, h->pop, h->pop_stride, h->pop_stride));
   }
   // P7-P9: critic backward (:137, :105-108)
@@ -1520,13 +1565,13 @@ static int enqueue_phase1(Ddpg* h, cudaStream_t st, float gscale, bool dp = fals
   const dim3 adam_grid((unsigned)((dc.n_params + 255) / 256), h->pop);  // one element per thread: the Float64 div/sqrt chains need TLP
   if (dp) {  // gradient exchange over NVLink fused into the optimiser step (critic segment = first nc floats of the flat buffer)
     TRY(launch_adam_dp(st, h->dp, 0, nullptr, 0, 0, h->grad[1], critic, h->adam_m[1], h->adam_v[1], dc.n_params, p.adam_beta1, p.adam_beta2, p.adam_eps,
-                       p.lr_critic, h->ctrl, 0, nullptr, 0.0f, nullptr, nullptr, 0, 0));
+                       h->ctrl, 0, nullptr, nullptr, nullptr, 0, 0));
   } else if (h->tc)
     adam_polyak_kernel<true><<<dim3((adam_grid.x + 3) / 4, h->pop), 256, 0, st>>>(critic, h->grad[1], h->adam_m[1], h->adam_v[1], dc.n_params, p.adam_beta1, p.adam_beta2,
-                                                       p.adam_eps, p.lr_critic, h->ctrl, 0, nullptr, 0.0f, nullptr, nullptr, 0, 0, gscale, h->pop_stride);
+                                                       p.adam_eps, h->ctrl, 0, nullptr, nullptr, nullptr, 0, 0, gscale, h->pop_stride);
   else
     adam_polyak_kernel<false><<<adam_grid, 256, 0, st>>>(critic, h->grad[1], h->adam_m[1], h->adam_v[1], dc.n_params, p.adam_beta1, p.adam_beta2,
-                                                        p.adam_eps, p.lr_critic, h->ctrl, 0, nullptr, 0.0f, nullptr, nullptr, 0, 0, gscale, h->pop_stride);
+                                                        p.adam_eps, h->ctrl, 0, nullptr, nullptr, nullptr, 0, 0, gscale, h->pop_stride);
   CUDA_TRY(cudaGetLastError());
   // P11-P13: critic(vcat(s_n, actor(s_n))) with the UPDATED critic (:116-119); loss_act = -mean(q) => dq = -1/B
   const bool chain = tc && h->chain;
@@ -1621,13 +1666,13 @@ static int enqueue_phase2(Ddpg* h, cudaStream_t st, float gscale, bool dp = fals
   // P19: ADAM(η_act) on the actor + soft_update! of both targets (:140-143)
   if (dp) {
     TRY(launch_adam_dp(st, h->dp, h->grad[0] - h->gradbuf, nullptr, 0, 0, h->grad[0], actor, h->adam_m[0], h->adam_v[0], da.n_params, p.adam_beta1,
-                       p.adam_beta2, p.adam_eps, p.lr_actor, h->ctrl, 1, actor_t, p.tau, critic_t, critic, dc.n_params, 1));
+                       p.adam_beta2, p.adam_eps, h->ctrl, 1, actor_t, critic_t, critic, dc.n_params, 1));
   } else if (h->tc)
     adam_polyak_kernel<true><<<dim3((adam_grid.x + 3) / 4, h->pop), 256, 0, st>>>(actor, h->grad[0], h->adam_m[0], h->adam_v[0], da.n_params, p.adam_beta1, p.adam_beta2,
-                                                       p.adam_eps, p.lr_actor, h->ctrl, 1, actor_t, p.tau, critic_t, critic, dc.n_params, 1, gscale, h->pop_stride);
+                                                       p.adam_eps, h->ctrl, 1, actor_t, critic_t, critic, dc.n_params, 1, gscale, h->pop_stride);
   else
     adam_polyak_kernel<false><<<adam_grid, 256, 0, st>>>(actor, h->grad[0], h->adam_m[0], h->adam_v[0], da.n_params, p.adam_beta1, p.adam_beta2,
-                                                        p.adam_eps, p.lr_actor, h->ctrl, 1, actor_t, p.tau, critic_t, critic, dc.n_params, 1, gscale, h->pop_stride);
+                                                        p.adam_eps, h->ctrl, 1, actor_t, critic_t, critic, dc.n_params, 1, gscale, h->pop_stride);
   CUDA_TRY(cudaGetLastError());
   return SHEMS_OK;
 }
@@ -1646,7 +1691,7 @@ static int enqueue_update_fused(Ddpg* h, cudaStream_t st, bool dp, const GatherS
   a.co = FusedNetOff{(int)dc.l[0].w_off, (int)dc.l[0].b_off, (int)dc.l[1].w_off, (int)dc.l[1].b_off, (int)dc.l[2].w_off, (int)dc.l[2].b_off};
   a.l1 = p.l1; a.l2 = p.l2; a.B = p.batch;
   a.xs = h->xs; a.xs2 = h->xs2; a.xspi = h->xspi; a.r = h->r; a.done = h->done; a.q = h->q; a.y = h->y; a.qpi = h->qpi;
-  a.gamma = p.gamma; a.inv_batch = 1.0f / (float)p.batch;
+  a.inv_batch = 1.0f / (float)p.batch;
   a.rings = src.from_rings ? h->rings_dev : nullptr;
   a.src_s = src.s; a.src_a = src.a; a.src_r = src.r; a.src_s2 = src.s2; a.src_d = src.done; a.src_ld = src.ld;
   a.ctrl = h->ctrl; a.idx = h->idx_dev; a.norm = h->norm; a.xs_w = h->xs;
@@ -1661,20 +1706,20 @@ static int enqueue_update_fused(Ddpg* h, cudaStream_t st, bool dp, const GatherS
   TRY(ddpg_fused_critic(st, a));
   if (dp) {  // partial-sum reduction, gradient exchange over NVLink and the optimiser step in ONE kernel
     TRY(launch_adam_dp(st, h->dp, 0, h->parts[1], nparts, dc.n_params, h->grad[1], critic, h->adam_m[1], h->adam_v[1], dc.n_params, p.adam_beta1,
-                       p.adam_beta2, p.adam_eps, p.lr_critic, h->ctrl, 0, nullptr, 0.0f, nullptr, nullptr, 0, 0));
+                       p.adam_beta2, p.adam_eps, h->ctrl, 0, nullptr, nullptr, nullptr, 0, 0));
   } else {
     adam_polyak_parts_kernel<<<ap_blocks, ADAM_PARTS_THREADS, 0, st>>>(critic, h->parts[1], nparts, dc.n_params, h->grad[1], h->adam_m[1], h->adam_v[1], dc.n_params,
-                                                           p.adam_beta1, p.adam_beta2, p.adam_eps, p.lr_critic, h->ctrl, 0, nullptr, 0.0f, nullptr, nullptr, 0, 0);
+                                                           p.adam_beta1, p.adam_beta2, p.adam_eps, h->ctrl, 0, nullptr, nullptr, nullptr, 0, 0);
   }
   CUDA_TRY(cudaGetLastError());
   a.part = h->parts[0]; a.part_stride = da.n_params;
   TRY(ddpg_fused_actor(st, a));
   if (dp) {
     TRY(launch_adam_dp(st, h->dp, h->grad[0] - h->gradbuf, h->parts[0], nparts, da.n_params, h->grad[0], actor, h->adam_m[0], h->adam_v[0], da.n_params,
-                       p.adam_beta1, p.adam_beta2, p.adam_eps, p.lr_actor, h->ctrl, 1, actor_t, p.tau, critic_t, critic, dc.n_params, 1));
+                       p.adam_beta1, p.adam_beta2, p.adam_eps, h->ctrl, 1, actor_t, critic_t, critic, dc.n_params, 1));
   } else {
     adam_polyak_parts_kernel<<<ap_blocks, ADAM_PARTS_THREADS, 0, st>>>(actor, h->parts[0], nparts, da.n_params, h->grad[0], h->adam_m[0], h->adam_v[0], da.n_params,
-                                                           p.adam_beta1, p.adam_beta2, p.adam_eps, p.lr_actor, h->ctrl, 1, actor_t, p.tau, critic_t, critic,
+                                                           p.adam_beta1, p.adam_beta2, p.adam_eps, h->ctrl, 1, actor_t, critic_t, critic,
                                                            dc.n_params, 1);
   }
   CUDA_TRY(cudaGetLastError());
@@ -1968,9 +2013,10 @@ ddpg_normalize_kernel(const float* __restrict__ obs, long long n, const float* _
     x[j * 9 + k] = __fdiv_rn(__fsub_rn(obs[k * osk + j], norm[k]), den);
   }
 }
-// clamp(actor + noise, -1, 1) and scale_action (DDPG.jl:172-184); noise: given, or σ·N(0,1) by Box-Muller on Philox
+// clamp(actor + noise, -1, 1) and scale_action (DDPG.jl:172-184); noise: given, or σ_eff·N(0,1) by Box-Muller on Philox, where
+// σ_eff = RN32(σ × noise_scale of the learner)
 __global__ void __launch_bounds__(256)
-ddpg_act_epilogue_kernel(const float* __restrict__ y /*[n][2]*/, long long n, float sigma, unsigned long long seed, long long step,
+ddpg_act_epilogue_kernel(const float* __restrict__ y /*[n][2]*/, long long n, float sigma, const DdpgCtrl* __restrict__ ctrl, unsigned long long seed, long long step,
                          long long env_id_base, const float* __restrict__ noise, float lo0, float lo1, float hi0, float hi1,
                          float* __restrict__ a_out, float* __restrict__ scaled_out, long long act_stride, long long asl, long long ask,
                          float* __restrict__ noise_acc, int noise_first) {
@@ -1981,6 +2027,7 @@ ddpg_act_epilogue_kernel(const float* __restrict__ y /*[n][2]*/, long long n, fl
      // (packed [P][2][n]: asl = 2n, ask = n; SoA over all instances: asl = n, ask = N); noise streams are keyed by the global env id
     const long long l = blockIdx.y;
     y += l * act_stride; a_out += l * asl; env_id_base += l * n;
+    sigma = __fmul_rn(sigma, ctrl[l].hp.noise_scale);
     if (noise) noise += l * asl;
     if (scaled_out) scaled_out += l * asl;
   }
@@ -1994,11 +2041,12 @@ ddpg_act_epilogue_kernel(const float* __restrict__ y /*[n][2]*/, long long n, fl
 
 // OUNoise (DDPG.jl:49-55, input.jl:190-234) with Julia's types: θ, μ, σ, dt and X are Float32, randn is Float64:
 //   dx = θ .* (μ .- X) .* dt              (Float32)
-//   dx .+= σ .* sqrt(dt) .* randn(2)      (Float32(σ·√dt) · z in Float64, added in Float64, stored Float32)
+//   dx .+= σ .* sqrt(dt) .* randn(2)      (Float32(σ·√dt) · z in Float64, added in Float64, stored Float32; σ = RN32(σ × noise_scale))
 //   X .+= dx;  noise = Float32.(X)        (X persists across steps AND episodes: the reference never resets it)
 // Every instance carries its own X (ou_x [2][n]); z: caller-supplied standard normal draws or Philox + Box-Muller.
 __global__ void __launch_bounds__(256)
-ddpg_act_ou_epilogue_kernel(const float* __restrict__ y /*[n][2]*/, long long n, float theta, float mu, float sigma, float dt, float* __restrict__ ou_x,
+ddpg_act_ou_epilogue_kernel(const float* __restrict__ y /*[n][2]*/, long long n, float theta, float mu, float sigma, const DdpgCtrl* __restrict__ ctrl,
+                            float dt, float* __restrict__ ou_x,
                             unsigned long long seed, long long step, long long env_id_base, const double* __restrict__ z, float lo0, float lo1,
                             float hi0, float hi1, float* __restrict__ a_out, float* __restrict__ scaled_out, long long act_stride,
                             long long asl, long long ask, float* __restrict__ noise_acc, int noise_first) {
@@ -2008,6 +2056,7 @@ ddpg_act_ou_epilogue_kernel(const float* __restrict__ y /*[n][2]*/, long long n,
   {  // learner l = blockIdx.y; component k of its instance j at [l*asl + k*ask + j] (packed: asl = 2n, ask = n; SoA: asl = n, ask = N)
     const long long l = blockIdx.y;
     y += l * act_stride; a_out += l * asl; ou_x += l * asl; env_id_base += l * n;
+    sigma = __fmul_rn(sigma, ctrl[l].hp.noise_scale);
     if (z) z += l * asl;
     if (scaled_out) scaled_out += l * asl;
   }
@@ -2107,7 +2156,7 @@ static int act_gauss(Ddpg* h, const float* obs_dev, int64_t n, float sigma, uint
   if (fused_act_ok(h, n)) {  // normalize, the actor's three layers, noise, clamp, scale_action (and the copy of s) in ONE cluster kernel
     FusedActArgs a = fused_act_args(h, obs_dev, n, n);   // one learner: packed [9][n] and SoA [9][N] coincide
     a.a_out = a_dev; a.scaled_out = scaled_dev; a.noise = noise_dev; a.ask = n;
-    a.sigma = sigma; a.seed = seed; a.step = step; a.env_id_base = env_id_base;
+    a.sigma = sigma * h->hp[0].noise_scale; a.seed = seed; a.step = step; a.env_id_base = env_id_base;   // RN32, as the kernels form it
     a.lo0 = h->p.act_lo[0]; a.lo1 = h->p.act_lo[1]; a.hi0 = h->p.act_hi[0]; a.hi1 = h->p.act_hi[1];
     a.sprev = sprev_dev; a.noise_acc = noise_acc; a.noise_first = noise_first;
     return ddpg_fused_act(h->stream, a);
@@ -2115,7 +2164,7 @@ static int act_gauss(Ddpg* h, const float* obs_dev, int64_t n, float sigma, uint
   if (sprev_dev) CUDA_TRY(cudaMemcpyAsync(sprev_dev, obs_dev, sizeof(float) * 9 * (size_t)N, cudaMemcpyDeviceToDevice, h->stream));
   TRY(act_forward(h, obs_dev, n, soa ? n : 9 * n, soa ? N : n));
   const dim3 gn((unsigned)((n + 255) / 256), h->pop);
-  ddpg_act_epilogue_kernel<<<gn, 256, 0, h->stream>>>(h->act_y, n, sigma, seed, step, env_id_base, noise_dev, h->p.act_lo[0], h->p.act_lo[1],
+  ddpg_act_epilogue_kernel<<<gn, 256, 0, h->stream>>>(h->act_y, n, sigma, h->ctrl, seed, step, env_id_base, noise_dev, h->p.act_lo[0], h->p.act_lo[1],
                                                       h->p.act_hi[0], h->p.act_hi[1], a_dev, scaled_dev, h->act_stride, soa ? n : 2 * n,
                                                       soa ? N : n, noise_acc, noise_first);
   CUDA_TRY(cudaGetLastError());
@@ -2142,7 +2191,7 @@ static int act_ou(Ddpg* h, const float* obs_dev, int64_t n, float theta, float m
   const long long N = (long long)n * h->pop;
   TRY(act_forward(h, obs_dev, n, soa ? n : 9 * n, soa ? N : n));
   const dim3 gn((unsigned)((n + 255) / 256), h->pop);
-  ddpg_act_ou_epilogue_kernel<<<gn, 256, 0, h->stream>>>(h->act_y, n, theta, mu, sigma, dt, ou_x_dev, seed, step, env_id_base, z_dev,
+  ddpg_act_ou_epilogue_kernel<<<gn, 256, 0, h->stream>>>(h->act_y, n, theta, mu, sigma, h->ctrl, dt, ou_x_dev, seed, step, env_id_base, z_dev,
                                                          h->p.act_lo[0], h->p.act_lo[1], h->p.act_hi[0], h->p.act_hi[1], a_dev, scaled_dev,
                                                          h->act_stride, soa ? n : 2 * n, soa ? N : n, noise_acc, noise_first);
   CUDA_TRY(cudaGetLastError());
@@ -2306,7 +2355,7 @@ extern "C" int32_t ddpg_rollout(Ddpg* h, ShemsEnv* env, int32_t n_steps, float s
     a.l1 = h->p.l1; a.l2 = h->p.l2;
     a.vec16 = (h->p.l2 % 4 == 0 && dA.l[1].w_off % 4 == 0 && dC.l[1].w_off % 4 == 0) ? 1 : 0;
     a.norm = h->norm; a.N = N; a.obs = env->obs; a.idx = env->idx; a.T = n_steps; a.step0 = env->step;
-    a.sigma = sigma; a.seed = seed; a.env_id_base = env_id_base;
+    a.sigma = sigma * h->hp[0].noise_scale; a.seed = seed; a.env_id_base = env_id_base;
     a.lo0 = h->p.act_lo[0]; a.lo1 = h->p.act_lo[1]; a.hi0 = h->p.act_hi[0]; a.hi1 = h->p.act_hi[1];
     a.ep_return = ep_return_dev; a.trace = trace_dev; a.act_traj = act_traj_dev;
     for (int g = 0; g < env->n_groups; ++g) {

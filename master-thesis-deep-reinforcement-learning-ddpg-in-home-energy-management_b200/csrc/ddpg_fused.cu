@@ -129,7 +129,7 @@ STAMP(0, 0);
   if (tid < 8) {  // y = r + γ(1-done) q'  (:133);  d mse / d q = 2 (q - y) / B
     const int r = tid;
     const float q2 = xch_sum(S, 2, r, 0) + b3ct;
-    const float y = S->rr[r] + (a.gamma * (1.0f - S->dd[r])) * q2;
+    const float y = S->rr[r] + (a.ctrl->hp.gamma * (1.0f - S->dd[r])) * q2;
     S->dout[r * 2] = 2.0f * (S->qv[r] - y) * a.inv_batch;
     S->dout[r * 2 + 1] = 0.0f;
     S->rr[r] = y;

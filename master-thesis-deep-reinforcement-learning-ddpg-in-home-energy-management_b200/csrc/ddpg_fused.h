@@ -11,6 +11,14 @@
 #define FUSED_MAX_L2 512
 #define FUSED_MAX_BATCH 256    // partial-gradient workspace = batch/8 copies of a net
 
+// per-learner hyper-parameters (ddpg_set_hparams).  The kernels of an update read them here, not as launch arguments: the update runs
+// as a captured CUDA graph, and a value baked into it would stay stale after a change.
+struct DdpgHparams {
+  float eta[2];         // ADAM learning rate per optimiser (0 critic, 1 actor), as bp below
+  float gamma, tau;     // discount of the TD target, Polyak rate of soft_update!
+  float noise_scale;    // exploration noise: σ_eff = RN32(σ of the call × noise_scale)
+};
+
 struct DdpgCtrl {  // device-side control block read by the gather kernel (graph replays need no host patching)
   unsigned long long seed;
   unsigned update;      // counts updates; Philox counter for minibatch draws
@@ -20,6 +28,7 @@ struct DdpgCtrl {  // device-side control block read by the gather kernel (graph
   unsigned blocks_done; // last-block-done counter of the final kernel of an update (advances the counters below)
   double bp[2][2];      // βp of Flux.ADAM per optimiser (0 critic, 1 actor): β^t, advanced after every update
   double rc[2][2];      // 1 / (1 - βp): correctly rounded reciprocals of the two bias-correction divisors
+  DdpgHparams hp;       // written by the host only (ddpg_create, ddpg_set_hparams); behind the prefix ddpg_episode rewrites by value
   unsigned dp_epoch;    // data-parallel learner: number of gradient exchanges completed (two per update)
   unsigned dp_blocks_done;
   int dp_error;         // set when a peer's signal did not arrive within DP_TIMEOUT_NS
@@ -38,7 +47,7 @@ struct FusedArgs {
   float *q, *y, *qpi;        // [B] critic(s,a), TD target, critic(s, actor(s))  (loss reporting)
   float* part;               // partial gradients of the net this pass differentiates: [B/8][n_params], one copy per cluster
   long long part_stride;     // = n_params of that net
-  float gamma, inv_batch;
+  float inv_batch;           // (γ of the TD target: ctrl->hp.gamma)
   int vec16;                  // W2 rows are 16-byte aligned in both nets: 16-byte staging copies and shared-memory reads (else 4-byte)
   // The critic pass samples and normalises its cluster's 8 transitions itself (what ddpg_gather_kernel does for the tiled path,
   // getData + normalize of src/memory_plotting_saving.jl:31-57) and leaves the (s_n | a) rows in xs for the actor pass.

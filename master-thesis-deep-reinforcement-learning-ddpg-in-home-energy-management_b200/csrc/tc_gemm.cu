@@ -401,6 +401,8 @@ tc_fwd_chain_kernel(const __grid_constant__ TcMaps maps, const TcFwdChainArgs p)
   const int K1 = p.K1[prob], J = p.J[prob];
   const int learner = blockIdx.y;                              // a population: the learner's slab starts lo floats further, TMA coordinate 2
   const long long lo = (long long)learner * p.pop_stride;
+  // γ of the TD target: requested now, used in the epilogue (loaded there, its latency would add to the kernel's tail)
+  const float td_gamma = p.out_mode[prob] == TC_OUT_TD ? p.td_gamma[learner * p.td_gamma_stride] : 0.0f;
   const int nkb = (p.L1 + BLOCK_K - 1) / BLOCK_K, nslab = (p.L1 + FC_BK - 1) / FC_BK;   // k-blocks of 32 / W2 slabs of 16 that hold real units
   if (warp == 2 && lane == 0) FC_STAMP(72);
   asm volatile("griddepcontrol.launch_dependents;\n" ::: "memory");   // see tc_gemm_kernel
@@ -608,7 +610,7 @@ tc_fwd_chain_kernel(const __grid_constant__ TcMaps maps, const TcFwdChainArgs p)
     } else if (p.out_mode[prob] == TC_OUT_ID) {
       p.out[prob][lo + (long long)erow * p.ldo[prob]] = z0;
     } else {  // TC_OUT_TD: y = r + gamma (1 - done) q'; dq = 2 (q - y) / B   (DDPG.jl:133, d mse / d q)
-      const float y = p.td_r[lo + erow] + (p.gamma * (1.0f - p.td_done[lo + erow])) * z0;
+      const float y = p.td_r[lo + erow] + (td_gamma * (1.0f - p.td_done[lo + erow])) * z0;
       p.out[prob][lo + (long long)erow * p.ldo[prob]] = y;
       p.td_dq[lo + erow] = 2.0f * (p.td_q[lo + erow] - y) * p.inv_batch;
     }

@@ -43,7 +43,8 @@ struct TcFwdChainArgs {
   float* H1[TC_MAX_PROBLEMS];                                      // [M][ldh1] layer-1 activations, or NULL (target nets: no backward pass)
   float* H2[TC_MAX_PROBLEMS];                                      // [M][ldh2] layer-2 activations, or NULL
   int out_mode[TC_MAX_PROBLEMS]; float* out[TC_MAX_PROBLEMS]; int ldo[TC_MAX_PROBLEMS];   // out[row*ldo + j]
-  const float *td_r, *td_done, *td_q; float* td_dq; float gamma, inv_batch;               // TC_OUT_TD
+  const float *td_r, *td_done, *td_q; float* td_dq; float inv_batch;                      // TC_OUT_TD
+  const float* td_gamma; long long td_gamma_stride;   // TC_OUT_TD: γ of learner l at td_gamma[l * td_gamma_stride] (its DDPG control block)
   int nsplit;                      // 2: a cluster of two CTAs per row tile, half of the layer-2 units each (for launches with few row tiles)
   int pdl, early_weights;          // programmatic dependent launch; early_weights: the predecessor in the stream did not write the net's weights
   int pop; long long pop_stride;   // a population of learners (grid.y): every pointer above moves by pop_stride floats per learner

@@ -153,6 +153,24 @@ class Learner:
         L.check(self.lib.ddpg_select_learner(self._h, int(learner)))
         return self
 
+    HPARAMS = ("lr_actor", "lr_critic", "gamma", "tau", "noise_scale")
+
+    def set_hparams(self, **kw):
+        """ddpg_set_hparams for the selected learner: any of lr_actor, lr_critic, gamma, tau, noise_scale (the others keep their
+        values).  Noise is drawn with σ_eff = float32(σ × noise_scale); the new values apply from the next launch on."""
+        bad = set(kw) - set(self.HPARAMS)
+        assert not bad, f"unknown hyper-parameters {sorted(bad)}"
+        hp = self.get_hparams()
+        hp.update({k: float(v) for k, v in kw.items()})
+        L.check(self.lib.ddpg_set_hparams(self._h, *[hp[k] for k in self.HPARAMS]))
+        return self
+
+    def get_hparams(self):
+        """ddpg_get_hparams: {lr_actor, lr_critic, gamma, tau, noise_scale} of the selected learner (float32 values)."""
+        v = [C.c_float() for _ in self.HPARAMS]
+        L.check(self.lib.ddpg_get_hparams(self._h, *[C.byref(x) for x in v]))
+        return {k: x.value for k, x in zip(self.HPARAMS, v)}
+
     def layer_shape(self, net, layer):
         S, A = self.p.state_size, self.p.action_size
         critic = net in (L.NET_CRITIC, L.NET_CRITIC_TARGET)
@@ -513,10 +531,13 @@ class PopulationDriver:
     run of equal chargers), so a vector step is: act (population) -> step (one launch per charger) -> remember (one launch)
     -> replay() (population).
 
-    chargers[l] is learner l's charger id (shems_LU1.jl:47-59), equal ids must be adjacent; seeds[l] its rng_run (input.jl:136)."""
+    chargers[l] is learner l's charger id (shems_LU1.jl:47-59), equal ids must be adjacent; seeds[l] its rng_run (input.jl:136).
+    hparams: per-learner hyper-parameters, a dict of lists of length P with keys from Learner.HPARAMS (lr_actor, lr_critic, gamma,
+    tau, noise_scale); missing keys keep the DdpgParams values (noise_scale: 1).  Learner l explores with σ_eff = sigma × noise_scale[l],
+    so a σ grid is sigma=1.0 with the grid values as noise_scale."""
 
     def __init__(self, series, chargers, seeds, n_envs=64, mem_size=24_000, ep_length=72, sigma=0.1, device=0, use_tensor_cores=1, native=True,
-                 **ddpg_kw):
+                 hparams=None, **ddpg_kw):
         from .env import Shems
         assert len(chargers) == len(seeds)
         self.native = bool(native)
@@ -535,6 +556,12 @@ class PopulationDriver:
         self.mems = [Replay(mem_size, device=device) for _ in range(self.P)]
         self.learner = Learner(params=L.default_ddpg_params(population=self.P, use_tensor_cores=use_tensor_cores, **ddpg_kw), device=device)
         self.learner.init(self.seeds[0])            # learner l: Philox(seeds[0] + l)
+        if hparams:
+            for k, v in hparams.items():
+                assert len(v) == self.P, f"hparams[{k!r}] has {len(v)} values for {self.P} learners"
+            for l in range(self.P):
+                self.learner.select(l).set_hparams(**{k: v[l] for k, v in hparams.items()})
+            self.learner.select(0)
         self._dev = torch.device("cuda", int(device))
         self._s_prev = torch.empty((9, self.N), dtype=torch.float32, device=self._dev)
         self.n_env_steps = 0

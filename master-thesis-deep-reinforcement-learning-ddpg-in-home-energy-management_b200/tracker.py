@@ -4,7 +4,8 @@
   (RL-SHEMS/src/memory_plotting_saving.jl:167-190; column order = the `results` row, shems_LU1.jl:476-478).
 * `save_checkpoint` / `load_checkpoint` — the reference saves the actor only (BSON, :263-270) and can therefore not resume
   training; here the whole state goes into one .npz: the 4 nets in Flux layout, both optimisers (ADAM moments, β powers, update
-  counter), normalisation constants, OU noise state, the replay memories — for every learner of a population handle.  The
+  counter), normalisation constants, per-learner hyper-parameters, OU noise state, the replay memories — for every learner of a
+  population handle.  The
   Julia shim turns the actor arrays back into a Flux Chain (same memory layout as Dense.W / Dense.b) for saveBSON.
 """
 import numpy as np
@@ -35,7 +36,7 @@ def save_checkpoint(path, learner, s_min=None, s_max=None, memories=None, **scor
     actor and the score arrays only, memory_plotting_saving.jl:263-270): for every learner l of the handle the four nets
     (Flux layout, `l{l}_actor_W1` ... — learner 0 also without the prefix, which is what the Julia shim turns into a Flux
     Chain), ADAM moments, β powers, update counter and normalisation constants (`l{l}_state`, `l{l}_opt`: ddpg_get_state),
-    OUNoise.X when OU episodes ran, and — with `memories` (one Replay per learner) — the replay memories in logical order."""
+    the hyper-parameters (`l{l}_hparams` = [lr_actor, lr_critic, gamma, tau, noise_scale] float32: ddpg_get_hparams), OUNoise.X when OU episodes ran, and — with `memories` (one Replay per learner) — the replay memories in logical order."""
     out = {}
     P = learner.population
     keep = getattr(learner, "_sel", 0)
@@ -44,6 +45,8 @@ def save_checkpoint(path, learner, s_min=None, s_max=None, memories=None, **scor
             learner.select(l)
         st, opt = learner.get_state()
         out[f"l{l}_state"], out[f"l{l}_opt"] = st, opt
+        hp = learner.get_hparams()
+        out[f"l{l}_hparams"] = np.array([hp[k] for k in learner.HPARAMS], np.float32)
         for net, name in NETS:
             for k in range(3):
                 i, o = learner.layer_shape(net, k)
@@ -74,7 +77,8 @@ def save_checkpoint(path, learner, s_min=None, s_max=None, memories=None, **scor
 def load_checkpoint(path, learner, memories=None):
     """Restores what save_checkpoint wrote: every learner's full state (a resumed run continues bit-identically,
     tests/test_resume_gpu.py) and, into the given EMPTY Replay objects, the replay memories.  Files holding only net
-    arrays (weights-only checkpoints) restore the nets of learner 0."""
+    arrays (weights-only checkpoints) restore the nets of learner 0; files without `l{l}_hparams` leave the hyper-parameters as
+    they are."""
     import torch
     z = np.load(path)
     P = learner.population
@@ -85,6 +89,8 @@ def load_checkpoint(path, learner, memories=None):
             if P > 1:
                 learner.select(l)
             learner.set_state(z[f"l{l}_state"], z[f"l{l}_opt"])
+            if f"l{l}_hparams" in z:
+                learner.set_hparams(**dict(zip(learner.HPARAMS, z[f"l{l}_hparams"].tolist())))
         if P > 1:
             learner.select(keep)
         if "ou_x" in z:

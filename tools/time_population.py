@@ -1,5 +1,7 @@
 """Times a population of independent DDPG learners (BASELINE configs[4]) advanced by one launch sequence.
-usage: python tools/time_population.py [P] [n_updates] [batch] [use_tensor_cores]"""
+usage: python tools/time_population.py [P] [n_updates] [batch] [use_tensor_cores] [mixed]
+mixed: also time the same population with distinct per-learner hyper-parameters (every learner its own lr_actor, lr_critic, gamma,
+tau: ddpg_set_hparams), alternating homogeneous and mixed windows, and report both."""
 import json
 import os
 import sys
@@ -13,6 +15,7 @@ P = int(sys.argv[1]) if len(sys.argv) > 1 else 80
 n_updates = int(sys.argv[2]) if len(sys.argv) > 2 else 100
 B = int(sys.argv[3]) if len(sys.argv) > 3 else 120
 tc = int(sys.argv[4]) if len(sys.argv) > 4 else 0
+mixed = len(sys.argv) > 5 and sys.argv[5] == "mixed"
 ser = sb.series.synth_charger98(4320, seed=98)
 mems = []
 for l in range(P):
@@ -28,16 +31,35 @@ for l in range(P):
     le.select(l).set_norm(mn, mx)
 le.replay(mems, rng_rpl=1, n_updates=10)
 torch.cuda.synchronize()
-res = []
+base = le.get_hparams()
+
+
+def set_all(mix):
+    for l in range(P):
+        f = 1.0 + 0.5 * (l % 4) if mix else 1.0   # four distinct tuples, cycled over the learners
+        le.select(l).set_hparams(lr_actor=base["lr_actor"] * f, lr_critic=base["lr_critic"] / f, gamma=base["gamma"] - 0.01 * (f - 1.0),
+                                 tau=base["tau"] * f)
+    le.select(0)
+
+
+res = {False: [], True: []}
 for rep in range(3):
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    le.replay(mems, rng_rpl=100 * rep, n_updates=n_updates)
-    e1.record()
-    torch.cuda.synchronize()
-    res.append(e0.elapsed_time(e1))
-ms = sorted(res)[1]
+    for mix in ((False, True) if mixed else (False,)):
+        if mixed:
+            set_all(mix)
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        le.replay(mems, rng_rpl=100 * rep, n_updates=n_updates)
+        e1.record()
+        torch.cuda.synchronize()
+        res[mix].append(e0.elapsed_time(e1))
+ms = sorted(res[False])[1]
 lc, la = le.select(P - 1).losses()
-print(json.dumps(dict(population=P, batch=B, tensor_cores=tc, n_updates=n_updates, us_per_population_update=1e3 * ms / n_updates,
-                      learner_updates_per_s=P * n_updates / ms * 1e3, tflops=10 * 256_500 * B * P * n_updates / ms / 1e9,
-                      loss_crit_last=lc, loss_act_last=la)))
+out = dict(population=P, batch=B, tensor_cores=tc, n_updates=n_updates, us_per_population_update=1e3 * ms / n_updates,
+           learner_updates_per_s=P * n_updates / ms * 1e3, tflops=10 * 256_500 * B * P * n_updates / ms / 1e9,
+           loss_crit_last=lc, loss_act_last=la)
+if mixed:
+    mm = sorted(res[True])[1]
+    out.update(us_per_population_update_mixed=1e3 * mm / n_updates, us_windows_homogeneous=[1e3 * x / n_updates for x in res[False]],
+               us_windows_mixed=[1e3 * x / n_updates for x in res[True]])
+print(json.dumps(out))
