@@ -440,6 +440,79 @@ shems_rollout_kernel(DevParams P, const float4* __restrict__ series, long long N
   if (S.ep_return) S.ep_return[n] = ret;
 }
 
+// The same rollout, trimmed for the launches that need none of the general kernel's options: FAST constants, a consistent env
+// (s[2..8] is series row idx, so only the four row fields the step reads are carried and the final obs write loads the last row
+// once), no trace, no obs trajectory, and either no ring or compact records with N and cap multiples of 32 (RingWalk).  One Philox
+// block serves two steps: the loop advances two steps per block, starting one step early when step0 is odd, and the round keys come
+// precomputed from the host.  Every output bit equals shems_rollout_kernel's.
+template <int POLICY, int MINB>
+__global__ void __launch_bounds__(ROLLOUT_THREADS, MINB)
+shems_rollout_lean_kernel(DevParams P, const float4* __restrict__ series, long long N, float* __restrict__ obs,
+                          int32_t* __restrict__ idx_arr, int T, int step0, PhiloxKeys K, long long env_id_base,
+                          const float* __restrict__ tape, int tape_unscaled, RolloutSinks S, long long n0, long long n1) {
+  const long long n = n0 + (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= n1) return;
+  int idx = idx_arr[n];
+  float Soc_b = obs[0 * N + n], Soc_ev = obs[1 * N + n];
+  float c_ev, d_e, g_e, p_buy;
+  { const Row8 r = load_row(series, idx); c_ev = r.cd; d_e = r.d_e; g_e = r.g_e; p_buy = r.p_buy; }
+  double ret = 0.0;
+  RingWalk ring{};
+  if (S.ring) { long long slot = S.head + n; if (slot >= S.cap) slot -= S.cap; ring = ring_walk(S.ring, slot, N, S.cap); }
+  const uint64_t id = (uint64_t)(env_id_base + n);
+  auto step = [&](int t, uint32_t w0, uint32_t w1) {
+    StepIn s;
+    s.Soc_b = Soc_b; s.Soc_ev = Soc_ev; s.c_ev = c_ev; s.d_e = d_e; s.g_e = g_e; s.p_buy = p_buy;
+    float B, EV, Bt, EVt, a_raw0, a_raw1;
+    bool track_neg = false;
+    if (POLICY == SHEMS_POLICY_RULE) {
+      shems_action_rule<true>(P, s.Soc_b, s.Soc_ev, s.d_e, s.g_e, B, EV);
+      Bt = 0.0f; EVt = 0.0f; a_raw0 = B; a_raw1 = EV; track_neg = true;
+    } else {
+      if (POLICY == SHEMS_POLICY_RANDOM) {
+        a_raw0 = action_from_word(w0);
+        a_raw1 = action_from_word(w1);
+        Bt = (a_raw0 + 1.0f) * 0.5f;
+        EVt = (a_raw1 + 1.0f) * 0.5f;
+      } else {
+        Bt = tape[((size_t)t * 2 + 0) * N + n];
+        EVt = tape[((size_t)t * 2 + 1) * N + n];
+        a_raw0 = Bt; a_raw1 = EVt;
+        if (tape_unscaled) {
+          Bt = (float)(((double)a_raw0 + 1.0) * 0.5);
+          EVt = (float)(((double)a_raw1 + 1.0) * 0.5);
+        }
+      }
+      shems_action_drl<true>(P, s.Soc_b, s.Soc_ev, s.c_ev, s.d_e, s.g_e, Bt, EVt, B, EV);
+    }
+    StepTrace tr;
+    const StepOut o = shems_flows<false, true>(P, s, B, EV, EVt, track_neg, &tr);
+    const Row8 nx = load_row(series, idx + 1);
+    float Soc_ev_new = o.Soc_ev;
+    if (nx.cd >= 0.0f && c_ev == -1.0f) Soc_ev_new = nx.soc_ev;
+    if (S.ring) {
+      ring_store_compact(ring.q, Soc_b, Soc_ev, a_raw0, a_raw1, (float)o.reward, o.Soc_b, Soc_ev_new, S.src_entry, idx);
+      ring_walk_next(ring);
+    }
+    if (S.reward_traj) S.reward_traj[(size_t)t * N + n] = (float)o.reward;
+    Soc_b = o.Soc_b; Soc_ev = Soc_ev_new; c_ev = nx.cd; d_e = nx.d_e; g_e = nx.g_e; p_buy = nx.p_buy;
+    idx += 1;
+    ret += o.reward;
+  };
+  // t is the step that uses words 0..1 of the block; with an odd step0 the first block's words 0..1 belong to step -1
+  for (int t = POLICY == SHEMS_POLICY_RANDOM ? -(step0 & 1) : 0; t < T; t += 2) {
+    uint32_t rw[4] = {0u, 0u, 0u, 0u};
+    if (POLICY == SHEMS_POLICY_RANDOM) philox4x32_10(K, id, (unsigned)(step0 + t) >> 1, STREAM_ACTION, rw);
+    if (t >= 0) step(t, rw[0], rw[1]);
+    if (t + 1 < T) step(t + 1, rw[2], rw[3]);
+  }
+  const Row8 r = load_row(series, idx);
+  obs[0 * N + n] = Soc_b; obs[1 * N + n] = Soc_ev; obs[2 * N + n] = r.cd; obs[3 * N + n] = r.d_e; obs[4 * N + n] = r.g_e;
+  obs[5 * N + n] = r.p_buy; obs[6 * N + n] = r.h_cos; obs[7 * N + n] = r.h_sin; obs[8 * N + n] = r.season;
+  idx_arr[n] = idx;
+  if (S.ep_return) S.ep_return[n] = ret;
+}
+
 // ----------------------------------------------------------------------------- C ABI
 static inline unsigned grid_for(long long n, int block) { return (unsigned)((n + block - 1) / block); }
 
@@ -449,12 +522,14 @@ static inline unsigned grid_for(long long n, int block) { return (unsigned)((n +
 // bound), times the per-instance penalty of the tighter register budget.  That model was measured on the store-bound kernel that
 // writes full ring records.  With compact records the kernel is issue bound and its MINB = 6 build needs only 66 registers (7 CTAs
 // per SM anyway); it was the fastest of 6 / 7 / 8 at 2^20 and at 2^17 instances (profiles/r3_ring_compact.md), so compact launches
-// take 6.  SHEMS_ROLLOUT_MIN_BLOCKS=6|7|8 overrides.
-static int rollout_min_blocks(int device, long long n, bool compact) {
+// take 6.  The trimmed kernel (shems_rollout_lean_kernel) needs 78 registers for the random policy at MINB 6, which leaves 6 CTAs per
+// SM; at MINB 7 it fits 72 without spilling and keeps 7, so its compact launches take 7 (profiles/r5_lean_rollout.md).
+// SHEMS_ROLLOUT_MIN_BLOCKS=6|7|8 overrides.
+static int rollout_min_blocks(int device, long long n, bool compact, bool lean) {
   static int forced = -1;
   if (forced < 0) { const char* ev = getenv("SHEMS_ROLLOUT_MIN_BLOCKS"); forced = ev ? atoi(ev) : 0; }
   if (forced == 6 || forced == 7 || forced == 8) return forced;
-  if (compact) return 6;
+  if (compact) return lean ? 7 : 6;
   static int sms[64];
   if (device >= 0 && device < 64 && sms[device] == 0) {
     int v = 0;
@@ -478,6 +553,13 @@ static int rollout_min_blocks(int device, long long n, bool compact) {
 // Compact ring records (see ring.cuh) unless SHEMS_RING_COMPACT=0 forces full ones (read at every rollout: the A/B switch).
 static bool ring_compact_enabled() {
   const char* ev = getenv("SHEMS_RING_COMPACT");
+  return !(ev && atoi(ev) == 0);
+}
+
+// shems_rollout_lean_kernel where it applies unless SHEMS_ROLLOUT_LEAN=0 forces the general kernel (read at every rollout: the
+// A/B switch for bit-equality tests and same-process timing)
+static bool rollout_lean_enabled() {
+  const char* ev = getenv("SHEMS_ROLLOUT_LEAN");
   return !(ev && atoi(ev) == 0);
 }
 
@@ -758,7 +840,18 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
     else if (mb == 8) LAUNCH_RO(POL, false, 8);                                                                                     \
     else LAUNCH_RO(POL, false, ROLLOUT_MIN_BLOCKS);                                                                                 \
   } while (0)
+#define LAUNCH_LEAN(POL, MB)                                                                                                        \
+  shems_rollout_lean_kernel<POL, MB><<<grid_for(n1 - n0, ROLLOUT_THREADS), ROLLOUT_THREADS, 0, e->stream>>>(                           \
+      e->gdp[g], e->gseries[g], e->n, e->obs, e->idx, a->n_steps, e->step, keys, a->env_id_base, a->tape_dev, a->tape_unscaled, S, n0, n1)
+#define LAUNCH_LEAN_MB(POL)                                                                                                         \
+  do {                                                                                                                              \
+    if (mb == 7) LAUNCH_LEAN(POL, 7);                                                                                               \
+    else if (mb == 8) LAUNCH_LEAN(POL, 8);                                                                                          \
+    else LAUNCH_LEAN(POL, ROLLOUT_MIN_BLOCKS);                                                                                      \
+  } while (0)
   const bool tr = a->trace_dev != nullptr;
+  const bool may_lean = !tr && !a->obs_traj_dev && e->consistent && rollout_lean_enabled();
+  const PhiloxKeys keys = philox_keys(a->seed);
   // compact records need s[2..8] == series row idx (consistent), a row that fits the tag and a series-table entry in the ring
   const bool may_compact = a->replay && e->consistent && e->nrows <= RING_TAG_MAX_ROW && ring_compact_enabled();
   for (int g = 0; g < e->n_groups; ++g) {
@@ -772,14 +865,25 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
       compact = entry >= 0;
       S.src_entry = compact ? ring_tag(entry, 0) : 0u;
     }
-    const int mb = rollout_min_blocks(e->device, n1 - n0, compact);
+    const bool lean = may_lean && e->gdp[g].fast_all && (!a->replay || (compact && e->n % 32 == 0 && S.cap % 32 == 0));
+    const int mb = rollout_min_blocks(e->device, n1 - n0, compact, lean);
     COUNT_LAUNCH();
+    if (lean) {
+      switch (a->policy) {
+        case SHEMS_POLICY_RULE: LAUNCH_LEAN_MB(SHEMS_POLICY_RULE); break;
+        case SHEMS_POLICY_RANDOM: LAUNCH_LEAN_MB(SHEMS_POLICY_RANDOM); break;
+        default: LAUNCH_LEAN_MB(SHEMS_POLICY_TAPE); break;
+      }
+      continue;
+    }
     switch (a->policy) {
       case SHEMS_POLICY_RULE: LAUNCH_RO_MB(SHEMS_POLICY_RULE); break;
       case SHEMS_POLICY_RANDOM: LAUNCH_RO_MB(SHEMS_POLICY_RANDOM); break;
       default: LAUNCH_RO_MB(SHEMS_POLICY_TAPE); break;
     }
   }
+#undef LAUNCH_LEAN_MB
+#undef LAUNCH_LEAN
 #undef LAUNCH_RO_MB
 #undef LAUNCH_RO
 #undef LAUNCH_RO_C

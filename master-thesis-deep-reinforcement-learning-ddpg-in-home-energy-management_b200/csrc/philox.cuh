@@ -18,20 +18,41 @@ __host__ __device__ __forceinline__ uint64_t mul_wide_u32(uint32_t a, uint32_t b
 #endif
 }
 
+__host__ __device__ __forceinline__ void philox_round(uint32_t& c0, uint32_t& c1, uint32_t& c2, uint32_t& c3, uint32_t k0, uint32_t k1) {
+  const uint64_t p0 = mul_wide_u32(0xD2511F53u, c0);
+  const uint64_t p1 = mul_wide_u32(0xCD9E8D57u, c2);
+  const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ k0;
+  const uint32_t n1 = (uint32_t)p1;
+  const uint32_t n2 = (uint32_t)(p0 >> 32) ^ c3 ^ k1;
+  const uint32_t n3 = (uint32_t)p0;
+  c0 = n0; c1 = n1; c2 = n2; c3 = n3;
+}
+
 __host__ __device__ __forceinline__ void philox4x32_10(uint64_t seed, uint64_t id, uint32_t ctr, uint32_t stream, uint32_t out[4]) {
   uint32_t c0 = (uint32_t)id, c1 = (uint32_t)(id >> 32), c2 = ctr, c3 = stream;
   uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
 #pragma unroll
   for (int r = 0; r < 10; ++r) {
-    const uint64_t p0 = mul_wide_u32(0xD2511F53u, c0);
-    const uint64_t p1 = mul_wide_u32(0xCD9E8D57u, c2);
-    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ k0;
-    const uint32_t n1 = (uint32_t)p1;
-    const uint32_t n2 = (uint32_t)(p0 >> 32) ^ c3 ^ k1;
-    const uint32_t n3 = (uint32_t)p0;
-    c0 = n0; c1 = n1; c2 = n2; c3 = n3;
+    philox_round(c0, c1, c2, c3, k0, k1);
     k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
   }
+  out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
+}
+
+// The 10 round keys of a seed, for a kernel that draws many blocks under one seed: passed as a kernel argument, the rounds read
+// them as constant-bank operands instead of adding the Weyl increments per thread and call.
+struct PhiloxKeys { uint32_t k0[10], k1[10]; };
+inline PhiloxKeys philox_keys(uint64_t seed) {
+  PhiloxKeys K;
+  uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+  for (int r = 0; r < 10; ++r, k0 += 0x9E3779B9u, k1 += 0xBB67AE85u) { K.k0[r] = k0; K.k1[r] = k1; }
+  return K;
+}
+// philox4x32_10(seed, id, ctr, stream, out) with K = philox_keys(seed)
+__device__ __forceinline__ void philox4x32_10(const PhiloxKeys& K, uint64_t id, uint32_t ctr, uint32_t stream, uint32_t out[4]) {
+  uint32_t c0 = (uint32_t)id, c1 = (uint32_t)(id >> 32), c2 = ctr, c3 = stream;
+#pragma unroll
+  for (int r = 0; r < 10; ++r) philox_round(c0, c1, c2, c3, K.k0[r], K.k1[r]);
   out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
 }
 // 53-bit uniform in [0,1) from two words (stands in for Julia's Float64 rand())

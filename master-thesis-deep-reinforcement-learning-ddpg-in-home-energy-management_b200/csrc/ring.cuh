@@ -84,6 +84,23 @@ __host__ __device__ __forceinline__ long long ring_push_slot(long long head, lon
   return slot - (slot / cap) * cap;
 }
 
+// The record addresses a writer visits at slots s, s + N, s + 2N, ... (mod cap) when N and cap are multiples of 32: slot + N keeps
+// the lane (slot & 31) and moves N / 32 tiles, so the address advances by a constant stride and wraps with one compare.
+struct RingWalk {
+  float* q;            // record of the current slot
+  const float* last;   // from here on the next slot wraps
+  ptrdiff_t stride, back;  // N / 32 tiles, and the same less the ring's cap / 32 tiles
+};
+__host__ __device__ __forceinline__ RingWalk ring_walk(float* ring, long long slot, long long N, long long cap) {
+  RingWalk w;
+  w.q = ring + ring_base(slot);
+  w.stride = (ptrdiff_t)(N >> 5) * RING_FIELDS * 32;
+  w.back = w.stride - (ptrdiff_t)(cap >> 5) * RING_FIELDS * 32;
+  w.last = ring - w.back;  // N <= cap: at most one wrap
+  return w;
+}
+__host__ __device__ __forceinline__ void ring_walk_next(RingWalk& w) { w.q += (w.q >= w.last) ? w.back : w.stride; }
+
 // minibatch row j of update `update`: Philox(seed, id = j, ctr = update, stream SAMPLE) -> logical index floor(u * len)
 __host__ __device__ __forceinline__ long long ring_draw(uint64_t seed, uint64_t j, uint32_t update, long long len) {
   uint32_t w[4];
