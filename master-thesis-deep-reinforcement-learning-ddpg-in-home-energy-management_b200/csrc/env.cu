@@ -445,11 +445,19 @@ shems_rollout_kernel(DevParams P, const float4* __restrict__ series, long long N
 // once), no trace, no obs trajectory, and either no ring or compact records with N and cap multiples of 32 (RingWalk).  One Philox
 // block serves two steps: the loop advances two steps per block, starting one step early when step0 is odd, and the round keys come
 // precomputed from the host.  Every output bit equals shems_rollout_kernel's.
+// Lock step: a warp whose instances all stand at the same row when the launch starts stays in step with itself (every instance
+// advances one row per step), so the row class (shems_device.cuh) is uniform across it at every step.  Such a warp (when `lockstep`
+// allows it) runs a loop that dispatches each step to the body compiled for the row's class.  That loop advances one step per
+// iteration, so each class body is inlined once (about 19 KB of loop); the Philox block is drawn on even steps and its words 2..3
+// serve the odd one.  Two steps per iteration with every body inlined twice was measured faster in lock step but slower on the
+// two-step loop (profiles/r6_lockstep_rollout.md).  Any other warp runs the two-step loop with the general body only.  Each lane
+// takes its own row's class, so the bits never depend on the vote: it only decides the speed.
+template <int CLS> struct RowTag { static constexpr int value = CLS; };
 template <int POLICY, int MINB>
 __global__ void __launch_bounds__(ROLLOUT_THREADS, MINB)
 shems_rollout_lean_kernel(DevParams P, const float4* __restrict__ series, long long N, float* __restrict__ obs,
                           int32_t* __restrict__ idx_arr, int T, int step0, PhiloxKeys K, long long env_id_base,
-                          const float* __restrict__ tape, int tape_unscaled, RolloutSinks S, long long n0, long long n1) {
+                          const float* __restrict__ tape, int tape_unscaled, RolloutSinks S, long long n0, long long n1, int lockstep) {
   const long long n = n0 + (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (n >= n1) return;
   int idx = idx_arr[n];
@@ -460,7 +468,8 @@ shems_rollout_lean_kernel(DevParams P, const float4* __restrict__ series, long l
   RingWalk ring{};
   if (S.ring) { long long slot = S.head + n; if (slot >= S.cap) slot -= S.cap; ring = ring_walk(S.ring, slot, N, S.cap); }
   const uint64_t id = (uint64_t)(env_id_base + n);
-  auto step = [&](int t, uint32_t w0, uint32_t w1) {
+  auto step = [&](auto cls, int t, uint32_t w0, uint32_t w1) {
+    constexpr int CLS = decltype(cls)::value;
     StepIn s;
     s.Soc_b = Soc_b; s.Soc_ev = Soc_ev; s.c_ev = c_ev; s.d_e = d_e; s.g_e = g_e; s.p_buy = p_buy;
     float B, EV, Bt, EVt, a_raw0, a_raw1;
@@ -483,13 +492,13 @@ shems_rollout_lean_kernel(DevParams P, const float4* __restrict__ series, long l
           EVt = (float)(((double)a_raw1 + 1.0) * 0.5);
         }
       }
-      shems_action_drl<true>(P, s.Soc_b, s.Soc_ev, s.c_ev, s.d_e, s.g_e, Bt, EVt, B, EV);
+      shems_action_drl<true, CLS>(P, s.Soc_b, s.Soc_ev, s.c_ev, s.d_e, s.g_e, Bt, EVt, B, EV);
     }
     StepTrace tr;
-    const StepOut o = shems_flows<false, true>(P, s, B, EV, EVt, track_neg, &tr);
+    const StepOut o = shems_flows<false, true, CLS>(P, s, B, EV, EVt, track_neg, &tr);
     const Row8 nx = load_row(series, idx + 1);
     float Soc_ev_new = o.Soc_ev;
-    if (nx.cd >= 0.0f && c_ev == -1.0f) Soc_ev_new = nx.soc_ev;
+    if (nx.cd >= 0.0f && (CLS == ROW_ANY ? c_ev == -1.0f : row_noev<CLS>)) Soc_ev_new = nx.soc_ev;
     if (S.ring) {
       ring_store_compact(ring.q, Soc_b, Soc_ev, a_raw0, a_raw1, (float)o.reward, o.Soc_b, Soc_ev_new, S.src_entry, idx);
       ring_walk_next(ring);
@@ -499,12 +508,32 @@ shems_rollout_lean_kernel(DevParams P, const float4* __restrict__ series, long l
     idx += 1;
     ret += o.reward;
   };
-  // t is the step that uses words 0..1 of the block; with an odd step0 the first block's words 0..1 belong to step -1
-  for (int t = POLICY == SHEMS_POLICY_RANDOM ? -(step0 & 1) : 0; t < T; t += 2) {
+  // the lanes that returned above are not in the mask (N need not be a multiple of 32 without a ring)
+  const unsigned mask = __activemask();
+  if (lockstep && __all_sync(mask, idx == __shfl_sync(mask, idx, __ffs(mask) - 1))) {
     uint32_t rw[4] = {0u, 0u, 0u, 0u};
-    if (POLICY == SHEMS_POLICY_RANDOM) philox4x32_10(K, id, (unsigned)(step0 + t) >> 1, STREAM_ACTION, rw);
-    if (t >= 0) step(t, rw[0], rw[1]);
-    if (t + 1 < T) step(t + 1, rw[2], rw[3]);
+    for (int t = 0; t < T; ++t) {
+      if (POLICY == SHEMS_POLICY_RANDOM) {  // words 0..1 of block (step0 + t) / 2 serve even steps, words 2..3 odd ones
+        const unsigned st_abs = (unsigned)(step0 + t);
+        if ((st_abs & 1u) == 0u || t == 0) philox4x32_10(K, id, st_abs >> 1, STREAM_ACTION, rw);
+        if (st_abs & 1u) { rw[0] = rw[2]; rw[1] = rw[3]; }
+      }
+      switch (row_class(P, c_ev, d_e, g_e)) {
+        case ROW_A_NOEV: step(RowTag<ROW_A_NOEV>{}, t, rw[0], rw[1]); break;
+        case ROW_B_NOEV: step(RowTag<ROW_B_NOEV>{}, t, rw[0], rw[1]); break;
+        case ROW_A_EV: step(RowTag<ROW_A_EV>{}, t, rw[0], rw[1]); break;
+        case ROW_B_EV: step(RowTag<ROW_B_EV>{}, t, rw[0], rw[1]); break;
+        default: step(RowTag<ROW_ANY>{}, t, rw[0], rw[1]); break;
+      }
+    }
+  } else {
+    // t is the step that uses words 0..1 of the block; with an odd step0 the first block's words 0..1 belong to step -1
+    for (int t = POLICY == SHEMS_POLICY_RANDOM ? -(step0 & 1) : 0; t < T; t += 2) {
+      uint32_t rw[4] = {0u, 0u, 0u, 0u};
+      if (POLICY == SHEMS_POLICY_RANDOM) philox4x32_10(K, id, (unsigned)(step0 + t) >> 1, STREAM_ACTION, rw);
+      if (t >= 0) step(RowTag<ROW_ANY>{}, t, rw[0], rw[1]);
+      if (t + 1 < T) step(RowTag<ROW_ANY>{}, t + 1, rw[2], rw[3]);
+    }
   }
   const Row8 r = load_row(series, idx);
   obs[0 * N + n] = Soc_b; obs[1 * N + n] = Soc_ev; obs[2 * N + n] = r.cd; obs[3 * N + n] = r.d_e; obs[4 * N + n] = r.g_e;
@@ -560,6 +589,13 @@ static bool ring_compact_enabled() {
 // A/B switch for bit-equality tests and same-process timing)
 static bool rollout_lean_enabled() {
   const char* ev = getenv("SHEMS_ROLLOUT_LEAN");
+  return !(ev && atoi(ev) == 0);
+}
+
+// the trimmed kernel's lock-step loop for warps that start on one row unless SHEMS_ROLLOUT_LOCKSTEP=0 keeps every warp on its
+// two-step loop (read at every rollout: the A/B switch)
+static bool rollout_lockstep_enabled() {
+  const char* ev = getenv("SHEMS_ROLLOUT_LOCKSTEP");
   return !(ev && atoi(ev) == 0);
 }
 
@@ -842,7 +878,8 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
   } while (0)
 #define LAUNCH_LEAN(POL, MB)                                                                                                        \
   shems_rollout_lean_kernel<POL, MB><<<grid_for(n1 - n0, ROLLOUT_THREADS), ROLLOUT_THREADS, 0, e->stream>>>(                           \
-      e->gdp[g], e->gseries[g], e->n, e->obs, e->idx, a->n_steps, e->step, keys, a->env_id_base, a->tape_dev, a->tape_unscaled, S, n0, n1)
+      e->gdp[g], e->gseries[g], e->n, e->obs, e->idx, a->n_steps, e->step, keys, a->env_id_base, a->tape_dev, a->tape_unscaled, S, n0, n1, \
+      lockstep)
 #define LAUNCH_LEAN_MB(POL)                                                                                                         \
   do {                                                                                                                              \
     if (mb == 7) LAUNCH_LEAN(POL, 7);                                                                                               \
@@ -852,6 +889,7 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
   const bool tr = a->trace_dev != nullptr;
   const bool may_lean = !tr && !a->obs_traj_dev && e->consistent && rollout_lean_enabled();
   const PhiloxKeys keys = philox_keys(a->seed);
+  const int lockstep = rollout_lockstep_enabled() ? 1 : 0;
   // compact records need s[2..8] == series row idx (consistent), a row that fits the tag and a series-table entry in the ring
   const bool may_compact = a->replay && e->consistent && e->nrows <= RING_TAG_MAX_ROW && ring_compact_enabled();
   for (int g = 0; g < e->n_groups; ++g) {

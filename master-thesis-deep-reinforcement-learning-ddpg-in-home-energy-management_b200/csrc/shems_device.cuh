@@ -59,6 +59,23 @@ __device__ __forceinline__ double ddiv_const(double x, double d, double r, int o
   return fma(e, r, q);
 }
 
+// Row class: the values of the step's predicates that depend only on the series row — A = Float32(g_e * pv_eta) > d_e (PV covers the
+// demand, :368), c_ev > -1 (EV present, :292), c_ev == 0 (departure hour, :438), c_ev < 0 (no EV, :445) and c_ev == -1 (arrival test,
+// :270).  ROW_ANY evaluates them at run time; every other class fixes them, so a body instantiated for it is the same code with those
+// predicates as constants.  row_class() derives the class from the very expressions the step evaluates, so a lane gets the same bits
+// from the body of its class as from the ROW_ANY body.  Departure hours, -0.0, values in (-1, 0) and NaN stay ROW_ANY.
+enum RowClass { ROW_ANY = 0, ROW_A_NOEV, ROW_B_NOEV, ROW_A_EV, ROW_B_EV };   // A / B: branch :368 / :388; NOEV: c_ev == -1; EV: c_ev > 0
+__device__ __forceinline__ int row_class(const DevParams& P, float c_ev, float d_e, float g_e) {
+  const bool A = g_e * P.pv_eta > d_e;
+  if (c_ev == -1.0f) return A ? ROW_A_NOEV : ROW_B_NOEV;
+  if (c_ev > 0.0f) return A ? ROW_A_EV : ROW_B_EV;
+  return ROW_ANY;
+}
+// what a class other than ROW_ANY fixes; the step writes each predicate as `CLS == ROW_ANY ? <run-time test> : <constant>` in place
+template <int CLS> constexpr bool row_A = CLS == ROW_A_NOEV || CLS == ROW_A_EV;         // A
+template <int CLS> constexpr bool row_ev = CLS == ROW_A_EV || CLS == ROW_B_EV;          // c_ev > 0: c_ev > -1, not == 0, not < 0, not == -1
+template <int CLS> constexpr bool row_noev = CLS == ROW_A_NOEV || CLS == ROW_B_NOEV;    // c_ev == -1: not > -1, not == 0, < 0, == -1
+
 // FAST (template parameter of everything below) = the constants are in their usual state — P.fast_all: Float32-valued divisors,
 // Float32 penalty weight, shems_LU1's reward form — so the flag tests, the fall-back branches and the guarded Float32 division
 // sequences are compiled out (the Float32 quotients go through fdiv_const_wide), and Float32 decisions against Float64 constants are
@@ -75,12 +92,12 @@ __device__ __forceinline__ float charge_request_f(const DevParams& P, float pv, 
 __device__ __forceinline__ float discharge_request_f(const DevParams& P, float x) { return -((x < P.R_up) ? x : P.R_f); }
 
 // action(env, a::ShemsAction) :283-316 -> Float32.([B, EV])
-template <bool FAST>
+template <bool FAST, int CLS = ROW_ANY>
 __device__ __forceinline__ void shems_action_drl(const DevParams& P, float Soc_b, float Soc_ev, float c_ev, float d_e,
                                                  float g_e, float Bt, float EVt, float& B, float& EV) {
   const float sb0 = Soc_b - P.smin;
   const float perc = FAST ? fdiv_const_wide((double)sb0, P.span_d, P.r_span_d) : fdiv_const(sb0, P.span, P.r_span_f, P.fast_span_f);   // :288
-  EV = (c_ev > -1.0f && Soc_ev < EVt) ? jl_minf(P.evR, (EVt - Soc_ev) * P.C) : 0.0f;      // :292-297
+  EV = ((CLS == ROW_ANY ? c_ev > -1.0f : row_ev<CLS>) && Soc_ev < EVt) ? jl_minf(P.evR, (EVt - Soc_ev) * P.C) : 0.0f;      // :292-297
   const float pv = (g_e - d_e) - EV;                                                      // :301
   // :304-313 evaluated branch-free: charge request / discharge request / nothing
   const float Btv = Bt * P.span + P.smin;                                                 // :306 (two roundings, fmad off)
@@ -96,7 +113,7 @@ __device__ __forceinline__ void shems_action_drl(const DevParams& P, float Soc_b
   B = (pv > 0.0f && perc < Bt) ? Bc : ((Soc_b > 1e-3f) ? Bd : 0.0f);
 }
 
-// action(env, track) rule-based controller :318-340 -> Float32.([B, EV])
+// action(env, track) rule-based controller :318-340 -> Float32.([B, EV]); it reads no row predicate, so it takes no row class
 template <bool FAST>
 __device__ __forceinline__ void shems_action_rule(const DevParams& P, float Soc_b, float Soc_ev, float d_e, float g_e,
                                                   float& B, float& EV) {
@@ -123,7 +140,7 @@ static __device__ __noinline__ double shems_discomfort_term(int reward_form, dou
   return (pot == 1.0) ? dwd : (pot == 2.0) ? dwd * dwd : pow(dwd, pot);
 }
 
-template <bool WANT_TRACE, bool FAST>
+template <bool WANT_TRACE, bool FAST, int CLS = ROW_ANY>
 __device__ __forceinline__ StepOut shems_flows(const DevParams& P, const StepIn& s, float B, float EV, float EVt,
                                                bool track_neg, StepTrace* tr) {
   const float eta = P.b_eta;
@@ -132,7 +149,7 @@ __device__ __forceinline__ StepOut shems_flows(const DevParams& P, const StepIn&
   const double BD0 = (B < -0.01f) ? jl_clampd((double)(-B), 0.001, jl_mind(P.R, (double)(P.one_m_l_e * s.Soc_b))) : 0.0;
   // :368-409  PV -> demand -> EV, then battery -> demand -> EV, grid takes the slack
   const float ge = s.g_e * P.pv_eta;
-  const bool A = ge > s.d_e;                 // :368 PV covers the demand      (else :388)
+  const bool A = CLS == ROW_ANY ? ge > s.d_e : row_A<CLS>;   // :368 PV covers the demand      (else :388)
   const float pvr = ge - s.d_e;              // :370 PV left after the demand   (branch A)
   const float dB = s.d_e - ge;               // :391 demand left after the PV   (branch B)
   const bool A1 = A && (pvr > EV);           // :371 PV also covers the EV
@@ -183,12 +200,12 @@ __device__ __forceinline__ StepOut shems_flows(const DevParams& P, const StepIn&
   // :438-449
   float disc = 0.0f, EX_EV = 0.0f;
   double pen = 0.0;
-  if (s.c_ev == 0.0f && Soc_ev_new < 1.0f) {
+  if ((CLS == ROW_ANY ? s.c_ev == 0.0f : false) && Soc_ev_new < 1.0f) {
     const float short_ = 1.0f - Soc_ev_new;
     disc = short_ * 100.0f;
     EX_EV = short_ * P.C;
     Soc_ev_new = 1.0f;
-  } else if (s.c_ev < 0.0f && EVt < 0.99f) {  // F32 < 0.99 (Float64) <=> F32 < 0.99f0
+  } else if ((CLS == ROW_ANY ? s.c_ev < 0.0f : row_noev<CLS>) && EVt < 0.99f) {  // F32 < 0.99 (Float64) <=> F32 < 0.99f0
     // shems_LU1: Float32 product with penalty_weight::Float32; LU7 / input0607: penalty_weight is a Float64 -> Float64 product
     const float om = 1.0f - EVt;
     pen = (double)(om * P.pw);
