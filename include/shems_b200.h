@@ -269,7 +269,9 @@ typedef struct DdpgParams {
                              * parallelism (RL-SHEMS_bs_scheduler_*.sh:73-81) folded into one handle */
 } DdpgParams;
 
-enum { DDPG_NET_ACTOR = 0, DDPG_NET_CRITIC = 1, DDPG_NET_ACTOR_TARGET = 2, DDPG_NET_CRITIC_TARGET = 3 };
+/* DDPG_NET_ACTOR_BEST: the best-actor slot of a learner (what ddpg_keep_best keeps; ddpg_evaluate can run it).  ddpg_get_layer,
+ * ddpg_set_layer and ddpg_num_params accept it; every other call that takes a net rejects it with SHEMS_ERR_INVALID. */
+enum { DDPG_NET_ACTOR = 0, DDPG_NET_CRITIC = 1, DDPG_NET_ACTOR_TARGET = 2, DDPG_NET_CRITIC_TARGET = 3, DDPG_NET_ACTOR_BEST = 4 };
 
 typedef struct Ddpg Ddpg;
 SHEMS_API int32_t ddpg_default_params(DdpgParams* out);
@@ -336,6 +338,23 @@ SHEMS_API int32_t ddpg_episode(Ddpg* h, ShemsEnv* env, ShemsReplay* const* rps, 
  *   (:207-208);  act_traj_dev [T][2][N] float or NULL: the unscaled actions a.  Seeds as ddpg_episode; reset! stays with the caller. */
 SHEMS_API int32_t ddpg_rollout(Ddpg* h, ShemsEnv* env, int32_t n_steps, float sigma, uint64_t seed, int64_t env_id_base,
                                double* ep_return_dev, double* trace_dev, float* act_traj_dev);
+/* Evaluation and best-actor bookkeeping of run_episodes (DDPG.jl:266-289) for EVERY learner of the handle (P = 1 included).
+ * ddpg_evaluate: episode!(env; train = false) / inference(env; track = 1) without noise, by ONE call: the persistent cluster kernel of
+ * ddpg_rollout with a learner dimension (8 instances of one learner per cluster, that learner's actor and s_min / s_max), so a learner
+ * evaluated inside a population gets the bits it gets on a one-learner handle.  net = DDPG_NET_ACTOR or DDPG_NET_ACTOR_BEST; env holds
+ * N = P*n instances, learner l owns l*n .. l*n+n-1, and for P > 1 no group boundary of env may split a learner's instances.  Outputs, env_id_base,
+ * preconditions (one stream, reset! first) and SHEMS_ERR_BOUNDS (nothing launched) as ddpg_rollout; SHEMS_ERR_INVALID also when l1 > 256
+ * or l2 > 512 or a group splits a learner of a population.  For P == 1 and net = ACTOR it equals ddpg_rollout with sigma = 0. */
+SHEMS_API int32_t ddpg_evaluate(Ddpg* h, ShemsEnv* env, int32_t net, int32_t n_steps, int64_t env_id_base, double* ep_return_dev,
+                                double* trace_dev, float* act_traj_dev);
+/* ddpg_keep_best: one enqueue, no host round trip.  For every learner l: score_l = (sum over k of ep_return_dev[l*n + k]) / n, summed in
+ * index order in Float64 (score_mean, :273) and written to score_dev [P] unless NULL; if score_l > best_score_l (strict: a tie or NaN
+ * never wins, :282) best_score_l = score_l, best_run_l = episode and learner l's actor is copied into its DDPG_NET_ACTOR_BEST slot.
+ * ddpg_create starts every learner at best_score = -100000, best_run = 0 and a zero best actor.  ddpg_get_best / ddpg_set_best move the
+ * [P] arrays (set: checkpoint restore, the start of run_episodes; the best-actor weights go through ddpg_set_layer(ACTOR_BEST)). */
+SHEMS_API int32_t ddpg_keep_best(Ddpg* h, const double* ep_return_dev, int64_t n, int32_t episode, double* score_dev);
+SHEMS_API int32_t ddpg_get_best(Ddpg* h, double* best_score_host, int32_t* best_run_host);
+SHEMS_API int32_t ddpg_set_best(Ddpg* h, const double* best_score_host, const int32_t* best_run_host);
 /* replay() (DDPG.jl:121-145) n_updates times: sample -> TD target -> critic step -> actor step
  * -> Polyak.  idx_host ([n_updates][batch], 0-based logical indices) or NULL -> Philox(seed, draw j, counter u = index of the
  * update inside this call): replay(rng_rpl = r) trains on the minibatch replay_sample(seed = r) returns, as getData(rng) is one

@@ -13,7 +13,7 @@ OK, ERR_INVALID, ERR_CUDA, ERR_BOUNDS, ERR_KEY, ERR_STATE = 0, -1, -2, -3, -4, -
 RESET_DETERMINISTIC, RESET_HOST_DRAWS, RESET_DEVICE_PHILOX = 0, 1, 2
 POLICY_RULE, POLICY_RANDOM, POLICY_TAPE = 0, 1, 2
 ENV_LU1, ENV_LU7, ENV_LU1_INPUT0607 = 0, 1, 2
-NET_ACTOR, NET_CRITIC, NET_ACTOR_TARGET, NET_CRITIC_TARGET = 0, 1, 2, 3
+NET_ACTOR, NET_CRITIC, NET_ACTOR_TARGET, NET_CRITIC_TARGET, NET_ACTOR_BEST = 0, 1, 2, 3, 4
 DP_HANDLE_BYTES = 192
 
 
@@ -132,6 +132,10 @@ SIGNATURES = {
     "shems_tc_gemm": (I32, [VP, I64, I32, VP, I64, I32, VP, I64, I32, I32, I32, I32, VP, VP, I64, I32, VP, VP]),
     "ddpg_grad_buffer": (I32, [VP, C.POINTER(VP), C.POINTER(I64)]),
     "ddpg_rollout": (I32, [VP, VP, I32, F32, U64, I64, VP, VP, VP]),
+    "ddpg_evaluate": (I32, [VP, VP, I32, I32, I64, VP, VP, VP]),
+    "ddpg_keep_best": (I32, [VP, VP, I64, I32, VP]),
+    "ddpg_get_best": (I32, [VP, PD, PI]),
+    "ddpg_set_best": (I32, [VP, PD, PI]),
     "ddpg_state_floats": (I64, [VP]),
     "ddpg_get_state": (I32, [VP, PF, PD]),
     "ddpg_set_state": (I32, [VP, PF, PD]),

@@ -28,30 +28,36 @@ actor_rollout_kernel(const ActorRolloutArgs a) {
   const Geo g = make_geo(a.l1, a.l2, a.vec16, cluster);
   const int l1 = a.l1, l2 = a.l2;
   const long long N = a.N;
-  const long long j0 = a.n0 + g.row0;    // first instance of this cluster
+  // The launch's instances n0 .. n1-1 are segments of a.seg instances; segment s is learner a.l0 + s and takes ceil(seg / 8)
+  // clusters, the rows past its end idle.  One learner: a single segment over the whole range (l0 = 0).
+  const long long cps = (a.seg + FUSED_ROWS - 1) / FUSED_ROWS, c = blockIdx.x / FUSED_CLUSTER, sg = c / cps;
+  const long long j0 = a.n0 + sg * a.seg + (c - sg * cps) * FUSED_ROWS;   // first instance of this cluster
+  const long long jend = a.n0 + (sg + 1) * a.seg;                          // end of its learner's instances
+  const float* actor = a.actor + (a.l0 + sg) * a.actor_stride;
+  const float* norm = a.norm + (a.l0 + sg) * a.norm_stride;
   float* raw = S->x[1];                  // env.state of the 8 instances [row][12]
   cluster_arrive();
-  stage_w2(S->W[0], a.actor + a.ao.w2, l1, l2, g.n0, g.nv, a.vec16 != 0, tid);
+  stage_w2(S->W[0], actor + a.ao.w2, l1, l2, g.n0, g.nv, a.vec16 != 0, tid);
   if (tid < 72) {
     const int r = tid / 9, k = tid - r * 9;
     const long long j = j0 + r;
-    raw[r * 12 + k] = (j < a.n1) ? a.obs[(long long)k * N + j] : 0.0f;
+    raw[r * 12 + k] = (j < jend) ? a.obs[(long long)k * N + j] : 0.0f;
   } else if (tid >= 96 && tid < 96 + FUSED_ROWS) {
     const int r = tid - 96;
     const long long j = j0 + r;
-    const int idx = (j < a.n1) ? a.idx[j] : 1;
+    const int idx = (j < jend) ? a.idx[j] : 1;
     s_idx[r] = idx;
     s_cd[r] = __ldg(&reinterpret_cast<const float*>(a.series)[8 * (size_t)(idx - 1) + 1]);
     s_ret[r] = 0.0;
   }
-  const L1Regs Ra = load_l1(a.actor + a.ao.w1, a.actor + a.ao.b1, 9, l1, tid);
-  const TailRegs Ta = load_tail(a.actor + a.ao.b2 + g.n0, a.actor + a.ao.w3 + g.n0 * 2, 2, g.nv, lane);
-  const float b3a0 = __ldg(a.actor + a.ao.b3), b3a1 = __ldg(a.actor + a.ao.b3 + 1);
+  const L1Regs Ra = load_l1(actor + a.ao.w1, actor + a.ao.b1, 9, l1, tid);
+  const TailRegs Ta = load_tail(actor + a.ao.b2 + g.n0, actor + a.ao.w3 + g.n0 * 2, 2, g.nv, lane);
+  const float b3a0 = __ldg(actor + a.ao.b3), b3a1 = __ldg(actor + a.ao.b3 + 1);
   float nlo = 0.0f, nden = 1.0f;         // normalize(): thread (row, field k) keeps its s_min[k] and s_max[k] - s_min[k] + 1f-8
   if (tid < 72) {
     const int k = tid % 9;
-    nlo = a.norm[k];
-    nden = __fadd_rn(__fsub_rn(a.norm[9 + k], nlo), 1e-8f);
+    nlo = norm[k];
+    nden = __fadd_rn(__fsub_rn(norm[9 + k], nlo), 1e-8f);
   }
   cp_wait<0>();
   __syncthreads();
@@ -59,7 +65,7 @@ actor_rollout_kernel(const ActorRolloutArgs a) {
   for (int t = 0; t < a.T; ++t) {
     if (tid < 72) {  // normalize(s) = (s - s_min) / (s_max - s_min + 1f-8)   (memory_plotting_saving.jl:55-57); idle rows stay zero
       const int r = tid / 9, k = tid - r * 9;
-      S->x[0][r * 12 + k] = (j0 + r < a.n1) ? __fdiv_rn(__fsub_rn(raw[r * 12 + k], nlo), nden) : 0.0f;
+      S->x[0][r * 12 + k] = (j0 + r < jend) ? __fdiv_rn(__fsub_rn(raw[r * 12 + k], nlo), nden) : 0.0f;
     }
     __syncthreads();
     f1(Ra, 9, l1, S->x[0], S->h1T[0], tid);
@@ -68,7 +74,7 @@ actor_rollout_kernel(const ActorRolloutArgs a) {
     const int buf = t & 1;   // two all-gather buffers alternate: a peer refills one only after the barrier that follows my reads of it
     f3_partial(Ta, S->h2s[0], S, buf, cluster, g.rank, tid);
     cluster.sync();
-    if (tid < FUSED_ROWS && j0 + tid < a.n1) {
+    if (tid < FUSED_ROWS && j0 + tid < jend) {
       const int r = tid;
       const long long j = j0 + r;
       const float y0 = tanhf(xch_sum(S, buf, r, 0) + b3a0), y1 = tanhf(xch_sum(S, buf, r, 1) + b3a1);
@@ -111,10 +117,10 @@ actor_rollout_kernel(const ActorRolloutArgs a) {
   if (g.rank == 0) {
     if (tid < 72) {
       const int r = tid / 9, k = tid - r * 9;
-      if (j0 + r < a.n1) a.obs[(long long)k * N + j0 + r] = raw[r * 12 + k];
+      if (j0 + r < jend) a.obs[(long long)k * N + j0 + r] = raw[r * 12 + k];
     } else if (tid >= 96 && tid < 96 + FUSED_ROWS) {
       const int r = tid - 96;
-      if (j0 + r < a.n1) {
+      if (j0 + r < jend) {
         a.idx[j0 + r] = s_idx[r];
         if (a.ep_return) a.ep_return[j0 + r] = s_ret[r];
       }
@@ -130,7 +136,8 @@ int actor_rollout_prepare() {
 int actor_rollout_launch(cudaStream_t st, const ActorRolloutArgs& a) {
   const long long n = a.n1 - a.n0;
   if (n <= 0) return SHEMS_OK;
-  const unsigned clusters = (unsigned)((n + FUSED_ROWS - 1) / FUSED_ROWS);
+  if (a.seg < 1 || n % a.seg != 0) { shems_set_error("actor_rollout: %lld instances are not whole segments of %lld", n, a.seg); return SHEMS_ERR_INVALID; }
+  const unsigned clusters = (unsigned)((n / a.seg) * ((a.seg + FUSED_ROWS - 1) / FUSED_ROWS));
   if (a.trace) actor_rollout_kernel<true><<<clusters * FUSED_CLUSTER, FT, sizeof(FusedSmem), st>>>(a);
   else actor_rollout_kernel<false><<<clusters * FUSED_CLUSTER, FT, sizeof(FusedSmem), st>>>(a);
   CUDA_TRY(cudaGetLastError());

@@ -541,7 +541,10 @@ struct Ddpg {
   float *ep_a, *ep_scaled, *ep_sprev, *ep_r; double* ep_r64; long long ep_cap;
   // cluster-fused small-batch update (csrc/ddpg_fused.cu): per-cluster partial gradients [batch/8][n_params] of actor / critic
   bool fused; float* parts[2];
-  bool rollout_ok;   // ddpg_rollout may run as the persistent cluster kernel (one learner, widths within the shared-memory plan)
+  bool rollout_ok;   // widths within the shared-memory plan of the persistent cluster kernel (ddpg_rollout: one learner; ddpg_evaluate: any)
+  // best actor of every learner (run_episodes' best_run, DDPG.jl:282-289): its own allocation outside the slabs, learner l's copy
+  // best_stride floats behind learner 0's; best_score [P] Float64 (start -100000, the reference's), best_run [P]
+  float* best; long long best_stride; double* best_score; int32_t* best_run;
   int noise_kind; float ou_theta, ou_mu, ou_dt;   // ddpg_set_noise
   DdpgHparams* hp;   // [pop] host copy of every learner's ctrl->hp (ddpg_get_hparams; σ_eff of the one-learner cluster kernels)
   float* ou_x; long long ou_cap;                   // OUNoise.X of every instance of ddpg_episode's environment ([2][N])
@@ -655,13 +658,22 @@ extern "C" int32_t ddpg_create(const DdpgParams* p, int32_t device, Ddpg** out) 
     DMALLOC(h->parts[1], (long long)(B / FUSED_ROWS) * nc);
     h->fused = !(ev && ev[0] == '0');
   }
-  if (pop == 1 && ddpg_fused_shape_ok(FUSED_ROWS, p->l1, p->l2)) {
+  if (ddpg_fused_shape_ok(FUSED_ROWS, p->l1, p->l2)) {
     int s_ = actor_rollout_prepare();
     if (s_) { ddpg_destroy(h); return s_; }
     h->rollout_ok = true;
   }
   DMALLOC(h->ctrl, pop);
   DMALLOC(h->rings_dev, pop);
+  h->best_stride = (na + 63) & ~63ll;   // every copy starts on a 256-byte boundary (float4 copies)
+  DMALLOC(h->best, h->best_stride * pop);
+  DMALLOC(h->best_score, pop);
+  DMALLOC(h->best_run, pop);
+  {
+    std::vector<double> bs((size_t)pop, -100000.0);   // best_score = -100000 (DDPG_reinforce_charger_v1.jl), best_run = 0, zero weights
+    const cudaError_t e_ = cudaMemcpy(h->best_score, bs.data(), sizeof(double) * (size_t)pop, cudaMemcpyHostToDevice);
+    if (e_ != cudaSuccess) { shems_set_error("ddpg_create: best_score -> %s", cudaGetErrorString(e_)); ddpg_destroy(h); return SHEMS_ERR_CUDA; }
+  }
   h->hp = (DdpgHparams*)malloc(sizeof(DdpgHparams) * (size_t)pop);
   if (!h->hp) { shems_set_error("ddpg_create: out of host memory"); ddpg_destroy(h); return SHEMS_ERR_INVALID; }
   {
@@ -700,6 +712,7 @@ extern "C" int32_t ddpg_destroy(Ddpg* h) {
   if (h->graph_dp_exec) cudaGraphExecDestroy(h->graph_dp_exec);
   if (h->graph_dp) cudaGraphDestroy(h->graph_dp);
   for (int i = 0; i < h->dp_n_opened; ++i) cudaIpcCloseMemHandle(h->dp_opened[i]);
+  cudaFree(h->best); cudaFree(h->best_score); cudaFree(h->best_run);
   cudaFree(h->ctrl); cudaFree(h->idx_dev); cudaFree(h->ws); cudaFree((void*)h->rings_dev); cudaFree(h->dp_box); cudaFree(h->counters);
   cudaFree(h->ws_side); cudaFree(h->counters_side);
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
@@ -775,24 +788,30 @@ extern "C" int32_t ddpg_set_fused(Ddpg* h, int32_t on) {
   return h->fused ? 1 : 0;
 }
 
-extern "C" int64_t ddpg_num_params(const Ddpg* h, int32_t net) { return (h && net >= 0 && net < 4) ? dims_of(h, net).n_params : 0; }
+extern "C" int64_t ddpg_num_params(const Ddpg* h, int32_t net) {
+  return (h && net >= 0 && net <= DDPG_NET_ACTOR_BEST) ? dims_of(h, net).n_params : 0;   // ACTOR_BEST has the actor's shape
+}
+// the selected learner's copy of a net; DDPG_NET_ACTOR_BEST: its best-actor slot (outside the slab)
+static inline float* net_of(const Ddpg* h, int net) {
+  return net == DDPG_NET_ACTOR_BEST ? h->best + (long long)h->sel * h->best_stride : h->net[net] + sel_off(h);
+}
 
 extern "C" int32_t ddpg_set_layer(Ddpg* h, int32_t net, int32_t layer, const float* w_host, const float* b_host) {
-  REQUIRE(h && net >= 0 && net < 4 && layer >= 0 && layer < 3, SHEMS_ERR_INVALID, "ddpg_set_layer: net=%d layer=%d", net, layer);
+  REQUIRE(h && net >= 0 && net <= DDPG_NET_ACTOR_BEST && layer >= 0 && layer < 3, SHEMS_ERR_INVALID, "ddpg_set_layer: net=%d layer=%d", net, layer);
   GUARD(h->device);
   const LayerDims& L = dims_of(h, net).l[layer];
   CUDA_TRY(cudaStreamSynchronize(h->stream));
-  if (w_host) CUDA_TRY(cudaMemcpy(h->net[net] + sel_off(h) + L.w_off, w_host, sizeof(float) * (size_t)L.in * L.out, cudaMemcpyHostToDevice));
-  if (b_host) CUDA_TRY(cudaMemcpy(h->net[net] + sel_off(h) + L.b_off, b_host, sizeof(float) * (size_t)L.out, cudaMemcpyHostToDevice));
+  if (w_host) CUDA_TRY(cudaMemcpy(net_of(h, net) + L.w_off, w_host, sizeof(float) * (size_t)L.in * L.out, cudaMemcpyHostToDevice));
+  if (b_host) CUDA_TRY(cudaMemcpy(net_of(h, net) + L.b_off, b_host, sizeof(float) * (size_t)L.out, cudaMemcpyHostToDevice));
   return SHEMS_OK;
 }
 extern "C" int32_t ddpg_get_layer(Ddpg* h, int32_t net, int32_t layer, float* w_host, float* b_host) {
-  REQUIRE(h && net >= 0 && net < 4 && layer >= 0 && layer < 3, SHEMS_ERR_INVALID, "ddpg_get_layer: net=%d layer=%d", net, layer);
+  REQUIRE(h && net >= 0 && net <= DDPG_NET_ACTOR_BEST && layer >= 0 && layer < 3, SHEMS_ERR_INVALID, "ddpg_get_layer: net=%d layer=%d", net, layer);
   GUARD(h->device);
   const LayerDims& L = dims_of(h, net).l[layer];
   CUDA_TRY(cudaStreamSynchronize(h->stream));
-  if (w_host) CUDA_TRY(cudaMemcpy(w_host, h->net[net] + sel_off(h) + L.w_off, sizeof(float) * (size_t)L.in * L.out, cudaMemcpyDeviceToHost));
-  if (b_host) CUDA_TRY(cudaMemcpy(b_host, h->net[net] + sel_off(h) + L.b_off, sizeof(float) * (size_t)L.out, cudaMemcpyDeviceToHost));
+  if (w_host) CUDA_TRY(cudaMemcpy(w_host, net_of(h, net) + L.w_off, sizeof(float) * (size_t)L.in * L.out, cudaMemcpyDeviceToHost));
+  if (b_host) CUDA_TRY(cudaMemcpy(b_host, net_of(h, net) + L.b_off, sizeof(float) * (size_t)L.out, cudaMemcpyDeviceToHost));
   return SHEMS_OK;
 }
 extern "C" int32_t ddpg_get_grad(Ddpg* h, int32_t net, int32_t layer, float* w_host, float* b_host) {
@@ -2328,6 +2347,33 @@ extern "C" int32_t ddpg_episode(Ddpg* h, ShemsEnv* env, ShemsReplay* const* rps,
   return SHEMS_OK;
 }
 
+// The persistent cluster kernel (csrc/actor_rollout.cu) over every instance group of `env`, one launch per group: ddpg_rollout's
+// one-learner branch and ddpg_evaluate share it.  actor: learner 0's copy of the net to run, actor_stride floats between learners'
+// copies.  One learner: the whole group is one segment; populations: learner l owns instances l*n .. l*n+n-1, which the caller has
+// checked lie inside one group.
+static int rollout_launch(Ddpg* h, ShemsEnv* env, const float* actor, long long actor_stride, int32_t n_steps, float sigma, uint64_t seed,
+                          int64_t env_id_base, double* ep_return_dev, double* trace_dev, float* act_traj_dev) {
+  const NetDims& dA = h->dims[0]; const NetDims& dC = h->dims[1];
+  const long long N = env->n, n = N / h->pop;
+  ActorRolloutArgs a; memset(&a, 0, sizeof(a));
+  a.actor = actor;
+  a.ao = FusedNetOff{(int)dA.l[0].w_off, (int)dA.l[0].b_off, (int)dA.l[1].w_off, (int)dA.l[1].b_off, (int)dA.l[2].w_off, (int)dA.l[2].b_off};
+  a.l1 = h->p.l1; a.l2 = h->p.l2;
+  a.vec16 = (h->p.l2 % 4 == 0 && dA.l[1].w_off % 4 == 0 && dC.l[1].w_off % 4 == 0) ? 1 : 0;
+  a.norm = h->norm; a.actor_stride = actor_stride; a.norm_stride = h->pop_stride;
+  a.N = N; a.obs = env->obs; a.idx = env->idx; a.T = n_steps; a.step0 = env->step;
+  a.sigma = sigma * h->hp[0].noise_scale; a.seed = seed; a.env_id_base = env_id_base;
+  a.lo0 = h->p.act_lo[0]; a.lo1 = h->p.act_lo[1]; a.hi0 = h->p.act_hi[0]; a.hi1 = h->p.act_hi[1];
+  a.ep_return = ep_return_dev; a.trace = trace_dev; a.act_traj = act_traj_dev;
+  for (int g = 0; g < env->n_groups; ++g) {
+    a.P = env->gdp[g]; a.series = env->gseries[g]; a.n0 = env->gstart[g]; a.n1 = env->gstart[g + 1];
+    a.seg = h->pop == 1 ? a.n1 - a.n0 : n;
+    a.l0 = h->pop == 1 ? 0 : a.n0 / n;
+    TRY(actor_rollout_launch(h->stream, a));
+  }
+  return SHEMS_OK;
+}
+
 // episode!(env; NUM_STEPS, train = false, track, rng_ep) (DDPG.jl:186-242) / inference(env; track = 1) (memory_plotting_saving.jl:62-89)
 // for every instance of `env`: act(normalize(s)) [+ GNoise when sigma > 0] -> scale_action -> step!, n_steps times, by ONE call.
 // One learner at the fused shapes: a single persistent cluster kernel per group of instances (csrc/actor_rollout.cu) — no launch,
@@ -2348,20 +2394,7 @@ extern "C" int32_t ddpg_rollout(Ddpg* h, ShemsEnv* env, int32_t n_steps, float s
   GUARD(h->device);
   const long long N = env->n, n = N / h->pop;
   if (h->pop == 1 && h->rollout_ok) {
-    const NetDims& dA = h->dims[0]; const NetDims& dC = h->dims[1];
-    ActorRolloutArgs a; memset(&a, 0, sizeof(a));
-    a.actor = h->net[DDPG_NET_ACTOR];
-    a.ao = FusedNetOff{(int)dA.l[0].w_off, (int)dA.l[0].b_off, (int)dA.l[1].w_off, (int)dA.l[1].b_off, (int)dA.l[2].w_off, (int)dA.l[2].b_off};
-    a.l1 = h->p.l1; a.l2 = h->p.l2;
-    a.vec16 = (h->p.l2 % 4 == 0 && dA.l[1].w_off % 4 == 0 && dC.l[1].w_off % 4 == 0) ? 1 : 0;
-    a.norm = h->norm; a.N = N; a.obs = env->obs; a.idx = env->idx; a.T = n_steps; a.step0 = env->step;
-    a.sigma = sigma * h->hp[0].noise_scale; a.seed = seed; a.env_id_base = env_id_base;
-    a.lo0 = h->p.act_lo[0]; a.lo1 = h->p.act_lo[1]; a.hi0 = h->p.act_hi[0]; a.hi1 = h->p.act_hi[1];
-    a.ep_return = ep_return_dev; a.trace = trace_dev; a.act_traj = act_traj_dev;
-    for (int g = 0; g < env->n_groups; ++g) {
-      a.P = env->gdp[g]; a.series = env->gseries[g]; a.n0 = env->gstart[g]; a.n1 = env->gstart[g + 1];
-      TRY(actor_rollout_launch(h->stream, a));
-    }
+    TRY(rollout_launch(h, env, h->net[DDPG_NET_ACTOR], 0, n_steps, sigma, seed, env_id_base, ep_return_dev, trace_dev, act_traj_dev));
     env->max_idx += n_steps; env->step += n_steps; env->consistent = true;
     return SHEMS_OK;
   }
@@ -2384,6 +2417,90 @@ extern "C" int32_t ddpg_rollout(Ddpg* h, ShemsEnv* env, int32_t n_steps, float s
       CUDA_TRY(cudaGetLastError());
     }
   }
+  return SHEMS_OK;
+}
+
+// episode!(env; train = false) (DDPG.jl:266-271) / inference(env; track = 1) for EVERY learner of the handle, noise-free, by one call: the
+// persistent cluster kernel with a learner dimension (every cluster serves 8 instances of one learner and reads that learner's actor and
+// s_min / s_max), so a learner's evaluation inside a population has the bits of its evaluation on a one-learner handle.
+// net: DDPG_NET_ACTOR or DDPG_NET_ACTOR_BEST (the slot ddpg_keep_best fills).
+extern "C" int32_t ddpg_evaluate(Ddpg* h, ShemsEnv* env, int32_t net, int32_t n_steps, int64_t env_id_base, double* ep_return_dev, double* trace_dev,
+                                 float* act_traj_dev) {
+  REQUIRE(h && env, SHEMS_ERR_INVALID, "ddpg_evaluate: NULL argument");
+  REQUIRE(net == DDPG_NET_ACTOR || net == DDPG_NET_ACTOR_BEST, SHEMS_ERR_INVALID, "ddpg_evaluate: net=%d (ACTOR or ACTOR_BEST)", net);
+  REQUIRE(n_steps >= 1, SHEMS_ERR_INVALID, "ddpg_evaluate: n_steps=%d", n_steps);
+  REQUIRE(env->device == h->device, SHEMS_ERR_INVALID, "ddpg_evaluate: env on device %d, learner on %d", env->device, h->device);
+  REQUIRE(env->n % h->pop == 0, SHEMS_ERR_INVALID, "ddpg_evaluate: %lld instances do not split over %d learners", (long long)env->n, h->pop);
+  REQUIRE(h->rollout_ok, SHEMS_ERR_INVALID, "ddpg_evaluate: widths l1=%d l2=%d outside the cluster kernel's plan (l1 <= %d, l2 <= %d)", h->p.l1,
+          h->p.l2, FUSED_MAX_L1, FUSED_MAX_L2);
+  const long long N = env->n, n = N / h->pop;
+  for (int g = 1; g < env->n_groups && h->pop > 1; ++g)   // one learner: every group is a segment of its own (as ddpg_rollout)
+    REQUIRE(env->gstart[g] % n == 0, SHEMS_ERR_INVALID, "ddpg_evaluate: the group starting at instance %lld splits the %lld instances of learner %lld",
+            (long long)env->gstart[g], n, (long long)(env->gstart[g] / n));
+  REQUIRE(env->stream == h->stream, SHEMS_ERR_STATE, "ddpg_evaluate: bind the environment and the learner to one CUDA stream");
+  REQUIRE(env->was_reset, SHEMS_ERR_STATE, "ddpg_evaluate: reset! must come first");
+  if (ensure_rows(env, n_steps)) {
+    shems_set_error("BoundsError: evaluation of %d steps from row %d leaves the %d-row series (next_state!, shems_LU1.jl:266-268)", n_steps, env->max_idx,
+                    env->nrows);
+    return SHEMS_ERR_BOUNDS;
+  }
+  GUARD(h->device);
+  const float* actor = net == DDPG_NET_ACTOR ? h->net[DDPG_NET_ACTOR] : h->best;
+  const long long stride = net == DDPG_NET_ACTOR ? h->pop_stride : h->best_stride;
+  TRY(rollout_launch(h, env, actor, stride, n_steps, 0.0f, 0, env_id_base, ep_return_dev, trace_dev, act_traj_dev));
+  env->max_idx += n_steps; env->step += n_steps; env->consistent = true;
+  return SHEMS_OK;
+}
+
+// run_episodes' bookkeeping after an evaluation round (DDPG.jl:273, :282-289) for every learner: one block per learner, so the
+// decision and the copy it gates are made by the same block.  Thread 0 forms score = (Σ_k ep_return[l·n + k]) / n in index order in
+// Float64 and, when score > best_score (strict: ties and NaN never win), records it with the episode; then the block copies the
+// learner's actor into its best-actor slot.
+__global__ void __launch_bounds__(256)
+ddpg_keep_best_kernel(const double* __restrict__ ep_return, long long n, int episode, double* __restrict__ score_out, double* __restrict__ best_score,
+                      int32_t* __restrict__ best_run, const float* __restrict__ actor, long long pop_stride, float* __restrict__ best,
+                      long long best_stride, long long na) {
+  __shared__ int take;
+  const long long l = blockIdx.x;
+  if (threadIdx.x == 0) {
+    double sum = 0.0;
+    for (long long k = 0; k < n; ++k) sum += ep_return[l * n + k];
+    const double score = sum / (double)n;
+    if (score_out) score_out[l] = score;
+    take = score > best_score[l];
+    if (take) { best_score[l] = score; best_run[l] = episode; }
+  }
+  __syncthreads();
+  if (!take) return;
+  const float* src = actor + l * pop_stride;   // both copies start on 256-byte boundaries
+  float* dst = best + l * best_stride;
+  const long long n4 = na / 4;
+  for (long long i = threadIdx.x; i < n4; i += blockDim.x) reinterpret_cast<float4*>(dst)[i] = reinterpret_cast<const float4*>(src)[i];
+  for (long long i = 4 * n4 + threadIdx.x; i < na; i += blockDim.x) dst[i] = src[i];
+}
+extern "C" int32_t ddpg_keep_best(Ddpg* h, const double* ep_return_dev, int64_t n, int32_t episode, double* score_dev) {
+  REQUIRE(h && ep_return_dev, SHEMS_ERR_INVALID, "ddpg_keep_best: NULL argument");
+  REQUIRE(n >= 1, SHEMS_ERR_INVALID, "ddpg_keep_best: n=%lld", (long long)n);
+  GUARD(h->device);
+  ddpg_keep_best_kernel<<<h->pop, 256, 0, h->stream>>>(ep_return_dev, n, episode, score_dev, h->best_score, h->best_run, h->net[DDPG_NET_ACTOR],
+                                                       h->pop_stride, h->best, h->best_stride, h->dims[0].n_params);
+  CUDA_TRY(cudaGetLastError());
+  return SHEMS_OK;
+}
+extern "C" int32_t ddpg_get_best(Ddpg* h, double* best_score_host, int32_t* best_run_host) {
+  REQUIRE(h && best_score_host && best_run_host, SHEMS_ERR_INVALID, "ddpg_get_best: NULL argument");
+  GUARD(h->device);
+  CUDA_TRY(cudaStreamSynchronize(h->stream));
+  CUDA_TRY(cudaMemcpy(best_score_host, h->best_score, sizeof(double) * (size_t)h->pop, cudaMemcpyDeviceToHost));
+  CUDA_TRY(cudaMemcpy(best_run_host, h->best_run, sizeof(int32_t) * (size_t)h->pop, cudaMemcpyDeviceToHost));
+  return SHEMS_OK;
+}
+extern "C" int32_t ddpg_set_best(Ddpg* h, const double* best_score_host, const int32_t* best_run_host) {
+  REQUIRE(h && best_score_host && best_run_host, SHEMS_ERR_INVALID, "ddpg_set_best: NULL argument");
+  GUARD(h->device);
+  CUDA_TRY(cudaStreamSynchronize(h->stream));
+  CUDA_TRY(cudaMemcpy(h->best_score, best_score_host, sizeof(double) * (size_t)h->pop, cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(h->best_run, best_run_host, sizeof(int32_t) * (size_t)h->pop, cudaMemcpyHostToDevice));
   return SHEMS_OK;
 }
 

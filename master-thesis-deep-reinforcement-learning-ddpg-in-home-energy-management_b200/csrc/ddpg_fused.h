@@ -80,10 +80,13 @@ int ddpg_fused_critic(cudaStream_t st, const FusedArgs& a);  // targets, TD targ
 int ddpg_fused_actor(cudaStream_t st, const FusedArgs& a);   // actor-loss forward/backward through the critic -> part (actor)
 
 // episode!(env; train = false) / inference(track = 1) for the instances n0 .. n1-1 of an environment handle as one persistent cluster
-// kernel (csrc/actor_rollout.cu): act(normalize(s)) -> scale_action -> step! for T steps, 8 instances per cluster
+// kernel (csrc/actor_rollout.cu): act(normalize(s)) -> scale_action -> step! for T steps, 8 instances per cluster.  Populations: the
+// range is (n1 - n0) / seg learners of seg instances each, learner l0 + s taking instances n0 + s*seg ..; a cluster serves one learner
+// and reads its actor at actor + l*actor_stride and its s_min / s_max at norm + l*norm_stride.  One learner: seg = n1 - n0, l0 = 0.
 struct ActorRolloutArgs {
   const float* actor; FusedNetOff ao; int l1, l2, vec16;
   const float* norm;
+  long long seg, l0, actor_stride, norm_stride;
   DevParams P; const float4* series;
   long long N, n0, n1;       // SoA stride of the handle's arrays; instance range of this launch (one group of constants)
   float* obs; int32_t* idx;  // env.state [9][N], env.idx [N]: read at the start, written back at the end

@@ -267,6 +267,40 @@ class Learner:
                                       _ptr(out["ep_return"]), _ptr(out.get("trace")), _ptr(out.get("actions"))))
         return out
 
+    def evaluate(self, env, n_steps, best=False, want_trace=False, want_actions=False):
+        """ddpg_evaluate: episode!(env; train = false) / inference(env; track = 1) for EVERY learner, noise-free, by one call — the
+        persistent cluster kernel with a learner dimension.  env holds N = P*n instances (learner l owns l*n .. l*n+n-1; for P > 1
+        no group may split a learner); best=True runs the best-actor slots.  reset! stays with the caller.  Returns the dict of rollout()."""
+        N, T = env.n_envs, int(n_steps)
+        out = {"ep_return": torch.empty(N, dtype=torch.float64, device=self._dev)}
+        if want_trace:
+            out["trace"] = torch.empty((T, 23, N), dtype=torch.float64, device=self._dev)
+        if want_actions:
+            out["actions"] = torch.empty((T, 2, N), dtype=torch.float32, device=self._dev)
+        L.check(self.lib.ddpg_evaluate(self._h, env._h, L.NET_ACTOR_BEST if best else L.NET_ACTOR, T, int(env.env_id_base),
+                                       _ptr(out["ep_return"]), _ptr(out.get("trace")), _ptr(out.get("actions"))))
+        return out
+
+    def keep_best(self, ep_return, n, episode):
+        """ddpg_keep_best: score_l = mean of ep_return[l*n .. l*n+n-1] (index order, Float64); where score_l > best_score_l (strict)
+        the learner's actor goes into its best-actor slot and best_run_l = episode.  Enqueued only; returns the scores [P] (device)."""
+        assert ep_return.dtype == torch.float64 and ep_return.numel() == int(n) * self.population
+        score = torch.empty(self.population, dtype=torch.float64, device=self._dev)
+        L.check(self.lib.ddpg_keep_best(self._h, _ptr(ep_return), int(n), int(episode), _ptr(score)))
+        return score
+
+    def best(self):
+        """ddpg_get_best: (best_score [P] float64, best_run [P] int32) of every learner."""
+        sc, run = np.empty(self.population, np.float64), np.empty(self.population, np.int32)
+        L.check(self.lib.ddpg_get_best(self._h, sc.ctypes.data_as(L.PD), run.ctypes.data_as(L.PI)))
+        return sc, run
+
+    def set_best(self, best_score, best_run):
+        """ddpg_set_best: every learner's best_score / best_run (the best-actor weights go through set_layer(NET_ACTOR_BEST, ...))."""
+        sc = np.ascontiguousarray(np.broadcast_to(np.asarray(best_score, np.float64), (self.population,)))
+        run = np.ascontiguousarray(np.broadcast_to(np.asarray(best_run, np.int32), (self.population,)))
+        L.check(self.lib.ddpg_set_best(self._h, sc.ctypes.data_as(L.PD), run.ctypes.data_as(L.PI)))
+
     # ---- full snapshot (nets, targets, ADAM moments, β powers, update counter, s_min/s_max): resume where the run stopped
     def get_state(self):
         n = int(self.lib.ddpg_state_floats(self._h))
@@ -481,6 +515,9 @@ class Driver:
         saveBSON(actor, ...; idx = i, path = "temp") (:282-289) — and sets best_run = i.  The evaluation episodes run as instances
         of ONE env_eval handle (the reference runs them one after the other): test_runs is rounded up to whole batches of
         env_eval.n_envs.  `state` / `start_ep` continue a loop that was interrupted (the returned dict is that state).
+        The evaluation rule is the reference's i % test_every == 1 as written, so test_every = 1 never evaluates here;
+        PopulationDriver.run_episodes evaluates at i = 1, 1 + test_every, ..., which is the same rule for test_every > 1 and
+        every episode for test_every = 1.
         Seeds: rng_ep = rng_run * 100003 + i, rng_test = seed_ini * 1000 + test_ep (Julia's string concatenation feeds
         MersenneTwister; here the integers key Philox streams)."""
         n = self.env_train.n_envs
@@ -534,10 +571,16 @@ class PopulationDriver:
     chargers[l] is learner l's charger id (shems_LU1.jl:47-59), equal ids must be adjacent; seeds[l] its rng_run (input.jl:136).
     hparams: per-learner hyper-parameters, a dict of lists of length P with keys from Learner.HPARAMS (lr_actor, lr_critic, gamma,
     tau, noise_scale); missing keys keep the DdpgParams values (noise_scale: 1).  Learner l explores with σ_eff = sigma × noise_scale[l],
-    so a σ grid is sigma=1.0 with the grid values as noise_scale."""
+    so a σ grid is sigma=1.0 with the grid values as noise_scale.
+
+    eval_series ([8][nrows], or [G][8][nrows] with one series per run of equal chargers) adds the reference's evaluation protocol
+    (run_episodes / inference): an evaluation handle of test_runs instances per learner, one group per charger run, with
+    maxsteps = nrows - 1 so that every reset! starts on row 1 (rand(1:nrows-maxsteps)).  Every learner is scored on the SAME test_runs
+    starts: learner l's k-th evaluation instance starts from the draw of instance k of a one-learner evaluation handle (test_runs
+    instances of its charger, env_id_base 0), as every run of the reference evaluates with the same rng."""
 
     def __init__(self, series, chargers, seeds, n_envs=64, mem_size=24_000, ep_length=72, sigma=0.1, device=0, use_tensor_cores=1, native=True,
-                 hparams=None, **ddpg_kw):
+                 hparams=None, eval_series=None, test_runs=100, **ddpg_kw):
         from .env import Shems
         assert len(chargers) == len(seeds)
         self.native = bool(native)
@@ -565,6 +608,40 @@ class PopulationDriver:
         self._dev = torch.device("cuda", int(device))
         self._s_prev = torch.empty((9, self.N), dtype=torch.float32, device=self._dev)
         self.n_env_steps = 0
+        self._runs = [(c, k // self.n_envs) for c, k in groups]    # (charger, learners) per run of equal chargers
+        self.test_runs = int(test_runs)
+        self.env_eval = None
+        if eval_series is not None:
+            ev = np.ascontiguousarray(eval_series, np.float32)
+            self.env_eval = Shems(ev.shape[-1] - 1, ev, device=device, groups=[(c, m * self.test_runs) for c, m in self._runs])
+            # per charger run: the one-learner evaluation handle whose reset! draws every learner of the run starts from
+            self._eval_starts, g0 = [], 0
+            for g, (c, m) in enumerate(self._runs):
+                ser_g = ev[g] if ev.ndim == 3 else ev
+                self._eval_starts.append((g0, m, Shems(ser_g.shape[-1] - 1, ser_g, n_envs=self.test_runs, charger_id=c, device=device)))
+                g0 += m * self.test_runs
+
+    def reset_eval(self, rng):
+        """reset!(env_eval; rng) with the same test_runs starts for every learner: each charger run's one-learner handle is reset
+        with `rng` and its states and rows are tiled over the run's learners (the population handle's own reset! sets its step and
+        bounds; its draws, keyed by the global instance index, are replaced)."""
+        from .env import _wrap_device
+        env, R = self.env_eval, self.test_runs
+        env.reset(rng=rng)
+        obs = env.state_tensor()
+        idx = _wrap_device(env._idx_ptr, (env.n_envs,), torch.int32, self._dev, env)
+        for g0, m, one in self._eval_starts:
+            one.reset(rng=rng)
+            one_idx = _wrap_device(one._idx_ptr, (R,), torch.int32, self._dev, one)
+            obs[:, g0:g0 + m * R].view(9, m, R).copy_(one.state_tensor().unsqueeze(1))
+            idx[g0:g0 + m * R].view(m, R).copy_(one_idx.unsqueeze(0))
+        return env
+
+    def _inference_env(self, series):
+        """one instance per learner on `series` (a charger run's learners share its group), reset! with rng = -1 by the caller"""
+        from .env import Shems
+        ser = np.ascontiguousarray(series, np.float32)
+        return Shems(ser.shape[-1] - 1, ser, device=self._dev.index, groups=list(self._runs))
 
     def populate_memory(self):                       # memory_plotting_saving.jl:9-29 for every learner: a = 2U-1 per step, rng += 1 per episode
         rng = self.seeds[0]
@@ -614,3 +691,51 @@ class PopulationDriver:
         self.env.reset(rng=rng)
         ret = self.env.rollout(L.POLICY_RULE, self.ep_length)["ep_return"]
         return ret.view(self.P, self.n_envs).mean(dim=1).cpu().numpy()
+
+    # run_episodes (DDPG.jl:244-298, driver DDPG_reinforce_charger_v1.jl:87-105) for every learner at once
+    def run_episodes(self, num_ep, test_every=100, seed_ini=123, on_best=None, start_ep=1, state=None):
+        """Driver.run_episodes for the population.  Training episode i (rng_ep = seeds[0] * 100003 + i) fills total_reward[i-1] [P];
+        every `test_every` episodes (i = 1, 1 + test_every, ...: the reference's i % test_every == 1, and every episode for
+        test_every = 1) one evaluation round runs on the evaluation handle: ONE reset! (rng = seed_ini * 1000 + 1), one ddpg_evaluate of
+        all P x test_runs instances (noise-free, ep_length steps from row 1) and one ddpg_keep_best, which forms score_mean and keeps
+        each learner's best actor on the device.  The host reads the P scores only to fill score_mean[ceil(i / test_every) - 1] and to
+        call on_best(l, i, score) for every learner that improved (the reference's "temp" saveBSON, :282-289).
+        Every learner plays the same test_runs starts (reset_eval), so score_mean[.][l] is what learner l's actor and norm score on
+        a one-learner handle with an evaluation env of test_runs instances after reset!(rng = seed_ini * 1000 + 1).
+        Returns {total_reward [num_ep][P], score_mean [ceil(num_ep / test_every)][P], best_run [P], best_score [P]}.  A fresh start
+        (state=None) sets best_score = -100000, best_run = 0 and zero best actors; `state` / `start_ep` continue an interrupted loop
+        (its best scores are written back to the handle; restore the best actors with tracker.load_checkpoint)."""
+        assert self.env_eval is not None, "run_episodes needs eval_series"
+        P, te = self.P, int(test_every)
+        st = state if state is not None else dict(total_reward=np.zeros((num_ep, P)), score_mean=np.zeros((-(-num_ep // te), P)),
+                                                  best_run=np.zeros(P, np.int32), best_score=np.full(P, -100000.0))
+        self.learner.set_best(st["best_score"], st["best_run"])
+        if state is None:   # no best actor left over from an earlier call on this handle
+            for l in range(P):
+                self.learner.select(l)
+                for k in range(3):
+                    i_, o_ = self.learner.layer_shape(L.NET_ACTOR, k)
+                    self.learner.set_layer(L.NET_ACTOR_BEST, k, np.zeros(i_ * o_, np.float32), np.zeros(o_, np.float32))
+            self.learner.select(0)
+        for i in range(start_ep, num_ep + 1):
+            r = self.episode(train=True, rng_ep=self.seeds[0] * 100003 + i)
+            st["total_reward"][i - 1] = r.cpu().numpy()
+            if (i - 1) % te == 0:
+                ret = self.learner.evaluate(self.reset_eval(seed_ini * 1000 + 1), self.ep_length)["ep_return"]
+                score = self.learner.keep_best(ret, self.test_runs, i).cpu().numpy()
+                st["score_mean"][-(-i // te) - 1] = score
+                for l in np.flatnonzero(score > st["best_score"]):     # the same strict rule ddpg_keep_best applied on the device
+                    if on_best is not None:
+                        on_best(int(l), i, float(score[l]))
+                    st["best_score"][l], st["best_run"][l] = score[l], i
+        return st
+
+    # inference(env; track = 1) — memory_plotting_saving.jl:62-89, driver :95-105: one deterministic instance per learner
+    def inference(self, series, num_steps=None, best=True):
+        """every learner's (best) actor over `series` ([8][nrows] or one per charger run) from reset!(rng = -1), num_steps steps
+        (default nrows - 1) by one ddpg_evaluate.  Returns (returns [P] float64, trace [T][23][P] float64), device tensors."""
+        env = self._inference_env(series)
+        T = env.nrows - 1 if num_steps is None else int(num_steps)
+        env.reset(rng=-1)
+        out = self.learner.evaluate(env, T, best=best, want_trace=True)
+        return out["ep_return"], out["trace"]

@@ -4,8 +4,8 @@
   (RL-SHEMS/src/memory_plotting_saving.jl:167-190; column order = the `results` row, shems_LU1.jl:476-478).
 * `save_checkpoint` / `load_checkpoint` — the reference saves the actor only (BSON, :263-270) and can therefore not resume
   training; here the whole state goes into one .npz: the 4 nets in Flux layout, both optimisers (ADAM moments, β powers, update
-  counter), normalisation constants, per-learner hyper-parameters, OU noise state, the replay memories — for every learner of a
-  population handle.  The
+  counter), normalisation constants, per-learner hyper-parameters, OU noise state, the best actors with their best_score /
+  best_run (run_episodes' "temp" saveBSON, DDPG.jl:282-289), the replay memories — for every learner of a population handle.  The
   Julia shim turns the actor arrays back into a Flux Chain (same memory layout as Dense.W / Dense.b) for saveBSON.
 """
 import numpy as np
@@ -28,6 +28,30 @@ def write_results_csv(path, trace, instance=0):
                 penalty=float(rows[:, 8].sum()))  # the sums write_to_tracker_file appends (:208-210)
 
 
+SUMMARY_HEADER = ["learner", "charger", "seed", "lr_actor", "lr_critic", "gamma", "tau", "noise_scale", "best_run", "best_score", "rewards",
+                  "profit", "discomfort", "penalty"]
+
+
+def write_population_results(out_dir, trace, chargers, seeds, best_run, best_score, hparams=None, prefix="results"):
+    """A population's inference (PopulationDriver.inference, trace [T][23][P]): one results CSV per learner,
+    `{prefix}_l{l}.csv` through write_results_csv, and `{prefix}_summary.csv` with a row per learner — index, charger, seed,
+    hyper-parameters (hparams: one dict per learner with Learner.HPARAMS keys, or None), best_run, best_score and the four sums
+    write_results_csv returns.  Returns the list of those sums."""
+    import os
+    os.makedirs(out_dir, exist_ok=True)
+    sums = []
+    with open(os.path.join(out_dir, f"{prefix}_summary.csv"), "w") as f:
+        f.write(",".join(SUMMARY_HEADER) + "\n")
+        for l in range(len(chargers)):
+            sm = write_results_csv(os.path.join(out_dir, f"{prefix}_l{l}.csv"), trace, instance=l)
+            sums.append(sm)
+            hp = hparams[l] if hparams is not None else {}
+            row = [l, int(chargers[l]), int(seeds[l])] + [repr(float(hp[k])) if k in hp else "" for k in SUMMARY_HEADER[3:8]]
+            row += [int(best_run[l]), repr(float(best_score[l]))] + [repr(sm[k]) for k in SUMMARY_HEADER[10:]]
+            f.write(",".join(str(x) for x in row) + "\n")
+    return sums
+
+
 NETS = ((L.NET_ACTOR, "actor"), (L.NET_CRITIC, "critic"), (L.NET_ACTOR_TARGET, "actor_target"), (L.NET_CRITIC_TARGET, "critic_target"))
 
 
@@ -36,7 +60,9 @@ def save_checkpoint(path, learner, s_min=None, s_max=None, memories=None, **scor
     actor and the score arrays only, memory_plotting_saving.jl:263-270): for every learner l of the handle the four nets
     (Flux layout, `l{l}_actor_W1` ... — learner 0 also without the prefix, which is what the Julia shim turns into a Flux
     Chain), ADAM moments, β powers, update counter and normalisation constants (`l{l}_state`, `l{l}_opt`: ddpg_get_state),
-    the hyper-parameters (`l{l}_hparams` = [lr_actor, lr_critic, gamma, tau, noise_scale] float32: ddpg_get_hparams), OUNoise.X when OU episodes ran, and — with `memories` (one Replay per learner) — the replay memories in logical order."""
+    the hyper-parameters (`l{l}_hparams` = [lr_actor, lr_critic, gamma, tau, noise_scale] float32: ddpg_get_hparams), the best
+    actors (`l{l}_actor_best_W1` ...) with `best_score` [P] / `best_run` [P] (ddpg_get_best; a score keyword of the same name
+    replaces them), OUNoise.X when OU episodes ran, and — with `memories` (one Replay per learner) — the replay memories in logical order."""
     out = {}
     P = learner.population
     keep = getattr(learner, "_sel", 0)
@@ -55,8 +81,13 @@ def save_checkpoint(path, learner, s_min=None, s_max=None, memories=None, **scor
                 out[f"l{l}_{name}_b{k + 1}"] = b
                 if l == 0:
                     out[f"{name}_W{k + 1}"], out[f"{name}_b{k + 1}"] = out[f"l0_{name}_W{k + 1}"], b
+        for k in range(3):
+            i, o = learner.layer_shape(L.NET_ACTOR, k)
+            w, b = learner.get_layer(L.NET_ACTOR_BEST, k)
+            out[f"l{l}_actor_best_W{k + 1}"], out[f"l{l}_actor_best_b{k + 1}"] = w.reshape(i, o).T.copy(), b
     if P > 1:
         learner.select(keep)
+    out["best_score"], out["best_run"] = learner.best()
     ou = learner.get_ou_state()
     if ou is not None:
         out["ou_x"] = ou
@@ -78,7 +109,7 @@ def load_checkpoint(path, learner, memories=None):
     """Restores what save_checkpoint wrote: every learner's full state (a resumed run continues bit-identically,
     tests/test_resume_gpu.py) and, into the given EMPTY Replay objects, the replay memories.  Files holding only net
     arrays (weights-only checkpoints) restore the nets of learner 0; files without `l{l}_hparams` leave the hyper-parameters as
-    they are."""
+    they are, files without the best actors leave those (and best_score / best_run) as they are."""
     import torch
     z = np.load(path)
     P = learner.population
@@ -91,8 +122,14 @@ def load_checkpoint(path, learner, memories=None):
             learner.set_state(z[f"l{l}_state"], z[f"l{l}_opt"])
             if f"l{l}_hparams" in z:
                 learner.set_hparams(**dict(zip(learner.HPARAMS, z[f"l{l}_hparams"].tolist())))
+            if f"l{l}_actor_best_W1" in z:
+                for k in range(3):
+                    learner.set_layer(L.NET_ACTOR_BEST, k, np.ascontiguousarray(z[f"l{l}_actor_best_W{k + 1}"].T).ravel(),
+                                      z[f"l{l}_actor_best_b{k + 1}"])
         if P > 1:
             learner.select(keep)
+        if "l0_actor_best_W1" in z and "best_score" in z and "best_run" in z:
+            learner.set_best(np.asarray(z["best_score"], np.float64).reshape(-1), np.asarray(z["best_run"]).astype(np.int32).reshape(-1))
         if "ou_x" in z:
             learner.set_ou_state(z["ou_x"])
     else:

@@ -5,7 +5,11 @@ Under torch.distributed.run (one process per GPU) every rank trains its block of
 --grid: the thesis's scalar hyper-parameter grid search (input.jl:58-100) inside the one population.  Names: lr_actor, lr_critic,
 gamma, tau, noise_scale, or sigma (the exploration σ itself: the episodes then pass σ = 1 and each learner's noise_scale is its σ).
 Learner g takes grid point g mod (number of points) of the cartesian product; the summary reports the eval return per grid point,
-averaged over the learners (seeds, chargers) that share it."""
+averaged over the learners (seeds, chargers) that share it.
+--test-every K --test-runs R --inference-dir DIR: the reference protocol (run_episodes, DDPG.jl:244-298; driver :87-105) on a synthetic
+evaluation series (1440 rows) and test series (3000 rows): every K episodes R noise-free evaluation episodes per learner from row 1,
+each learner's best actor kept on the device, then inference of every best actor over the test series, one results CSV per learner
+and a summary CSV in DIR.  The report adds best score, best run and test-set return per learner and per grid point."""
 import argparse
 import itertools
 import json
@@ -25,6 +29,9 @@ ap.add_argument("--episodes", type=int, default=20)
 ap.add_argument("--tc", type=int, default=1)
 ap.add_argument("--eval-every", type=int, default=0)
 ap.add_argument("--grid", nargs="*", default=[], metavar="NAME=V1,V2", help="per-learner hyper-parameter grid (cartesian product)")
+ap.add_argument("--test-every", type=int, default=0, help="evaluate every K episodes and keep each learner's best actor (run_episodes)")
+ap.add_argument("--test-runs", type=int, default=100, help="evaluation episodes per learner and round")
+ap.add_argument("--inference-dir", default=None, help="write the test-set inference CSVs of the best actors here (needs --test-every)")
 args = ap.parse_args()
 GRID_NAMES = ("lr_actor", "lr_critic", "gamma", "tau", "noise_scale", "sigma")
 grid = {}
@@ -52,6 +59,10 @@ grid_of = [g % len(points) for g in learner_ids]
 hparams = {("noise_scale" if k == "sigma" else k): [points[i][k] for i in grid_of] for k in grid}
 drv_kw = dict(sigma=1.0) if "sigma" in grid else {}
 ser = sb.series.synth_charger98(4320, seed=98)
+assert args.inference_dir is None or args.test_every > 0, "--inference-dir runs the best actors: give --test-every K to choose them"
+protocol = args.test_every > 0
+if protocol:
+    drv_kw.update(eval_series=sb.series.synth_charger98(1440, seed=1440), test_runs=args.test_runs)
 drv = sb.PopulationDriver(ser, chargers=chargers, seeds=seeds, n_envs=args.envs, device=local, use_tensor_cores=args.tc, hparams=hparams, **drv_kw)
 t0 = time.time()
 drv.populate_memory()
@@ -62,6 +73,33 @@ rule = drv.evaluate_rule_based()
 first = drv.episode(train=False, rng_ep=999).cpu().numpy()
 t1 = time.time()
 t_eval = 0.0
+if protocol:   # run_episodes: training episodes with an evaluation round every --test-every episodes
+    import numpy as np
+    st = drv.run_episodes(args.episodes, test_every=args.test_every)
+    torch.cuda.synchronize()
+    dt = time.time() - t1
+    rets, trace = drv.inference(sb.series.synth_charger98(3000, seed=3000))
+    test_ret = rets.cpu().numpy()
+    if args.inference_dir:
+        hp_rows = [{k: v[l] for k, v in hparams.items()} for l in range(P)]
+        sb.tracker.write_population_results(os.path.join(args.inference_dir, f"rank{rank}"), trace, chargers, seeds, st["best_run"],
+                                            st["best_score"], hparams=hp_rows)
+    best = dict(best_score=st["best_score"].tolist(), best_run=[int(x) for x in st["best_run"]], test_return=test_ret.tolist(), grid_of=grid_of)
+    if dist is not None:
+        every = [None] * world if rank == 0 else None
+        dist.gather_object(best, every, dst=0)
+        if rank == 0:
+            best = {k: [v for x in every for v in x[k]] for k in best}
+        dist.barrier()
+        dist.destroy_process_group()
+    if rank == 0:
+        gi, bs, tr = (np.asarray(best[k]) for k in ("grid_of", "best_score", "test_return"))
+        print(json.dumps(dict(learners=len(gi), episodes=args.episodes, test_every=args.test_every, test_runs=args.test_runs, train_seconds=dt,
+                              best_score=best["best_score"], best_run=best["best_run"], test_return=best["test_return"],
+                              grid=[dict(point=pt, learners=int((gi == i).sum()), best_score=float(bs[gi == i].mean()),
+                                         best_score_max=float(bs[gi == i].max()), test_return=float(tr[gi == i].mean()))
+                                    for i, pt in enumerate(points) if (gi == i).any()])), flush=True)
+    sys.exit(0)
 for ep in range(1, args.episodes + 1):
     r = drv.episode(train=True, rng_ep=ep)
     if args.eval_every and ep % args.eval_every == 0:
