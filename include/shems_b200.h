@@ -355,6 +355,34 @@ SHEMS_API int32_t ddpg_evaluate(Ddpg* h, ShemsEnv* env, int32_t net, int32_t n_s
 SHEMS_API int32_t ddpg_keep_best(Ddpg* h, const double* ep_return_dev, int64_t n, int32_t episode, double* score_dev);
 SHEMS_API int32_t ddpg_get_best(Ddpg* h, double* best_score_host, int32_t* best_run_host);
 SHEMS_API int32_t ddpg_set_best(Ddpg* h, const double* best_score_host, const int32_t* best_run_host);
+/* Population-based training (no reference counterpart: the reference runs one process per grid point and its author picks the best
+ * seeds afterwards).  ddpg_exploit: one enqueue, no host allocation, no synchronisation (it fits between ddpg_keep_best and the next
+ * ddpg_episode).  Learners split into contiguous groups [group_start[g], group_start[g+1]) (n_groups = 0: one group of all P);
+ * nothing crosses a group.  In a group of m learners: key_l = score_dev[l] with NaN as -inf, rank_l = position in descending key order
+ * with ties to the lower index, k = floor(frac * m) in double.  Every learner d with rank_d >= m - k (the bottom set) draws
+ * w[4] = Philox4x32-10(seed, id = d, ctr = round, stream = 0x5042) and takes as its source s the learner of rank
+ * (uint32)(((uint64)w[0] * k) >> 32) (the top set rank < k; the two sets are disjoint).  From s to d are copied exactly what
+ * ddpg_get_state / ddpg_set_state move: actor, critic, both targets, the four ADAM moment arrays, s_min / s_max, and the β powers
+ * (with their reciprocals) of both optimisers.  d keeps its own Philox seed and update counter, its replay memory, its best-actor
+ * slot, best_score / best_run, OU state, gradients and scratch; the handle-wide update counter is unchanged.  Then each
+ * hyper-parameter j with bit j of keys set (0 lr_actor, 1 lr_critic, 2 gamma, 3 tau, 4 noise_scale) becomes RN32(value_s * f), f =
+ * factor_hi if bit j of w[1] is set else factor_lo, gamma and tau then min(x, 1); the others are copied.  parent_dev [P] (or NULL)
+ * receives s for a replaced learner and -1 for the others.  k = 0 or m = 1 changes nothing in that group; P = 1 is valid.
+ * ddpg_get_hparams after the call synchronises and shows the device values.  SHEMS_ERR_INVALID, with nothing launched: NULL h,
+ * score_dev or p, frac NaN or outside [0, 0.5], a factor not finite or <= 0, keys outside 0..31, n_groups outside 0..16, group
+ * starts that do not begin at 0, increase strictly and end at P. */
+#define DDPG_EXPLOIT_MAX_GROUPS 16
+typedef struct DdpgExploitParams DdpgExploitParams;
+struct DdpgExploitParams {
+  double frac;                 /* share of each group replaced and share it is drawn from, [0, 0.5] */
+  float factor_lo, factor_hi;  /* perturbation factors, finite and > 0 */
+  int32_t keys;                /* bit j set: perturb hyper-parameter j (0 lr_actor, 1 lr_critic, 2 gamma, 3 tau, 4 noise_scale) */
+  uint32_t round;              /* Philox counter: the evaluation round */
+  uint64_t seed;
+  int32_t n_groups;            /* 0: one group of all P learners */
+  int32_t group_start[DDPG_EXPLOIT_MAX_GROUPS + 1];
+};
+SHEMS_API int32_t ddpg_exploit(Ddpg* h, const double* score_dev, const DdpgExploitParams* p, int32_t* parent_dev);
 /* replay() (DDPG.jl:121-145) n_updates times: sample -> TD target -> critic step -> actor step
  * -> Polyak.  idx_host ([n_updates][batch], 0-based logical indices) or NULL -> Philox(seed, draw j, counter u = index of the
  * update inside this call): replay(rng_rpl = r) trains on the minibatch replay_sample(seed = r) returns, as getData(rng) is one

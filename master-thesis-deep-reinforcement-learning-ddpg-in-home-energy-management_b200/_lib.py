@@ -44,6 +44,16 @@ class ShemsRolloutArgs(C.Structure):
     ]
 
 
+EXPLOIT_MAX_GROUPS = 16
+
+
+class DdpgExploitParams(C.Structure):
+    _fields_ = [
+        ("frac", C.c_double), ("factor_lo", C.c_float), ("factor_hi", C.c_float), ("keys", C.c_int32), ("round", C.c_uint32),
+        ("seed", C.c_uint64), ("n_groups", C.c_int32), ("group_start", C.c_int32 * (EXPLOIT_MAX_GROUPS + 1)),
+    ]
+
+
 class ShemsError(RuntimeError):
     def __init__(self, code, msg):
         super().__init__(f"[{code}] {msg}")
@@ -136,6 +146,7 @@ SIGNATURES = {
     "ddpg_keep_best": (I32, [VP, VP, I64, I32, VP]),
     "ddpg_get_best": (I32, [VP, PD, PI]),
     "ddpg_set_best": (I32, [VP, PD, PI]),
+    "ddpg_exploit": (I32, [VP, VP, C.POINTER(DdpgExploitParams), VP]),
     "ddpg_state_floats": (I64, [VP]),
     "ddpg_get_state": (I32, [VP, PF, PD]),
     "ddpg_set_state": (I32, [VP, PF, PD]),

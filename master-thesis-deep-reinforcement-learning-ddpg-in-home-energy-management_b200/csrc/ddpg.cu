@@ -547,6 +547,7 @@ struct Ddpg {
   float* best; long long best_stride; double* best_score; int32_t* best_run;
   int noise_kind; float ou_theta, ou_mu, ou_dt;   // ddpg_set_noise
   DdpgHparams* hp;   // [pop] host copy of every learner's ctrl->hp (ddpg_get_hparams; σ_eff of the one-learner cluster kernels)
+  bool hp_stale;     // ddpg_exploit rewrote ctrl->hp on the device: ddpg_get_hparams reloads hp before it answers
   float* ou_x; long long ou_cap;                   // OUNoise.X of every instance of ddpg_episode's environment ([2][N])
 };
 static inline int round_ld(int x) { return (x + 31) & ~31; }  // activation rows start on 128-byte lines: one L2 request per TMA box row
@@ -754,6 +755,13 @@ extern "C" int32_t ddpg_set_hparams(Ddpg* h, float lr_actor, float lr_critic, fl
 }
 extern "C" int32_t ddpg_get_hparams(Ddpg* h, float* lr_actor, float* lr_critic, float* gamma, float* tau, float* noise_scale) {
   REQUIRE(h && lr_actor && lr_critic && gamma && tau && noise_scale, SHEMS_ERR_INVALID, "ddpg_get_hparams: NULL argument");
+  if (h->hp_stale) {   // after ddpg_exploit: the device values of every learner (a ddpg_set_hparams enqueued later has landed too)
+    GUARD(h->device);
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    CUDA_TRY(cudaMemcpy2D(h->hp, sizeof(DdpgHparams), (const char*)h->ctrl + offsetof(DdpgCtrl, hp), sizeof(DdpgCtrl), sizeof(DdpgHparams),
+                          (size_t)h->pop, cudaMemcpyDeviceToHost));
+    h->hp_stale = false;
+  }
   const DdpgHparams& v = h->hp[h->sel];
   *lr_actor = v.eta[1]; *lr_critic = v.eta[0]; *gamma = v.gamma; *tau = v.tau; *noise_scale = v.noise_scale;
   return SHEMS_OK;
@@ -2501,6 +2509,157 @@ extern "C" int32_t ddpg_set_best(Ddpg* h, const double* best_score_host, const i
   CUDA_TRY(cudaStreamSynchronize(h->stream));
   CUDA_TRY(cudaMemcpy(h->best_score, best_score_host, sizeof(double) * (size_t)h->pop, cudaMemcpyHostToDevice));
   CUDA_TRY(cudaMemcpy(h->best_run, best_run_host, sizeof(int32_t) * (size_t)h->pop, cudaMemcpyHostToDevice));
+  return SHEMS_OK;
+}
+
+// ----------------------------------------------------------------------------- population-based training (exploit + explore)
+// ddpg_exploit: inside every group of learners the bottom share takes over the learner state of a learner drawn from the top share and
+// perturbs its hyper-parameters.  Grid (copy chunks x P), blockIdx.y = learner d.  Every block works out d's decision itself from the
+// scores (a pure function of scores, seed, round and d), so all blocks of d agree without talking to each other and the call is one
+// launch.  Top (rank < k) and bottom (rank >= m - k) sets are disjoint for k <= m / 2: no learner is read and written in one call.
+#define EXPLOIT_THREADS 256
+#define EXPLOIT_UNROLL 8
+#define EXPLOIT_CHUNK (EXPLOIT_THREADS * EXPLOIT_UNROLL)   // float4 per block
+#define EXPLOIT_PARTS 9
+struct ExploitArgs {
+  const double* score; float* slab; long long pop_stride; DdpgCtrl* ctrl; int32_t* parent;
+  long long part_off[EXPLOIT_PARTS], part_n4[EXPLOIT_PARTS];   // float4 offset of a part inside a learner's slab, float4 count
+  double frac; float factor_lo, factor_hi; int keys; unsigned round; unsigned long long seed;
+  int n_groups; int group_start[DDPG_EXPLOIT_MAX_GROUPS + 1];
+};
+// the sort key: the score with NaN as -inf; learner i ranks before learner j on a larger key, ties to the lower index
+__device__ __forceinline__ double pbt_key(double s) { return isnan(s) ? -INFINITY : s; }
+__device__ __forceinline__ bool pbt_before(double ki, int i, double kj, int j) { return ki > kj || (ki == kj && i < j); }
+// hyper-parameter j of the source (bit j of keys set): x * factor in one fp32 multiply; gamma and tau then at most 1
+__device__ __forceinline__ float pbt_perturb(float x, int j, int keys, unsigned w1, float lo, float hi) {
+  if (!((keys >> j) & 1)) return x;
+  const float y = __fmul_rn(x, ((w1 >> j) & 1u) ? hi : lo);
+  return (j == 2 || j == 3) ? fminf(y, 1.0f) : y;
+}
+__device__ __forceinline__ int block_sum(int v, int* red) {
+  v = __reduce_add_sync(0xffffffffu, v);
+  __syncthreads();   // red may still be read from an earlier call
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  int s = 0;
+#pragma unroll
+  for (int w = 0; w < EXPLOIT_THREADS / 32; ++w) s += red[w];
+  return s;
+}
+
+__global__ void __launch_bounds__(EXPLOIT_THREADS) ddpg_exploit_kernel(const ExploitArgs a) {
+  __shared__ int red[EXPLOIT_THREADS / 32];
+  __shared__ int s_src;
+  const int d = blockIdx.y, tid = threadIdx.x;
+  int g = 0;
+  while (d >= a.group_start[g + 1]) ++g;
+  const int g0 = a.group_start[g], m = a.group_start[g + 1] - g0;
+  const int k = (int)floor(a.frac * (double)m);
+  // rank of d inside its group: the learners that rank before it
+  const double kd = pbt_key(a.score[d]);
+  int c = 0;
+  for (int i = g0 + tid; i < g0 + m; i += EXPLOIT_THREADS) c += pbt_before(pbt_key(a.score[i]), i, kd, d);
+  const int rank = block_sum(c, red);
+  if (k == 0 || rank < m - k) {   // kept
+    if (blockIdx.x == 0 && tid == 0 && a.parent) a.parent[d] = -1;
+    return;
+  }
+  uint32_t w[4];
+  philox4x32_10(a.seed, (uint64_t)d, a.round, STREAM_PBT, w);
+  const int r_src = (int)(uint32_t)(((uint64_t)w[0] * (uint64_t)k) >> 32);
+  // the source is the group's learner of rank r_src: every thread ranks its candidates (ranks are a permutation: one thread finds it)
+  for (int j = g0 + tid; j < g0 + m; j += EXPLOIT_THREADS) {
+    const double kj = pbt_key(a.score[j]);
+    int rj = 0;
+    for (int i = g0; i < g0 + m && rj <= r_src; ++i) rj += pbt_before(pbt_key(a.score[i]), i, kj, j);
+    if (rj == r_src) s_src = j;
+  }
+  __syncthreads();
+  const int src = s_src;
+  if (blockIdx.x == 0 && tid == 0) {   // optimiser β powers and their reciprocals, perturbed hyper-parameters, lineage
+    const DdpgCtrl& cs = a.ctrl[src];
+    DdpgCtrl& cd = a.ctrl[d];
+#pragma unroll
+    for (int n = 0; n < 2; ++n)
+#pragma unroll
+      for (int b = 0; b < 2; ++b) { cd.bp[n][b] = cs.bp[n][b]; cd.rc[n][b] = cs.rc[n][b]; }
+    const DdpgHparams hs = cs.hp;
+    DdpgHparams hd;   // bits of keys in Learner.HPARAMS order: 0 lr_actor (eta[1]), 1 lr_critic (eta[0]), 2 gamma, 3 tau, 4 noise_scale
+    hd.eta[1] = pbt_perturb(hs.eta[1], 0, a.keys, w[1], a.factor_lo, a.factor_hi);
+    hd.eta[0] = pbt_perturb(hs.eta[0], 1, a.keys, w[1], a.factor_lo, a.factor_hi);
+    hd.gamma = pbt_perturb(hs.gamma, 2, a.keys, w[1], a.factor_lo, a.factor_hi);
+    hd.tau = pbt_perturb(hs.tau, 3, a.keys, w[1], a.factor_lo, a.factor_hi);
+    hd.noise_scale = pbt_perturb(hs.noise_scale, 4, a.keys, w[1], a.factor_lo, a.factor_hi);
+    cd.hp = hd;
+    if (a.parent) a.parent[d] = src;
+  }
+  // this block's chunk of the concatenated parts: every part starts on a 256-byte boundary of the slab and its float4 count covers
+  // the part (the tail float4 stays inside the part's 64-float carve), so the copy is float4 only
+  const float4* __restrict__ from = reinterpret_cast<const float4*>(a.slab + (long long)src * a.pop_stride);
+  float4* __restrict__ to = reinterpret_cast<float4*>(a.slab + (long long)d * a.pop_stride);
+  const long long c0 = (long long)blockIdx.x * EXPLOIT_CHUNK, c1 = c0 + EXPLOIT_CHUNK;
+  long long p0 = 0;
+#pragma unroll 1
+  for (int p = 0; p < EXPLOIT_PARTS; ++p) {
+    const long long p1 = p0 + a.part_n4[p], lo = max(c0, p0), hi = min(c1, p1);
+    if (lo < hi) {
+      const float4* s = from + a.part_off[p] + (lo - p0);
+      float4* t = to + a.part_off[p] + (lo - p0);
+      const long long n = hi - lo;
+      float4 v[EXPLOIT_UNROLL];
+#pragma unroll
+      for (int u = 0; u < EXPLOIT_UNROLL; ++u) {
+        const long long i = tid + (long long)u * EXPLOIT_THREADS;
+        if (i < n) v[u] = __ldg(s + i);
+      }
+#pragma unroll
+      for (int u = 0; u < EXPLOIT_UNROLL; ++u) {
+        const long long i = tid + (long long)u * EXPLOIT_THREADS;
+        if (i < n) t[i] = v[u];
+      }
+    }
+    p0 = p1;
+  }
+}
+
+extern "C" int32_t ddpg_exploit(Ddpg* h, const double* score_dev, const DdpgExploitParams* p, int32_t* parent_dev) {
+  REQUIRE(h && score_dev && p, SHEMS_ERR_INVALID, "ddpg_exploit: NULL argument");
+  REQUIRE(p->frac >= 0.0 && p->frac <= 0.5, SHEMS_ERR_INVALID, "ddpg_exploit: frac=%g outside [0, 0.5]", p->frac);
+  REQUIRE(isfinite(p->factor_lo) && isfinite(p->factor_hi) && p->factor_lo > 0.0f && p->factor_hi > 0.0f, SHEMS_ERR_INVALID,
+          "ddpg_exploit: factors %g, %g must be finite and > 0", (double)p->factor_lo, (double)p->factor_hi);
+  REQUIRE(p->keys >= 0 && p->keys <= 31, SHEMS_ERR_INVALID, "ddpg_exploit: keys=%d outside 0..31", p->keys);
+  REQUIRE(p->n_groups >= 0 && p->n_groups <= DDPG_EXPLOIT_MAX_GROUPS, SHEMS_ERR_INVALID, "ddpg_exploit: n_groups=%d outside 0..%d", p->n_groups,
+          DDPG_EXPLOIT_MAX_GROUPS);
+  ExploitArgs a;
+  memset(&a, 0, sizeof(a));
+  if (p->n_groups == 0) {
+    a.n_groups = 1; a.group_start[0] = 0; a.group_start[1] = h->pop;
+  } else {
+    REQUIRE(p->group_start[0] == 0 && p->group_start[p->n_groups] == h->pop, SHEMS_ERR_INVALID,
+            "ddpg_exploit: group starts must begin at 0 and end at P = %d (%d .. %d)", h->pop, p->group_start[0], p->group_start[p->n_groups]);
+    for (int g = 0; g < p->n_groups; ++g)
+      REQUIRE(p->group_start[g] < p->group_start[g + 1], SHEMS_ERR_INVALID, "ddpg_exploit: group starts do not increase at group %d (%d, %d)", g,
+              p->group_start[g], p->group_start[g + 1]);
+    a.n_groups = p->n_groups;
+    for (int g = 0; g <= p->n_groups; ++g) a.group_start[g] = p->group_start[g];
+  }
+  GUARD(h->device);
+  // what ddpg_get_state / ddpg_set_state move: the four nets, the four ADAM moment arrays, s_min | s_max
+  const long long na = h->dims[0].n_params, nc = h->dims[1].n_params;
+  float* const parts[EXPLOIT_PARTS] = {h->net[0], h->net[1], h->net[2], h->net[3], h->adam_m[0], h->adam_v[0], h->adam_m[1], h->adam_v[1], h->norm};
+  const long long counts[EXPLOIT_PARTS] = {na, nc, na, nc, na, na, nc, nc, 18};
+  long long total = 0;
+  for (int i = 0; i < EXPLOIT_PARTS; ++i) {
+    a.part_off[i] = (parts[i] - h->slab) / 4;   // every part starts on a 256-byte boundary
+    a.part_n4[i] = (counts[i] + 3) / 4;
+    total += a.part_n4[i];
+  }
+  a.score = score_dev; a.slab = h->slab; a.pop_stride = h->pop_stride; a.ctrl = h->ctrl; a.parent = parent_dev;
+  a.frac = p->frac; a.factor_lo = p->factor_lo; a.factor_hi = p->factor_hi; a.keys = p->keys; a.round = p->round; a.seed = p->seed;
+  const dim3 grid((unsigned)((total + EXPLOIT_CHUNK - 1) / EXPLOIT_CHUNK), (unsigned)h->pop);
+  ddpg_exploit_kernel<<<grid, EXPLOIT_THREADS, 0, h->stream>>>(a);
+  CUDA_TRY(cudaGetLastError());
+  h->hp_stale = true;
   return SHEMS_OK;
 }
 

@@ -301,6 +301,28 @@ class Learner:
         run = np.ascontiguousarray(np.broadcast_to(np.asarray(best_run, np.int32), (self.population,)))
         L.check(self.lib.ddpg_set_best(self._h, sc.ctypes.data_as(L.PD), run.ctypes.data_as(L.PI)))
 
+    def exploit(self, score, frac, factors=(0.8, 1.25), keys=HPARAMS, seed=0, round=0, groups=None):
+        """ddpg_exploit (population-based training): in every group the learners ranked in the bottom floor(frac * m) by `score`
+        (the [P] float64 device tensor keep_best returns; NaN ranks last) take over the learner state (nets, targets, ADAM moments
+        and β powers, s_min / s_max) of a learner drawn from the top floor(frac * m), and the hyper-parameters named in `keys` become
+        float32(source value × factors[0] or factors[1]), γ and τ at most 1.  groups: learners per group in order (summing to P) or
+        None for one group.  Enqueued only; returns parent [P] int32 (device): the source of a replaced learner, -1 otherwise."""
+        assert score.dtype == torch.float64 and score.numel() == self.population and score.is_cuda and score.is_contiguous()
+        bad = set(keys) - set(self.HPARAMS)
+        assert not bad, f"unknown hyper-parameters {sorted(bad)}"
+        p = L.DdpgExploitParams()
+        p.frac, p.factor_lo, p.factor_hi = float(frac), float(factors[0]), float(factors[1])
+        p.keys = sum(1 << self.HPARAMS.index(k) for k in set(keys))
+        p.round, p.seed = int(round) & 0xFFFFFFFF, int(seed) & (2**64 - 1)
+        if groups is not None:
+            sizes = [int(x) for x in groups]
+            assert len(sizes) <= L.EXPLOIT_MAX_GROUPS, f"{len(sizes)} groups, at most {L.EXPLOIT_MAX_GROUPS}"
+            p.n_groups = len(sizes)
+            p.group_start[:len(sizes) + 1] = np.concatenate([[0], np.cumsum(sizes)]).astype(int).tolist()
+        parent = torch.empty(self.population, dtype=torch.int32, device=self._dev)
+        L.check(self.lib.ddpg_exploit(self._h, _ptr(score), C.byref(p), _ptr(parent)))
+        return parent
+
     # ---- full snapshot (nets, targets, ADAM moments, β powers, update counter, s_min/s_max): resume where the run stopped
     def get_state(self):
         n = int(self.lib.ddpg_state_floats(self._h))
@@ -693,7 +715,7 @@ class PopulationDriver:
         return ret.view(self.P, self.n_envs).mean(dim=1).cpu().numpy()
 
     # run_episodes (DDPG.jl:244-298, driver DDPG_reinforce_charger_v1.jl:87-105) for every learner at once
-    def run_episodes(self, num_ep, test_every=100, seed_ini=123, on_best=None, start_ep=1, state=None):
+    def run_episodes(self, num_ep, test_every=100, seed_ini=123, on_best=None, start_ep=1, state=None, pbt=None):
         """Driver.run_episodes for the population.  Training episode i (rng_ep = seeds[0] * 100003 + i) fills total_reward[i-1] [P];
         every `test_every` episodes (i = 1, 1 + test_every, ...: the reference's i % test_every == 1, and every episode for
         test_every = 1) one evaluation round runs on the evaluation handle: ONE reset! (rng = seed_ini * 1000 + 1), one ddpg_evaluate of
@@ -704,11 +726,25 @@ class PopulationDriver:
         a one-learner handle with an evaluation env of test_runs instances after reset!(rng = seed_ini * 1000 + 1).
         Returns {total_reward [num_ep][P], score_mean [ceil(num_ep / test_every)][P], best_run [P], best_score [P]}.  A fresh start
         (state=None) sets best_score = -100000, best_run = 0 and zero best actors; `state` / `start_ep` continue an interrupted loop
-        (its best scores are written back to the handle; restore the best actors with tracker.load_checkpoint)."""
+        (its best scores are written back to the handle; restore the best actors with tracker.load_checkpoint).
+        pbt = dict(every, frac, factors=(0.8, 1.25), keys=Learner.HPARAMS, seed=0) adds population-based training: after the
+        keep_best of every `every`-th evaluation round r (0-based: r = every - 1, 2 every - 1, ...) one Learner.exploit with the
+        runs of equal chargers as groups (an actor never moves to another household's battery) and round = r, so a resumed run
+        draws the same choices.  st then also holds parent [rounds][P] int32 (-1: kept, or a round without exploit) and hparams
+        [rounds][P][5] float32 (Learner.HPARAMS order), the values after the round; save them with the scores
+        (tracker.save_checkpoint(**st))."""
         assert self.env_eval is not None, "run_episodes needs eval_series"
         P, te = self.P, int(test_every)
-        st = state if state is not None else dict(total_reward=np.zeros((num_ep, P)), score_mean=np.zeros((-(-num_ep // te), P)),
+        rounds = -(-num_ep // te)
+        st = state if state is not None else dict(total_reward=np.zeros((num_ep, P)), score_mean=np.zeros((rounds, P)),
                                                   best_run=np.zeros(P, np.int32), best_score=np.full(P, -100000.0))
+        if pbt is not None:
+            every = int(pbt["every"])
+            assert every >= 1, "pbt['every'] counts evaluation rounds (>= 1)"
+            pkw = dict(frac=float(pbt["frac"]), factors=tuple(pbt.get("factors", (0.8, 1.25))), keys=tuple(pbt.get("keys", Learner.HPARAMS)),
+                       seed=int(pbt.get("seed", 0)), groups=[m for _, m in self._runs])
+            st.setdefault("parent", np.full((rounds, P), -1, np.int32))
+            st.setdefault("hparams", np.zeros((rounds, P, len(Learner.HPARAMS)), np.float32))
         self.learner.set_best(st["best_score"], st["best_run"])
         if state is None:   # no best actor left over from an earlier call on this handle
             for l in range(P):
@@ -722,12 +758,23 @@ class PopulationDriver:
             st["total_reward"][i - 1] = r.cpu().numpy()
             if (i - 1) % te == 0:
                 ret = self.learner.evaluate(self.reset_eval(seed_ini * 1000 + 1), self.ep_length)["ep_return"]
-                score = self.learner.keep_best(ret, self.test_runs, i).cpu().numpy()
-                st["score_mean"][-(-i // te) - 1] = score
+                score_dev = self.learner.keep_best(ret, self.test_runs, i)
+                rnd = -(-i // te) - 1
+                parent = None
+                if pbt is not None and (rnd + 1) % every == 0:
+                    parent = self.learner.exploit(score_dev, round=rnd, **pkw)
+                score = score_dev.cpu().numpy()
+                st["score_mean"][rnd] = score
                 for l in np.flatnonzero(score > st["best_score"]):     # the same strict rule ddpg_keep_best applied on the device
                     if on_best is not None:
                         on_best(int(l), i, float(score[l]))
                     st["best_score"][l], st["best_run"][l] = score[l], i
+                if pbt is not None:
+                    st["parent"][rnd] = parent.cpu().numpy() if parent is not None else -1
+                    for l in range(P):
+                        hp = self.learner.select(l).get_hparams()
+                        st["hparams"][rnd, l] = [hp[k] for k in Learner.HPARAMS]
+                    self.learner.select(0)
         return st
 
     # inference(env; track = 1) — memory_plotting_saving.jl:62-89, driver :95-105: one deterministic instance per learner

@@ -9,7 +9,12 @@ averaged over the learners (seeds, chargers) that share it.
 --test-every K --test-runs R --inference-dir DIR: the reference protocol (run_episodes, DDPG.jl:244-298; driver :87-105) on a synthetic
 evaluation series (1440 rows) and test series (3000 rows): every K episodes R noise-free evaluation episodes per learner from row 1,
 each learner's best actor kept on the device, then inference of every best actor over the test series, one results CSV per learner
-and a summary CSV in DIR.  The report adds best score, best run and test-set return per learner and per grid point."""
+and a summary CSV in DIR.  The report adds best score, best run and test-set return per learner and per grid point.
+--pbt EVERY,FRAC [--pbt-factors LO,HI] [--pbt-keys name,...] (needs --test-every): population-based training inside every run of equal
+chargers (PopulationDriver.run_episodes(pbt=...)): after every EVERY-th evaluation round the worst floor(FRAC * m) learners of a run take
+over the state of one of its best floor(FRAC * m) and perturb the named hyper-parameters by LO or HI.  Under torch.distributed each rank
+does this over its own shard.  The report adds every learner's final hyper-parameters and how often it was replaced; the grid
+table stays keyed by each learner's starting grid point."""
 import argparse
 import itertools
 import json
@@ -32,6 +37,9 @@ ap.add_argument("--grid", nargs="*", default=[], metavar="NAME=V1,V2", help="per
 ap.add_argument("--test-every", type=int, default=0, help="evaluate every K episodes and keep each learner's best actor (run_episodes)")
 ap.add_argument("--test-runs", type=int, default=100, help="evaluation episodes per learner and round")
 ap.add_argument("--inference-dir", default=None, help="write the test-set inference CSVs of the best actors here (needs --test-every)")
+ap.add_argument("--pbt", default=None, metavar="EVERY,FRAC", help="population-based training every EVERY evaluation rounds, share FRAC (needs --test-every)")
+ap.add_argument("--pbt-factors", default="0.8,1.25", metavar="LO,HI", help="perturbation factors of --pbt")
+ap.add_argument("--pbt-keys", default=",".join(sb.Learner.HPARAMS), metavar="NAME,...", help="hyper-parameters --pbt perturbs")
 args = ap.parse_args()
 GRID_NAMES = ("lr_actor", "lr_critic", "gamma", "tau", "noise_scale", "sigma")
 grid = {}
@@ -61,6 +69,12 @@ drv_kw = dict(sigma=1.0) if "sigma" in grid else {}
 ser = sb.series.synth_charger98(4320, seed=98)
 assert args.inference_dir is None or args.test_every > 0, "--inference-dir runs the best actors: give --test-every K to choose them"
 protocol = args.test_every > 0
+assert args.pbt is None or protocol, "--pbt exploits the evaluation scores: give --test-every K"
+pbt = None
+if args.pbt:
+    p_every, p_frac = args.pbt.split(",")
+    lo, hi = (float(x) for x in args.pbt_factors.split(","))
+    pbt = dict(every=int(p_every), frac=float(p_frac), factors=(lo, hi), keys=tuple(k for k in args.pbt_keys.split(",") if k), seed=rank)
 if protocol:
     drv_kw.update(eval_series=sb.series.synth_charger98(1440, seed=1440), test_runs=args.test_runs)
 drv = sb.PopulationDriver(ser, chargers=chargers, seeds=seeds, n_envs=args.envs, device=local, use_tensor_cores=args.tc, hparams=hparams, **drv_kw)
@@ -75,16 +89,20 @@ t1 = time.time()
 t_eval = 0.0
 if protocol:   # run_episodes: training episodes with an evaluation round every --test-every episodes
     import numpy as np
-    st = drv.run_episodes(args.episodes, test_every=args.test_every)
+    st = drv.run_episodes(args.episodes, test_every=args.test_every, pbt=pbt)
     torch.cuda.synchronize()
     dt = time.time() - t1
     rets, trace = drv.inference(sb.series.synth_charger98(3000, seed=3000))
     test_ret = rets.cpu().numpy()
     if args.inference_dir:
         hp_rows = [{k: v[l] for k, v in hparams.items()} for l in range(P)]
+        if pbt is not None:   # the values the best actors' lineages ended with
+            hp_rows = [dict(zip(sb.Learner.HPARAMS, st["hparams"][-1, l].tolist())) for l in range(P)]
         sb.tracker.write_population_results(os.path.join(args.inference_dir, f"rank{rank}"), trace, chargers, seeds, st["best_run"],
                                             st["best_score"], hparams=hp_rows)
     best = dict(best_score=st["best_score"].tolist(), best_run=[int(x) for x in st["best_run"]], test_return=test_ret.tolist(), grid_of=grid_of)
+    if pbt is not None:
+        best.update(hparams_final=st["hparams"][-1].tolist(), replaced=[int(x) for x in (st["parent"] >= 0).sum(axis=0)])
     if dist is not None:
         every = [None] * world if rank == 0 else None
         dist.gather_object(best, every, dst=0)
@@ -96,6 +114,8 @@ if protocol:   # run_episodes: training episodes with an evaluation round every 
         gi, bs, tr = (np.asarray(best[k]) for k in ("grid_of", "best_score", "test_return"))
         print(json.dumps(dict(learners=len(gi), episodes=args.episodes, test_every=args.test_every, test_runs=args.test_runs, train_seconds=dt,
                               best_score=best["best_score"], best_run=best["best_run"], test_return=best["test_return"],
+                              **({k: best[k] for k in ("hparams_final", "replaced")} if pbt is not None else {}),
+                              pbt=pbt,
                               grid=[dict(point=pt, learners=int((gi == i).sum()), best_score=float(bs[gi == i].mean()),
                                          best_score_max=float(bs[gi == i].max()), test_return=float(tr[gi == i].mean()))
                                     for i, pt in enumerate(points) if (gi == i).any()])), flush=True)
