@@ -570,6 +570,8 @@ static void make_dims(NetDims& d, int in, int l1, int l2, int out) {
   d.n_params = off;
 }
 static inline const NetDims& dims_of(const Ddpg* h, int net) { return h->dims[(net == DDPG_NET_CRITIC || net == DDPG_NET_CRITIC_TARGET) ? 1 : 0]; }
+// every slab buffer starts on a 256-byte boundary: W2 rows are 16-byte aligned iff l2 and both W2 offsets are multiples of 4 floats
+static inline bool w2_vec16(const Ddpg* h) { return h->p.l2 % 4 == 0 && h->dims[0].l[1].w_off % 4 == 0 && h->dims[1].l[1].w_off % 4 == 0; }
 
 extern "C" int32_t ddpg_default_params(DdpgParams* p) {
   REQUIRE(p, SHEMS_ERR_INVALID, "ddpg_default_params: NULL");
@@ -609,7 +611,7 @@ extern "C" int32_t ddpg_create(const DdpgParams* p, int32_t device, Ddpg** out) 
   h->ld1 = round_ld(p->l1); h->ld2 = round_ld(p->l2);
   const int l1 = h->ld1, l2 = h->ld2;  // allocation strides
   // W2 of both nets must start on a 16-byte boundary and have 16-byte rows for the TMA descriptors
-  h->tc = p->use_tensor_cores && (p->l2 % 4 == 0) && (h->dims[0].l[1].w_off % 4 == 0) && (h->dims[1].l[1].w_off % 4 == 0);
+  h->tc = p->use_tensor_cores && w2_vec16(h);
   h->ws_floats = (long long)SPLITK_MAX * ((long long)p->l1 * p->l2 + p->l2 + (long long)C * p->l1 + p->l1 + (long long)p->l2 * A + A);
   DMALLOC(h->ws, h->ws_floats);
   DMALLOC(h->counters, WS_COUNTERS);
@@ -1337,6 +1339,10 @@ static int launch_gemms(cudaStream_t st, const GemmProblem* ps, int count, int p
   CUDA_TRY(cudaGetLastError());
   return SHEMS_OK;
 }
+// the same problems for every learner of the handle, each on the weights and activations of its own slab
+static inline int slab_gemms(const Ddpg* h, cudaStream_t st, const GemmProblem* ps, int count) {
+  return launch_gemms(st, ps, count, h->pop, h->pop_stride, h->pop_stride);
+}
 #define TRY(x) do { int _s = (x); if (_s) return _s; } while (0)
 
 // dW-type product (K = batch) with its bias gradient.  From SPLITK_MIN_BATCH rows on the batch dimension is split over
@@ -1344,7 +1350,7 @@ static int launch_gemms(cudaStream_t st, const GemmProblem* ps, int count, int p
 static int launch_dw(Ddpg* h, cudaStream_t st, const GemmProblem& g, bool side = false) {
   const int B = g.K;
   float* const ws = side ? h->ws_side : h->ws;
-  if (B < SPLITK_MIN_BATCH) return launch_gemms(st, &g, 1, h->pop, h->pop_stride, h->pop_stride);
+  if (B < SPLITK_MIN_BATCH) return slab_gemms(h, st, &g, 1);
   const long long mn = (long long)g.M * g.N, stride = mn + g.N;
   REQUIRE(g.ldc == g.N && g.dbias == g.C + mn && g.epi == EPI_NONE, SHEMS_ERR_INVALID, "launch_dw: not a contiguous [W|b] gradient block");
   const int ksplit = min(SPLITK_MAX, B / 256);
@@ -1363,14 +1369,8 @@ static int launch_dw(Ddpg* h, cudaStream_t st, const GemmProblem& g, bool side =
 
 // ---- layer-2 contractions on TF32 tensor cores (csrc/tc_gemm.cu); operands are used where they lie in HBM.  A population
 // handle runs all learners' products in one launch (grid.z = learner): weights/gradients/activations of learner l sit
-// l*pop_stride floats behind learner 0's; act() scratch uses its own stride (xs).
-// Y = relu(X · W + b):  X [M][ldx] K-major, Flux weight Wt[in][out] MN-major
-static int tc_fwd(const Ddpg* h, cudaStream_t st, const float* X, int ldx, int M, const float* net, const LayerDims& L, float* Y, int ldy, long long xstride) {
-  TcOperand A{X, ldx, false}, Bo{net + L.w_off, L.out, true};
-  TcBatch bt; bt.count = h->pop; bt.sA = xstride; bt.sB = h->pop_stride; bt.sD = xstride; bt.sBias = h->pop_stride;
-  return tc_gemm(st, A, Bo, Y, ldy, M, L.out, L.in, TC_EPI_BIAS_RELU, net + L.b_off, nullptr, 0, 1, nullptr, bt);
-}
-// dX = (dZ · W^T) masked by relu'(H):  dZ [M][lddz] K-major, Wt[in][out] K-major (k = out)
+// l*pop_stride floats behind learner 0's; act() scratch uses its own stride (enqueue_forward's xstride).
+// dX =(dZ · W^T) masked by relu'(H):  dZ [M][lddz] K-major, Wt[in][out] K-major (k = out)
 static int tc_dx(const Ddpg* h, cudaStream_t st, const float* dZ, int lddz, int M, const float* net, const LayerDims& L, float* dX, int lddx, const float* H, int ldh) {
   TcOperand A{dZ, lddz, false}, Bo{net + L.w_off, L.out, false};
   TcBatch bt; bt.count = h->pop; bt.sA = bt.sB = bt.sD = bt.sAux = h->pop_stride;
@@ -1399,16 +1399,19 @@ static int tc_dw(Ddpg* h, cudaStream_t st, const float* X, int ldx, const float*
   CUDA_TRY(cudaGetLastError());
   return SHEMS_OK;
 }
-// large-batch first layer (up to 3 problems): see l1_fwd_kernel
-static int big_l1(cudaStream_t st, int count, const float* const* X, int ldx, int M, const float* const* net, const LayerDims* const* L,
-                  float* const* Y, int ldy, int pop = 1, long long ls_w = 0, long long ls_x = 0) {
+// one net of a forward pass: inputs X -> h1 -> h2 -> output layer (out: TC_OUT_TANH / TC_OUT_ID / TC_OUT_TD) into y [rows][ldy].
+// keep: a backward pass reads h1 and h2 (the chain kernel stores them only then; the layer-by-layer products always go through them)
+struct FwdNet { const float* X; const float* w; const NetDims* d; float *h1, *h2; bool keep; int out; float* y; int ldy; };
+// large-batch first layer (up to 3 nets): see l1_fwd_kernel
+static int big_l1(cudaStream_t st, const FwdNet* nets, int count, int ldx, int M, int ldy, int pop, long long ls_w, long long ls_x) {
   L1Batch a; memset(&a, 0, sizeof(a));
   a.count = count; a.ls_w = ls_w; a.ls_x = ls_x;
   for (int i = 0; i < count; ++i) {
-    a.X[i] = X[i]; a.W[i] = net[i] + L[i]->w_off; a.bias[i] = net[i] + L[i]->b_off; a.Y[i] = Y[i]; a.K[i] = L[i]->in;
-    REQUIRE(L[i]->in <= 12 && L[i]->out == L[0]->out, SHEMS_ERR_INVALID, "big_l1: unsupported first-layer shape");
+    const LayerDims& L = nets[i].d->l[0];
+    a.X[i] = nets[i].X; a.W[i] = nets[i].w + L.w_off; a.bias[i] = nets[i].w + L.b_off; a.Y[i] = nets[i].h1; a.K[i] = L.in;
+    REQUIRE(L.in <= 12 && L.out == nets[0].d->l[0].out, SHEMS_ERR_INVALID, "big_l1: unsupported first-layer shape");
   }
-  a.M = M; a.N = L[0]->out; a.ldx = ldx; a.ldy = ldy;
+  a.M = M; a.N = nets[0].d->l[0].out; a.ldx = ldx; a.ldy = ldy;
   l1_fwd_kernel<<<dim3((M + 31) / 32, (a.N + 255) / 256, count * pop), 256, 0, st>>>(a);
   CUDA_TRY(cudaGetLastError());
   return SHEMS_OK;
@@ -1450,20 +1453,143 @@ static int side_join(Ddpg* h, cudaStream_t st) {                     // `st` con
   return SHEMS_OK;
 }
 static inline bool use_tc(const Ddpg* h, long long rows) { return h->tc && rows * h->pop >= TC_MIN_ROWS; }
-// forward-chain problem q: net `w` (flat Flux buffer, dims d) on the inputs X [B][11] (first K1 columns)
-static inline void chain_set(TcFwdChainArgs& a, int q, const float* X, const float* w, const NetDims& d, float* H1, float* H2, int mode, float* out, int ldo) {
-  a.X[q] = X; a.K1[q] = d.l[0].in;
-  a.W1[q] = w + d.l[0].w_off; a.b1[q] = w + d.l[0].b_off; a.W2[q] = w + d.l[1].w_off; a.b2[q] = w + d.l[1].b_off;
-  a.W3[q] = w + d.l[2].w_off; a.b3[q] = w + d.l[2].b_off; a.J[q] = d.l[2].out;
-  a.H1[q] = H1; a.H2[q] = H2; a.out_mode[q] = mode; a.out[q] = out; a.ldo[q] = ldo;
+// how the passes of a call run, as the caller decides it: chain: a net's whole forward pass is one kernel (tc_fwd_chain); tc: the
+// layer-2 products on TF32 tensor cores; big: streaming kernels for the thin products, the weight gradients of a backward pass on the
+// side stream
+struct Regime { bool chain, tc, big; };
+static inline Regime update_regime(const Ddpg* h) {
+  const int B = h->p.batch;
+  const bool tc = use_tc(h, B);
+  return Regime{tc && h->chain, tc, tc || B >= SPLITK_MIN_BATCH || h->pop > 1};
 }
-static inline TcFwdChainArgs chain_args(const Ddpg* h, int nprob) {
-  TcFwdChainArgs a; memset(&a, 0, sizeof(a));
-  a.M = h->p.batch; a.L1 = h->p.l1; a.L2 = h->p.l2; a.nprob = nprob; a.ldx = 11; a.ldh1 = h->ld1; a.ldh2 = h->ld2;
-  a.pop = h->pop; a.pop_stride = h->pop_stride;
-  // few row tiles: two CTAs (a cluster) per tile, half of the layer-2 units each, so that the launch covers the SMs
-  a.nsplit = (long long)((h->p.batch + 127) / 128) * nprob * h->pop * 2 <= 148 ? 2 : 1;
-  return a;
+
+// The forward passes of up to 3 nets of one width on M rows of inputs [M][ldx], sharing launches: layer 1 -> layer 2 -> output layer,
+// or with rg.chain one whole-net kernel (csrc/tc_gemm.cu tc_fwd_chain_kernel) launched with the flags pdl / early_weights.  The
+// activations of learner l lie xstride floats behind learner 0's, its weights pop_stride.  defer_out: without the chain kernel the
+// output layer is left to the caller.
+static int enqueue_forward(const Ddpg* h, cudaStream_t st, const Regime& rg, const FwdNet* nets, int count, int ldx, int M, long long xstride,
+                           int pdl = 0, int early_weights = 0, bool defer_out = false) {
+  if (rg.chain) {
+    TcFwdChainArgs a; memset(&a, 0, sizeof(a));
+    a.M = M; a.L1 = h->p.l1; a.L2 = h->p.l2; a.nprob = count; a.ldx = ldx; a.ldh1 = h->ld1; a.ldh2 = h->ld2;
+    a.pop = h->pop; a.pop_stride = h->pop_stride;
+    // few row tiles: two CTAs (a cluster) per tile, half of the layer-2 units each, so that the launch covers the SMs
+    a.nsplit = (long long)((M + 127) / 128) * count * h->pop * 2 <= 148 ? 2 : 1;
+    for (int q = 0; q < count; ++q) {
+      const FwdNet& n = nets[q]; const NetDims& d = *n.d;
+      a.X[q] = n.X; a.K1[q] = d.l[0].in;
+      a.W1[q] = n.w + d.l[0].w_off; a.b1[q] = n.w + d.l[0].b_off; a.W2[q] = n.w + d.l[1].w_off; a.b2[q] = n.w + d.l[1].b_off;
+      a.W3[q] = n.w + d.l[2].w_off; a.b3[q] = n.w + d.l[2].b_off; a.J[q] = d.l[2].out;
+      a.H1[q] = n.keep ? n.h1 : nullptr; a.H2[q] = n.keep ? n.h2 : nullptr; a.out_mode[q] = n.out; a.out[q] = n.y; a.ldo[q] = n.ldy;
+      if (n.out == TC_OUT_TD) {
+        a.td_r = h->r; a.td_done = h->done; a.td_q = h->q; a.td_dq = h->dq; a.inv_batch = 1.0f / (float)M;
+        a.td_gamma = &h->ctrl->hp.gamma; a.td_gamma_stride = sizeof(DdpgCtrl) / sizeof(float);
+      }
+    }
+    a.pdl = pdl; a.early_weights = early_weights;
+    return tc_fwd_chain(st, a);
+  }
+  const int l1 = h->ld1, l2 = h->ld2;
+  GemmProblem g[TC_MAX_PROBLEMS];
+  if (rg.big) TRY(big_l1(st, nets, count, ldx, M, l1, h->pop, h->pop_stride, xstride));
+  else {
+    for (int q = 0; q < count; ++q) g[q] = gp_fwd(nets[q].X, ldx, M, nets[q].w, nets[q].d->l[0], nets[q].h1, l1, EPI_BIAS_RELU);
+    TRY(launch_gemms(st, g, count, h->pop, h->pop_stride, xstride));
+  }
+  if (rg.tc) {  // the layer-2 products have one shape: a single persistent launch deals their tiles over the SMs
+    TcOperand A[TC_MAX_PROBLEMS], W[TC_MAX_PROBLEMS]; float* D[TC_MAX_PROBLEMS]; const float* bias[TC_MAX_PROBLEMS];
+    for (int q = 0; q < count; ++q) {   // Y = relu(X · W + b):  X [M][ld1] K-major, Flux weight Wt[in][out] MN-major
+      const LayerDims& L = nets[q].d->l[1];
+      A[q] = TcOperand{nets[q].h1, l1, false}; W[q] = TcOperand{nets[q].w + L.w_off, L.out, true};
+      D[q] = nets[q].h2; bias[q] = nets[q].w + L.b_off;
+    }
+    TcBatch bt; bt.count = h->pop; bt.sA = bt.sD = xstride; bt.sB = bt.sBias = h->pop_stride;
+    const LayerDims& L = nets[0].d->l[1];
+    TRY(tc_gemm_multi(st, count, A, W, D, l2, M, L.out, L.in, TC_EPI_BIAS_RELU, bias, nullptr, 0, 1, nullptr, bt));
+  } else {
+    for (int q = 0; q < count; ++q) g[q] = gp_fwd(nets[q].h1, l1, M, nets[q].w, nets[q].d->l[1], nets[q].h2, l2, EPI_BIAS_RELU);
+    TRY(launch_gemms(st, g, count, h->pop, h->pop_stride, xstride));
+  }
+  if (defer_out) return SHEMS_OK;
+  for (int q = 0; q < count; ++q) {
+    const FwdNet& n = nets[q];
+    g[q] = gp_fwd(n.h2, l2, M, n.w, n.d->l[2], n.y, n.ldy, n.out == TC_OUT_TANH ? EPI_BIAS_TANH : n.out == TC_OUT_ID ? EPI_BIAS_ID : EPI_TD_TARGET);
+    if (n.out == TC_OUT_TD) { g[q].aux = h->r; g[q].aux2 = h->done; g[q].aux3 = h->q; g[q].out2 = h->dq; g[q].ctrl = h->ctrl; g[q].inv_batch = 1.0f / (float)M; }
+  }
+  return launch_gemms(st, g, count, h->pop, h->pop_stride, xstride);
+}
+
+// The backward pass of one net from dout = d loss / d output [B][J] to its weight gradients in grad, through dz2 [B][ld2] and dz1 [B][ld1],
+// on the activations h1, h2 of its forward pass and the minibatch xs (the actor's first layer reads its 9 state columns).  extra: a
+// product that is no part of the pass (the actor's reporting-only q(s, actor(s))), enqueued off the critical path.
+static int enqueue_backward(Ddpg* h, cudaStream_t st, const Regime& rg, const float* w, const NetDims& d, const float* h1, const float* h2,
+                            const float* dout, float* dz2, float* dz1, float* grad, const GemmProblem* extra = nullptr) {
+  const int B = h->p.batch, l1 = h->ld1, l2 = h->ld2, J = d.l[2].out;
+  GemmProblem g[2];
+  if (rg.big) {
+    // the dX chain (dz2 -> dz1 -> dW1) is the critical path; dW3, dW2 and their bias sums run beside it on the side stream
+    TRY(side_after(h, st, h->ev_fork));                                                                       // dout, h2 are ready
+    TRY(out_bwd_dw(h, h->side, h2, l2, dout, J, B, d.l[2], grad, true));
+    if (extra) TRY(slab_gemms(h, h->side, extra, 1));
+    TRY(launch_outer_mask(h, st, dout, J, w + d.l[2].w_off, h2, l2, B, d.l[2].in, dz2));
+    TRY(side_after(h, st, h->ev_mid));                                                                        // dz2 is ready
+    if (rg.tc) {
+      TRY(tc_dw(h, h->side, h1, l1, dz2, l2, B, d.l[1], grad, true));
+      TRY(tc_dx(h, st, dz2, l2, B, w, d.l[1], dz1, l1, h1, l1));
+    } else {
+      g[0] = gp_dw(h1, l1, dz2, l2, B, d.l[1], grad);
+      g[1] = gp_dx(dz2, l2, B, w, d.l[1], 0, d.l[1].in, dz1, l1, EPI_RELU_MASK, h1, l1);
+      TRY(launch_dw(h, h->side, g[0], true));
+      TRY(slab_gemms(h, st, g + 1, 1));
+    }
+    TRY(launch_dw(h, st, gp_dw(h->xs, 11, dz1, l1, B, d.l[0], grad)));
+    return side_join(h, st);
+  }
+  g[0] = gp_dw(h2, l2, dout, J, B, d.l[2], grad);
+  g[1] = gp_dx(dout, J, B, w, d.l[2], 0, d.l[2].in, dz2, l2, EPI_RELU_MASK, h2, l2);
+  TRY(slab_gemms(h, st, g, 2));
+  g[0] = gp_dw(h1, l1, dz2, l2, B, d.l[1], grad);
+  g[1] = gp_dx(dz2, l2, B, w, d.l[1], 0, d.l[1].in, dz1, l1, EPI_RELU_MASK, h1, l1);
+  TRY(slab_gemms(h, st, g, 2));
+  TRY(launch_dw(h, st, gp_dw(h->xs, 11, dz1, l1, B, d.l[0], grad)));
+  if (extra) TRY(slab_gemms(h, st, extra, 1));
+  return SHEMS_OK;
+}
+
+// ADAM on the critic (opt 0) or on the actor (opt 1: with soft_update! of both targets and the advance of the update counters).
+// dp: the gradient exchange over NVLink fused into the step; parts: the gradient is the sum of the cluster-fused passes' per-cluster
+// partials, added in the same kernel.  One element per thread (the Float64 div/sqrt chains need TLP); the grids of both steps are sized
+// from the critic's parameter count.
+#ifndef ADAM_PARTS_THREADS
+#define ADAM_PARTS_THREADS 256
+#endif
+static int enqueue_adam(Ddpg* h, cudaStream_t st, int opt, float gscale, bool dp, bool parts) {
+  const DdpgParams& p = h->p;
+  const int k = opt == 0 ? 1 : 0;   // index of the net in grad, adam_m, adam_v, parts and dims (0 actor, 1 critic)
+  const long long n = h->dims[k].n_params, nc = h->dims[1].n_params;
+  float* const x = h->net[opt == 0 ? DDPG_NET_CRITIC : DDPG_NET_ACTOR];
+  float* const target = opt ? h->net[DDPG_NET_ACTOR_TARGET] : nullptr;
+  float* const target2 = opt ? h->net[DDPG_NET_CRITIC_TARGET] : nullptr;   // the critic target moves with the actor step (DDPG.jl:142-143)
+  const float* const model2 = opt ? h->net[DDPG_NET_CRITIC] : nullptr;
+  const long long n2 = opt ? nc : 0;
+  const int nparts = parts ? p.batch / FUSED_ROWS : 0;
+  const float* const part = parts ? h->parts[k] : nullptr;
+  if (dp)  // the flat gradient buffer holds the critic's segment, then the actor's
+    return launch_adam_dp(st, h->dp, h->grad[k] - h->gradbuf, part, nparts, parts ? n : 0, h->grad[k], x, h->adam_m[k], h->adam_v[k], n,
+                          p.adam_beta1, p.adam_beta2, p.adam_eps, h->ctrl, opt, target, target2, model2, n2, opt);
+  const unsigned blocks = (unsigned)((nc + 255) / 256);
+  if (parts)
+    adam_polyak_parts_kernel<<<(unsigned)((nc + ADAM_PARTS_THREADS - 1) / ADAM_PARTS_THREADS), ADAM_PARTS_THREADS, 0, st>>>(
+        x, part, nparts, n, h->grad[k], h->adam_m[k], h->adam_v[k], n, p.adam_beta1, p.adam_beta2, p.adam_eps, h->ctrl, opt, target, target2,
+        model2, n2, opt);
+  else if (h->tc)
+    adam_polyak_kernel<true><<<dim3((blocks + 3) / 4, h->pop), 256, 0, st>>>(x, h->grad[k], h->adam_m[k], h->adam_v[k], n, p.adam_beta1, p.adam_beta2,
+                                                                            p.adam_eps, h->ctrl, opt, target, target2, model2, n2, opt, gscale, h->pop_stride);
+  else
+    adam_polyak_kernel<false><<<dim3(blocks, h->pop), 256, 0, st>>>(x, h->grad[k], h->adam_m[k], h->adam_v[k], n, p.adam_beta1, p.adam_beta2,
+                                                                   p.adam_eps, h->ctrl, opt, target, target2, model2, n2, opt, gscale, h->pop_stride);
+  CUDA_TRY(cudaGetLastError());
+  return SHEMS_OK;
 }
 
 // one replay() after the minibatch has been gathered (DESIGN.md, "DDPG update"), in three phases so that a data-parallel
@@ -1475,152 +1601,44 @@ static inline TcFwdChainArgs chain_args(const Ddpg* h, int nprob) {
 // Large batches run one problem per launch; the 250x500 contractions go to the TF32 tensor-core kernel when enabled and
 // every product whose K is the batch is split over the batch.
 static int enqueue_phase0(Ddpg* h, cudaStream_t st) {
-  const DdpgParams& p = h->p;
-  const int B = p.batch, l1 = h->ld1, l2 = h->ld2;
-  const bool tc = use_tc(h, B), big = tc || B >= SPLITK_MIN_BATCH || h->pop > 1;  // streaming kernels for the thin products
+  const Regime rg = update_regime(h);
+  const int B = h->p.batch;
   const NetDims& da = h->dims[0]; const NetDims& dc = h->dims[1];
   float *actor = h->net[DDPG_NET_ACTOR], *critic = h->net[DDPG_NET_CRITIC], *actor_t = h->net[DDPG_NET_ACTOR_TARGET], *critic_t = h->net[DDPG_NET_CRITIC_TARGET];
-  GemmProblem g[4];
-  if (tc && h->chain) {
-    // the forward passes as whole-net kernels (csrc/tc_gemm.cu tc_fwd_chain_kernel): layer 1 -> tcgen05 layer 2 -> output layer
-    // actor_target(s'_n) -> a' | critic(s_n, a) -> q | actor(s_n) -> vcat(s_n, actions)      (DDPG.jl:131, :114, :117)
-    TcFwdChainArgs a = chain_args(h, 3);
-    chain_set(a, 0, h->xs2, actor_t, da, nullptr, nullptr, TC_OUT_TANH, h->xs2 + 9, 11);
-    chain_set(a, 1, h->xs, critic, dc, h->c_h1, h->c_h2, TC_OUT_ID, h->q, 1);
-    chain_set(a, 2, h->xs, actor, da, h->a_h1, h->a_h2, TC_OUT_TANH, h->xspi + 9, 11);
-    // Programmatic dependent launches (the tcgen05 kernels only: their set-up is worth hiding, and a CTA of theirs fills an SM, so
-    // a grid scheduled early takes nothing from the side branch.  The thin kernels as dependents were measured and dropped: their
-    // early-resident blocks starve the side branch, 209 -> 226 us).  After the gather only the rows' inputs are its output:
-    a.pdl = 1; a.early_weights = 1;
-    TRY(tc_fwd_chain(st, a));
-    // q' = critic_target(vcat(s'_n, a'));  y = r + gamma (1 - done) q';  dq = 2 (q - y) / B     (:132-133)
-    TcFwdChainArgs t = chain_args(h, 1);
-    chain_set(t, 0, h->xs2, critic_t, dc, nullptr, nullptr, TC_OUT_TD, h->y, 1);
-    t.td_r = h->r; t.td_done = h->done; t.td_q = h->q; t.td_dq = h->dq; t.inv_batch = 1.0f / (float)B;
-    t.td_gamma = &h->ctrl->hp.gamma; t.td_gamma_stride = sizeof(DdpgCtrl) / sizeof(float);
-    t.pdl = 1; t.early_weights = 1;   // after the three-net launch: a' and q are its output, critic_target's weights are not
-    TRY(tc_fwd_chain(st, t));
-  } else {
-  // P1-P3: actor_target(s'_n) | critic(s_n, a) | actor(s_n)     (DDPG.jl:131, :114, :117)
-  if (big) {
-    const float* X[3] = {h->xs2, h->xs, h->xs}; const float* nets[3] = {actor_t, critic, actor};
-    const LayerDims* Ls[3] = {&da.l[0], &dc.l[0], &da.l[0]}; float* Y[3] = {h->t_h1, h->c_h1, h->a_h1};
-    TRY(big_l1(st, 3, X, 11, B, nets, Ls, Y, l1, h->pop, h->pop_stride, h->pop_stride));
-  } else {
-    g[0] = gp_fwd(h->xs2, 11, B, actor_t, da.l[0], h->t_h1, l1, EPI_BIAS_RELU);
-    g[1] = gp_fwd(h->xs, 11, B, critic, dc.l[0], h->c_h1, l1, EPI_BIAS_RELU);
-    g[2] = gp_fwd(h->xs, 11, B, actor, da.l[0], h->a_h1, l1, EPI_BIAS_RELU);
-    TRY(launch_gemms(st, g, 3, h->pop, h->pop_stride, h->pop_stride));
-  }
-  if (tc) {  // the three layer-2 forward products have one shape: a single persistent launch deals their tiles over the SMs
-    const TcOperand As[3] = {{h->t_h1, l1, false}, {h->c_h1, l1, false}, {h->a_h1, l1, false}};
-    const TcOperand Bs[3] = {{actor_t + da.l[1].w_off, da.l[1].out, true}, {critic + dc.l[1].w_off, dc.l[1].out, true}, {actor + da.l[1].w_off, da.l[1].out, true}};
-    float* Ds[3] = {h->t_h2, h->c_h2, h->a_h2};
-    const float* bs[3] = {actor_t + da.l[1].b_off, critic + dc.l[1].b_off, actor + da.l[1].b_off};
-    TcBatch bt; bt.count = h->pop; bt.sA = bt.sB = bt.sD = bt.sBias = h->pop_stride;
-    TRY(tc_gemm_multi(st, 3, As, Bs, Ds, l2, B, da.l[1].out, da.l[1].in, TC_EPI_BIAS_RELU, bs, nullptr, 0, 1, nullptr, bt));
-  } else {
-    g[0] = gp_fwd(h->t_h1, l1, B, actor_t, da.l[1], h->t_h2, l2, EPI_BIAS_RELU);
-    g[1] = gp_fwd(h->c_h1, l1, B, critic, dc.l[1], h->c_h2, l2, EPI_BIAS_RELU);
-    g[2] = gp_fwd(h->a_h1, l1, B, actor, da.l[1], h->a_h2, l2, EPI_BIAS_RELU);
-    TRY(launch_gemms(st, g, 3, h->pop, h->pop_stride, h->pop_stride));
-  }
-  g[0] = gp_fwd(h->t_h2, l2, B, actor_t, da.l[2], h->xs2 + 9, 11, EPI_BIAS_TANH);   // a' -> vcat(s'_n, a')
-  g[1] = gp_fwd(h->c_h2, l2, B, critic, dc.l[2], h->q, 1, EPI_BIAS_ID);
-  g[2] = gp_fwd(h->a_h2, l2, B, actor, da.l[2], h->xspi + 9, 11, EPI_BIAS_TANH);    // actor(s_n) -> vcat(s_n, actions)
-  TRY(launch_gemms(st, g, 3, h->pop, h->pop_stride, h->pop_stride));
+  // P1-P3: actor_target(s'_n) -> a' | critic(s_n, a) -> q | actor(s_n) -> vcat(s_n, actions)      (DDPG.jl:131, :114, :117)
+  // Programmatic dependent launches (the tcgen05 kernels only: their set-up is worth hiding, and a CTA of theirs fills an SM, so
+  // a grid scheduled early takes nothing from the side branch.  The thin kernels as dependents were measured and dropped: their
+  // early-resident blocks starve the side branch, 209 -> 226 us).  After the gather only the rows' inputs are its output.
+  const FwdNet fwd[3] = {{h->xs2, actor_t, &da, h->t_h1, h->t_h2, false, TC_OUT_TANH, h->xs2 + 9, 11},
+                         {h->xs, critic, &dc, h->c_h1, h->c_h2, true, TC_OUT_ID, h->q, 1},
+                         {h->xs, actor, &da, h->a_h1, h->a_h2, true, TC_OUT_TANH, h->xspi + 9, 11}};
+  TRY(enqueue_forward(h, st, rg, fwd, 3, 11, B, h->pop_stride, 1, 1));
   // P4-P6: q' = critic_target(vcat(s'_n, a'));  y = r + γ(1-done) q';  dq = 2(q-y)/B     (:132-133)
-  if (big) {
-    const float* X[1] = {h->xs2}; const float* nets[1] = {critic_t}; const LayerDims* Ls[1] = {&dc.l[0]}; float* Y[1] = {h->tc_h1};
-    TRY(big_l1(st, 1, X, 11, B, nets, Ls, Y, l1, h->pop, h->pop_stride, h->pop_stride));
-  } else {
-    g[0] = gp_fwd(h->xs2, 11, B, critic_t, dc.l[0], h->tc_h1, l1, EPI_BIAS_RELU);
-    TRY(launch_gemms(st, g, 1, h->pop, h->pop_stride, h->pop_stride));
-  }
-  if (tc) TRY(tc_fwd(h, st, h->tc_h1, l1, B, critic_t, dc.l[1], h->tc_h2, l2, h->pop_stride));
-  else {
-    g[0] = gp_fwd(h->tc_h1, l1, B, critic_t, dc.l[1], h->tc_h2, l2, EPI_BIAS_RELU);
-    TRY(launch_gemms(st, g, 1, h->pop, h->pop_stride, h->pop_stride));
-  }
-  g[0] = gp_fwd(h->tc_h2, l2, B, critic_t, dc.l[2], h->y, 1, EPI_TD_TARGET);
-  g[0].aux = h->r; g[0].aux2 = h->done; g[0].aux3 = h->q; g[0].out2 = h->dq; g[0].ctrl = h->ctrl; g[0].inv_batch = 1.0f / (float)B;
-  TRY(launch_gemms(st, g, 1, h->pop, h->pop_stride, h->pop_stride));
-  }
+  // (after the three-net launch: a' and q are its output, critic_target's weights are not)
+  const FwdNet td = {h->xs2, critic_t, &dc, h->tc_h1, h->tc_h2, false, TC_OUT_TD, h->y, 1};
+  TRY(enqueue_forward(h, st, rg, &td, 1, 11, B, h->pop_stride, 1, 1));
   // P7-P9: critic backward (:137, :105-108)
-  if (big) {
-    // the dX chain (dz2 -> dz1 -> dW1) is the critical path; dW3, dW2 and their bias sums run beside it on the side stream
-    TRY(side_after(h, st, h->ev_fork));                                                                       // dq, c_h2 are ready
-    TRY(out_bwd_dw(h, h->side, h->c_h2, l2, h->dq, 1, B, dc.l[2], h->grad[1], true));
-    TRY(launch_outer_mask(h, st, h->dq, 1, critic + dc.l[2].w_off, h->c_h2, l2, B, p.l2, h->dz2));
-    TRY(side_after(h, st, h->ev_mid));                                                                        // dz2 is ready
-    if (tc) {
-      TRY(tc_dw(h, h->side, h->c_h1, l1, h->dz2, l2, B, dc.l[1], h->grad[1], true));
-      TRY(tc_dx(h, st, h->dz2, l2, B, critic, dc.l[1], h->dz1, l1, h->c_h1, l1));
-    } else {
-      g[0] = gp_dw(h->c_h1, l1, h->dz2, l2, B, dc.l[1], h->grad[1]);
-      g[1] = gp_dx(h->dz2, l2, B, critic, dc.l[1], 0, p.l1, h->dz1, l1, EPI_RELU_MASK, h->c_h1, l1);
-      TRY(launch_dw(h, h->side, g[0], true));
-      TRY(launch_gemms(st, g + 1, 1, h->pop, h->pop_stride, h->pop_stride));
-    }
-    g[0] = gp_dw(h->xs, 11, h->dz1, l1, B, dc.l[0], h->grad[1]);
-    TRY(launch_dw(h, st, g[0]));
-    TRY(side_join(h, st));
-    return SHEMS_OK;
-  }
-  g[0] = gp_dw(h->c_h2, l2, h->dq, 1, B, dc.l[2], h->grad[1]);
-  g[1] = gp_dx(h->dq, 1, B, critic, dc.l[2], 0, p.l2, h->dz2, l2, EPI_RELU_MASK, h->c_h2, l2);
-  TRY(launch_gemms(st, g, 2, h->pop, h->pop_stride, h->pop_stride));
-  g[0] = gp_dw(h->c_h1, l1, h->dz2, l2, B, dc.l[1], h->grad[1]);
-  g[1] = gp_dx(h->dz2, l2, B, critic, dc.l[1], 0, p.l1, h->dz1, l1, EPI_RELU_MASK, h->c_h1, l1);
-  TRY(launch_gemms(st, g, 2, h->pop, h->pop_stride, h->pop_stride));
-  g[0] = gp_dw(h->xs, 11, h->dz1, l1, B, dc.l[0], h->grad[1]);
-  TRY(launch_dw(h, st, g[0]));
-  return SHEMS_OK;
+  return enqueue_backward(h, st, rg, critic, dc, h->c_h1, h->c_h2, h->dq, h->dz2, h->dz1, h->grad[1]);
 }
 
 static int enqueue_phase1(Ddpg* h, cudaStream_t st, float gscale, bool dp = false) {
+  const Regime rg = update_regime(h);
   const DdpgParams& p = h->p;
   const int B = p.batch, l1 = h->ld1, l2 = h->ld2;
-  const bool tc = use_tc(h, B), big = tc || B >= SPLITK_MIN_BATCH || h->pop > 1;  // streaming kernels for the thin products
   const NetDims& da = h->dims[0]; const NetDims& dc = h->dims[1];
   float *actor = h->net[DDPG_NET_ACTOR], *critic = h->net[DDPG_NET_CRITIC];
-  GemmProblem g[4];
   // the fused dX chain through the critic below: with few row tiles two CTAs share a tile and ADD their shares of the action-input gradient
-  const int bwd_split = (tc && h->chain && h->pop == 1 && ((B + 127) / 128) * 2 <= 148) ? 2 : 1;
+  const int bwd_split = (rg.chain && h->pop == 1 && ((B + 127) / 128) * 2 <= 148) ? 2 : 1;
   if (bwd_split == 2) CUDA_TRY(cudaMemsetAsync(h->dza3, 0, sizeof(float) * 2 * (size_t)B, st));
   // P10: ADAM(η_crit) on the critic
-  const dim3 adam_grid((unsigned)((dc.n_params + 255) / 256), h->pop);  // one element per thread: the Float64 div/sqrt chains need TLP
-  if (dp) {  // gradient exchange over NVLink fused into the optimiser step (critic segment = first nc floats of the flat buffer)
-    TRY(launch_adam_dp(st, h->dp, 0, nullptr, 0, 0, h->grad[1], critic, h->adam_m[1], h->adam_v[1], dc.n_params, p.adam_beta1, p.adam_beta2, p.adam_eps,
-                       h->ctrl, 0, nullptr, nullptr, nullptr, 0, 0));
-  } else if (h->tc)
-    adam_polyak_kernel<true><<<dim3((adam_grid.x + 3) / 4, h->pop), 256, 0, st>>>(critic, h->grad[1], h->adam_m[1], h->adam_v[1], dc.n_params, p.adam_beta1, p.adam_beta2,
-                                                       p.adam_eps, h->ctrl, 0, nullptr, nullptr, nullptr, 0, 0, gscale, h->pop_stride);
-  else
-    adam_polyak_kernel<false><<<adam_grid, 256, 0, st>>>(critic, h->grad[1], h->adam_m[1], h->adam_v[1], dc.n_params, p.adam_beta1, p.adam_beta2,
-                                                        p.adam_eps, h->ctrl, 0, nullptr, nullptr, nullptr, 0, 0, gscale, h->pop_stride);
-  CUDA_TRY(cudaGetLastError());
-  // P11-P13: critic(vcat(s_n, actor(s_n))) with the UPDATED critic (:116-119); loss_act = -mean(q) => dq = -1/B
-  const bool chain = tc && h->chain;
-  if (chain) {  // one kernel: p_h1, p_h2 (for the backward pass) and q(s, actor(s)) itself (reporting)
-    TcFwdChainArgs a = chain_args(h, 1);
-    chain_set(a, 0, h->xspi, critic, dc, h->p_h1, h->p_h2, TC_OUT_ID, h->qpi, 1);
-    a.pdl = 1; a.early_weights = 0;   // after ADAM(critic): the weights are the predecessor's output
-    TRY(tc_fwd_chain(st, a));
-  } else if (big) {
-    const float* X[1] = {h->xspi}; const float* nets[1] = {critic}; const LayerDims* Ls[1] = {&dc.l[0]}; float* Y[1] = {h->p_h1};
-    TRY(big_l1(st, 1, X, 11, B, nets, Ls, Y, l1, h->pop, h->pop_stride, h->pop_stride));
-  } else {
-    g[0] = gp_fwd(h->xspi, 11, B, critic, dc.l[0], h->p_h1, l1, EPI_BIAS_RELU);
-    TRY(launch_gemms(st, g, 1, h->pop, h->pop_stride, h->pop_stride));
-  }
-  if (chain) { }
-  else if (tc) TRY(tc_fwd(h, st, h->p_h1, l1, B, critic, dc.l[1], h->p_h2, l2, h->pop_stride));
-  else {
-    g[0] = gp_fwd(h->p_h1, l1, B, critic, dc.l[1], h->p_h2, l2, EPI_BIAS_RELU);
-    TRY(launch_gemms(st, g, 1, h->pop, h->pop_stride, h->pop_stride));
-  }
-  if (chain) {
+  TRY(enqueue_adam(h, st, 0, gscale, dp, false));
+  // P11-P13: critic(vcat(s_n, actor(s_n))) with the UPDATED critic (:116-119); loss_act = -mean(q) => dq = -1/B.  The chain kernel
+  // also yields q(s, actor(s)) itself (reporting); layer by layer, that product is left for the actor's backward pass below
+  // (chain: after ADAM(critic), the weights are the predecessor's output)
+  const FwdNet fwd = {h->xspi, critic, &dc, h->p_h1, h->p_h2, true, TC_OUT_ID, h->qpi, 1};
+  TRY(enqueue_forward(h, st, rg, &fwd, 1, 11, B, h->pop_stride, 1, 0, true));
+  GemmProblem g;
+  if (rg.chain) {
     // dX through the critic only, as ONE kernel (csrc/tc_gemm.cu tc_bwd_chain_kernel): dq -> dz2 -> dz1 -> the action inputs, times tanh';
     // nothing of it is kept (no weight gradient of the critic in the actor's loss)
     TcBwdChainArgs b; memset(&b, 0, sizeof(b));
@@ -1630,127 +1648,57 @@ static int enqueue_phase1(Ddpg* h, cudaStream_t st, float gscale, bool dp = fals
     b.pop = h->pop; b.pop_stride = h->pop_stride;
     TRY(tc_bwd_chain(st, b));
   } else {
-    if (big) {                                                                                               // dX through the critic only
+    if (rg.big) {                                                                                            // dX through the critic only
       TRY(launch_outer_mask(h, st, h->dqpi, 1, critic + dc.l[2].w_off, h->p_h2, l2, B, p.l2, h->dzp2));
     } else {
-      g[0] = gp_dx(h->dqpi, 1, B, critic, dc.l[2], 0, p.l2, h->dzp2, l2, EPI_RELU_MASK, h->p_h2, l2);
-      TRY(launch_gemms(st, g, 1, h->pop, h->pop_stride, h->pop_stride));
+      g = gp_dx(h->dqpi, 1, B, critic, dc.l[2], 0, p.l2, h->dzp2, l2, EPI_RELU_MASK, h->p_h2, l2);
+      TRY(slab_gemms(h, st, &g, 1));
     }
     // P14-P15: back through critic layers 2, 1 down to the action inputs, times tanh'
-    if (tc) TRY(tc_dx(h, st, h->dzp2, l2, B, critic, dc.l[1], h->dzp1, l1, h->p_h1, l1));
+    if (rg.tc) TRY(tc_dx(h, st, h->dzp2, l2, B, critic, dc.l[1], h->dzp1, l1, h->p_h1, l1));
     else {
-      g[0] = gp_dx(h->dzp2, l2, B, critic, dc.l[1], 0, p.l1, h->dzp1, l1, EPI_RELU_MASK, h->p_h1, l1);
-      TRY(launch_gemms(st, g, 1, h->pop, h->pop_stride, h->pop_stride));
+      g = gp_dx(h->dzp2, l2, B, critic, dc.l[1], 0, p.l1, h->dzp1, l1, EPI_RELU_MASK, h->p_h1, l1);
+      TRY(slab_gemms(h, st, &g, 1));
     }
-    g[0] = gp_dx(h->dzp1, l1, B, critic, dc.l[0], 9, 2, h->dza3, 2, EPI_TANH_GRAD, h->xspi + 9, 11);
-    TRY(launch_gemms(st, g, 1, h->pop, h->pop_stride, h->pop_stride));
+    g = gp_dx(h->dzp1, l1, B, critic, dc.l[0], 9, 2, h->dza3, 2, EPI_TANH_GRAD, h->xspi + 9, 11);
+    TRY(slab_gemms(h, st, &g, 1));
   }
-  // P16-P18: actor backward
-  if (big) {  // as in the critic's backward pass: dW3, dW2 (and the reporting-only q(s, actor(s))) beside the dX chain
-    TRY(side_after(h, st, h->ev_fork));                                                                       // dza3 is ready
-    TRY(out_bwd_dw(h, h->side, h->a_h2, l2, h->dza3, 2, B, da.l[2], h->grad[0], true));
-    if (!chain) {
-      g[0] = gp_fwd(h->p_h2, l2, B, critic, dc.l[2], h->qpi, 1, EPI_BIAS_ID);
-      TRY(launch_gemms(h->side, g, 1, h->pop, h->pop_stride, h->pop_stride));
-    }
-    TRY(launch_outer_mask(h, st, h->dza3, 2, actor + da.l[2].w_off, h->a_h2, l2, B, p.l2, h->dza2));
-    TRY(side_after(h, st, h->ev_mid));                                                                        // dza2 is ready
-    if (tc) {
-      TRY(tc_dw(h, h->side, h->a_h1, l1, h->dza2, l2, B, da.l[1], h->grad[0], true));
-      TRY(tc_dx(h, st, h->dza2, l2, B, actor, da.l[1], h->dza1, l1, h->a_h1, l1));
-    } else {
-      g[0] = gp_dw(h->a_h1, l1, h->dza2, l2, B, da.l[1], h->grad[0]);
-      g[1] = gp_dx(h->dza2, l2, B, actor, da.l[1], 0, p.l1, h->dza1, l1, EPI_RELU_MASK, h->a_h1, l1);
-      TRY(launch_dw(h, h->side, g[0], true));
-      TRY(launch_gemms(st, g + 1, 1, h->pop, h->pop_stride, h->pop_stride));
-    }
-    g[0] = gp_dw(h->xs, 11, h->dza1, l1, B, da.l[0], h->grad[0]);
-    g[0].M = 9;  // only the 9 state columns of xs feed the actor
-    TRY(launch_dw(h, st, g[0]));
-    TRY(side_join(h, st));
-    return SHEMS_OK;
-  }
-  g[0] = gp_dw(h->a_h2, l2, h->dza3, 2, B, da.l[2], h->grad[0]);
-  g[1] = gp_dx(h->dza3, 2, B, actor, da.l[2], 0, p.l2, h->dza2, l2, EPI_RELU_MASK, h->a_h2, l2);
-  TRY(launch_gemms(st, g, 2, h->pop, h->pop_stride, h->pop_stride));
-  g[0] = gp_dw(h->a_h1, l1, h->dza2, l2, B, da.l[1], h->grad[0]);
-  g[1] = gp_dx(h->dza2, l2, B, actor, da.l[1], 0, p.l1, h->dza1, l1, EPI_RELU_MASK, h->a_h1, l1);
-  TRY(launch_gemms(st, g, 2, h->pop, h->pop_stride, h->pop_stride));
-  g[0] = gp_dw(h->xs, 11, h->dza1, l1, B, da.l[0], h->grad[0]);
-  g[0].M = 9;  // only the 9 state columns of xs feed the actor
-  TRY(launch_dw(h, st, g[0]));
-  // q(s, actor(s)) itself only feeds loss_act (reporting): off the critical path, skinny kernel
-  g[0] = gp_fwd(h->p_h2, l2, B, critic, dc.l[2], h->qpi, 1, EPI_BIAS_ID);
-  TRY(launch_gemms(st, g, 1, h->pop, h->pop_stride, h->pop_stride));
-  return SHEMS_OK;
+  // P16-P18: actor backward, with q(s, actor(s)) beside it when the chain kernel has not produced it
+  const GemmProblem qpi = gp_fwd(h->p_h2, l2, B, critic, dc.l[2], h->qpi, 1, EPI_BIAS_ID);
+  return enqueue_backward(h, st, rg, actor, da, h->a_h1, h->a_h2, h->dza3, h->dza2, h->dza1, h->grad[0], rg.chain ? nullptr : &qpi);
 }
 
 static int enqueue_phase2(Ddpg* h, cudaStream_t st, float gscale, bool dp = false) {
-  const DdpgParams& p = h->p;
-  const NetDims& da = h->dims[0]; const NetDims& dc = h->dims[1];
-  float *actor = h->net[DDPG_NET_ACTOR], *critic = h->net[DDPG_NET_CRITIC], *actor_t = h->net[DDPG_NET_ACTOR_TARGET], *critic_t = h->net[DDPG_NET_CRITIC_TARGET];
-  const dim3 adam_grid((unsigned)((dc.n_params + 255) / 256), h->pop);
   // P19: ADAM(η_act) on the actor + soft_update! of both targets (:140-143)
-  if (dp) {
-    TRY(launch_adam_dp(st, h->dp, h->grad[0] - h->gradbuf, nullptr, 0, 0, h->grad[0], actor, h->adam_m[0], h->adam_v[0], da.n_params, p.adam_beta1,
-                       p.adam_beta2, p.adam_eps, h->ctrl, 1, actor_t, critic_t, critic, dc.n_params, 1));
-  } else if (h->tc)
-    adam_polyak_kernel<true><<<dim3((adam_grid.x + 3) / 4, h->pop), 256, 0, st>>>(actor, h->grad[0], h->adam_m[0], h->adam_v[0], da.n_params, p.adam_beta1, p.adam_beta2,
-                                                       p.adam_eps, h->ctrl, 1, actor_t, critic_t, critic, dc.n_params, 1, gscale, h->pop_stride);
-  else
-    adam_polyak_kernel<false><<<adam_grid, 256, 0, st>>>(actor, h->grad[0], h->adam_m[0], h->adam_v[0], da.n_params, p.adam_beta1, p.adam_beta2,
-                                                        p.adam_eps, h->ctrl, 1, actor_t, critic_t, critic, dc.n_params, 1, gscale, h->pop_stride);
-  CUDA_TRY(cudaGetLastError());
-  return SHEMS_OK;
+  return enqueue_adam(h, st, 1, gscale, dp, false);
 }
 
 // One learner at a small batch: critic pass -> ADAM(critic) -> actor pass -> ADAM(actor) + soft_update!, the two passes as
 // thread-block-cluster kernels that keep a row's whole forward/backward chain on chip (csrc/ddpg_fused.cu)
 static inline bool use_fused(const Ddpg* h) { return h->fused && h->parts[0] && h->parts[1]; }
+static inline FusedNetOff fused_off(const NetDims& d) {
+  return FusedNetOff{(int)d.l[0].w_off, (int)d.l[0].b_off, (int)d.l[1].w_off, (int)d.l[1].b_off, (int)d.l[2].w_off, (int)d.l[2].b_off};
+}
 struct GatherSrc { bool from_rings; const float *s, *a, *r, *s2, *done; long long ld; };
 static int enqueue_update_fused(Ddpg* h, cudaStream_t st, bool dp, const GatherSrc& src) {
   const DdpgParams& p = h->p;
-  const NetDims& da = h->dims[0]; const NetDims& dc = h->dims[1];
-  float *actor = h->net[DDPG_NET_ACTOR], *critic = h->net[DDPG_NET_CRITIC], *actor_t = h->net[DDPG_NET_ACTOR_TARGET], *critic_t = h->net[DDPG_NET_CRITIC_TARGET];
   FusedArgs a; memset(&a, 0, sizeof(a));
-  a.actor = actor; a.critic = critic; a.actor_t = actor_t; a.critic_t = critic_t;
-  a.ao = FusedNetOff{(int)da.l[0].w_off, (int)da.l[0].b_off, (int)da.l[1].w_off, (int)da.l[1].b_off, (int)da.l[2].w_off, (int)da.l[2].b_off};
-  a.co = FusedNetOff{(int)dc.l[0].w_off, (int)dc.l[0].b_off, (int)dc.l[1].w_off, (int)dc.l[1].b_off, (int)dc.l[2].w_off, (int)dc.l[2].b_off};
+  a.actor = h->net[DDPG_NET_ACTOR]; a.critic = h->net[DDPG_NET_CRITIC]; a.actor_t = h->net[DDPG_NET_ACTOR_TARGET]; a.critic_t = h->net[DDPG_NET_CRITIC_TARGET];
+  a.ao = fused_off(h->dims[0]); a.co = fused_off(h->dims[1]);
   a.l1 = p.l1; a.l2 = p.l2; a.B = p.batch;
   a.xs = h->xs; a.xs2 = h->xs2; a.xspi = h->xspi; a.r = h->r; a.done = h->done; a.q = h->q; a.y = h->y; a.qpi = h->qpi;
   a.inv_batch = 1.0f / (float)p.batch;
   a.rings = src.from_rings ? h->rings_dev : nullptr;
   a.src_s = src.s; a.src_a = src.a; a.src_r = src.r; a.src_s2 = src.s2; a.src_d = src.done; a.src_ld = src.ld;
   a.ctrl = h->ctrl; a.idx = h->idx_dev; a.norm = h->norm; a.xs_w = h->xs;
-  // every slab buffer starts on a 256-byte boundary: W2 rows are 16-byte aligned iff l2 and both W2 offsets are multiples of 4 floats
-  a.vec16 = (p.l2 % 4 == 0 && da.l[1].w_off % 4 == 0 && dc.l[1].w_off % 4 == 0) ? 1 : 0;
-  const int nparts = p.batch / FUSED_ROWS;
-#ifndef ADAM_PARTS_THREADS
-#define ADAM_PARTS_THREADS 256
-#endif
-  const unsigned ap_blocks = (unsigned)((dc.n_params + ADAM_PARTS_THREADS - 1) / ADAM_PARTS_THREADS);   // one element per thread
-  a.part = h->parts[1]; a.part_stride = dc.n_params;
+  a.vec16 = w2_vec16(h) ? 1 : 0;
+  // each pass is followed by the reduction of its partial sums and the optimiser step (dp: with the gradient exchange) in ONE kernel
+  a.part = h->parts[1]; a.part_stride = h->dims[1].n_params;
   TRY(ddpg_fused_critic(st, a));
-  if (dp) {  // partial-sum reduction, gradient exchange over NVLink and the optimiser step in ONE kernel
-    TRY(launch_adam_dp(st, h->dp, 0, h->parts[1], nparts, dc.n_params, h->grad[1], critic, h->adam_m[1], h->adam_v[1], dc.n_params, p.adam_beta1,
-                       p.adam_beta2, p.adam_eps, h->ctrl, 0, nullptr, nullptr, nullptr, 0, 0));
-  } else {
-    adam_polyak_parts_kernel<<<ap_blocks, ADAM_PARTS_THREADS, 0, st>>>(critic, h->parts[1], nparts, dc.n_params, h->grad[1], h->adam_m[1], h->adam_v[1], dc.n_params,
-                                                           p.adam_beta1, p.adam_beta2, p.adam_eps, h->ctrl, 0, nullptr, nullptr, nullptr, 0, 0);
-  }
-  CUDA_TRY(cudaGetLastError());
-  a.part = h->parts[0]; a.part_stride = da.n_params;
+  TRY(enqueue_adam(h, st, 0, 1.0f, dp, true));
+  a.part = h->parts[0]; a.part_stride = h->dims[0].n_params;
   TRY(ddpg_fused_actor(st, a));
-  if (dp) {
-    TRY(launch_adam_dp(st, h->dp, h->grad[0] - h->gradbuf, h->parts[0], nparts, da.n_params, h->grad[0], actor, h->adam_m[0], h->adam_v[0], da.n_params,
-                       p.adam_beta1, p.adam_beta2, p.adam_eps, h->ctrl, 1, actor_t, critic_t, critic, dc.n_params, 1));
-  } else {
-    adam_polyak_parts_kernel<<<ap_blocks, ADAM_PARTS_THREADS, 0, st>>>(actor, h->parts[0], nparts, da.n_params, h->grad[0], h->adam_m[0], h->adam_v[0], da.n_params,
-                                                           p.adam_beta1, p.adam_beta2, p.adam_eps, h->ctrl, 1, actor_t, critic_t, critic,
-                                                           dc.n_params, 1);
-  }
-  CUDA_TRY(cudaGetLastError());
-  return SHEMS_OK;
+  return enqueue_adam(h, st, 1, 1.0f, dp, true);
 }
 
 static int enqueue_update_body(Ddpg* h, cudaStream_t st, bool dp = false) {
@@ -2124,12 +2072,11 @@ ddpg_act_ou_epilogue_kernel(const float* __restrict__ y /*[n][2]*/, long long n,
 // act() on a handful of states of one learner runs as one cluster kernel (csrc/ddpg_fused.cu)
 static inline bool fused_act_ok(const Ddpg* h, int64_t n) { return use_fused(h) && h->pop == 1 && n <= FUSED_ACT_MAX_ROWS; }
 static FusedActArgs fused_act_args(const Ddpg* h, const float* obs_dev, int64_t n, long long osk) {
-  const NetDims& dA = h->dims[0]; const NetDims& dC = h->dims[1];
   FusedActArgs a; memset(&a, 0, sizeof(a));
   a.actor = h->net[DDPG_NET_ACTOR];
-  a.ao = FusedNetOff{(int)dA.l[0].w_off, (int)dA.l[0].b_off, (int)dA.l[1].w_off, (int)dA.l[1].b_off, (int)dA.l[2].w_off, (int)dA.l[2].b_off};
+  a.ao = fused_off(h->dims[0]);
   a.l1 = h->p.l1; a.l2 = h->p.l2;
-  a.vec16 = (h->p.l2 % 4 == 0 && dA.l[1].w_off % 4 == 0 && dC.l[1].w_off % 4 == 0) ? 1 : 0;
+  a.vec16 = w2_vec16(h) ? 1 : 0;
   a.n = n; a.obs = obs_dev; a.osk = osk; a.norm = h->norm; a.y = h->act_y;
   return a;
 }
@@ -2152,24 +2099,9 @@ static int act_forward(Ddpg* h, const float* obs_dev, int64_t n, long long osl, 
   const dim3 gn((unsigned)((n + 255) / 256), pop);
   ddpg_normalize_kernel<<<gn, 256, 0, h->stream>>>(obs_dev, n, h->norm, h->act_x, h->pop_stride, h->act_stride, osl, osk);
   CUDA_TRY(cudaGetLastError());
-  const NetDims& da = h->dims[0];
-  const float* actor = h->net[DDPG_NET_ACTOR];
-  GemmProblem g[1];
-  if (n * pop >= SPLITK_MIN_BATCH) {
-    const float* X[1] = {h->act_x}; const float* nets[1] = {actor}; const LayerDims* Ls[1] = {&da.l[0]}; float* Y[1] = {h->act_h1};
-    TRY(big_l1(h->stream, 1, X, 9, (int)n, nets, Ls, Y, l1, pop, h->pop_stride, h->act_stride));
-  } else {
-    g[0] = gp_fwd(h->act_x, 9, (int)n, actor, da.l[0], h->act_h1, l1, EPI_BIAS_RELU);
-    TRY(launch_gemms(h->stream, g, 1, pop, h->pop_stride, h->act_stride));
-  }
-  if (use_tc(h, n)) TRY(tc_fwd(h, h->stream, h->act_h1, l1, (int)n, actor, da.l[1], h->act_h2, l2, h->act_stride));
-  else {
-    g[0] = gp_fwd(h->act_h1, l1, (int)n, actor, da.l[1], h->act_h2, l2, EPI_BIAS_RELU);
-    TRY(launch_gemms(h->stream, g, 1, pop, h->pop_stride, h->act_stride));
-  }
-  g[0] = gp_fwd(h->act_h2, l2, (int)n, actor, da.l[2], h->act_y, 2, EPI_BIAS_TANH);
-  TRY(launch_gemms(h->stream, g, 1, pop, h->pop_stride, h->act_stride));
-  return SHEMS_OK;
+  const Regime rg{false, use_tc(h, n), n * pop >= SPLITK_MIN_BATCH};
+  const FwdNet fwd = {h->act_x, h->net[DDPG_NET_ACTOR], &h->dims[0], h->act_h1, h->act_h2, false, TC_OUT_TANH, h->act_y, 2};
+  return enqueue_forward(h, h->stream, rg, &fwd, 1, 9, (int)n, h->act_stride);
 }
 
 // sprev_dev (optional, [9][N]): receives a copy of the raw states — the episode loop's s for `remember`
@@ -2361,13 +2293,12 @@ extern "C" int32_t ddpg_episode(Ddpg* h, ShemsEnv* env, ShemsReplay* const* rps,
 // checked lie inside one group.
 static int rollout_launch(Ddpg* h, ShemsEnv* env, const float* actor, long long actor_stride, int32_t n_steps, float sigma, uint64_t seed,
                           int64_t env_id_base, double* ep_return_dev, double* trace_dev, float* act_traj_dev) {
-  const NetDims& dA = h->dims[0]; const NetDims& dC = h->dims[1];
   const long long N = env->n, n = N / h->pop;
   ActorRolloutArgs a; memset(&a, 0, sizeof(a));
   a.actor = actor;
-  a.ao = FusedNetOff{(int)dA.l[0].w_off, (int)dA.l[0].b_off, (int)dA.l[1].w_off, (int)dA.l[1].b_off, (int)dA.l[2].w_off, (int)dA.l[2].b_off};
+  a.ao = fused_off(h->dims[0]);
   a.l1 = h->p.l1; a.l2 = h->p.l2;
-  a.vec16 = (h->p.l2 % 4 == 0 && dA.l[1].w_off % 4 == 0 && dC.l[1].w_off % 4 == 0) ? 1 : 0;
+  a.vec16 = w2_vec16(h) ? 1 : 0;
   a.norm = h->norm; a.actor_stride = actor_stride; a.norm_stride = h->pop_stride;
   a.N = N; a.obs = env->obs; a.idx = env->idx; a.T = n_steps; a.step0 = env->step;
   a.sigma = sigma * h->hp[0].noise_scale; a.seed = seed; a.env_id_base = env_id_base;
