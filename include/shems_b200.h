@@ -49,6 +49,8 @@ SHEMS_API const char* shems_last_error(void);
 SHEMS_API int32_t shems_version(void);
 /* environment kernels (reset / step / action / rollout) this process has launched so far — a real counter for benchmarks' launch counts */
 SHEMS_API int64_t shems_env_kernel_launches(void);
+/* of those, rollouts that ran two instances per thread (all instances on one row; see DESIGN.md, rollout) */
+SHEMS_API int64_t shems_rollout_pair_launches(void);
 /* number of visible CUDA devices (0 on a CPU-only box; never an error) */
 SHEMS_API int32_t shems_device_count(void);
 

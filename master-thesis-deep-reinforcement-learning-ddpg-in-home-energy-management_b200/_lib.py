@@ -77,6 +77,7 @@ SIGNATURES = {
     "shems_version": (I32, []),
     "shems_device_count": (I32, []),
     "shems_env_kernel_launches": (I64, []),
+    "shems_rollout_pair_launches": (I64, []),
     "shems_params_for_charger": (I32, [I32, C.POINTER(ShemsParams)]),
     "shems_params_for_env": (I32, [I32, I32, C.POINTER(ShemsParams)]),
     "shems_series_from_csv": (I32, [C.c_char_p, PF, I32, PI]),

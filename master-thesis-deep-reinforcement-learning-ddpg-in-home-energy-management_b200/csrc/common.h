@@ -112,6 +112,8 @@ struct ShemsEnv {
   unsigned long long serial;  // unique per env handle of the process (keys the replay rings' series tables)
   bool was_reset;
   bool consistent;    // state fields 2..8 equal series row idx (false after shems_set_state)
+  bool uniform_row;   // every instance stands on the same row (steps keep it: each instance advances one row per step); like
+                      // `consistent`, writes through shems_state_ptr must keep it true
   int32_t* scratch_i; float* scratch_f; // staging for reset host draws
   // groups of instances with their own constants (several chargers in one handle): group g = instances gstart[g] .. gstart[g+1]-1
   int n_groups;

@@ -452,6 +452,8 @@ shems_rollout_kernel(DevParams P, const float4* __restrict__ series, long long N
 // serve the odd one.  Two steps per iteration with every body inlined twice was measured faster in lock step but slower on the
 // two-step loop (profiles/r6_lockstep_rollout.md).  Any other warp runs the two-step loop with the general body only.  Each lane
 // takes its own row's class, so the bits never depend on the vote: it only decides the speed.
+// When the host knows that every instance of the launch stands on one row (ShemsEnv::uniform_row) and the grid is large enough,
+// shems_rollout_pair_kernel below runs this lock-step loop with two instances per thread instead (profiles/r10_pair_rollout.md).
 template <int CLS> struct RowTag { static constexpr int value = CLS; };
 template <int POLICY, int MINB>
 __global__ void __launch_bounds__(ROLLOUT_THREADS, MINB)
@@ -542,6 +544,106 @@ shems_rollout_lean_kernel(DevParams P, const float4* __restrict__ series, long l
   if (S.ep_return) S.ep_return[n] = ret;
 }
 
+// The lock-step loop of shems_rollout_lean_kernel with two instances per thread, for launches in which every instance stands on the
+// same row (ShemsEnv::uniform_row, so no vote and no other loop).  Thread k carries instances n0 + 2k and n0 + 2k + 1: the row class
+// and its dispatch, the next row's load, the terms of the step that depend on the row only (both instances' bodies sit in one class
+// body, so the compiler computes those once), the loop control and the ring walk are paid once for two instances.  Each instance keeps
+// its own Soc_b, Soc_ev, return and Philox stream (id = env_id_base + its index).  With a ring, head + n0 is even, so the two records
+// sit in adjacent slots of one tile and each field of both is one 8-byte store.  Every output bit equals shems_rollout_lean_kernel's.
+template <int POLICY, int MINB>
+__global__ void __launch_bounds__(ROLLOUT_THREADS, MINB)
+shems_rollout_pair_kernel(DevParams P, const float4* __restrict__ series, long long N, float* __restrict__ obs,
+                          int32_t* __restrict__ idx_arr, int T, int step0, PhiloxKeys K, long long env_id_base,
+                          const float* __restrict__ tape, int tape_unscaled, RolloutSinks S, long long n0, long long n1) {
+  const long long n = n0 + 2 * ((long long)blockIdx.x * blockDim.x + threadIdx.x);
+  if (n >= n1) return;  // n1 - n0 is even
+  int idx = idx_arr[n];
+  float Soc_b[2] = {obs[n], obs[n + 1]}, Soc_ev[2] = {obs[N + n], obs[N + n + 1]};
+  float c_ev, d_e, g_e, p_buy;
+  { const Row8 r = load_row(series, idx); c_ev = r.cd; d_e = r.d_e; g_e = r.g_e; p_buy = r.p_buy; }
+  double ret[2] = {0.0, 0.0};
+  RingWalk ring{};
+  if (S.ring) { long long slot = S.head + n; if (slot >= S.cap) slot -= S.cap; ring = ring_walk(S.ring, slot, N, S.cap); }
+  const uint64_t id = (uint64_t)(env_id_base + n);
+  auto step = [&](auto cls, int t, const uint32_t (&rw)[2][4]) {
+    constexpr int CLS = decltype(cls)::value;
+    const Row8 nx = load_row(series, idx + 1);
+    float a_raw0[2], a_raw1[2], r32[2], Soc_b2[2], Soc_ev2[2];
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {
+      StepIn s;
+      s.Soc_b = Soc_b[i]; s.Soc_ev = Soc_ev[i]; s.c_ev = c_ev; s.d_e = d_e; s.g_e = g_e; s.p_buy = p_buy;
+      float B, EV, Bt, EVt;
+      bool track_neg = false;
+      if (POLICY == SHEMS_POLICY_RULE) {
+        shems_action_rule<true>(P, s.Soc_b, s.Soc_ev, s.d_e, s.g_e, B, EV);
+        Bt = 0.0f; EVt = 0.0f; a_raw0[i] = B; a_raw1[i] = EV; track_neg = true;
+      } else {
+        if (POLICY == SHEMS_POLICY_RANDOM) {
+          a_raw0[i] = action_from_word(rw[i][0]);
+          a_raw1[i] = action_from_word(rw[i][1]);
+          Bt = (a_raw0[i] + 1.0f) * 0.5f;
+          EVt = (a_raw1[i] + 1.0f) * 0.5f;
+        } else {
+          Bt = tape[((size_t)t * 2 + 0) * N + n + i];
+          EVt = tape[((size_t)t * 2 + 1) * N + n + i];
+          a_raw0[i] = Bt; a_raw1[i] = EVt;
+          if (tape_unscaled) {
+            Bt = (float)(((double)a_raw0[i] + 1.0) * 0.5);
+            EVt = (float)(((double)a_raw1[i] + 1.0) * 0.5);
+          }
+        }
+        shems_action_drl<true, CLS>(P, s.Soc_b, s.Soc_ev, s.c_ev, s.d_e, s.g_e, Bt, EVt, B, EV);
+      }
+      StepTrace tr;
+      const StepOut o = shems_flows<false, true, CLS>(P, s, B, EV, EVt, track_neg, &tr);
+      Soc_ev2[i] = (nx.cd >= 0.0f && (CLS == ROW_ANY ? c_ev == -1.0f : row_noev<CLS>)) ? nx.soc_ev : o.Soc_ev;
+      Soc_b2[i] = o.Soc_b;
+      r32[i] = (float)o.reward;
+      ret[i] += o.reward;
+    }
+    if (S.ring) {
+      ring_store_compact_pair(ring.q, Soc_b, Soc_ev, a_raw0, a_raw1, r32, Soc_b2, Soc_ev2, S.src_entry, idx);
+      ring_walk_next(ring);
+    }
+    if (S.reward_traj) { S.reward_traj[(size_t)t * N + n] = r32[0]; S.reward_traj[(size_t)t * N + n + 1] = r32[1]; }
+#pragma unroll
+    for (int i = 0; i < 2; ++i) { Soc_b[i] = Soc_b2[i]; Soc_ev[i] = Soc_ev2[i]; }
+    c_ev = nx.cd; d_e = nx.d_e; g_e = nx.g_e; p_buy = nx.p_buy;
+    idx += 1;
+  };
+  uint32_t rw[2][4] = {};
+  for (int t = 0; t < T; ++t) {
+    if (POLICY == SHEMS_POLICY_RANDOM) {  // as the lean kernel's lock-step loop, once per instance
+      const unsigned st_abs = (unsigned)(step0 + t);
+      if ((st_abs & 1u) == 0u || t == 0) {
+        philox4x32_10(K, id, st_abs >> 1, STREAM_ACTION, rw[0]);
+        philox4x32_10(K, id + 1, st_abs >> 1, STREAM_ACTION, rw[1]);
+      }
+      if (st_abs & 1u) {
+#pragma unroll
+        for (int i = 0; i < 2; ++i) { rw[i][0] = rw[i][2]; rw[i][1] = rw[i][3]; }
+      }
+    }
+    switch (row_class(P, c_ev, d_e, g_e)) {
+      case ROW_A_NOEV: step(RowTag<ROW_A_NOEV>{}, t, rw); break;
+      case ROW_B_NOEV: step(RowTag<ROW_B_NOEV>{}, t, rw); break;
+      case ROW_A_EV: step(RowTag<ROW_A_EV>{}, t, rw); break;
+      case ROW_B_EV: step(RowTag<ROW_B_EV>{}, t, rw); break;
+      default: step(RowTag<ROW_ANY>{}, t, rw); break;
+    }
+  }
+  const Row8 r = load_row(series, idx);
+#pragma unroll
+  for (int i = 0; i < 2; ++i) {
+    const long long m = n + i;
+    obs[0 * N + m] = Soc_b[i]; obs[1 * N + m] = Soc_ev[i]; obs[2 * N + m] = r.cd; obs[3 * N + m] = r.d_e; obs[4 * N + m] = r.g_e;
+    obs[5 * N + m] = r.p_buy; obs[6 * N + m] = r.h_cos; obs[7 * N + m] = r.h_sin; obs[8 * N + m] = r.season;
+    idx_arr[m] = idx;
+    if (S.ep_return) S.ep_return[m] = ret[i];
+  }
+}
+
 // ----------------------------------------------------------------------------- C ABI
 static inline unsigned grid_for(long long n, int block) { return (unsigned)((n + block - 1) / block); }
 
@@ -554,18 +656,21 @@ static inline unsigned grid_for(long long n, int block) { return (unsigned)((n +
 // take 6.  The trimmed kernel (shems_rollout_lean_kernel) needs 78 registers for the random policy at MINB 6, which leaves 6 CTAs per
 // SM; at MINB 7 it fits 72 without spilling and keeps 7, so its compact launches take 7 (profiles/r5_lean_rollout.md).
 // SHEMS_ROLLOUT_MIN_BLOCKS=6|7|8 overrides.
-static int rollout_min_blocks(int device, long long n, bool compact, bool lean) {
-  static int forced = -1;
-  if (forced < 0) { const char* ev = getenv("SHEMS_ROLLOUT_MIN_BLOCKS"); forced = ev ? atoi(ev) : 0; }
-  if (forced == 6 || forced == 7 || forced == 8) return forced;
-  if (compact) return lean ? 7 : 6;
+static int sm_count(int device) {
   static int sms[64];
   if (device >= 0 && device < 64 && sms[device] == 0) {
     int v = 0;
     if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || v <= 0) { cudaGetLastError(); v = 148; }
     sms[device] = v;
   }
-  const int nsm = (device >= 0 && device < 64) ? sms[device] : 148;
+  return (device >= 0 && device < 64) ? sms[device] : 148;
+}
+static int rollout_min_blocks(int device, long long n, bool compact, bool lean) {
+  static int forced = -1;
+  if (forced < 0) { const char* ev = getenv("SHEMS_ROLLOUT_MIN_BLOCKS"); forced = ev ? atoi(ev) : 0; }
+  if (forced == 6 || forced == 7 || forced == 8) return forced;
+  if (compact) return lean ? 7 : 6;
+  const int nsm = sm_count(device);
   const double ctas = (double)((n + ROLLOUT_THREADS - 1) / ROLLOUT_THREADS);
   int best = ROLLOUT_MIN_BLOCKS; double best_cost = 1e300;
   for (int b = 6; b <= 8; ++b) {
@@ -598,6 +703,31 @@ static bool rollout_lockstep_enabled() {
   const char* ev = getenv("SHEMS_ROLLOUT_LOCKSTEP");
   return !(ev && atoi(ev) == 0);
 }
+
+// The pair kernel (shems_rollout_pair_kernel) applies to a launch the trimmed kernel would take in lock step whose instances all stand
+// on one row, with an even count and, with a ring, an even first slot.  It is taken there when its grid of half as many threads fills
+// at least ROLLOUT_PAIR_MIN_WAVES waves of ROLLOUT_PAIR_MIN_BLOCKS CTAs per SM: below that, the trimmed kernel's grid of twice the
+// warps hides the step's latencies better (profiles/r10_pair_rollout.md).  SHEMS_ROLLOUT_PAIR=0 forces the trimmed kernel and
+// SHEMS_ROLLOUT_PAIR=2 takes the pair kernel wherever it applies, whatever the grid (read at every rollout: the A/B switch, and
+// small launches for bit-equality tests).
+#ifndef ROLLOUT_PAIR_MIN_BLOCKS
+#define ROLLOUT_PAIR_MIN_BLOCKS 4
+#endif
+#ifndef ROLLOUT_PAIR_MIN_WAVES
+#define ROLLOUT_PAIR_MIN_WAVES 1
+#endif
+static int rollout_pair_mode() {
+  const char* ev = getenv("SHEMS_ROLLOUT_PAIR");
+  return ev ? atoi(ev) : 1;
+}
+static bool rollout_pair_fills(int device, long long n, int mode) {
+  if (mode == 2) return true;
+  const long long ctas = (n / 2 + ROLLOUT_THREADS - 1) / ROLLOUT_THREADS;
+  return ctas >= (long long)ROLLOUT_PAIR_MIN_WAVES * sm_count(device) * ROLLOUT_PAIR_MIN_BLOCKS;
+}
+// pair-kernel launches this process has made (tests use it to tell which kernel ran)
+static long long g_pair_launches = 0;
+extern "C" int64_t shems_rollout_pair_launches(void) { return __atomic_load_n(&g_pair_launches, __ATOMIC_RELAXED); }
 
 // Shems(maxsteps, path) for G groups of instances (group g: group_sizes[g] consecutive instances with params[g] and, when
 // series_per_group, its own series): several chargers in one handle.  Every kernel is launched once per group on its slice.
@@ -746,6 +876,13 @@ extern "C" int32_t shems_reset(ShemsEnv* e, int32_t mode, const int32_t* idx0_ho
   e->step = 0;          // :210
   e->was_reset = true;
   e->consistent = true;
+  // one row for every instance: rng = -1, a single admissible start row, or host draws that all name the same row (the window shift
+  // of :227-246 depends on the start row only)
+  e->uniform_row = mode == SHEMS_RESET_DETERMINISTIC || hi == 1;
+  if (mode == SHEMS_RESET_HOST_DRAWS) {
+    e->uniform_row = true;
+    for (int64_t i = 1; i < e->n && e->uniform_row; ++i) e->uniform_row = idx0_host[i] == idx0_host[0];
+  }
   return SHEMS_OK;
 }
 
@@ -828,6 +965,8 @@ extern "C" int32_t shems_set_state(ShemsEnv* e, const float* obs_host, const int
   e->max_idx = mx; e->max_pending = false;
   e->was_reset = true;
   e->consistent = false;
+  e->uniform_row = true;
+  for (int64_t i = 1; i < e->n && e->uniform_row; ++i) e->uniform_row = idx_host[i] == idx_host[0];
   return SHEMS_OK;
 }
 
@@ -880,6 +1019,9 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
   shems_rollout_lean_kernel<POL, MB><<<grid_for(n1 - n0, ROLLOUT_THREADS), ROLLOUT_THREADS, 0, e->stream>>>(                           \
       e->gdp[g], e->gseries[g], e->n, e->obs, e->idx, a->n_steps, e->step, keys, a->env_id_base, a->tape_dev, a->tape_unscaled, S, n0, n1, \
       lockstep)
+#define LAUNCH_PAIR(POL)                                                                                                            \
+  shems_rollout_pair_kernel<POL, ROLLOUT_PAIR_MIN_BLOCKS><<<grid_for((n1 - n0) / 2, ROLLOUT_THREADS), ROLLOUT_THREADS, 0, e->stream>>>( \
+      e->gdp[g], e->gseries[g], e->n, e->obs, e->idx, a->n_steps, e->step, keys, a->env_id_base, a->tape_dev, a->tape_unscaled, S, n0, n1)
 #define LAUNCH_LEAN_MB(POL)                                                                                                         \
   do {                                                                                                                              \
     if (mb == 7) LAUNCH_LEAN(POL, 7);                                                                                               \
@@ -890,6 +1032,7 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
   const bool may_lean = !tr && !a->obs_traj_dev && e->consistent && rollout_lean_enabled();
   const PhiloxKeys keys = philox_keys(a->seed);
   const int lockstep = rollout_lockstep_enabled() ? 1 : 0;
+  const int pair_mode = lockstep ? rollout_pair_mode() : 0;
   // compact records need s[2..8] == series row idx (consistent), a row that fits the tag and a series-table entry in the ring
   const bool may_compact = a->replay && e->consistent && e->nrows <= RING_TAG_MAX_ROW && ring_compact_enabled();
   for (int g = 0; g < e->n_groups; ++g) {
@@ -904,8 +1047,19 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
       S.src_entry = compact ? ring_tag(entry, 0) : 0u;
     }
     const bool lean = may_lean && e->gdp[g].fast_all && (!a->replay || (compact && e->n % 32 == 0 && S.cap % 32 == 0));
+    const bool pair = lean && e->uniform_row && pair_mode != 0 && (n1 - n0) % 2 == 0 && (!a->replay || (S.head + n0) % 2 == 0) &&
+                      rollout_pair_fills(e->device, n1 - n0, pair_mode);
     const int mb = rollout_min_blocks(e->device, n1 - n0, compact, lean);
     COUNT_LAUNCH();
+    if (pair) {
+      __atomic_add_fetch(&g_pair_launches, 1, __ATOMIC_RELAXED);
+      switch (a->policy) {
+        case SHEMS_POLICY_RULE: LAUNCH_PAIR(SHEMS_POLICY_RULE); break;
+        case SHEMS_POLICY_RANDOM: LAUNCH_PAIR(SHEMS_POLICY_RANDOM); break;
+        default: LAUNCH_PAIR(SHEMS_POLICY_TAPE); break;
+      }
+      continue;
+    }
     if (lean) {
       switch (a->policy) {
         case SHEMS_POLICY_RULE: LAUNCH_LEAN_MB(SHEMS_POLICY_RULE); break;
@@ -921,6 +1075,7 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
     }
   }
 #undef LAUNCH_LEAN_MB
+#undef LAUNCH_PAIR
 #undef LAUNCH_LEAN
 #undef LAUNCH_RO_MB
 #undef LAUNCH_RO

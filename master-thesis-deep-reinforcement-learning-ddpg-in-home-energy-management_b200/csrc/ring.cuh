@@ -132,3 +132,15 @@ __device__ __forceinline__ void ring_store_compact(float* q, float sb, float sev
   ring_store_own(q, sb, sev, a0, a1, r, sb2, sev2);
   q[RING_SRC * 32] = __uint_as_float(series_tag | (uint32_t)row);
 }
+// ring_store_compact for two records of the same series row in slots s and s + 1, s even (so both sit in one tile): q is slot s's
+// record, element i of each argument belongs to slot s + i, and each field of both is one 8-byte store
+__device__ __forceinline__ void ring_store_compact_pair(float* q, const float sb[2], const float sev[2], const float a0[2], const float a1[2],
+                                                        const float r[2], const float sb2[2], const float sev2[2], uint32_t series_tag, int row) {
+  auto st2 = [q](int f, float x, float y) { *reinterpret_cast<float2*>(q + f * 32) = make_float2(x, y); };
+  st2(RING_S + 0, sb[0], sb[1]); st2(RING_S + 1, sev[0], sev[1]);
+  st2(RING_A + 0, a0[0], a0[1]); st2(RING_A + 1, a1[0], a1[1]);
+  st2(RING_R, r[0], r[1]);
+  st2(RING_S2 + 0, sb2[0], sb2[1]); st2(RING_S2 + 1, sev2[0], sev2[1]);
+  const float tag = __uint_as_float(series_tag | (uint32_t)row);
+  st2(RING_SRC, tag, tag);
+}
