@@ -224,6 +224,9 @@ SHEMS_API int32_t replay_destroy(ShemsReplay* rp);
 SHEMS_API int32_t replay_set_stream(ShemsReplay* rp, void* cuda_stream);
 SHEMS_API int64_t replay_length(const ShemsReplay* rp);
 SHEMS_API int64_t replay_capacity(const ShemsReplay* rp);
+/* physical slot the next push writes (a full memory's oldest record sits there): checkpoints of a memory with priorities restore
+ * the same slot order, which the tree's sums follow */
+SHEMS_API int64_t replay_head(const ShemsReplay* rp);
 /* number of env series the ring holds copies of: a rollout from a series-consistent env stores 32-byte compact records that
  * name a row of such a copy instead of the 88-byte transition (SHEMS_RING_COMPACT=0 forces full records) */
 SHEMS_API int32_t replay_series_count(const ShemsReplay* rp);
@@ -242,6 +245,23 @@ SHEMS_API int32_t replay_push_groups(ShemsReplay* const* rps, int32_t n_groups, 
  * Outputs are device arrays [9][B], [2][B], [B], [9][B], [B]. */
 SHEMS_API int32_t replay_sample(ShemsReplay* rp, int32_t batch, const int32_t* idx_host, uint64_t seed,
                                 float* s_dev, float* a_dev, float* r_dev, float* s2_dev, float* done_dev);
+/* Proportional prioritized replay (Schaul et al., 2016; no reference counterpart).  replay_enable_priorities gives the memory a sum
+ * tree of per-slot priorities: every filled slot gets p_max (which starts at 1), and from then on every slot a writer fills
+ * (replay_push, replay_push_groups, shems_rollout with this replay, ddpg_episode) gets the p_max current in stream order.  Internal
+ * nodes are always RN32(left + right) of their children.  A memory without priorities pays nothing. */
+SHEMS_API int32_t replay_enable_priorities(ShemsReplay* rp);
+/* priorities of the len records in logical order (0 = oldest) and p_max; synchronises the memory's stream.  SHEMS_ERR_STATE
+ * without priorities. */
+SHEMS_API int32_t replay_get_priorities(ShemsReplay* rp, float* prio_host /*[len]*/, float* p_max);
+/* checkpoint restore: the len priorities in logical order and p_max, then the whole tree is recomputed.  Priorities must be finite
+ * and >= 0 with at least one > 0, p_max finite and > 0; else SHEMS_ERR_INVALID and nothing changes. */
+SHEMS_API int32_t replay_set_priorities(ShemsReplay* rp, const float* prio_host /*[len]*/, float p_max);
+/* what update 0 of ddpg_update(seed) on a prioritized learner draws and weighs, enqueued on the memory's stream: draw j is
+ * U = u53(Philox(seed, j, 0, STREAM_PER)), x = RN32((j + U) root / batch), then down the tree (left if x < L or R == 0, else
+ * x = RN32(x - L) and right); idx_dev[j] = its logical index; w_dev[j] = RN32(x_j^-beta / max_k x_k^-beta) with
+ * x_j = leaf_j len / root in Float64.  batch <= the memory's length is not required (draws are with replacement). */
+SHEMS_API int32_t replay_sample_prioritized(ShemsReplay* rp, int32_t batch, uint64_t seed, float beta, int32_t* idx_dev /*[batch]*/,
+                                            float* w_dev /*[batch]*/);
 /* min_max_buffer(n) (memory_plotting_saving.jl:50-53): min/max of s over a with-replacement
  * sample of size n_samples -> s_min_host[9], s_max_host[9]. */
 SHEMS_API int32_t replay_minmax(ShemsReplay* rp, int64_t n_samples, const int32_t* idx_host, uint64_t seed,
@@ -289,6 +309,18 @@ SHEMS_API int32_t ddpg_sync(Ddpg* h);
  * path populations, large batches and the data-parallel learner use).  Both are fp32 and deterministic; they differ by summation
  * order.  Returns the resulting state (1 fused, 0 not) or a negative status. */
 SHEMS_API int32_t ddpg_set_fused(Ddpg* h, int32_t on);
+/* Prioritized replay for every learner of the handle (on != 0) or uniform draws (on = 0, the default).  A prioritized update draws
+ * its minibatch from the memory's sum tree (replay_sample_prioritized), scales the critic's output gradient of row j by its
+ * importance weight (dq_j = RN32(dq_j w_j); the reported critic loss stays the unweighted mse) and writes the priority
+ * p_j = RN32((|RN32(y_j - q_j)| + eps)^alpha) back to the slot it drew (a slot drawn twice takes the larger), p_max = max(p_max, p_j).
+ * Caller-supplied indices (idx_host) are weighed and written back the same way.  Its updates take the tiled-GEMM sequence, never the
+ * cluster-fused passes; act(), ddpg_rollout and ddpg_evaluate are unchanged.  alpha >= 0, beta in [0, 1], eps > 0, all finite, else
+ * SHEMS_ERR_INVALID and nothing changes (the values are ignored for on = 0).  alpha, beta, eps are handle-wide and written in
+ * stream order like ddpg_set_hparams (a beta schedule needs no re-capture).  Every update and training episode then needs memories
+ * with priorities, one per learner (else SHEMS_ERR_STATE / SHEMS_ERR_INVALID, nothing launched); ddpg_update_batch,
+ * ddpg_update_phase, ddpg_dp_connect and ddpg_update_dp return SHEMS_ERR_STATE on a prioritized handle. */
+SHEMS_API int32_t ddpg_set_prioritized(Ddpg* h, int32_t on, float alpha, float beta, float eps);
+SHEMS_API int32_t ddpg_get_prioritized(Ddpg* h, int32_t* on, float* alpha, float* beta, float* eps);
 /* glorot_uniform hidden layers, U(-3e-3,3e-3) last layers, zero biases, targets = copies
  * (DDPG.jl:21-22, 30-46) from Philox(seed) (Julia's MersenneTwister stream is not reproduced); fresh optimisers
  * (ADAM moments zero, βp = β, update counter 0: input.jl:126-127). */

@@ -103,18 +103,25 @@ SIGNATURES = {
     "replay_set_stream": (I32, [VP, VP]),
     "replay_length": (I64, [VP]),
     "replay_capacity": (I64, [VP]),
+    "replay_head": (I64, [VP]),
     "replay_series_count": (I32, [VP]),
     "replay_push": (I32, [VP, VP, VP, VP, VP, VP, I64]),
     "replay_push_groups": (I32, [C.POINTER(VP), I32, VP, VP, VP, VP, VP, I64]),
     "replay_sample": (I32, [VP, I32, PI, U64, VP, VP, VP, VP, VP]),
     "replay_minmax": (I32, [VP, I64, PI, U64, PF, PF]),
     "replay_get": (I32, [VP, PF, PF, PF, PF, PF]),
+    "replay_enable_priorities": (I32, [VP]),
+    "replay_get_priorities": (I32, [VP, PF, PF]),
+    "replay_set_priorities": (I32, [VP, PF, F32]),
+    "replay_sample_prioritized": (I32, [VP, I32, U64, F32, VP, VP]),
     "ddpg_default_params": (I32, [C.POINTER(DdpgParams)]),
     "ddpg_create": (I32, [C.POINTER(DdpgParams), I32, C.POINTER(VP)]),
     "ddpg_destroy": (I32, [VP]),
     "ddpg_set_stream": (I32, [VP, VP]),
     "ddpg_sync": (I32, [VP]),
     "ddpg_set_fused": (I32, [VP, I32]),
+    "ddpg_set_prioritized": (I32, [VP, I32, F32, F32, F32]),
+    "ddpg_get_prioritized": (I32, [VP, PI, PF, PF, PF]),
     "ddpg_init": (I32, [VP, U64]),
     "ddpg_set_layer": (I32, [VP, I32, I32, PF, PF]),
     "ddpg_get_layer": (I32, [VP, I32, I32, PF, PF]),

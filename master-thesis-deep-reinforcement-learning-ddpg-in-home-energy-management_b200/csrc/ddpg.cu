@@ -549,6 +549,10 @@ struct Ddpg {
   DdpgHparams* hp;   // [pop] host copy of every learner's ctrl->hp (ddpg_get_hparams; σ_eff of the one-learner cluster kernels)
   bool hp_stale;     // ddpg_exploit rewrote ctrl->hp on the device: ddpg_get_hparams reloads hp before it answers
   float* ou_x; long long ou_cap;                   // OUNoise.X of every instance of ddpg_episode's environment ([2][N])
+  // prioritized replay (ddpg_set_prioritized): the updates draw from every learner's sum tree (trees_dev, staged beside rings_dev),
+  // weigh the critic's dq and write the rows' priorities back.  per_knobs: α, β, ε on the device (handle-wide, written in stream order);
+  // per_slot / per_leaf [pop][B]: the slot each row of the current update drew and its priority at the draw
+  bool per; float per_host[3]; float* per_knobs; float** trees_dev; int32_t* per_slot; float* per_leaf;
 };
 static inline int round_ld(int x) { return (x + 31) & ~31; }  // activation rows start on 128-byte lines: one L2 request per TMA box row
 #ifndef TC_MIN_ROWS
@@ -668,6 +672,10 @@ extern "C" int32_t ddpg_create(const DdpgParams* p, int32_t device, Ddpg** out) 
   }
   DMALLOC(h->ctrl, pop);
   DMALLOC(h->rings_dev, pop);
+  DMALLOC(h->trees_dev, pop);
+  DMALLOC(h->per_knobs, 3);
+  DMALLOC(h->per_slot, (long long)pop * B);
+  DMALLOC(h->per_leaf, (long long)pop * B);
   h->best_stride = (na + 63) & ~63ll;   // every copy starts on a 256-byte boundary (float4 copies)
   DMALLOC(h->best, h->best_stride * pop);
   DMALLOC(h->best_score, pop);
@@ -716,8 +724,9 @@ extern "C" int32_t ddpg_destroy(Ddpg* h) {
   if (h->graph_dp) cudaGraphDestroy(h->graph_dp);
   for (int i = 0; i < h->dp_n_opened; ++i) cudaIpcCloseMemHandle(h->dp_opened[i]);
   cudaFree(h->best); cudaFree(h->best_score); cudaFree(h->best_run);
-  cudaFree(h->ctrl); cudaFree(h->idx_dev); cudaFree(h->ws); cudaFree((void*)h->rings_dev); cudaFree(h->dp_box); cudaFree(h->counters);
+  cudaFree(h->ctrl); cudaFree(h->idx_dev); cudaFree(h->ws); cudaFree((void*)h->rings_dev); cudaFree(h->trees_dev); cudaFree(h->dp_box); cudaFree(h->counters);
   cudaFree(h->ws_side); cudaFree(h->counters_side);
+  cudaFree(h->per_knobs); cudaFree(h->per_slot); cudaFree(h->per_leaf);
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
   if (h->ev_mid) cudaEventDestroy(h->ev_mid);
   if (h->ev_join) cudaEventDestroy(h->ev_join);
@@ -796,6 +805,33 @@ extern "C" int32_t ddpg_set_fused(Ddpg* h, int32_t on) {
     h->fused = want;
   }
   return h->fused ? 1 : 0;
+}
+extern "C" int32_t ddpg_set_prioritized(Ddpg* h, int32_t on, float alpha, float beta, float eps) {
+  REQUIRE(h, SHEMS_ERR_INVALID, "ddpg_set_prioritized: NULL handle");
+  if (on) {
+    REQUIRE(isfinite(alpha) && isfinite(beta) && isfinite(eps) && alpha >= 0.0f && beta >= 0.0f && beta <= 1.0f && eps > 0.0f, SHEMS_ERR_INVALID,
+            "ddpg_set_prioritized: alpha=%g beta=%g eps=%g (finite, alpha >= 0, beta in [0, 1], eps > 0)", (double)alpha, (double)beta, (double)eps);
+    REQUIRE(!h->dp_on, SHEMS_ERR_STATE, "ddpg_set_prioritized: not available for a data-parallel learner");
+  }
+  GUARD(h->device);
+  if (on) {
+    const float v[3] = {alpha, beta, eps};
+    // pageable source: staged before the call returns; ordered like ddpg_set_hparams, so a captured update reads the new values
+    CUDA_TRY(cudaMemcpyAsync(h->per_knobs, v, sizeof(v), cudaMemcpyHostToDevice, h->stream));
+    memcpy(h->per_host, v, sizeof(v));
+  }
+  if ((on != 0) != h->per) {   // the update's graph gains or loses the prioritized kernels: re-captured by the next update
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }
+    h->per = on != 0;
+  }
+  return SHEMS_OK;
+}
+extern "C" int32_t ddpg_get_prioritized(Ddpg* h, int32_t* on, float* alpha, float* beta, float* eps) {
+  REQUIRE(h && on && alpha && beta && eps, SHEMS_ERR_INVALID, "ddpg_get_prioritized: NULL argument");
+  *on = h->per ? 1 : 0;
+  *alpha = h->per_host[0]; *beta = h->per_host[1]; *eps = h->per_host[2];
+  return SHEMS_OK;
 }
 
 extern "C" int64_t ddpg_num_params(const Ddpg* h, int32_t net) {
@@ -893,11 +929,15 @@ extern "C" int32_t ddpg_init(Ddpg* h, uint64_t seed) {
 // xspi[:, :9] = s_n, r, done for the B sampled transitions.  src arrays are SoA with leading dim `ld`.
 // src: either the replay ring (tiled layout, ring != NULL) or caller-supplied SoA arrays with leading dim ld (direct).
 // One thread per (sample j, state field k): thread k == 0 also moves a, r, done.
-__global__ void __launch_bounds__(128)
-ddpg_gather_kernel(const float* const* __restrict__ rings, const float* __restrict__ rs, const float* __restrict__ ra, const float* __restrict__ rr,
-                   const float* __restrict__ rs2, const float* __restrict__ rd, long long ld, DdpgCtrl* __restrict__ ctrl,
-                   const int32_t* __restrict__ idx, long long idx_stride, const float* __restrict__ norm, int B, float* __restrict__ xs,
-                   float* __restrict__ xs2, float* __restrict__ xspi, float* __restrict__ r, float* __restrict__ done, long long pop_stride) {
+// PER: the ring rows come from the learner's sum tree (trees[blockIdx.y], ring_draw_prioritized; caller-supplied indices as they are),
+// and thread k == 0 of row j records its slot and priority in per_slot / per_leaf [pop][B] for ddpg_per_kernel.
+template <bool PER>
+__device__ __forceinline__ void gather_body(const float* const* __restrict__ rings, const float* __restrict__ rs, const float* __restrict__ ra,
+                                            const float* __restrict__ rr, const float* __restrict__ rs2, const float* __restrict__ rd, long long ld,
+                                            DdpgCtrl* __restrict__ ctrl, const int32_t* __restrict__ idx, long long idx_stride,
+                                            const float* __restrict__ norm, int B, float* __restrict__ xs, float* __restrict__ xs2,
+                                            float* __restrict__ xspi, float* __restrict__ r, float* __restrict__ done, long long pop_stride,
+                                            const float* const* __restrict__ trees, int32_t* __restrict__ per_slot, float* __restrict__ per_leaf) {
   asm volatile("griddepcontrol.launch_dependents;\n" ::: "memory");   // the forward-chain launch after it stages its weights under this kernel
   const unsigned g = blockIdx.x * blockDim.x + threadIdx.x;
   const int j = g / 9, k = g % 9;  // unsigned: k is known to be < 9, which folds ring_field's field-range tests
@@ -911,8 +951,23 @@ ddpg_gather_kernel(const float* const* __restrict__ rings, const float* __restri
   float sv, s2v, a0 = 0.f, a1 = 0.f, rv = 0.f, dv = 0.f;
   if (ring) {
     const long long len = ctrl->len, head = ctrl->head, cap = ctrl->cap;
-    const long long li = ctrl->use_idx ? idx[(long long)ctrl->idx_cursor * B + j] : ring_draw(ctrl->seed, j, ctrl->update, len);
-    const float* q = ring + ring_base(ring_slot(li, head, len, cap));
+    long long slot;
+    if (PER) {
+      const float* tree = trees[blockIdx.y];
+      const long long p2 = prio_p2(cap);
+      float leaf;
+      if (ctrl->use_idx) {
+        slot = ring_slot(idx[(long long)ctrl->idx_cursor * B + j], head, len, cap);
+        leaf = tree[p2 + slot];
+      } else {
+        slot = ring_draw_prioritized(tree, p2, ctrl->seed, j, ctrl->update, B, &leaf);
+      }
+      if (k == 0) { per_slot[(long long)blockIdx.y * B + j] = (int32_t)slot; per_leaf[(long long)blockIdx.y * B + j] = leaf; }
+    } else {
+      const long long li = ctrl->use_idx ? idx[(long long)ctrl->idx_cursor * B + j] : ring_draw(ctrl->seed, j, ctrl->update, len);
+      slot = ring_slot(li, head, len, cap);
+    }
+    const float* q = ring + ring_base(slot);
     const float* row = ring_row(ring_table(ring), q);
     sv = ring_field(q, row, RING_S + k); s2v = ring_field(q, row, RING_S2 + k);
     if (k == 0) {
@@ -927,6 +982,70 @@ ddpg_gather_kernel(const float* const* __restrict__ rings, const float* __restri
   const float s2n = __fdiv_rn(__fsub_rn(s2v, norm[k]), den);
   xs[j * 11 + k] = sn; xspi[j * 11 + k] = sn; xs2[j * 11 + k] = s2n;
   if (k == 0) { xs[j * 11 + 9] = a0; xs[j * 11 + 10] = a1; r[j] = rv; done[j] = dv; }
+}
+__global__ void __launch_bounds__(128)
+ddpg_gather_kernel(const float* const* __restrict__ rings, const float* __restrict__ rs, const float* __restrict__ ra, const float* __restrict__ rr,
+                   const float* __restrict__ rs2, const float* __restrict__ rd, long long ld, DdpgCtrl* __restrict__ ctrl,
+                   const int32_t* __restrict__ idx, long long idx_stride, const float* __restrict__ norm, int B, float* __restrict__ xs,
+                   float* __restrict__ xs2, float* __restrict__ xspi, float* __restrict__ r, float* __restrict__ done, long long pop_stride) {
+  gather_body<false>(rings, rs, ra, rr, rs2, rd, ld, ctrl, idx, idx_stride, norm, B, xs, xs2, xspi, r, done, pop_stride, nullptr, nullptr, nullptr);
+}
+__global__ void __launch_bounds__(128)
+ddpg_gather_per_kernel(const float* const* __restrict__ rings, DdpgCtrl* __restrict__ ctrl, const int32_t* __restrict__ idx, long long idx_stride,
+                       const float* __restrict__ norm, int B, float* __restrict__ xs, float* __restrict__ xs2, float* __restrict__ xspi,
+                       float* __restrict__ r, float* __restrict__ done, long long pop_stride, const float* const* __restrict__ trees,
+                       int32_t* __restrict__ per_slot, float* __restrict__ per_leaf) {
+  gather_body<true>(rings, nullptr, nullptr, nullptr, nullptr, nullptr, 0, ctrl, idx, idx_stride, norm, B, xs, xs2, xspi, r, done, pop_stride, trees,
+                    per_slot, per_leaf);
+}
+
+// Prioritized replay between the TD target and the critic's backward pass, one block per learner (blockIdx.y):
+//   w_j = RN32((leaf_j len / root)^-β / max_k (leaf_k len / root)^-β)  (Float64, the max over the B rows);  dq_j = RN32(dq_j w_j)
+//   p_j = RN32((|RN32(y_j - q_j)| + ε)^α);  each drawn slot's leaf = the largest p_j of the rows that drew it;  p_max = max(p_max, p_j)
+//   then the nodes above the drawn leaves, level by level (every node from its two children, as a full rebuild computes it)
+#define PER_THREADS 1024
+__global__ void __launch_bounds__(PER_THREADS)
+ddpg_per_kernel(float* const* __restrict__ trees, const DdpgCtrl* __restrict__ ctrl, const float* __restrict__ knobs, const int32_t* __restrict__ per_slot,
+                const float* __restrict__ per_leaf, const float* __restrict__ q, const float* __restrict__ y, float* __restrict__ dq, int B,
+                long long pop_stride) {
+  __shared__ double red_w[PER_THREADS / 32];
+  __shared__ float red_p[PER_THREADS / 32];
+  const long long lo = (long long)blockIdx.y * pop_stride;
+  float* const tree = trees[blockIdx.y];
+  ctrl += blockIdx.y; per_slot += (long long)blockIdx.y * B; per_leaf += (long long)blockIdx.y * B;
+  q += lo; y += lo; dq += lo;
+  const long long len = ctrl->len, p2 = prio_p2(ctrl->cap);
+  const float alpha = knobs[0], beta = knobs[1], eps = knobs[2];
+  const float root = tree[1];
+  double wmax = 0.0;
+  float pmax = 0.0f;
+  for (int j = threadIdx.x; j < B; j += blockDim.x) {
+    wmax = fmax(wmax, ring_is_weight(per_leaf[j], len, root, beta));
+    pmax = fmaxf(pmax, ring_priority(y[j], q[j], alpha, eps));
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    wmax = fmax(wmax, __shfl_xor_sync(0xffffffffu, wmax, o));
+    pmax = fmaxf(pmax, __shfl_xor_sync(0xffffffffu, pmax, o));
+  }
+  if ((threadIdx.x & 31) == 0) { red_w[threadIdx.x >> 5] = wmax; red_p[threadIdx.x >> 5] = pmax; }
+  __syncthreads();   // also: every thread has read the root before a leaf changes
+  for (int i = 0; i < (int)(blockDim.x >> 5); ++i) { wmax = fmax(wmax, red_w[i]); pmax = fmaxf(pmax, red_p[i]); }
+  for (int j = threadIdx.x; j < B; j += blockDim.x) {
+    dq[j] = __fmul_rn(dq[j], (float)(ring_is_weight(per_leaf[j], len, root, beta) / wmax));
+    tree[p2 + per_slot[j]] = 0.0f;
+  }
+  __syncthreads();
+  for (int j = threadIdx.x; j < B; j += blockDim.x)   // priorities are >= 0: their bits order as signed integers
+    atomicMax(reinterpret_cast<int*>(tree + p2 + per_slot[j]), __float_as_int(ring_priority(y[j], q[j], alpha, eps)));
+  if (threadIdx.x == 0) prio_header(tree)[PRIO_PMAX] = fmaxf(prio_header(tree)[PRIO_PMAX], pmax);
+  for (long long level = p2 >> 1; level >= 1; level >>= 1) {
+    __syncthreads();
+    const int shift = 63 - __clzll(p2 / level);
+    for (int j = threadIdx.x; j < B; j += blockDim.x) {
+      const long long n = (p2 + per_slot[j]) >> shift;
+      tree[n] = __fadd_rn(tree[2 * n], tree[2 * n + 1]);
+    }
+  }
 }
 
 // ----------------------------------------------------------------------------- Adam + Polyak
@@ -1617,6 +1736,11 @@ static int enqueue_phase0(Ddpg* h, cudaStream_t st) {
   // (after the three-net launch: a' and q are its output, critic_target's weights are not)
   const FwdNet td = {h->xs2, critic_t, &dc, h->tc_h1, h->tc_h2, false, TC_OUT_TD, h->y, 1};
   TRY(enqueue_forward(h, st, rg, &td, 1, 11, B, h->pop_stride, 1, 1));
+  if (h->per) {   // prioritized replay: importance weights on dq, the rows' priorities back into the sum trees
+    ddpg_per_kernel<<<dim3(1, h->pop), PER_THREADS, 0, st>>>(h->trees_dev, h->ctrl, h->per_knobs, h->per_slot, h->per_leaf, h->q, h->y, h->dq, B,
+                                                             h->pop_stride);
+    CUDA_TRY(cudaGetLastError());
+  }
   // P7-P9: critic backward (:137, :105-108)
   return enqueue_backward(h, st, rg, critic, dc, h->c_h1, h->c_h2, h->dq, h->dz2, h->dz1, h->grad[1]);
 }
@@ -1712,6 +1836,13 @@ static int enqueue_update_body(Ddpg* h, cudaStream_t st, bool dp = false) {
 static int enqueue_gather(Ddpg* h, cudaStream_t st, bool from_rings, const float* s, const float* a, const float* r, const float* s2,
                           const float* done, long long ld) {
   const int B = h->p.batch;
+  if (h->per && from_rings) {
+    ddpg_gather_per_kernel<<<dim3((B * 9 + 127) / 128, h->pop), 128, 0, st>>>(h->rings_dev, h->ctrl, h->idx_dev, h->idx_stride, h->norm, B, h->xs,
+                                                                             h->xs2, h->xspi, h->r, h->done, h->pop_stride, h->trees_dev,
+                                                                             h->per_slot, h->per_leaf);
+    CUDA_TRY(cudaGetLastError());
+    return SHEMS_OK;
+  }
   ddpg_gather_kernel<<<dim3((B * 9 + 127) / 128, from_rings ? h->pop : 1), 128, 0, st>>>(from_rings ? h->rings_dev : nullptr, s, a, r, s2, done, ld,
                                                                                      h->ctrl, h->idx_dev, h->idx_stride, h->norm, B, h->xs,
                                                                                      h->xs2, h->xspi, h->r, h->done, h->pop_stride);
@@ -1722,7 +1853,8 @@ static int enqueue_gather(Ddpg* h, cudaStream_t st, bool from_rings, const float
 // one whole replay(): sample + update.  Fused path: 4 launches (the critic pass gathers); tiled path: gather kernel + the GEMM sequence
 static int enqueue_update(Ddpg* h, cudaStream_t st, bool dp, bool from_rings, const float* s, const float* a, const float* r, const float* s2,
                           const float* done, long long ld) {
-  if (use_fused(h)) return enqueue_update_fused(h, st, dp, GatherSrc{from_rings, s, a, r, s2, done, ld});
+  // prioritized replay weighs dq between the passes of the tiled sequence: its updates never take the fused passes
+  if (use_fused(h) && !h->per) return enqueue_update_fused(h, st, dp, GatherSrc{from_rings, s, a, r, s2, done, ld});
   TRY(enqueue_gather(h, st, from_rings, s, a, r, s2, done, ld));
   return enqueue_update_body(h, st, dp);
 }
@@ -1746,6 +1878,18 @@ static int ensure_graph(Ddpg* h, bool dp = false) {
   return SHEMS_OK;
 }
 
+// a prioritized learner writes priorities back into its memory's tree: every learner needs a memory with priorities of its own
+static int per_memories_ok(const Ddpg* h, ShemsReplay* const* rps, const char* who) {
+  if (!h->per) return SHEMS_OK;
+  for (int l = 0; l < h->pop; ++l) {
+    REQUIRE(rps[l], SHEMS_ERR_INVALID, "%s: learner %d has no replay memory", who, l);
+    REQUIRE(rps[l]->prio, SHEMS_ERR_STATE, "%s: prioritized learner, but the memory of learner %d has no priorities (replay_enable_priorities)", who, l);
+    for (int k = 0; k < l; ++k)
+      REQUIRE(rps[k] != rps[l], SHEMS_ERR_INVALID, "%s: prioritized learners %d and %d share one memory", who, k, l);
+  }
+  return SHEMS_OK;
+}
+
 struct CtrlHostPart { unsigned long long seed; unsigned update; int use_idx; long long len, head, cap; int idx_cursor; unsigned blocks_done; };
 static_assert(sizeof(CtrlHostPart) == offsetof(DdpgCtrl, bp), "control block layout");
 
@@ -1755,11 +1899,14 @@ static int stage_update_inputs(Ddpg* h, ShemsReplay* const* rps, const uint64_t*
   const int pop = h->pop;
   std::vector<CtrlHostPart> hp((size_t)pop);
   std::vector<const float*> rings((size_t)pop);
+  std::vector<float*> trees((size_t)pop);
+  TRY(per_memories_ok(h, rps, "ddpg_update"));
   for (int l = 0; l < pop; ++l) {
     ShemsReplay* rp = rps[l];
     REQUIRE(rp, SHEMS_ERR_INVALID, "ddpg_update: learner %d has no replay memory", l);
     REQUIRE(rp->device == h->device, SHEMS_ERR_INVALID, "ddpg_update: replay on device %d, learner on %d", rp->device, h->device);
     REQUIRE(rp->length > 0, SHEMS_ERR_STATE, "ddpg_update: memory is empty");
+    trees[l] = rp->prio;
     if (idx_host)
       for (long long j = 0; j < per_learner; ++j) {
         const int32_t v = idx_host[(long long)l * per_learner + j];
@@ -1791,6 +1938,7 @@ static int stage_update_inputs(Ddpg* h, ShemsReplay* const* rps, const uint64_t*
   // pageable sources: the runtime stages these small copies before returning, so the vectors may go out of scope
   CUDA_TRY(cudaMemcpy2DAsync(h->ctrl, sizeof(DdpgCtrl), hp.data(), sizeof(CtrlHostPart), sizeof(CtrlHostPart), (size_t)pop, cudaMemcpyHostToDevice, h->stream));
   CUDA_TRY(cudaMemcpyAsync((void*)h->rings_dev, rings.data(), sizeof(const float*) * (size_t)pop, cudaMemcpyHostToDevice, h->stream));
+  if (h->per) CUDA_TRY(cudaMemcpyAsync(h->trees_dev, trees.data(), sizeof(float*) * (size_t)pop, cudaMemcpyHostToDevice, h->stream));
   return SHEMS_OK;
 }
 
@@ -1817,6 +1965,7 @@ extern "C" int32_t ddpg_update_phase(Ddpg* h, ShemsReplay* rp, int32_t phase, co
   REQUIRE(h, SHEMS_ERR_INVALID, "ddpg_update_phase: NULL handle");
   REQUIRE(phase >= 0 && phase <= 2, SHEMS_ERR_INVALID, "ddpg_update_phase: phase=%d", phase);
   REQUIRE(h->pop == 1, SHEMS_ERR_INVALID, "ddpg_update_phase: not available for a population handle");
+  REQUIRE(!h->per, SHEMS_ERR_STATE, "ddpg_update_phase: not available for a prioritized learner");
   GUARD(h->device);
   if (phase == 0) {
     REQUIRE(rp, SHEMS_ERR_STATE, "ddpg_update_phase: replay missing");
@@ -1864,6 +2013,7 @@ extern "C" int32_t ddpg_dp_connect(Ddpg* h, int32_t rank, int32_t world, const v
   REQUIRE(h && handles, SHEMS_ERR_INVALID, "ddpg_dp_connect: NULL argument");
   REQUIRE(world >= 1 && world <= DP_MAX_WORLD && rank >= 0 && rank < world, SHEMS_ERR_INVALID, "ddpg_dp_connect: rank=%d world=%d (max %d)", rank, world, DP_MAX_WORLD);
   REQUIRE(h->pop == 1 && !h->dp_on, SHEMS_ERR_STATE, "ddpg_dp_connect: population handle, or already connected");
+  REQUIRE(!h->per, SHEMS_ERR_STATE, "ddpg_dp_connect: not available for a prioritized learner");
   REQUIRE(h->dp_box, SHEMS_ERR_STATE, "ddpg_dp_connect: call ddpg_dp_export on this handle first");
   GUARD(h->device);
   memset(&h->dp, 0, sizeof(h->dp));
@@ -1925,6 +2075,7 @@ extern "C" int32_t ddpg_dp_prepare(Ddpg* h, int64_t idx_ints) {
 extern "C" int32_t ddpg_update_dp(Ddpg* h, ShemsReplay* rp, int32_t n_updates, const int32_t* idx_host, uint64_t seed) {
   REQUIRE(h && rp, SHEMS_ERR_INVALID, "ddpg_update_dp: NULL argument");
   REQUIRE(h->dp_on, SHEMS_ERR_STATE, "ddpg_update_dp: call ddpg_dp_connect first");
+  REQUIRE(!h->per, SHEMS_ERR_STATE, "ddpg_update_dp: not available for a prioritized learner");
   REQUIRE(n_updates >= 1, SHEMS_ERR_INVALID, "ddpg_update_dp: n_updates=%d", n_updates);
   GUARD(h->device);
   TRY(stage_update_inputs(h, &rp, &seed, idx_host, (long long)n_updates * h->p.batch));
@@ -1947,6 +2098,7 @@ extern "C" int32_t ddpg_dp_status(Ddpg* h, int32_t* error_out) {
 extern "C" int32_t ddpg_update_batch(Ddpg* h, const float* s_dev, const float* a_dev, const float* r_dev, const float* s2_dev, const float* done_dev) {
   REQUIRE(h && s_dev && a_dev && r_dev && s2_dev, SHEMS_ERR_INVALID, "ddpg_update_batch: NULL argument");
   REQUIRE(h->pop == 1, SHEMS_ERR_INVALID, "ddpg_update_batch: not available for a population handle");
+  REQUIRE(!h->per, SHEMS_ERR_STATE, "ddpg_update_batch: a prioritized learner samples its replay memory (no priorities come with a caller's minibatch)");
   GUARD(h->device);
   TRY(enqueue_update(h, h->stream, false, false, s_dev, a_dev, r_dev, s2_dev, done_dev, h->p.batch));
   h->n_updates += 1;
@@ -2214,6 +2366,7 @@ extern "C" int32_t ddpg_episode(Ddpg* h, ShemsEnv* env, ShemsReplay* const* rps,
   REQUIRE(env->stream == h->stream && (!train || rps[0]->stream == h->stream), SHEMS_ERR_STATE,
           "ddpg_episode: bind the environment, the learner and the replay memories to one CUDA stream");
   REQUIRE(env->was_reset, SHEMS_ERR_STATE, "ddpg_episode: reset! must come first");
+  if (train) TRY(per_memories_ok(h, rps, "ddpg_episode"));
   if (ensure_rows(env, n_steps)) {  // nothing is enqueued for an episode that would leave the series
     shems_set_error("BoundsError: episode of %d steps from row %d leaves the %d-row series (next_state!, shems_LU1.jl:266-268)", n_steps, env->max_idx,
                     env->nrows);
@@ -2237,6 +2390,8 @@ extern "C" int32_t ddpg_episode(Ddpg* h, ShemsEnv* env, ShemsReplay* const* rps,
     h->ou_cap = N;
   }
   std::vector<uint64_t> seeds((size_t)h->pop);
+  if (train && h->per && h->pop == 1 && updates_per_step > 0)   // the post-step kernel below stages the ring, not the tree
+    CUDA_TRY(cudaMemcpyAsync(h->trees_dev, &rps[0]->prio, sizeof(float*), cudaMemcpyHostToDevice, h->stream));
   for (int step = 1; step <= n_steps; ++step) {
     const uint64_t rng_step = (seed * 1000003ull + (uint64_t)step) & 0x7fffffffffffffffull;
     if (train && h->noise_kind == 1) {
@@ -2253,7 +2408,7 @@ extern "C" int32_t ddpg_episode(Ddpg* h, ShemsEnv* env, ShemsReplay* const* rps,
       REQUIRE(rp && rp->device == h->device, SHEMS_ERR_INVALID, "ddpg_episode: replay memory missing or on another device");
       REQUIRE(N <= rp->capacity, SHEMS_ERR_INVALID, "ddpg_episode: %lld instances exceed the memory's capacity %lld", N, (long long)rp->capacity);
       const long long head = rp->head;
-      replay_after_rollout(rp, N);
+      TRY(replay_after_rollout(rp, N, h->stream));
       CtrlHostPart hp; memset(&hp, 0, sizeof(hp));
       hp.seed = rng_step; hp.update = 0u; hp.use_idx = 0;
       hp.len = rp->length; hp.head = rp->head; hp.cap = rp->capacity;

@@ -1085,6 +1085,6 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
   e->max_idx += a->n_steps;
   e->step += a->n_steps;
   e->consistent = true;
-  if (a->replay) return replay_after_rollout(a->replay, total);
+  if (a->replay) return replay_after_rollout(a->replay, total, e->stream);
   return SHEMS_OK;
 }

@@ -5,7 +5,7 @@
 #include <stdint.h>
 
 enum : uint32_t { STREAM_RESET = 0x5245u, STREAM_ACTION = 0x4143u, STREAM_NOISE = 0x4e4fu, STREAM_SAMPLE = 0x534du, STREAM_INIT = 0x494eu,
-                  STREAM_PBT = 0x5042u };
+                  STREAM_PBT = 0x5042u, STREAM_PER = 0x5052u };
 
 // the 64-bit product of two words.  On the device one mul.wide.u32 (a single IMAD.WIDE.U32): the compiler's lowering of the
 // C expression adds a zero high word to every product, one wasted instruction each.

@@ -10,6 +10,8 @@
 
 #include "common.h"
 
+#define TRY_PRIO(expr) do { const int _s = (expr); if (_s) return _s; } while (0)
+
 extern "C" int32_t replay_create(int64_t capacity, int32_t device, ShemsReplay** out) {
   REQUIRE(out && capacity >= 1, SHEMS_ERR_INVALID, "replay_create: capacity=%lld", (long long)capacity);
   REQUIRE(shems_device_count() > 0, SHEMS_ERR_CUDA, "replay_create: no CUDA device (this library has no CPU fallback)");
@@ -35,7 +37,7 @@ extern "C" int32_t replay_destroy(ShemsReplay* rp) {
   if (!rp) return SHEMS_OK;
   GUARD(rp->device);
   for (int i = 0; i < rp->n_src; ++i) cudaFree(rp->src[i].rows);
-  cudaFree(rp->alloc); cudaFree(rp->idx_scratch); cudaFree(rp->minmax_scratch); cudaFree(rp->group_refs);
+  cudaFree(rp->alloc); cudaFree(rp->prio_alloc); cudaFree(rp->idx_scratch); cudaFree(rp->minmax_scratch); cudaFree(rp->group_refs);
   delete rp;
   return SHEMS_OK;
 }
@@ -46,11 +48,159 @@ extern "C" int32_t replay_set_stream(ShemsReplay* rp, void* s) {
 }
 extern "C" int64_t replay_length(const ShemsReplay* rp) { return rp ? rp->length : 0; }
 extern "C" int64_t replay_capacity(const ShemsReplay* rp) { return rp ? rp->capacity : 0; }
+extern "C" int64_t replay_head(const ShemsReplay* rp) { return rp ? rp->head : 0; }
 extern "C" int32_t replay_series_count(const ShemsReplay* rp) { return rp ? rp->n_src : 0; }
 
-int replay_after_rollout(ShemsReplay* rp, int64_t n_written) {
+// ---- priorities (ring.cuh: the sum tree)
+// One launch rebuilds the tree after leaves changed.  Block c owns the chunk of `sub` = min(P2, PRIO_SUB) slots from c * sub: with
+// m >= 0 it gives the slots (s0 + i) mod cap, i < m, that fall in its chunk the leaf p_max and recomputes the chunk's subtree; with
+// m < 0 it recomputes every chunk's subtree from the leaves as they are.  The last block to arrive recomputes the nodes above the
+// chunk roots.
+#define PRIO_SUB 1024
+#define PRIO_THREADS 512
+__global__ void __launch_bounds__(PRIO_THREADS)
+replay_prio_refresh_kernel(float* __restrict__ tree, long long p2, long long cap, long long s0, long long m) {
+  const long long sub = p2 < PRIO_SUB ? p2 : PRIO_SUB;
+  const long long first = (long long)blockIdx.x * sub, last = first + sub < cap ? first + sub : cap;
+  const long long end1 = s0 + m < cap ? s0 + m : cap;   // the written slots are [s0, end1) and, after a wrap, [0, s0 + m - cap)
+  const bool touched = m < 0 || (first < end1 && s0 < last) || (s0 + m > cap && first < s0 + m - cap);
+  if (touched) {
+    if (m >= 0) {
+      const float pmax = prio_header(tree)[PRIO_PMAX];
+      for (long long s = first + threadIdx.x; s < last; s += blockDim.x) {
+        long long d = s - s0;
+        if (d < 0) d += cap;
+        if (d < m) tree[p2 + s] = pmax;
+      }
+    }
+    long long lo = p2 + first;
+    for (long long width = sub >> 1; width >= 1; width >>= 1) {
+      __syncthreads();
+      lo >>= 1;
+      for (long long t = threadIdx.x; t < width; t += blockDim.x) tree[lo + t] = __fadd_rn(tree[2 * (lo + t)], tree[2 * (lo + t) + 1]);
+    }
+  }
+  __shared__ bool last_block;
+  __syncthreads();
+  unsigned* arrived = reinterpret_cast<unsigned*>(prio_header(tree) + PRIO_ARRIVED);
+  if (threadIdx.x == 0) {
+    __threadfence();
+    last_block = atomicAdd(arrived, 1u) == gridDim.x - 1;
+  }
+  __syncthreads();
+  if (!last_block) return;
+  __threadfence();
+  long long lo = p2 / sub;   // the chunk roots are nodes p2/sub .. 2 p2/sub - 1
+  for (long long width = lo >> 1; width >= 1; width >>= 1) {
+    lo >>= 1;
+    for (long long t = threadIdx.x; t < width; t += blockDim.x) tree[lo + t] = __fadd_rn(__ldcg(tree + 2 * (lo + t)), __ldcg(tree + 2 * (lo + t) + 1));
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) *arrived = 0u;
+}
+
+static int prio_refresh(ShemsReplay* rp, long long s0, long long m, cudaStream_t st) {
+  const long long sub = rp->prio_p2 < PRIO_SUB ? rp->prio_p2 : PRIO_SUB;
+  replay_prio_refresh_kernel<<<(unsigned)((rp->capacity + sub - 1) / sub), PRIO_THREADS, 0, st>>>(rp->prio, rp->prio_p2, rp->capacity, s0, m);
+  CUDA_TRY(cudaGetLastError());
+  return SHEMS_OK;
+}
+
+int replay_after_rollout(ShemsReplay* rp, int64_t n_written, cudaStream_t st) {
+  const int64_t m = n_written < rp->capacity ? n_written : rp->capacity;   // the slots that survive the push
+  const int64_t s0 = (rp->head + n_written - m) % rp->capacity;
   rp->head = (rp->head + n_written) % rp->capacity;
   rp->length = rp->length + n_written > rp->capacity ? rp->capacity : rp->length + n_written;
+  if (rp->prio && m > 0) return prio_refresh(rp, s0, m, st);
+  return SHEMS_OK;
+}
+
+extern "C" int32_t replay_enable_priorities(ShemsReplay* rp) {
+  REQUIRE(rp, SHEMS_ERR_INVALID, "replay_enable_priorities: NULL handle");
+  if (rp->prio) return SHEMS_OK;
+  GUARD(rp->device);
+  const size_t floats = prio_alloc_floats(rp->capacity);
+  CUDA_TRY(cudaStreamSynchronize(rp->stream));
+  CUDA_TRY(cudaMalloc(&rp->prio_alloc, sizeof(float) * floats));
+  rp->prio = rp->prio_alloc + PRIO_HEADER_FLOATS;
+  rp->prio_p2 = prio_p2(rp->capacity);
+  const float pmax = 1.0f;
+  CUDA_TRY(cudaMemsetAsync(rp->prio_alloc, 0, sizeof(float) * floats, rp->stream));
+  CUDA_TRY(cudaMemcpyAsync(rp->prio_alloc + PRIO_PMAX, &pmax, sizeof(float), cudaMemcpyHostToDevice, rp->stream));
+  TRY_PRIO(prio_refresh(rp, ring_slot(0, rp->head, rp->length, rp->capacity), rp->length, rp->stream));   // every filled slot gets p_max
+  CUDA_TRY(cudaStreamSynchronize(rp->stream));   // &pmax is on this stack frame
+  return SHEMS_OK;
+}
+
+extern "C" int32_t replay_get_priorities(ShemsReplay* rp, float* prio_host, float* p_max) {
+  REQUIRE(rp && prio_host && p_max, SHEMS_ERR_INVALID, "replay_get_priorities: NULL argument");
+  REQUIRE(rp->prio, SHEMS_ERR_STATE, "replay_get_priorities: the memory has no priorities (replay_enable_priorities)");
+  GUARD(rp->device);
+  const int64_t cap = rp->capacity, len = rp->length;
+  std::vector<float> leaves((size_t)cap);
+  CUDA_TRY(cudaStreamSynchronize(rp->stream));
+  CUDA_TRY(cudaMemcpy(leaves.data(), rp->prio + rp->prio_p2, sizeof(float) * (size_t)cap, cudaMemcpyDeviceToHost));
+  CUDA_TRY(cudaMemcpy(p_max, rp->prio_alloc + PRIO_PMAX, sizeof(float), cudaMemcpyDeviceToHost));
+  for (int64_t i = 0; i < len; ++i) prio_host[i] = leaves[(size_t)ring_slot(i, rp->head, len, cap)];
+  return SHEMS_OK;
+}
+
+extern "C" int32_t replay_set_priorities(ShemsReplay* rp, const float* prio_host, float p_max) {
+  REQUIRE(rp && prio_host, SHEMS_ERR_INVALID, "replay_set_priorities: NULL argument");
+  REQUIRE(rp->prio, SHEMS_ERR_STATE, "replay_set_priorities: the memory has no priorities (replay_enable_priorities)");
+  REQUIRE(isfinite(p_max) && p_max > 0.0f, SHEMS_ERR_INVALID, "replay_set_priorities: p_max=%g must be finite and > 0", (double)p_max);
+  const int64_t cap = rp->capacity, len = rp->length;
+  bool mass = false;
+  for (int64_t i = 0; i < len; ++i) {
+    REQUIRE(isfinite(prio_host[i]) && prio_host[i] >= 0.0f, SHEMS_ERR_INVALID, "replay_set_priorities: prio[%lld]=%g must be finite and >= 0",
+            (long long)i, (double)prio_host[i]);
+    mass = mass || prio_host[i] > 0.0f;
+  }
+  REQUIRE(mass || len == 0, SHEMS_ERR_INVALID, "replay_set_priorities: every priority is 0 (nothing could be drawn)");
+  GUARD(rp->device);
+  std::vector<float> leaves((size_t)rp->prio_p2, 0.0f);
+  for (int64_t i = 0; i < len; ++i) leaves[(size_t)ring_slot(i, rp->head, len, cap)] = prio_host[i];
+  CUDA_TRY(cudaMemcpyAsync(rp->prio + rp->prio_p2, leaves.data(), sizeof(float) * leaves.size(), cudaMemcpyHostToDevice, rp->stream));
+  CUDA_TRY(cudaMemcpyAsync(rp->prio_alloc + PRIO_PMAX, &p_max, sizeof(float), cudaMemcpyHostToDevice, rp->stream));
+  TRY_PRIO(prio_refresh(rp, 0, -1, rp->stream));
+  CUDA_TRY(cudaStreamSynchronize(rp->stream));   // the host sources live on this stack frame
+  return SHEMS_OK;
+}
+
+// the B draws and importance weights of update 0 of ddpg_update(seed) on this memory: one block (the weights are normalised by the
+// largest of the B)
+#define PRIO_SAMPLE_THREADS 1024
+__global__ void __launch_bounds__(PRIO_SAMPLE_THREADS)
+replay_sample_prioritized_kernel(const float* __restrict__ tree, long long p2, long long cap, long long head, long long len, unsigned long long seed,
+                                 int B, float beta, int32_t* __restrict__ idx, float* __restrict__ w) {
+  __shared__ double red[PRIO_SAMPLE_THREADS / 32];
+  const float root = tree[1];
+  double wmax = 0.0;
+  for (int j = threadIdx.x; j < B; j += blockDim.x) {
+    float leaf;
+    const long long slot = ring_draw_prioritized(tree, p2, seed, (uint64_t)j, 0u, B, &leaf);
+    idx[j] = (int32_t)ring_logical(slot, head, len, cap);
+    w[j] = leaf;   // the same thread turns it into the weight below
+    wmax = fmax(wmax, ring_is_weight(leaf, len, root, beta));
+  }
+  for (int o = 16; o > 0; o >>= 1) wmax = fmax(wmax, __shfl_xor_sync(0xffffffffu, wmax, o));
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = wmax;
+  __syncthreads();
+  wmax = 0.0;
+  for (int i = 0; i < (int)(blockDim.x >> 5); ++i) wmax = fmax(wmax, red[i]);
+  for (int j = threadIdx.x; j < B; j += blockDim.x) w[j] = (float)(ring_is_weight(w[j], len, root, beta) / wmax);
+}
+
+extern "C" int32_t replay_sample_prioritized(ShemsReplay* rp, int32_t batch, uint64_t seed, float beta, int32_t* idx_dev, float* w_dev) {
+  REQUIRE(rp && idx_dev && w_dev, SHEMS_ERR_INVALID, "replay_sample_prioritized: NULL argument");
+  REQUIRE(batch >= 1, SHEMS_ERR_INVALID, "replay_sample_prioritized: batch=%d", batch);
+  REQUIRE(isfinite(beta) && beta >= 0.0f && beta <= 1.0f, SHEMS_ERR_INVALID, "replay_sample_prioritized: beta=%g outside [0, 1]", (double)beta);
+  REQUIRE(rp->prio, SHEMS_ERR_STATE, "replay_sample_prioritized: the memory has no priorities (replay_enable_priorities)");
+  REQUIRE(rp->length > 0, SHEMS_ERR_STATE, "replay_sample_prioritized: memory is empty");
+  GUARD(rp->device);
+  replay_sample_prioritized_kernel<<<1, PRIO_SAMPLE_THREADS, 0, rp->stream>>>(rp->prio, rp->prio_p2, rp->capacity, rp->head, rp->length, seed, batch,
+                                                                             beta, idx_dev, w_dev);
+  CUDA_TRY(cudaGetLastError());
   return SHEMS_OK;
 }
 
@@ -105,7 +255,7 @@ extern "C" int32_t replay_push(ShemsReplay* rp, const float* s_dev, const float*
   replay_push_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, rp->stream>>>(rp->ring, rp->capacity, rp->head, s_dev, a_dev, r_dev, s2_dev,
                                                                            done_dev, n, first);
   CUDA_TRY(cudaGetLastError());
-  return replay_after_rollout(rp, n);
+  return replay_after_rollout(rp, n, rp->stream);
 }
 
 // remember() for a population: arrays are SoA over all N = P*n_per instances, learner l = instances l*n_per .. l*n_per+n_per-1
@@ -151,7 +301,7 @@ extern "C" int32_t replay_push_groups(ShemsReplay* const* rps, int32_t n_groups,
                                                                                                 r_dev, s2_dev, done_dev, n_per,
                                                                                                 n_per * n_groups);
   CUDA_TRY(cudaGetLastError());
-  for (int g = 0; g < n_groups; ++g) replay_after_rollout(rps[g], n_per);
+  for (int g = 0; g < n_groups; ++g) TRY_PRIO(replay_after_rollout(rps[g], n_per, r0->stream));
   return SHEMS_OK;
 }
 

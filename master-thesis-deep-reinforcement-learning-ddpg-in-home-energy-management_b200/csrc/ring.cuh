@@ -16,6 +16,7 @@
 //
 // Logical index i (0 = oldest) of a ring holding len records lives in physical slot (head - len + i) mod cap.
 #pragma once
+#include <math.h>
 #include <stddef.h>
 #include <stdint.h>
 #include <string.h>
@@ -108,6 +109,57 @@ __host__ __device__ __forceinline__ long long ring_draw(uint64_t seed, uint64_t 
   long long li = (long long)(u53(w[0], w[1]) * (double)len);
   if (li >= len) li = len - 1;
   return li;
+}
+
+// ---- proportional prioritized replay (replay_enable_priorities; Schaul et al., 2016)
+// A memory with priorities keeps a sum tree beside the ring: P2 = the next power of two >= cap, nodes 0 .. 2 P2 - 1 (node 0 unused),
+// node 1 the root, node i the parent of 2i and 2i+1, the leaf of slot s node P2 + s.  Every internal node is RN32(left + right),
+// always recomputed from its children (never updated by deltas), so the tree's bits are a function of its leaves alone.  Unfilled
+// slots and the padding past cap are 0.  PRIO_HEADER_FLOATS floats in front of node 0 hold p_max and the arrival counter of
+// replay_prio_refresh_kernel.
+#define PRIO_HEADER_FLOATS 32
+#define PRIO_PMAX 0      // header float: the largest priority ever written (starts at 1)
+#define PRIO_ARRIVED 1   // header word: blocks of the running refresh launch that are done
+__host__ __device__ __forceinline__ long long prio_p2(long long cap) {
+  long long p = 1;
+  while (p < cap) p <<= 1;
+  return p;
+}
+__host__ __device__ __forceinline__ size_t prio_alloc_floats(long long cap) { return PRIO_HEADER_FLOATS + 2 * (size_t)prio_p2(cap); }
+__host__ __device__ __forceinline__ float* prio_header(float* tree) { return tree - PRIO_HEADER_FLOATS; }
+
+// prioritized minibatch row j of B of update `update`: U = u53(Philox(seed, id = j, ctr = update, stream PER)), x = RN32((j + U) root / B)
+// (stratified: one draw per B-th of the mass), then down from the root: left if x < L or R == 0, else x = RN32(x - L) and right.  A
+// subtree without mass is never entered, so the draw lands on a slot of positive priority even when x rounds up to the root.  Returns
+// the physical slot; *leaf = its priority.
+__host__ __device__ __forceinline__ long long ring_draw_prioritized(const float* tree, long long p2, uint64_t seed, uint64_t j, uint32_t update,
+                                                                   int B, float* leaf) {
+  uint32_t w[4];
+  philox4x32_10(seed, j, update, STREAM_PER, w);
+  float x = (float)(((double)j + u53(w[0], w[1])) * (double)tree[1] / (double)B);
+  long long n = 1;
+  while (n < p2) {
+    const float L = tree[2 * n], R = tree[2 * n + 1];
+    if (x < L || R == 0.0f) n = 2 * n;
+    else { x = x - L; n = 2 * n + 1; }
+  }
+  *leaf = tree[n];
+  return n - p2;
+}
+// logical index (0 = oldest) of physical slot `slot` of a ring of len records whose next push goes to slot head
+__host__ __device__ __forceinline__ long long ring_logical(long long slot, long long head, long long len, long long cap) {
+  long long li = (slot - head + len) % cap;
+  if (li < 0) li += cap;
+  return li;
+}
+// importance weight before the normalisation by the minibatch's largest: (leaf len / root)^-beta in Float64
+__host__ __device__ __forceinline__ double ring_is_weight(float leaf, long long len, float root, float beta) {
+  return pow((double)leaf * (double)len / (double)root, -(double)beta);
+}
+// priority of a row after its TD target: RN32((|RN32(y - q)| + eps)^alpha)
+__host__ __device__ __forceinline__ float ring_priority(float y, float q, float alpha, float eps) {
+  const float d = y - q;
+  return (float)pow((double)fabsf(d) + (double)eps, (double)alpha);
 }
 
 // the words both record forms store; a compact record adds its tag, a full one the other 14 fields

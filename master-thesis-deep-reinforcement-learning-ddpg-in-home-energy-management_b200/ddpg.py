@@ -60,6 +60,11 @@ class Replay:
         return int(self.lib.replay_capacity(self._h))
 
     @property
+    def head(self):
+        """physical slot of the next push"""
+        return int(self.lib.replay_head(self._h))
+
+    @property
     def series_copies(self):
         """env series the ring holds copies of (rollouts store compact records that point into them)"""
         return int(self.lib.replay_series_count(self._h))
@@ -95,6 +100,35 @@ class Replay:
             ip = idx.ctypes.data_as(L.PI)
         L.check(self.lib.replay_minmax(self._h, int(n_samples), ip, int(rng_mm) & (2**64 - 1), mn.ctypes.data_as(L.PF), mx.ctypes.data_as(L.PF)))
         return mn, mx
+
+    # ---- proportional prioritized replay (replay_enable_priorities): a sum tree of per-slot priorities beside the ring
+    def enable_priorities(self):
+        """every filled slot gets p_max (1 at first), every slot written from now on the p_max current at its write"""
+        L.check(self.lib.replay_enable_priorities(self._h))
+        self.prioritized = True
+        return self
+
+    prioritized = False
+
+    def priorities(self):
+        """(priorities [len] float32 in logical order, oldest first; p_max)"""
+        p, pm = np.empty(len(self), np.float32), C.c_float()
+        L.check(self.lib.replay_get_priorities(self._h, p.ctypes.data_as(L.PF), C.byref(pm)))
+        return p, pm.value
+
+    def set_priorities(self, prio, p_max):
+        """checkpoint restore: prio [len] in logical order (finite, >= 0, not all 0), p_max > 0; the tree is recomputed"""
+        p = np.ascontiguousarray(prio, np.float32)
+        assert p.size == len(self)
+        L.check(self.lib.replay_set_priorities(self._h, p.ctypes.data_as(L.PF), float(p_max)))
+
+    def sample_prioritized(self, batch, seed=0, beta=0.4):
+        """what update 0 of a prioritized Learner.replay(rng_rpl=seed) draws: (logical indices [B] int32, importance weights [B]
+        float32), device tensors"""
+        idx = torch.empty(batch, dtype=torch.int32, device=self._dev)
+        w = torch.empty(batch, dtype=torch.float32, device=self._dev)
+        L.check(self.lib.replay_sample_prioritized(self._h, int(batch), int(seed) & (2**64 - 1), float(beta), _ptr(idx), _ptr(w)))
+        return idx, w
 
     def get(self):
         n = len(self)
@@ -147,6 +181,21 @@ class Learner:
         if r < 0:
             L.check(r)
         return bool(r)
+
+    def set_prioritized(self, alpha=0.6, beta=0.4, eps=1e-6):
+        """ddpg_set_prioritized: proportional prioritized replay for every learner of the handle (alpha=None turns it off).
+        Updates then need memories with priorities (Replay.enable_priorities), one per learner."""
+        if alpha is None:
+            L.check(self.lib.ddpg_set_prioritized(self._h, 0, 0.0, 0.0, 0.0))
+        else:
+            L.check(self.lib.ddpg_set_prioritized(self._h, 1, float(alpha), float(beta), float(eps)))
+        return self
+
+    def get_prioritized(self):
+        """None, or {alpha, beta, eps} (float32 values)"""
+        on, a, b, e = C.c_int32(), C.c_float(), C.c_float(), C.c_float()
+        L.check(self.lib.ddpg_get_prioritized(self._h, C.byref(on), C.byref(a), C.byref(b), C.byref(e)))
+        return dict(alpha=a.value, beta=b.value, eps=e.value) if on.value else None
 
     def select(self, learner):
         """ddpg_select_learner: the learner of a population that set/get_layer, get_grad, set_norm and losses address."""
@@ -437,6 +486,22 @@ class Learner:
         return _wrap_device(p.value, (n.value,), torch.float32, self._dev, self)
 
 
+def per_beta(beta0, episode, num_ep):
+    """the importance-sampling exponent of training episode `episode` (1-based) of num_ep: linear from beta0 at the first to 1 at
+    the last (Schaul et al., 2016)"""
+    if episode >= num_ep:
+        return 1.0
+    return float(beta0) + (1.0 - float(beta0)) * (episode - 1) / (num_ep - 1)
+
+
+def _per_args(per):
+    """per = (alpha, beta0[, eps]) or dict(alpha, beta0, eps) -> dict, or None"""
+    if per is None:
+        return None
+    d = dict(per) if isinstance(per, dict) else dict(zip(("alpha", "beta0", "eps"), per))
+    return dict(alpha=float(d["alpha"]), beta0=float(d.get("beta0", 0.4)), eps=float(d.get("eps", 1e-6)))
+
+
 class Driver:
     """DDPG_reinforce_charger_v1.jl + DDPG.jl loop glue for N lock-stepped instances.
 
@@ -444,7 +509,9 @@ class Driver:
     (Julia's string-concatenated MersenneTwister seeds cannot be reproduced)."""
 
     def __init__(self, env_train, env_eval=None, learner=None, mem_size=24_000, ep_length=72, sigma=0.1, updates_per_step=1,
-                 rng_run=1231, noise_type="gn", theta=0.15, ou_dt=1e-2, native=True):
+                 rng_run=1231, noise_type="gn", theta=0.15, ou_dt=1e-2, native=True, per=None):
+        """per = (alpha, beta0[, eps]) or a dict of them: proportional prioritized replay, β annealed linearly from beta0 to 1
+        over the episodes of run_episodes (per_beta)"""
         self.env_train, self.env_eval = env_train, env_eval
         self.learner = learner if learner is not None else Learner(device=env_train.device)
         self.memory = Replay(mem_size, device=env_train.device)
@@ -458,6 +525,15 @@ class Driver:
         self.noise_type, self.theta, self.ou_dt = noise_type, float(theta), float(ou_dt)
         self._ou_x = None  # OUNoise.X per training instance; like the reference's global `ou` it is never reset (input.jl:234)
         self.learner.set_noise(noise_type, theta=self.theta, mu=0.0, dt=self.ou_dt)
+        self.per = _per_args(per)
+        if self.per is not None:
+            self.memory.enable_priorities()
+            self.learner.set_prioritized(self.per["alpha"], self.per["beta0"], self.per["eps"])
+
+    def set_beta(self, episode, num_ep):
+        """prioritized replay: β of training episode `episode` of num_ep (per_beta); run_episodes calls it before every episode"""
+        if self.per is not None:
+            self.learner.set_prioritized(self.per["alpha"], per_beta(self.per["beta0"], episode, num_ep), self.per["eps"])
 
     # populate_memory(env; rng) — memory_plotting_saving.jl:9-29 (fused random-policy rollouts)
     def populate_memory(self, rng=None):
@@ -547,6 +623,7 @@ class Driver:
                                                   score_mean=np.zeros(-(-num_ep // test_every)), best_run=0, best_score=-100000.0)
         for i in range(start_ep, num_ep + 1):
             rng_ep = self.rng_run * 100003 + i                                        # :252
+            self.set_beta(i, num_ep)
             r, _, nz = self.episode(self.env_train, train=True, rng_ep=rng_ep)        # :255
             st["total_reward"][i - 1] = r.cpu().numpy()
             st["noise_mean"][i - 1] = nz.cpu().numpy() if torch.is_tensor(nz) else nz
@@ -593,7 +670,8 @@ class PopulationDriver:
     chargers[l] is learner l's charger id (shems_LU1.jl:47-59), equal ids must be adjacent; seeds[l] its rng_run (input.jl:136).
     hparams: per-learner hyper-parameters, a dict of lists of length P with keys from Learner.HPARAMS (lr_actor, lr_critic, gamma,
     tau, noise_scale); missing keys keep the DdpgParams values (noise_scale: 1).  Learner l explores with σ_eff = sigma × noise_scale[l],
-    so a σ grid is sigma=1.0 with the grid values as noise_scale.
+    so a σ grid is sigma=1.0 with the grid values as noise_scale.  per = (alpha, beta0[, eps]): prioritized replay for every learner,
+    β annealed from beta0 to 1 over the episodes of run_episodes, as Driver(per=...).
 
     eval_series ([8][nrows], or [G][8][nrows] with one series per run of equal chargers) adds the reference's evaluation protocol
     (run_episodes / inference): an evaluation handle of test_runs instances per learner, one group per charger run, with
@@ -602,7 +680,7 @@ class PopulationDriver:
     instances of its charger, env_id_base 0), as every run of the reference evaluates with the same rng."""
 
     def __init__(self, series, chargers, seeds, n_envs=64, mem_size=24_000, ep_length=72, sigma=0.1, device=0, use_tensor_cores=1, native=True,
-                 hparams=None, eval_series=None, test_runs=100, **ddpg_kw):
+                 hparams=None, eval_series=None, test_runs=100, per=None, **ddpg_kw):
         from .env import Shems
         assert len(chargers) == len(seeds)
         self.native = bool(native)
@@ -627,6 +705,11 @@ class PopulationDriver:
             for l in range(self.P):
                 self.learner.select(l).set_hparams(**{k: v[l] for k, v in hparams.items()})
             self.learner.select(0)
+        self.per = _per_args(per)   # prioritized replay for every learner, as Driver(per=...)
+        if self.per is not None:
+            for m in self.mems:
+                m.enable_priorities()
+            self.learner.set_prioritized(self.per["alpha"], self.per["beta0"], self.per["eps"])
         self._dev = torch.device("cuda", int(device))
         self._s_prev = torch.empty((9, self.N), dtype=torch.float32, device=self._dev)
         self.n_env_steps = 0
@@ -642,6 +725,8 @@ class PopulationDriver:
                 ser_g = ev[g] if ev.ndim == 3 else ev
                 self._eval_starts.append((g0, m, Shems(ser_g.shape[-1] - 1, ser_g, n_envs=self.test_runs, charger_id=c, device=device)))
                 g0 += m * self.test_runs
+
+    set_beta = Driver.set_beta
 
     def reset_eval(self, rng):
         """reset!(env_eval; rng) with the same test_runs starts for every learner: each charger run's one-learner handle is reset
@@ -754,6 +839,7 @@ class PopulationDriver:
                     self.learner.set_layer(L.NET_ACTOR_BEST, k, np.zeros(i_ * o_, np.float32), np.zeros(o_, np.float32))
             self.learner.select(0)
         for i in range(start_ep, num_ep + 1):
+            self.set_beta(i, num_ep)
             r = self.episode(train=True, rng_ep=self.seeds[0] * 100003 + i)
             st["total_reward"][i - 1] = r.cpu().numpy()
             if (i - 1) % te == 0:

@@ -62,7 +62,8 @@ def save_checkpoint(path, learner, s_min=None, s_max=None, memories=None, **scor
     Chain), ADAM moments, β powers, update counter and normalisation constants (`l{l}_state`, `l{l}_opt`: ddpg_get_state),
     the hyper-parameters (`l{l}_hparams` = [lr_actor, lr_critic, gamma, tau, noise_scale] float32: ddpg_get_hparams), the best
     actors (`l{l}_actor_best_W1` ...) with `best_score` [P] / `best_run` [P] (ddpg_get_best; a score keyword of the same name
-    replaces them), OUNoise.X when OU episodes ran, and — with `memories` (one Replay per learner) — the replay memories in logical order."""
+    replaces them), OUNoise.X when OU episodes ran, and — with `memories` (one Replay per learner) — the replay memories in logical order,
+    with their priorities and p_max when they have them."""
     out = {}
     P = learner.population
     keep = getattr(learner, "_sel", 0)
@@ -98,6 +99,10 @@ def save_checkpoint(path, learner, s_min=None, s_max=None, memories=None, **scor
             S, A, R, S2, D = m.get()
             out[f"mem{l}_s"], out[f"mem{l}_a"], out[f"mem{l}_r"], out[f"mem{l}_s2"], out[f"mem{l}_done"] = S, A, R, S2, D
             out[f"mem{l}_capacity"] = np.int64(m.capacity)
+            if m.prioritized:   # the priorities, p_max and the ring's head (the tree's sums follow the slots' physical order)
+                out[f"mem{l}_prio"], pm = m.priorities()
+                out[f"mem{l}_pmax"] = np.float32(pm)
+                out[f"mem{l}_head"] = np.int64(m.head)
     if s_min is not None:
         out["s_min"], out["s_max"] = np.asarray(s_min, np.float32), np.asarray(s_max, np.float32)
     for k, v in scores.items():
@@ -144,6 +149,15 @@ def load_checkpoint(path, learner, memories=None):
         for l, m in enumerate(mems):
             assert len(m) == 0 and m.capacity == int(z[f"mem{l}_capacity"]), "restore into an empty memory of the saved capacity"
             dev = lambda x: torch.as_tensor(np.ascontiguousarray(x), device=m._dev)
-            if z[f"mem{l}_r"].size:
-                m.push(dev(z[f"mem{l}_s"]), dev(z[f"mem{l}_a"]), dev(z[f"mem{l}_r"]), dev(z[f"mem{l}_s2"]), dev(z[f"mem{l}_done"]))
+            rec = [z[f"mem{l}_{k}"] for k in ("s", "a", "r", "s2", "done")]
+            if f"mem{l}_head" in z and rec[2].size == m.capacity:
+                # a full memory whose oldest record sat at slot head: the first `head` pushes only move the ring there
+                head = int(z[f"mem{l}_head"])
+                if head:
+                    m.push(*[dev(x[..., :head]) for x in rec])
+            if rec[2].size:
+                m.push(*[dev(x) for x in rec])
+            if f"mem{l}_prio" in z:
+                m.enable_priorities()
+                m.set_priorities(z[f"mem{l}_prio"], float(z[f"mem{l}_pmax"]))
     return z

@@ -25,6 +25,7 @@ ap.add_argument("--seed", type=int, default=1231)
 ap.add_argument("--sigma", type=float, default=0.1)
 ap.add_argument("--tc", type=int, default=1, help="TF32 tensor cores for the 250x500 products")
 ap.add_argument("--noise", default="gn", choices=["gn", "ou"])
+ap.add_argument("--per", default=None, metavar="ALPHA,BETA0", help="prioritized replay, beta annealed from BETA0 to 1 over the episodes")
 args = ap.parse_args()
 
 train = sb.series.synth_charger98(4320, seed=98)
@@ -34,7 +35,7 @@ ev = sb.Shems(72, evals, n_envs=1024)          # evaluation: 1024 random 72-step
 le = sb.Learner(params=sb.default_ddpg_params(batch=args.batch, use_tensor_cores=args.tc))   # γ=0.99, τ=1e-3, η=1e-4/1e-3, 250/500 (README.md:68-86)
 le.init(args.seed)
 drv = sb.Driver(env, ev, learner=le, mem_size=args.mem, ep_length=72, sigma=args.sigma, updates_per_step=args.updates_per_step,
-                rng_run=args.seed, noise_type=args.noise)
+                rng_run=args.seed, noise_type=args.noise, per=tuple(float(x) for x in args.per.split(",")) if args.per else None)
 t0 = time.time()
 drv.populate_memory()
 drv.min_max_buffer()
@@ -56,6 +57,7 @@ print(json.dumps(hist[-1]), flush=True)
 t1 = time.time()
 steps0 = drv.n_env_steps
 for ep in range(1, args.episodes + 1):
+    drv.set_beta(ep, args.episodes)
     r, _, _ = drv.episode(env, train=True, rng_ep=args.seed * 100003 + ep)
     if ep % args.eval_every == 0 or ep == args.episodes:
         lc, la = le.losses()

@@ -38,6 +38,7 @@ ap.add_argument("--test-every", type=int, default=0, help="evaluate every K epis
 ap.add_argument("--test-runs", type=int, default=100, help="evaluation episodes per learner and round")
 ap.add_argument("--inference-dir", default=None, help="write the test-set inference CSVs of the best actors here (needs --test-every)")
 ap.add_argument("--pbt", default=None, metavar="EVERY,FRAC", help="population-based training every EVERY evaluation rounds, share FRAC (needs --test-every)")
+ap.add_argument("--per", default=None, metavar="ALPHA,BETA0", help="prioritized replay for every learner, beta annealed from BETA0 to 1")
 ap.add_argument("--pbt-factors", default="0.8,1.25", metavar="LO,HI", help="perturbation factors of --pbt")
 ap.add_argument("--pbt-keys", default=",".join(sb.Learner.HPARAMS), metavar="NAME,...", help="hyper-parameters --pbt perturbs")
 args = ap.parse_args()
@@ -77,6 +78,8 @@ if args.pbt:
     pbt = dict(every=int(p_every), frac=float(p_frac), factors=(lo, hi), keys=tuple(k for k in args.pbt_keys.split(",") if k), seed=rank)
 if protocol:
     drv_kw.update(eval_series=sb.series.synth_charger98(1440, seed=1440), test_runs=args.test_runs)
+if args.per:
+    drv_kw["per"] = tuple(float(x) for x in args.per.split(","))
 drv = sb.PopulationDriver(ser, chargers=chargers, seeds=seeds, n_envs=args.envs, device=local, use_tensor_cores=args.tc, hparams=hparams, **drv_kw)
 t0 = time.time()
 drv.populate_memory()
@@ -121,6 +124,7 @@ if protocol:   # run_episodes: training episodes with an evaluation round every 
                                     for i, pt in enumerate(points) if (gi == i).any()])), flush=True)
     sys.exit(0)
 for ep in range(1, args.episodes + 1):
+    drv.set_beta(ep, args.episodes)
     r = drv.episode(train=True, rng_ep=ep)
     if args.eval_every and ep % args.eval_every == 0:
         torch.cuda.synchronize()
