@@ -90,25 +90,15 @@ actor_rollout_kernel(const ActorRolloutArgs a) {
       StepTrace tr;
       const StepOut so = shems_flows<WANT_TRACE, false>(a.P, s, B, EV, o.s1, false, &tr);
       const int idx = s_idx[r];
-      const float4 ra = __ldg(a.series + 2 * (size_t)idx), rb = __ldg(a.series + 2 * (size_t)idx + 1);   // row idx + 1 (next_state! :264-281)
-      float Soc_ev_new = so.Soc_ev;
-      if (ra.y >= 0.0f && s_cd[r] == -1.0f) Soc_ev_new = ra.x;   // EV newly connected :270-272
+      const Row8 nx = load_row(a.series, idx + 1);   // next_state! :264-281
+      const float Soc_ev_new = next_soc_ev(so.Soc_ev, nx, s_cd[r]);
       if (g.rank == 0) {
-        if (WANT_TRACE) {  // the `results` row :476-478
-          double* q = a.trace + (size_t)t * SHEMS_TRACE_COLS * N + j;
-          q[SHEMS_T_INDEX * N] = (double)(idx + 1); q[SHEMS_T_C_EV * N] = (double)s.c_ev; q[SHEMS_T_EV_TARGET * N] = (double)o.s1;
-          q[SHEMS_T_EV * N] = tr.EV; q[SHEMS_T_SOC_EV * N] = (double)s.Soc_ev; q[SHEMS_T_REWARD * N] = so.reward;
-          q[SHEMS_T_PROFIT * N] = tr.profit; q[SHEMS_T_DISCOMFORT * N] = tr.discomfort; q[SHEMS_T_PENALTY * N] = tr.penalty;
-          q[SHEMS_T_PV_DE * N] = tr.PV_DE; q[SHEMS_T_B_DE * N] = tr.B_DE; q[SHEMS_T_GR_DE * N] = tr.GR_DE; q[SHEMS_T_PV_B * N] = tr.PV_B;
-          q[SHEMS_T_PV_GR * N] = tr.PV_GR; q[SHEMS_T_PV_EV * N] = tr.PV_EV; q[SHEMS_T_B_EV * N] = tr.B_EV; q[SHEMS_T_GR_EV * N] = tr.GR_EV;
-          q[SHEMS_T_EX_EV * N] = tr.EX_EV; q[SHEMS_T_GR_B * N] = 0.0; q[SHEMS_T_B_GR * N] = 0.0; q[SHEMS_T_B * N] = tr.B;
-          q[SHEMS_T_B_TARGET * N] = (double)o.s0; q[SHEMS_T_SOC_B * N] = (double)s.Soc_b;
-        }
+        if (WANT_TRACE) store_trace_row(a.trace + (size_t)t * SHEMS_TRACE_COLS * N + j, N, idx, s, o.s0, o.s1, so, tr);
         if (a.act_traj) { a.act_traj[((size_t)t * 2 + 0) * N + j] = o.a0; a.act_traj[((size_t)t * 2 + 1) * N + j] = o.a1; }
       }
-      raw[r * 12 + 0] = so.Soc_b; raw[r * 12 + 1] = Soc_ev_new; raw[r * 12 + 2] = ra.y; raw[r * 12 + 3] = ra.z; raw[r * 12 + 4] = ra.w;
-      raw[r * 12 + 5] = rb.x; raw[r * 12 + 6] = rb.y; raw[r * 12 + 7] = rb.z; raw[r * 12 + 8] = rb.w;
-      s_cd[r] = ra.y;
+      raw[r * 12 + 0] = so.Soc_b; raw[r * 12 + 1] = Soc_ev_new; raw[r * 12 + 2] = nx.cd; raw[r * 12 + 3] = nx.d_e; raw[r * 12 + 4] = nx.g_e;
+      raw[r * 12 + 5] = nx.p_buy; raw[r * 12 + 6] = nx.h_cos; raw[r * 12 + 7] = nx.h_sin; raw[r * 12 + 8] = nx.season;
+      s_cd[r] = nx.cd;
       s_idx[r] = idx + 1;
       s_ret[r] += so.reward;   // reward_eps += r, Float64 (DDPG.jl:223)
     }

@@ -165,16 +165,6 @@ static DevParams make_dev_params(const ShemsParams& p) {
   return d;
 }
 
-// ----------------------------------------------------------------------------- series rows
-struct Row8 { float soc_ev, cd, d_e, g_e, p_buy, h_cos, h_sin, season; };
-__device__ __forceinline__ Row8 load_row(const float4* __restrict__ series, int row1 /*1-based*/) {
-  const float4 a = __ldg(series + 2 * (size_t)(row1 - 1));
-  const float4 b = __ldg(series + 2 * (size_t)(row1 - 1) + 1);
-  Row8 r;
-  r.soc_ev = a.x; r.cd = a.y; r.d_e = a.z; r.g_e = a.w; r.p_buy = b.x; r.h_cos = b.y; r.h_sin = b.z; r.season = b.w;
-  return r;
-}
-
 // ----------------------------------------------------------------------------- reset
 // reset!/reset_state! (shems_LU1.jl:206-262).  mode: SHEMS_RESET_*.
 __global__ void __launch_bounds__(256)
@@ -214,15 +204,7 @@ shems_reset_kernel(DevParams P, const float4* __restrict__ series, int nrows, in
       }
     }
     const Row8 r = load_row(series, idx);  // :251-260
-    obs[0 * N + n] = Soc_b;
-    obs[1 * N + n] = r.soc_ev;
-    obs[2 * N + n] = r.cd;
-    obs[3 * N + n] = r.d_e;
-    obs[4 * N + n] = r.g_e;
-    obs[5 * N + n] = r.p_buy;
-    obs[6 * N + n] = r.h_cos;
-    obs[7 * N + n] = r.h_sin;
-    obs[8 * N + n] = r.season;
+    store_obs(obs, N, n, Soc_b, r.soc_ev, r);
     idx_out[n] = idx;
   }
   // max idx of the block -> one atomic (bounds pre-check of the following steps)
@@ -275,35 +257,13 @@ shems_step_kernel(DevParams P, const float4* __restrict__ series, long long N, f
   const StepOut o = shems_flows<WANT_TRACE, FAST>(P, s, B, EV, EVt, track_neg != 0, &tr);
   // next_state! :264-281
   const Row8 nx = load_row(series, idx + 1);
-  float Soc_ev_new = o.Soc_ev;
-  if (nx.cd >= 0.0f && cd_here == -1.0f) Soc_ev_new = nx.soc_ev;  // EV newly connected :270-272
-  obs[0 * N + n] = o.Soc_b;
-  obs[1 * N + n] = Soc_ev_new;
-  obs[2 * N + n] = nx.cd;
-  obs[3 * N + n] = nx.d_e;
-  obs[4 * N + n] = nx.g_e;
-  obs[5 * N + n] = nx.p_buy;
-  obs[6 * N + n] = nx.h_cos;
-  obs[7 * N + n] = nx.h_sin;
-  obs[8 * N + n] = nx.season;
+  const float Soc_ev_new = next_soc_ev(o.Soc_ev, nx, cd_here);
+  store_obs(obs, N, n, o.Soc_b, Soc_ev_new, nx);
   idx_arr[n] = idx + 1;  // :456
   if (reward_out) reward_out[n] = (float)o.reward;
   if (reward64_out) reward64_out[n] = o.reward;  // env.reward::Float64 (:171, :467-470)
-  if (obs_out) {
-    obs_out[0 * N + n] = o.Soc_b; obs_out[1 * N + n] = Soc_ev_new; obs_out[2 * N + n] = nx.cd; obs_out[3 * N + n] = nx.d_e;
-    obs_out[4 * N + n] = nx.g_e; obs_out[5 * N + n] = nx.p_buy; obs_out[6 * N + n] = nx.h_cos; obs_out[7 * N + n] = nx.h_sin;
-    obs_out[8 * N + n] = nx.season;
-  }
-  if (WANT_TRACE) {  // :476-478
-    double* t = trace + n;
-    t[SHEMS_T_INDEX * N] = (double)(idx + 1); t[SHEMS_T_C_EV * N] = (double)s.c_ev; t[SHEMS_T_EV_TARGET * N] = (double)EVt;
-    t[SHEMS_T_EV * N] = tr.EV; t[SHEMS_T_SOC_EV * N] = (double)s.Soc_ev; t[SHEMS_T_REWARD * N] = o.reward;
-    t[SHEMS_T_PROFIT * N] = tr.profit; t[SHEMS_T_DISCOMFORT * N] = tr.discomfort; t[SHEMS_T_PENALTY * N] = tr.penalty;
-    t[SHEMS_T_PV_DE * N] = tr.PV_DE; t[SHEMS_T_B_DE * N] = tr.B_DE; t[SHEMS_T_GR_DE * N] = tr.GR_DE; t[SHEMS_T_PV_B * N] = tr.PV_B;
-    t[SHEMS_T_PV_GR * N] = tr.PV_GR; t[SHEMS_T_PV_EV * N] = tr.PV_EV; t[SHEMS_T_B_EV * N] = tr.B_EV; t[SHEMS_T_GR_EV * N] = tr.GR_EV;
-    t[SHEMS_T_EX_EV * N] = tr.EX_EV; t[SHEMS_T_GR_B * N] = 0.0; t[SHEMS_T_B_GR * N] = 0.0; t[SHEMS_T_B * N] = tr.B;
-    t[SHEMS_T_B_TARGET * N] = (double)Bt; t[SHEMS_T_SOC_B * N] = (double)s.Soc_b;
-  }
+  if (obs_out) store_obs(obs_out, N, n, o.Soc_b, Soc_ev_new, nx);
+  if (WANT_TRACE) store_trace_row(trace + n, N, idx, s, Bt, EVt, o, tr);
 }
 
 // action(env, track) / action(env, a) for all instances
@@ -345,6 +305,40 @@ struct RolloutSinks {
 // MINB = resident CTAs per SM the register budget is cut for (6: 80 registers, 7: 72, 8: 64).  6 is the fastest per wave; 7 or 8 are
 // chosen when they save a mostly empty last wave (e.g. 2^20 instances over 8 GPUs = 1024 CTAs per GPU: 1.15 waves of 148 x 6 CTAs,
 // but ONE wave of 148 x 7) — see rollout_min_blocks().
+// The rollout policy's action for instance n at step t of a launch, from state s on a row of class CLS: the feasible (B, EV), the
+// targets (Bt, EVt) step! records, the action remember() stores (a_raw) and track < 0.  The random policy takes Philox words w0, w1.
+struct RolloutAction { float B, EV, Bt, EVt, a_raw0, a_raw1; bool track_neg; };
+template <int POLICY, bool FAST, int CLS = ROW_ANY>
+__device__ __forceinline__ RolloutAction rollout_action(const DevParams& P, const StepIn& s, uint32_t w0, uint32_t w1,
+                                                        const float* __restrict__ tape, int tape_unscaled, long long N, long long n, int t) {
+  RolloutAction a;
+  a.track_neg = false;
+  if (POLICY == SHEMS_POLICY_RULE) {  // DDPG.jl:209-212
+    shems_action_rule<FAST>(P, s.Soc_b, s.Soc_ev, s.d_e, s.g_e, a.B, a.EV);
+    a.Bt = 0.0f; a.EVt = 0.0f; a.a_raw0 = a.B; a.a_raw1 = a.EV; a.track_neg = true;
+    return a;
+  }
+  if (POLICY == SHEMS_POLICY_RANDOM) {  // memory_plotting_saving.jl:14-19: u = w * 2^-32; a = Float32(2u - 1) (action_from_word, philox.cuh)
+    a.a_raw0 = action_from_word(w0);
+    a.a_raw1 = action_from_word(w1);
+    // scale_action with bounds (0,0)/(1,1) (DDPG.jl:178-184, input.jl:182-183): Float32((Float64(a) + 1.0) * 0.5).
+    // a is a multiple of 2^-31, so a + 1.0 and the halving are exact in Float64 and the single final rounding
+    // equals the Float32 add followed by the exact halving.
+    a.Bt = (a.a_raw0 + 1.0f) * 0.5f;
+    a.EVt = (a.a_raw1 + 1.0f) * 0.5f;
+  } else {
+    a.Bt = tape[((size_t)t * 2 + 0) * N + n];
+    a.EVt = tape[((size_t)t * 2 + 1) * N + n];
+    a.a_raw0 = a.Bt; a.a_raw1 = a.EVt;
+    if (tape_unscaled) {  // the tape holds what `remember` stores (DDPG.jl:229): a in [-1,1]; scale_action with bounds (0,0)/(1,1)
+      a.Bt = (float)(((double)a.a_raw0 + 1.0) * 0.5);   // Float32.(lo .+ (a .+ ones(2)) .* 0.5 .* (hi .- lo))  (:178-184)
+      a.EVt = (float)(((double)a.a_raw1 + 1.0) * 0.5);
+    }
+  }
+  shems_action_drl<FAST, CLS>(P, s.Soc_b, s.Soc_ev, s.c_ev, s.d_e, s.g_e, a.Bt, a.EVt, a.B, a.EV);
+  return a;
+}
+
 // COMPACT: the ring sink stores 8 words per transition (Soc_b, Soc_ev, a, r, Soc_b', Soc_ev', series tag; ring.cuh) instead of 23 —
 // only when s[2..8] is series row idx, i.e. the env is consistent.
 template <int POLICY, bool WANT_TRACE, int MINB, bool FAST, bool COMPACT>
@@ -366,63 +360,31 @@ shems_rollout_kernel(DevParams P, const float4* __restrict__ series, long long N
   for (int t = 0; t < T; ++t) {
     StepIn s;
     s.Soc_b = st[0]; s.Soc_ev = st[1]; s.c_ev = st[2]; s.d_e = st[3]; s.g_e = st[4]; s.p_buy = st[5];
-    float B, EV, Bt, EVt, a_raw0, a_raw1;
-    bool track_neg = false;
-    if (POLICY == SHEMS_POLICY_RULE) {  // DDPG.jl:209-212
-      shems_action_rule<FAST>(P, s.Soc_b, s.Soc_ev, s.d_e, s.g_e, B, EV);
-      Bt = 0.0f; EVt = 0.0f; a_raw0 = B; a_raw1 = EV; track_neg = true;
-    } else {
-      if (POLICY == SHEMS_POLICY_RANDOM) {  // memory_plotting_saving.jl:14-19
-        // one Philox block per two steps; u = w * 2^-32; a = Float32(2u - 1) (action_from_word, philox.cuh)
-        const unsigned st_abs = (unsigned)(step0 + t);
-        if (t == 0 || (st_abs & 1u) == 0u) philox4x32_10(seed, (uint64_t)(env_id_base + n), st_abs >> 1, STREAM_ACTION, rw);
-        const uint32_t w0 = (st_abs & 1u) ? rw[2] : rw[0], w1 = (st_abs & 1u) ? rw[3] : rw[1];
-        a_raw0 = action_from_word(w0);
-        a_raw1 = action_from_word(w1);
-        // scale_action with bounds (0,0)/(1,1) (DDPG.jl:178-184, input.jl:182-183): Float32((Float64(a) + 1.0) * 0.5).
-        // a is a multiple of 2^-31, so a + 1.0 and the halving are exact in Float64 and the single final rounding
-        // equals the Float32 add followed by the exact halving.
-        Bt = (a_raw0 + 1.0f) * 0.5f;
-        EVt = (a_raw1 + 1.0f) * 0.5f;
-      } else {
-        Bt = tape[((size_t)t * 2 + 0) * N + n];
-        EVt = tape[((size_t)t * 2 + 1) * N + n];
-        a_raw0 = Bt; a_raw1 = EVt;
-        if (tape_unscaled) {  // the tape holds what `remember` stores (DDPG.jl:229): a in [-1,1]; scale_action with bounds (0,0)/(1,1)
-          Bt = (float)(((double)a_raw0 + 1.0) * 0.5);   // Float32.(lo .+ (a .+ ones(2)) .* 0.5 .* (hi .- lo))  (:178-184)
-          EVt = (float)(((double)a_raw1 + 1.0) * 0.5);
-        }
-      }
-      shems_action_drl<FAST>(P, s.Soc_b, s.Soc_ev, s.c_ev, s.d_e, s.g_e, Bt, EVt, B, EV);
+    uint32_t w0 = 0u, w1 = 0u;
+    if (POLICY == SHEMS_POLICY_RANDOM) {  // one Philox block per two steps: words 0..1 serve the even step, words 2..3 the odd one
+      const unsigned st_abs = (unsigned)(step0 + t);
+      if (t == 0 || (st_abs & 1u) == 0u) philox4x32_10(seed, (uint64_t)(env_id_base + n), st_abs >> 1, STREAM_ACTION, rw);
+      w0 = (st_abs & 1u) ? rw[2] : rw[0]; w1 = (st_abs & 1u) ? rw[3] : rw[1];
     }
+    const RolloutAction a = rollout_action<POLICY, FAST>(P, s, w0, w1, tape, tape_unscaled, N, n, t);
     StepTrace tr;
-    const StepOut o = shems_flows<WANT_TRACE, FAST>(P, s, B, EV, EVt, track_neg, &tr);
+    const StepOut o = shems_flows<WANT_TRACE, FAST>(P, s, a.B, a.EV, a.EVt, a.track_neg, &tr);
     const Row8 nx = load_row(series, idx + 1);
-    float Soc_ev_new = o.Soc_ev;
-    if (nx.cd >= 0.0f && cd_here == -1.0f) Soc_ev_new = nx.soc_ev;
+    const float Soc_ev_new = next_soc_ev(o.Soc_ev, nx, cd_here);
     if (S.ring) {  // remember(s, a, r, s', finished) — memory_plotting_saving.jl:46-47; stores at fixed 128-byte strides
       float* q = S.ring + ring_base(slot);
       if (COMPACT) {  // s[2..8] = series row idx, s'[2..8] = row idx + 1, done = 0: the tag names them
-        ring_store_compact(q, st[0], st[1], a_raw0, a_raw1, (float)o.reward, o.Soc_b, Soc_ev_new, S.src_entry, idx);
+        ring_store_compact(q, st[0], st[1], a.a_raw0, a.a_raw1, (float)o.reward, o.Soc_b, Soc_ev_new, S.src_entry, idx);
       } else {
         // sv copies st: passing st itself takes its address, and the kernel then compiles to a different register allocation
         const float sv[9] = {st[0], st[1], st[2], st[3], st[4], st[5], st[6], st[7], st[8]};
         const float s2v[9] = {o.Soc_b, Soc_ev_new, nx.cd, nx.d_e, nx.g_e, nx.p_buy, nx.h_cos, nx.h_sin, nx.season};
-        ring_store_full(q, sv, a_raw0, a_raw1, (float)o.reward, s2v, 0.0f);  // finished() is always false (shems_LU1.jl:487-502)
+        ring_store_full(q, sv, a.a_raw0, a.a_raw1, (float)o.reward, s2v, 0.0f);  // finished() is always false (shems_LU1.jl:487-502)
       }
       slot += N;
       if (slot >= S.cap) slot -= S.cap;
     }
-    if (WANT_TRACE) {
-      double* q = S.trace + (size_t)t * SHEMS_TRACE_COLS * N + n;
-      q[SHEMS_T_INDEX * N] = (double)(idx + 1); q[SHEMS_T_C_EV * N] = (double)s.c_ev; q[SHEMS_T_EV_TARGET * N] = (double)EVt;
-      q[SHEMS_T_EV * N] = tr.EV; q[SHEMS_T_SOC_EV * N] = (double)s.Soc_ev; q[SHEMS_T_REWARD * N] = o.reward;
-      q[SHEMS_T_PROFIT * N] = tr.profit; q[SHEMS_T_DISCOMFORT * N] = tr.discomfort; q[SHEMS_T_PENALTY * N] = tr.penalty;
-      q[SHEMS_T_PV_DE * N] = tr.PV_DE; q[SHEMS_T_B_DE * N] = tr.B_DE; q[SHEMS_T_GR_DE * N] = tr.GR_DE; q[SHEMS_T_PV_B * N] = tr.PV_B;
-      q[SHEMS_T_PV_GR * N] = tr.PV_GR; q[SHEMS_T_PV_EV * N] = tr.PV_EV; q[SHEMS_T_B_EV * N] = tr.B_EV; q[SHEMS_T_GR_EV * N] = tr.GR_EV;
-      q[SHEMS_T_EX_EV * N] = tr.EX_EV; q[SHEMS_T_GR_B * N] = 0.0; q[SHEMS_T_B_GR * N] = 0.0; q[SHEMS_T_B * N] = tr.B;
-      q[SHEMS_T_B_TARGET * N] = (double)Bt; q[SHEMS_T_SOC_B * N] = (double)s.Soc_b;
-    }
+    if (WANT_TRACE) store_trace_row(S.trace + (size_t)t * SHEMS_TRACE_COLS * N + n, N, idx, s, a.Bt, a.EVt, o, tr);
     st[0] = o.Soc_b; st[1] = Soc_ev_new; st[2] = nx.cd; st[3] = nx.d_e; st[4] = nx.g_e; st[5] = nx.p_buy;
     st[6] = nx.h_cos; st[7] = nx.h_sin; st[8] = nx.season;
     cd_here = nx.cd;
@@ -455,6 +417,32 @@ shems_rollout_kernel(DevParams P, const float4* __restrict__ series, long long N
 // When the host knows that every instance of the launch stands on one row (ShemsEnv::uniform_row) and the grid is large enough,
 // shems_rollout_pair_kernel below runs this lock-step loop with two instances per thread instead (profiles/r10_pair_rollout.md).
 template <int CLS> struct RowTag { static constexpr int value = CLS; };
+// f(RowTag<cls>{}): the body of f compiled for the row class cls
+template <class F>
+__device__ __forceinline__ void with_row_class(int cls, F&& f) {
+  switch (cls) {
+    case ROW_A_NOEV: f(RowTag<ROW_A_NOEV>{}); break;
+    case ROW_B_NOEV: f(RowTag<ROW_B_NOEV>{}); break;
+    case ROW_A_EV: f(RowTag<ROW_A_EV>{}); break;
+    case ROW_B_EV: f(RowTag<ROW_B_EV>{}); break;
+    default: f(RowTag<ROW_ANY>{}); break;
+  }
+}
+// The lock-step loops' random words for step t of I consecutive instances (Philox ids id, id + 1, ...): rw holds I blocks of 4 words,
+// and words 0..1 of block i serve instance i.  Block (step0 + t) / 2 is drawn on an even step (and at t = 0); an odd step moves its
+// words 2..3 to 0..1.  rw is a flat pointer: taken as an array of I blocks, the trimmed kernel's random-policy builds compile differently.
+template <int I>
+__device__ __forceinline__ void lockstep_words(const PhiloxKeys& K, uint64_t id, int step0, int t, uint32_t* rw) {
+  const unsigned st_abs = (unsigned)(step0 + t);
+  if ((st_abs & 1u) == 0u || t == 0) {
+#pragma unroll
+    for (int i = 0; i < I; ++i) philox4x32_10(K, id + i, st_abs >> 1, STREAM_ACTION, rw + 4 * i);
+  }
+  if (st_abs & 1u) {
+#pragma unroll
+    for (int i = 0; i < I; ++i) { rw[4 * i + 0] = rw[4 * i + 2]; rw[4 * i + 1] = rw[4 * i + 3]; }
+  }
+}
 template <int POLICY, int MINB>
 __global__ void __launch_bounds__(ROLLOUT_THREADS, MINB)
 shems_rollout_lean_kernel(DevParams P, const float4* __restrict__ series, long long N, float* __restrict__ obs,
@@ -474,35 +462,13 @@ shems_rollout_lean_kernel(DevParams P, const float4* __restrict__ series, long l
     constexpr int CLS = decltype(cls)::value;
     StepIn s;
     s.Soc_b = Soc_b; s.Soc_ev = Soc_ev; s.c_ev = c_ev; s.d_e = d_e; s.g_e = g_e; s.p_buy = p_buy;
-    float B, EV, Bt, EVt, a_raw0, a_raw1;
-    bool track_neg = false;
-    if (POLICY == SHEMS_POLICY_RULE) {
-      shems_action_rule<true>(P, s.Soc_b, s.Soc_ev, s.d_e, s.g_e, B, EV);
-      Bt = 0.0f; EVt = 0.0f; a_raw0 = B; a_raw1 = EV; track_neg = true;
-    } else {
-      if (POLICY == SHEMS_POLICY_RANDOM) {
-        a_raw0 = action_from_word(w0);
-        a_raw1 = action_from_word(w1);
-        Bt = (a_raw0 + 1.0f) * 0.5f;
-        EVt = (a_raw1 + 1.0f) * 0.5f;
-      } else {
-        Bt = tape[((size_t)t * 2 + 0) * N + n];
-        EVt = tape[((size_t)t * 2 + 1) * N + n];
-        a_raw0 = Bt; a_raw1 = EVt;
-        if (tape_unscaled) {
-          Bt = (float)(((double)a_raw0 + 1.0) * 0.5);
-          EVt = (float)(((double)a_raw1 + 1.0) * 0.5);
-        }
-      }
-      shems_action_drl<true, CLS>(P, s.Soc_b, s.Soc_ev, s.c_ev, s.d_e, s.g_e, Bt, EVt, B, EV);
-    }
+    const RolloutAction a = rollout_action<POLICY, true, CLS>(P, s, w0, w1, tape, tape_unscaled, N, n, t);
     StepTrace tr;
-    const StepOut o = shems_flows<false, true, CLS>(P, s, B, EV, EVt, track_neg, &tr);
+    const StepOut o = shems_flows<false, true, CLS>(P, s, a.B, a.EV, a.EVt, a.track_neg, &tr);
     const Row8 nx = load_row(series, idx + 1);
-    float Soc_ev_new = o.Soc_ev;
-    if (nx.cd >= 0.0f && (CLS == ROW_ANY ? c_ev == -1.0f : row_noev<CLS>)) Soc_ev_new = nx.soc_ev;
+    const float Soc_ev_new = next_soc_ev<CLS>(o.Soc_ev, nx, c_ev);
     if (S.ring) {
-      ring_store_compact(ring.q, Soc_b, Soc_ev, a_raw0, a_raw1, (float)o.reward, o.Soc_b, Soc_ev_new, S.src_entry, idx);
+      ring_store_compact(ring.q, Soc_b, Soc_ev, a.a_raw0, a.a_raw1, (float)o.reward, o.Soc_b, Soc_ev_new, S.src_entry, idx);
       ring_walk_next(ring);
     }
     if (S.reward_traj) S.reward_traj[(size_t)t * N + n] = (float)o.reward;
@@ -515,18 +481,8 @@ shems_rollout_lean_kernel(DevParams P, const float4* __restrict__ series, long l
   if (lockstep && __all_sync(mask, idx == __shfl_sync(mask, idx, __ffs(mask) - 1))) {
     uint32_t rw[4] = {0u, 0u, 0u, 0u};
     for (int t = 0; t < T; ++t) {
-      if (POLICY == SHEMS_POLICY_RANDOM) {  // words 0..1 of block (step0 + t) / 2 serve even steps, words 2..3 odd ones
-        const unsigned st_abs = (unsigned)(step0 + t);
-        if ((st_abs & 1u) == 0u || t == 0) philox4x32_10(K, id, st_abs >> 1, STREAM_ACTION, rw);
-        if (st_abs & 1u) { rw[0] = rw[2]; rw[1] = rw[3]; }
-      }
-      switch (row_class(P, c_ev, d_e, g_e)) {
-        case ROW_A_NOEV: step(RowTag<ROW_A_NOEV>{}, t, rw[0], rw[1]); break;
-        case ROW_B_NOEV: step(RowTag<ROW_B_NOEV>{}, t, rw[0], rw[1]); break;
-        case ROW_A_EV: step(RowTag<ROW_A_EV>{}, t, rw[0], rw[1]); break;
-        case ROW_B_EV: step(RowTag<ROW_B_EV>{}, t, rw[0], rw[1]); break;
-        default: step(RowTag<ROW_ANY>{}, t, rw[0], rw[1]); break;
-      }
+      if (POLICY == SHEMS_POLICY_RANDOM) lockstep_words<1>(K, id, step0, t, rw);
+      with_row_class(row_class(P, c_ev, d_e, g_e), [&](auto cls) { step(cls, t, rw[0], rw[1]); });
     }
   } else {
     // t is the step that uses words 0..1 of the block; with an odd step0 the first block's words 0..1 belong to step -1
@@ -537,9 +493,7 @@ shems_rollout_lean_kernel(DevParams P, const float4* __restrict__ series, long l
       if (t + 1 < T) step(RowTag<ROW_ANY>{}, t + 1, rw[2], rw[3]);
     }
   }
-  const Row8 r = load_row(series, idx);
-  obs[0 * N + n] = Soc_b; obs[1 * N + n] = Soc_ev; obs[2 * N + n] = r.cd; obs[3 * N + n] = r.d_e; obs[4 * N + n] = r.g_e;
-  obs[5 * N + n] = r.p_buy; obs[6 * N + n] = r.h_cos; obs[7 * N + n] = r.h_sin; obs[8 * N + n] = r.season;
+  store_obs(obs, N, n, Soc_b, Soc_ev, load_row(series, idx));
   idx_arr[n] = idx;
   if (S.ep_return) S.ep_return[n] = ret;
 }
@@ -573,31 +527,11 @@ shems_rollout_pair_kernel(DevParams P, const float4* __restrict__ series, long l
     for (int i = 0; i < 2; ++i) {
       StepIn s;
       s.Soc_b = Soc_b[i]; s.Soc_ev = Soc_ev[i]; s.c_ev = c_ev; s.d_e = d_e; s.g_e = g_e; s.p_buy = p_buy;
-      float B, EV, Bt, EVt;
-      bool track_neg = false;
-      if (POLICY == SHEMS_POLICY_RULE) {
-        shems_action_rule<true>(P, s.Soc_b, s.Soc_ev, s.d_e, s.g_e, B, EV);
-        Bt = 0.0f; EVt = 0.0f; a_raw0[i] = B; a_raw1[i] = EV; track_neg = true;
-      } else {
-        if (POLICY == SHEMS_POLICY_RANDOM) {
-          a_raw0[i] = action_from_word(rw[i][0]);
-          a_raw1[i] = action_from_word(rw[i][1]);
-          Bt = (a_raw0[i] + 1.0f) * 0.5f;
-          EVt = (a_raw1[i] + 1.0f) * 0.5f;
-        } else {
-          Bt = tape[((size_t)t * 2 + 0) * N + n + i];
-          EVt = tape[((size_t)t * 2 + 1) * N + n + i];
-          a_raw0[i] = Bt; a_raw1[i] = EVt;
-          if (tape_unscaled) {
-            Bt = (float)(((double)a_raw0[i] + 1.0) * 0.5);
-            EVt = (float)(((double)a_raw1[i] + 1.0) * 0.5);
-          }
-        }
-        shems_action_drl<true, CLS>(P, s.Soc_b, s.Soc_ev, s.c_ev, s.d_e, s.g_e, Bt, EVt, B, EV);
-      }
+      const RolloutAction a = rollout_action<POLICY, true, CLS>(P, s, rw[i][0], rw[i][1], tape, tape_unscaled, N, n + i, t);
+      a_raw0[i] = a.a_raw0; a_raw1[i] = a.a_raw1;
       StepTrace tr;
-      const StepOut o = shems_flows<false, true, CLS>(P, s, B, EV, EVt, track_neg, &tr);
-      Soc_ev2[i] = (nx.cd >= 0.0f && (CLS == ROW_ANY ? c_ev == -1.0f : row_noev<CLS>)) ? nx.soc_ev : o.Soc_ev;
+      const StepOut o = shems_flows<false, true, CLS>(P, s, a.B, a.EV, a.EVt, a.track_neg, &tr);
+      Soc_ev2[i] = next_soc_ev<CLS>(o.Soc_ev, nx, c_ev);
       Soc_b2[i] = o.Soc_b;
       r32[i] = (float)o.reward;
       ret[i] += o.reward;
@@ -614,38 +548,28 @@ shems_rollout_pair_kernel(DevParams P, const float4* __restrict__ series, long l
   };
   uint32_t rw[2][4] = {};
   for (int t = 0; t < T; ++t) {
-    if (POLICY == SHEMS_POLICY_RANDOM) {  // as the lean kernel's lock-step loop, once per instance
-      const unsigned st_abs = (unsigned)(step0 + t);
-      if ((st_abs & 1u) == 0u || t == 0) {
-        philox4x32_10(K, id, st_abs >> 1, STREAM_ACTION, rw[0]);
-        philox4x32_10(K, id + 1, st_abs >> 1, STREAM_ACTION, rw[1]);
-      }
-      if (st_abs & 1u) {
-#pragma unroll
-        for (int i = 0; i < 2; ++i) { rw[i][0] = rw[i][2]; rw[i][1] = rw[i][3]; }
-      }
-    }
-    switch (row_class(P, c_ev, d_e, g_e)) {
-      case ROW_A_NOEV: step(RowTag<ROW_A_NOEV>{}, t, rw); break;
-      case ROW_B_NOEV: step(RowTag<ROW_B_NOEV>{}, t, rw); break;
-      case ROW_A_EV: step(RowTag<ROW_A_EV>{}, t, rw); break;
-      case ROW_B_EV: step(RowTag<ROW_B_EV>{}, t, rw); break;
-      default: step(RowTag<ROW_ANY>{}, t, rw); break;
-    }
+    if (POLICY == SHEMS_POLICY_RANDOM) lockstep_words<2>(K, id, step0, t, &rw[0][0]);
+    with_row_class(row_class(P, c_ev, d_e, g_e), [&](auto cls) { step(cls, t, rw); });
   }
   const Row8 r = load_row(series, idx);
 #pragma unroll
   for (int i = 0; i < 2; ++i) {
-    const long long m = n + i;
-    obs[0 * N + m] = Soc_b[i]; obs[1 * N + m] = Soc_ev[i]; obs[2 * N + m] = r.cd; obs[3 * N + m] = r.d_e; obs[4 * N + m] = r.g_e;
-    obs[5 * N + m] = r.p_buy; obs[6 * N + m] = r.h_cos; obs[7 * N + m] = r.h_sin; obs[8 * N + m] = r.season;
-    idx_arr[m] = idx;
-    if (S.ep_return) S.ep_return[m] = ret[i];
+    store_obs(obs, N, n + i, Soc_b[i], Soc_ev[i], r);
+    idx_arr[n + i] = idx;
+    if (S.ep_return) S.ep_return[n + i] = ret[i];
   }
 }
 
 // ----------------------------------------------------------------------------- C ABI
 static inline unsigned grid_for(long long n, int block) { return (unsigned)((n + block - 1) / block); }
+
+// The integer value of environment variable `name`, `dflt` when it is unset.  The A/B switches of the rollout (SHEMS_RING_COMPACT,
+// SHEMS_ROLLOUT_LEAN, SHEMS_ROLLOUT_LOCKSTEP, SHEMS_ROLLOUT_PAIR; see shems_rollout) are read at every rollout, so that bit-equality
+// tests and same-process timings can flip them between calls.
+static int env_int(const char* name, int dflt) {
+  const char* ev = getenv(name);
+  return ev ? atoi(ev) : dflt;
+}
 
 // Resident CTAs per SM for a rollout over n instances.  A wave of 148 x b CTAs takes about the same time for b = 6, 7, 8 per CTA slot
 // (measured: 6 is 1-3 % faster per instance, profiles/r1_rollout_sweep.md), but a sparsely filled LAST wave runs its few warps at a
@@ -666,8 +590,7 @@ static int sm_count(int device) {
   return (device >= 0 && device < 64) ? sms[device] : 148;
 }
 static int rollout_min_blocks(int device, long long n, bool compact, bool lean) {
-  static int forced = -1;
-  if (forced < 0) { const char* ev = getenv("SHEMS_ROLLOUT_MIN_BLOCKS"); forced = ev ? atoi(ev) : 0; }
+  static const int forced = env_int("SHEMS_ROLLOUT_MIN_BLOCKS", 0);
   if (forced == 6 || forced == 7 || forced == 8) return forced;
   if (compact) return lean ? 7 : 6;
   const int nsm = sm_count(device);
@@ -684,26 +607,6 @@ static int rollout_min_blocks(int device, long long n, bool compact, bool lean) 
   return best;
 }
 
-// Compact ring records (see ring.cuh) unless SHEMS_RING_COMPACT=0 forces full ones (read at every rollout: the A/B switch).
-static bool ring_compact_enabled() {
-  const char* ev = getenv("SHEMS_RING_COMPACT");
-  return !(ev && atoi(ev) == 0);
-}
-
-// shems_rollout_lean_kernel where it applies unless SHEMS_ROLLOUT_LEAN=0 forces the general kernel (read at every rollout: the
-// A/B switch for bit-equality tests and same-process timing)
-static bool rollout_lean_enabled() {
-  const char* ev = getenv("SHEMS_ROLLOUT_LEAN");
-  return !(ev && atoi(ev) == 0);
-}
-
-// the trimmed kernel's lock-step loop for warps that start on one row unless SHEMS_ROLLOUT_LOCKSTEP=0 keeps every warp on its
-// two-step loop (read at every rollout: the A/B switch)
-static bool rollout_lockstep_enabled() {
-  const char* ev = getenv("SHEMS_ROLLOUT_LOCKSTEP");
-  return !(ev && atoi(ev) == 0);
-}
-
 // The pair kernel (shems_rollout_pair_kernel) applies to a launch the trimmed kernel would take in lock step whose instances all stand
 // on one row, with an even count and, with a ring, an even first slot.  It is taken there when its grid of half as many threads fills
 // at least ROLLOUT_PAIR_MIN_WAVES waves of ROLLOUT_PAIR_MIN_BLOCKS CTAs per SM: below that, the trimmed kernel's grid of twice the
@@ -716,10 +619,6 @@ static bool rollout_lockstep_enabled() {
 #ifndef ROLLOUT_PAIR_MIN_WAVES
 #define ROLLOUT_PAIR_MIN_WAVES 1
 #endif
-static int rollout_pair_mode() {
-  const char* ev = getenv("SHEMS_ROLLOUT_PAIR");
-  return ev ? atoi(ev) : 1;
-}
 static bool rollout_pair_fills(int device, long long n, int mode) {
   if (mode == 2) return true;
   const long long ctas = (n / 2 + ROLLOUT_THREADS - 1) / ROLLOUT_THREADS;
@@ -970,6 +869,42 @@ extern "C" int32_t shems_set_state(ShemsEnv* e, const float* obs_host, const int
   return SHEMS_OK;
 }
 
+// shems_rollout_kernel<POL, TR, MB, FAST, COMPACT> for the run-time COMPACT and, without a trace, the run-time MINB mb
+using RolloutKernel = void (*)(DevParams, const float4*, long long, float*, int32_t*, int, int, unsigned long long, long long, const float*, int,
+                               RolloutSinks, long long, long long);
+template <int POL, bool TR, int MB, bool FAST>
+static RolloutKernel general_rollout_kernel(bool compact) {
+  return compact ? shems_rollout_kernel<POL, TR, MB, FAST, true> : shems_rollout_kernel<POL, TR, MB, FAST, false>;
+}
+template <int POL, bool FAST>
+static RolloutKernel general_rollout_kernel(int mb, bool compact) {
+  return mb == 7   ? general_rollout_kernel<POL, false, 7, FAST>(compact)
+         : mb == 8 ? general_rollout_kernel<POL, false, 8, FAST>(compact)
+                   : general_rollout_kernel<POL, false, ROLLOUT_MIN_BLOCKS, FAST>(compact);
+}
+
+// shems_rollout's launch on group g for policy POL: the pair kernel, the trimmed kernel at MINB mb, or the general kernel (a trace
+// takes its Float64-constant build at ROLLOUT_MIN_BLOCKS; otherwise MINB mb and FAST when the group's constants allow it)
+template <int POL>
+static void launch_rollout(const ShemsEnv* e, const ShemsRolloutArgs* a, const RolloutSinks& S, const PhiloxKeys& keys, int lockstep, int g,
+                           bool pair, bool lean, bool compact, int mb) {
+  const long long n0 = e->gstart[g], n1 = e->gstart[g + 1];
+  if (pair) {
+    shems_rollout_pair_kernel<POL, ROLLOUT_PAIR_MIN_BLOCKS><<<grid_for((n1 - n0) / 2, ROLLOUT_THREADS), ROLLOUT_THREADS, 0, e->stream>>>(
+        e->gdp[g], e->gseries[g], e->n, e->obs, e->idx, a->n_steps, e->step, keys, a->env_id_base, a->tape_dev, a->tape_unscaled, S, n0, n1);
+  } else if (lean) {
+    const auto k = mb == 7 ? shems_rollout_lean_kernel<POL, 7> : mb == 8 ? shems_rollout_lean_kernel<POL, 8> : shems_rollout_lean_kernel<POL, ROLLOUT_MIN_BLOCKS>;
+    k<<<grid_for(n1 - n0, ROLLOUT_THREADS), ROLLOUT_THREADS, 0, e->stream>>>(e->gdp[g], e->gseries[g], e->n, e->obs, e->idx, a->n_steps, e->step,
+                                                                           keys, a->env_id_base, a->tape_dev, a->tape_unscaled, S, n0, n1, lockstep);
+  } else {
+    const RolloutKernel k = a->trace_dev           ? general_rollout_kernel<POL, true, ROLLOUT_MIN_BLOCKS, false>(compact)
+                            : e->gdp[g].fast_all ? general_rollout_kernel<POL, true>(mb, compact)
+                                                 : general_rollout_kernel<POL, false>(mb, compact);
+    k<<<grid_for(n1 - n0, ROLLOUT_THREADS), ROLLOUT_THREADS, 0, e->stream>>>(e->gdp[g], e->gseries[g], e->n, e->obs, e->idx, a->n_steps, e->step,
+                                                                           a->seed, a->env_id_base, a->tape_dev, a->tape_unscaled, S, n0, n1);
+  }
+}
+
 extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
   REQUIRE(e && a, SHEMS_ERR_INVALID, "shems_rollout: NULL argument");
   REQUIRE(e->was_reset, SHEMS_ERR_STATE, "shems_rollout: reset! must come first");
@@ -1001,40 +936,15 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
     REQUIRE(e->n <= rp->capacity, SHEMS_ERR_INVALID, "shems_rollout: replay capacity %lld < n_envs %lld", (long long)rp->capacity, (long long)e->n);
     S.ring = rp->ring; S.cap = rp->capacity; S.head = rp->head;
   }
-#define LAUNCH_RO_F(POL, TR, MB, FA, CO)                                                                                            \
-  shems_rollout_kernel<POL, TR, MB, FA, CO><<<grid_for(n1 - n0, ROLLOUT_THREADS), ROLLOUT_THREADS, 0, e->stream>>>(                      \
-      e->gdp[g], e->gseries[g], e->n, e->obs, e->idx, a->n_steps, e->step, a->seed, a->env_id_base, a->tape_dev, a->tape_unscaled, S, n0, n1)
-#define LAUNCH_RO_C(POL, TR, MB, FA)                                                                                                \
-  do { if (compact) LAUNCH_RO_F(POL, TR, MB, FA, true); else LAUNCH_RO_F(POL, TR, MB, FA, false); } while (0)
-#define LAUNCH_RO(POL, TR, MB)                                                                                                      \
-  do { if (!TR && e->gdp[g].fast_all) LAUNCH_RO_C(POL, false, MB, true); else LAUNCH_RO_C(POL, TR, MB, false); } while (0)
-#define LAUNCH_RO_MB(POL)                                                                                                           \
-  do {                                                                                                                              \
-    if (tr) LAUNCH_RO(POL, true, ROLLOUT_MIN_BLOCKS);                                                                               \
-    else if (mb == 7) LAUNCH_RO(POL, false, 7);                                                                                     \
-    else if (mb == 8) LAUNCH_RO(POL, false, 8);                                                                                     \
-    else LAUNCH_RO(POL, false, ROLLOUT_MIN_BLOCKS);                                                                                 \
-  } while (0)
-#define LAUNCH_LEAN(POL, MB)                                                                                                        \
-  shems_rollout_lean_kernel<POL, MB><<<grid_for(n1 - n0, ROLLOUT_THREADS), ROLLOUT_THREADS, 0, e->stream>>>(                           \
-      e->gdp[g], e->gseries[g], e->n, e->obs, e->idx, a->n_steps, e->step, keys, a->env_id_base, a->tape_dev, a->tape_unscaled, S, n0, n1, \
-      lockstep)
-#define LAUNCH_PAIR(POL)                                                                                                            \
-  shems_rollout_pair_kernel<POL, ROLLOUT_PAIR_MIN_BLOCKS><<<grid_for((n1 - n0) / 2, ROLLOUT_THREADS), ROLLOUT_THREADS, 0, e->stream>>>( \
-      e->gdp[g], e->gseries[g], e->n, e->obs, e->idx, a->n_steps, e->step, keys, a->env_id_base, a->tape_dev, a->tape_unscaled, S, n0, n1)
-#define LAUNCH_LEAN_MB(POL)                                                                                                         \
-  do {                                                                                                                              \
-    if (mb == 7) LAUNCH_LEAN(POL, 7);                                                                                               \
-    else if (mb == 8) LAUNCH_LEAN(POL, 8);                                                                                          \
-    else LAUNCH_LEAN(POL, ROLLOUT_MIN_BLOCKS);                                                                                      \
-  } while (0)
-  const bool tr = a->trace_dev != nullptr;
-  const bool may_lean = !tr && !a->obs_traj_dev && e->consistent && rollout_lean_enabled();
+  // SHEMS_ROLLOUT_LEAN=0 forces the general kernel where the trimmed one would apply
+  const bool may_lean = !a->trace_dev && !a->obs_traj_dev && e->consistent && env_int("SHEMS_ROLLOUT_LEAN", 1) != 0;
   const PhiloxKeys keys = philox_keys(a->seed);
-  const int lockstep = rollout_lockstep_enabled() ? 1 : 0;
-  const int pair_mode = lockstep ? rollout_pair_mode() : 0;
-  // compact records need s[2..8] == series row idx (consistent), a row that fits the tag and a series-table entry in the ring
-  const bool may_compact = a->replay && e->consistent && e->nrows <= RING_TAG_MAX_ROW && ring_compact_enabled();
+  // SHEMS_ROLLOUT_LOCKSTEP=0 keeps every warp of the trimmed kernel on its two-step loop, and so never takes the pair kernel
+  const int lockstep = env_int("SHEMS_ROLLOUT_LOCKSTEP", 1) != 0 ? 1 : 0;
+  const int pair_mode = lockstep ? env_int("SHEMS_ROLLOUT_PAIR", 1) : 0;
+  // compact records need s[2..8] == series row idx (consistent), a row that fits the tag and a series-table entry in the ring;
+  // SHEMS_RING_COMPACT=0 forces full ones
+  const bool may_compact = a->replay && e->consistent && e->nrows <= RING_TAG_MAX_ROW && env_int("SHEMS_RING_COMPACT", 1) != 0;
   for (int g = 0; g < e->n_groups; ++g) {
     const long long n0 = e->gstart[g], n1 = e->gstart[g + 1];
     bool compact = false;
@@ -1051,36 +961,13 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
                       rollout_pair_fills(e->device, n1 - n0, pair_mode);
     const int mb = rollout_min_blocks(e->device, n1 - n0, compact, lean);
     COUNT_LAUNCH();
-    if (pair) {
-      __atomic_add_fetch(&g_pair_launches, 1, __ATOMIC_RELAXED);
-      switch (a->policy) {
-        case SHEMS_POLICY_RULE: LAUNCH_PAIR(SHEMS_POLICY_RULE); break;
-        case SHEMS_POLICY_RANDOM: LAUNCH_PAIR(SHEMS_POLICY_RANDOM); break;
-        default: LAUNCH_PAIR(SHEMS_POLICY_TAPE); break;
-      }
-      continue;
-    }
-    if (lean) {
-      switch (a->policy) {
-        case SHEMS_POLICY_RULE: LAUNCH_LEAN_MB(SHEMS_POLICY_RULE); break;
-        case SHEMS_POLICY_RANDOM: LAUNCH_LEAN_MB(SHEMS_POLICY_RANDOM); break;
-        default: LAUNCH_LEAN_MB(SHEMS_POLICY_TAPE); break;
-      }
-      continue;
-    }
+    if (pair) __atomic_add_fetch(&g_pair_launches, 1, __ATOMIC_RELAXED);
     switch (a->policy) {
-      case SHEMS_POLICY_RULE: LAUNCH_RO_MB(SHEMS_POLICY_RULE); break;
-      case SHEMS_POLICY_RANDOM: LAUNCH_RO_MB(SHEMS_POLICY_RANDOM); break;
-      default: LAUNCH_RO_MB(SHEMS_POLICY_TAPE); break;
+      case SHEMS_POLICY_RULE: launch_rollout<SHEMS_POLICY_RULE>(e, a, S, keys, lockstep, g, pair, lean, compact, mb); break;
+      case SHEMS_POLICY_RANDOM: launch_rollout<SHEMS_POLICY_RANDOM>(e, a, S, keys, lockstep, g, pair, lean, compact, mb); break;
+      default: launch_rollout<SHEMS_POLICY_TAPE>(e, a, S, keys, lockstep, g, pair, lean, compact, mb); break;
     }
   }
-#undef LAUNCH_LEAN_MB
-#undef LAUNCH_PAIR
-#undef LAUNCH_LEAN
-#undef LAUNCH_RO_MB
-#undef LAUNCH_RO
-#undef LAUNCH_RO_C
-#undef LAUNCH_RO_F
   CUDA_TRY(cudaGetLastError());
   e->max_idx += a->n_steps;
   e->step += a->n_steps;

@@ -24,6 +24,16 @@ struct StepTrace {  // the remaining `results` columns (:476-478); all values ex
   double EV, profit, discomfort, penalty, PV_DE, B_DE, GR_DE, PV_B, PV_GR, PV_EV, B_EV, GR_EV, EX_EV, B;
 };
 
+// one 32-byte series row (env.cu: the series layout)
+struct Row8 { float soc_ev, cd, d_e, g_e, p_buy, h_cos, h_sin, season; };
+__device__ __forceinline__ Row8 load_row(const float4* __restrict__ series, int row1 /*1-based*/) {
+  const float4 a = __ldg(series + 2 * (size_t)(row1 - 1));
+  const float4 b = __ldg(series + 2 * (size_t)(row1 - 1) + 1);
+  Row8 r;
+  r.soc_ev = a.x; r.cd = a.y; r.d_e = a.z; r.g_e = a.w; r.p_buy = b.x; r.h_cos = b.y; r.h_sin = b.z; r.season = b.w;
+  return r;
+}
+
 __device__ __forceinline__ float jl_minf(float x, float y) { return (y < x) ? y : x; }     // Base.min(x, y), no NaN
 __device__ __forceinline__ double jl_mind(double x, double y) { return (y < x) ? y : x; }
 // Base.clamp(x, lo, hi) = ifelse(x > hi, hi, ifelse(x < lo, lo, x))
@@ -75,6 +85,15 @@ __device__ __forceinline__ int row_class(const DevParams& P, float c_ev, float d
 template <int CLS> constexpr bool row_A = CLS == ROW_A_NOEV || CLS == ROW_A_EV;         // A
 template <int CLS> constexpr bool row_ev = CLS == ROW_A_EV || CLS == ROW_B_EV;          // c_ev > 0: c_ev > -1, not == 0, not < 0, not == -1
 template <int CLS> constexpr bool row_noev = CLS == ROW_A_NOEV || CLS == ROW_B_NOEV;    // c_ev == -1: not > -1, not == 0, < 0, == -1
+
+// next_state! :264-281: Soc_ev of s' after a step from a row with countdown cd_here (class CLS) to row nx — the row's soc_ev when an
+// EV arrives there (:270-272), else the step's own.  nx is taken by value (by reference the lean and pair rollout kernels compile the
+// select with its operands swapped) and cd_here by reference (so that actor_rollout_kernel reads it from shared memory only when
+// nx.cd >= 0, as it always has).
+template <int CLS = ROW_ANY>
+__device__ __forceinline__ float next_soc_ev(float step_soc_ev, Row8 nx, const float& cd_here) {
+  return (nx.cd >= 0.0f && (CLS == ROW_ANY ? cd_here == -1.0f : row_noev<CLS>)) ? nx.soc_ev : step_soc_ev;
+}
 
 // FAST (template parameter of everything below) = the constants are in their usual state — P.fast_all: Float32-valued divisors,
 // Float32 penalty weight, shems_LU1's reward form — so the flag tests, the fall-back branches and the guarded Float32 division
@@ -228,4 +247,22 @@ __device__ __forceinline__ StepOut shems_flows(const DevParams& P, const StepIn&
     tr->PV_EV = (double)PV_EV; tr->B_EV = B_EV; tr->GR_EV = GR_EV; tr->EX_EV = (double)EX_EV; tr->B = (double)B;
   }
   return o;
+}
+
+// the `results` row :476-478 of a step from row idx, column c at q[c * N]
+__device__ __forceinline__ void store_trace_row(double* __restrict__ q, long long N, int idx, const StepIn& s, float Bt, float EVt,
+                                                const StepOut& o, const StepTrace& tr) {
+  q[SHEMS_T_INDEX * N] = (double)(idx + 1); q[SHEMS_T_C_EV * N] = (double)s.c_ev; q[SHEMS_T_EV_TARGET * N] = (double)EVt;
+  q[SHEMS_T_EV * N] = tr.EV; q[SHEMS_T_SOC_EV * N] = (double)s.Soc_ev; q[SHEMS_T_REWARD * N] = o.reward;
+  q[SHEMS_T_PROFIT * N] = tr.profit; q[SHEMS_T_DISCOMFORT * N] = tr.discomfort; q[SHEMS_T_PENALTY * N] = tr.penalty;
+  q[SHEMS_T_PV_DE * N] = tr.PV_DE; q[SHEMS_T_B_DE * N] = tr.B_DE; q[SHEMS_T_GR_DE * N] = tr.GR_DE; q[SHEMS_T_PV_B * N] = tr.PV_B;
+  q[SHEMS_T_PV_GR * N] = tr.PV_GR; q[SHEMS_T_PV_EV * N] = tr.PV_EV; q[SHEMS_T_B_EV * N] = tr.B_EV; q[SHEMS_T_GR_EV * N] = tr.GR_EV;
+  q[SHEMS_T_EX_EV * N] = tr.EX_EV; q[SHEMS_T_GR_B * N] = 0.0; q[SHEMS_T_B_GR * N] = 0.0; q[SHEMS_T_B * N] = tr.B;
+  q[SHEMS_T_B_TARGET * N] = (double)Bt; q[SHEMS_T_SOC_B * N] = (double)s.Soc_b;
+}
+
+// env.state of instance n into the structure-of-arrays obs [9][N]: (Soc_b, Soc_ev) and the exogenous fields of series row r
+__device__ __forceinline__ void store_obs(float* __restrict__ obs, long long N, long long n, float Soc_b, float Soc_ev, const Row8& r) {
+  obs[0 * N + n] = Soc_b; obs[1 * N + n] = Soc_ev; obs[2 * N + n] = r.cd; obs[3 * N + n] = r.d_e; obs[4 * N + n] = r.g_e;
+  obs[5 * N + n] = r.p_buy; obs[6 * N + n] = r.h_cos; obs[7 * N + n] = r.h_sin; obs[8 * N + n] = r.season;
 }

@@ -125,7 +125,63 @@ def record():
         out[f"update_dp world 1 {name} B={B}"] = dict(graph=True, work=profile(lambda: le.replay_fused_dp(mem, rng_rpl=next(seeds))))
         assert le.dp_status() == 0
     os.environ.pop("SHEMS_TC_CHAIN", None)
+    record_rollouts(sb, out)
     return dict(lib=os.path.basename(os.environ.get("SHEMS_B200_LIB", "libshems_b200.so")), card=card(), regimes=out)
+
+
+def record_rollouts(sb, out):
+    """one rollout per branch of shems_rollout's kernel choice: pair, trimmed (lean) at MINB 6 / 7 / 8 with and without a ring, and
+    the general kernel with a trace, an obs trajectory, after set_state, with full records, with N not a multiple of 32 and with
+    Float64 constants; two groups; every policy.  Every profiled call resets the env first (profile() calls it twice)."""
+    import torch
+    ser = sb.series.synth_charger98(600, seed=98)
+    pair_n = 2 * 128 * 148 * 4   # the smallest launch whose paired grid fills a wave of 148 SMs x 4 CTAs
+
+    def rollout(name, n=1024, policy=sb.POLICY_RANDOM, T=4, ring=False, rng=-1, set_state=False, groups=None, params=None, env=(), **kw):
+        e = sb.Shems(64, ser, n_envs=n, groups=groups, params=params)
+        mem = sb.Replay(e.n_envs * 8) if ring else None
+        tape = torch.rand((T, 2, e.n_envs), device="cuda") * 2 - 1 if policy == sb.POLICY_TAPE else None
+        if set_state:
+            e.reset(rng=-1)
+            obs, idx = e.state, e.idx
+
+        def fn():
+            if set_state:
+                e.set_state(obs, idx)
+            else:
+                e.reset(rng=rng)
+            e.rollout(policy, T, seed=1, tape=tape, tape_unscaled=True, replay=mem, **kw)
+
+        saved = {k: os.environ.get(k) for k, _ in env}
+        os.environ.update(dict(env))
+        try:
+            out["rollout " + name] = dict(graph=False, work=profile(fn))
+        finally:
+            for k, v in saved.items():
+                if v is None:
+                    os.environ.pop(k, None)
+                else:
+                    os.environ[k] = v
+
+    for pol, pname in ((sb.POLICY_RULE, "rule"), (sb.POLICY_RANDOM, "random"), (sb.POLICY_TAPE, "tape")):
+        rollout(f"{pname} pair ring", n=pair_n, policy=pol, ring=True)
+        rollout(f"{pname} lean ring", policy=pol, ring=True)
+        rollout(f"{pname} general trace", n=1000, policy=pol, want_trace=True)
+        rollout(f"{pname} general full records", policy=pol, ring=True, env=[("SHEMS_RING_COMPACT", "0")])
+    rollout("pair no ring", n=pair_n)
+    rollout("pair forced, small", env=[("SHEMS_ROLLOUT_PAIR", "2")])
+    rollout("pair off: lean", n=pair_n, env=[("SHEMS_ROLLOUT_PAIR", "0")])
+    rollout("lockstep off: lean", n=pair_n, env=[("SHEMS_ROLLOUT_LOCKSTEP", "0")])
+    rollout("lean random windows", n=pair_n, ring=True, rng=1)
+    for n in (1024, 1024 * 128, 1100 * 128):   # the wave cost model picks MINB 6, 7 and 8
+        rollout(f"lean no ring n={n}", n=n)
+        rollout(f"general obs trajectory n={n}", n=n, want_obs=True)
+    rollout("lean off: general compact", ring=True, env=[("SHEMS_ROLLOUT_LEAN", "0")])
+    rollout("general compact N=1000", n=1000, ring=True)
+    rollout("general after set_state", ring=True, set_state=True)
+    rollout("general Float64 constants", params=sb.params_for_env(sb.ENV_LU7, 98), ring=True)
+    rollout("two groups ring", groups=[(98, 512), (4, 512)], ring=True)
+    rollout("two groups odd counts", groups=[(98, 33), (4, 64)], want_reward=True)
 
 
 def canonical(entry):
