@@ -7,14 +7,17 @@ Wt[in][out] (Flux).  The formulas are those of oracle/ddpg_oracle.c and tests/te
 relu'(0) = 0 (Zygote's x > 0) everywhere.
 
 critic_pass() and actor_pass() are separate: the actor's gradients are taken through the UPDATED critic (phase 2 of an update only
-moves the targets), so a test can hand actor_pass() the critic the device holds after the step.
+moves the targets), so a test can hand actor_pass() the critic the device holds after the step.  actor_out() is the forward-only
+half that act() and the evaluation kernels compute: tanh(z3) of the actor on normalised states.  lsb_exp / sig_bits / tf32_exact /
+grid_units state when data is exact on every path (TF32 operands, fp32 sums in any order).
 
 track=True adds a running error bound to every gradient: each product is bounded by
   |got - ref| <= |eA|·|B| + |A|·|eB| + |eA|·|eB| + eps_K · (|A| + eA)·(|B| + eB),   eps_K = U_TF32 + K · 2^-24,
 the magnitude pass (the same chain on |W|, |x| and |upstream gradient|, with the reference's relu masks) carrying the operands'
 own bounds.  U_TF32 = 2^-9 covers truncating or rounding both operands of a product to TF32 (10 explicit bits); K · 2^-24 covers
 fp32 accumulation of K terms in any order or split.  The same eps is used for every product, so the bound holds whichever of the
-fp32 SIMT or TF32 tensor-core kernels computed it.  A relu unit whose reference pre-activation lies within its own bound may flip
+fp32 SIMT or TF32 tensor-core kernels computed it.  forward() takes per layer whether it may run on TF32 (actor_out: layer 2 only);
+a layer that is fp32 on every path gets eps_K = (K + 2) · 2^-24.  A relu unit whose reference pre-activation lies within its own bound may flip
 on the device: its full upstream |gradient| is added to the bound of what it feeds.
 """
 import numpy as np
@@ -24,8 +27,9 @@ U_FP32 = 2.0 ** -24
 STATE = 9
 
 
-def eps(K):
-    return U_TF32 + K * U_FP32
+def eps(K, tf32=True):
+    """relative bound of one product of K terms: TF32 operands (if tf32) and fp32 accumulation in any order"""
+    return (U_TF32 if tf32 else 2 * U_FP32) + K * U_FP32
 
 
 def normalize(s, s_min, s_max):
@@ -47,8 +51,8 @@ class Val:
         self.v, self.err = v, err
 
 
-def _prod(A, B, K, track):
-    """A @ B, and its bound when tracked (A, B: Val)"""
+def _prod(A, B, K, track, tf32=True):
+    """A @ B, and its bound when tracked (A, B: Val); tf32=False: a product computed in fp32 throughout"""
     v = A.v @ B.v
     if not track:
         return Val(v)
@@ -56,16 +60,16 @@ def _prod(A, B, K, track):
     eA = A.err if A.err is not None else np.zeros_like(aA)
     eB = B.err if B.err is not None else np.zeros_like(aB)
     if B.err is None:                     # exact operand (weights): two of the four products vanish
-        return Val(v, eA @ aB + eps(K) * ((aA + eA) @ aB))
-    e = eA @ aB + aA @ eB + eA @ eB + eps(K) * ((aA + eA) @ (aB + eB))
+        return Val(v, eA @ aB + eps(K, tf32) * ((aA + eA) @ aB))
+    e = eA @ aB + aA @ eB + eA @ eB + eps(K, tf32) * ((aA + eA) @ (aB + eB))
     return Val(v, e)
 
 
-def _add_bias(z, b, K, track):
+def _add_bias(z, b, K, track, tf32=True):
     v = z.v + b[None, :]
     if not track:
         return Val(v)
-    return Val(v, z.err + eps(K) * np.abs(b)[None, :])
+    return Val(v, z.err + eps(K, tf32) * np.abs(b)[None, :])
 
 
 def _colsum(d, track):
@@ -77,15 +81,16 @@ def _colsum(d, track):
     return Val(v, d.err.sum(0) + eps(B) * (np.abs(d.v) + d.err).sum(0))
 
 
-def forward(net, x, track=False):
-    """x: Val [B][in].  Returns the pre-activations z1, z2, z3 and activations h1, h2 (Val)."""
+def forward(net, x, track=False, tf32=(True, True, True)):
+    """x: Val [B][in].  Returns the pre-activations z1, z2, z3 and activations h1, h2 (Val).
+    tf32[k]: layer k + 1 may run on TF32 tensor cores (else its bound is that of fp32 arithmetic alone)."""
     (W1, b1), (W2, b2), (W3, b3) = net
     f = {"x": x}
-    z1 = _add_bias(_prod(x, Val(W1), W1.shape[0], track), b1, W1.shape[0], track)
+    z1 = _add_bias(_prod(x, Val(W1), W1.shape[0], track, tf32[0]), b1, W1.shape[0], track, tf32[0])
     h1 = Val(np.where(z1.v > 0, z1.v, 0.0), z1.err)           # relu is 1-Lipschitz: the bound carries over, flipped or not
-    z2 = _add_bias(_prod(h1, Val(W2), W2.shape[0], track), b2, W2.shape[0], track)
+    z2 = _add_bias(_prod(h1, Val(W2), W2.shape[0], track, tf32[1]), b2, W2.shape[0], track, tf32[1])
     h2 = Val(np.where(z2.v > 0, z2.v, 0.0), z2.err)
-    z3 = _add_bias(_prod(h2, Val(W3), W3.shape[0], track), b3, W3.shape[0], track)
+    z3 = _add_bias(_prod(h2, Val(W3), W3.shape[0], track, tf32[2]), b3, W3.shape[0], track, tf32[2])
     f.update(z1=z1, h1=h1, z2=z2, h2=h2, z3=z3)
     return f
 
@@ -127,6 +132,14 @@ def _tanh(z, track):
     if not track:
         return Val(v)
     return Val(v, z.err + 4 * U_FP32)   # tanh is 1-Lipschitz; tanhf is within a few ulp of |tanh| <= 1
+
+
+def actor_out(actor, s_min, s_max, obs, track=False, tf32=True):
+    """tanh(z3) of `actor` on the states obs [9][n] (float32): Val [n][2], with its bound when tracked.  act() computes layers 1
+    and 3 in fp32 on every path; tf32: layer 2 may run on TF32 tensor cores"""
+    sn = normalize(obs, s_min, s_max)
+    f = forward(actor, Val(sn, 2 * U_FP32 * np.abs(sn) if track else None), track, (False, tf32, False))
+    return _tanh(f["z3"], track)
 
 
 def critic_pass(actor_t, critic, critic_t, s_min, s_max, s, a, r, s2, done=None, gamma=0.99, track=False):
@@ -174,3 +187,55 @@ def actor_pass(actor, critic, s_min, s_max, s, track=False):
     loss = float(-np.mean(fp["z3"].v[:, 0]))
     return {"grads": ba["grads"], "loss": loss, "api": api.v, "dA": dA.v, "qpi": fp["z3"].v[:, 0], "fwd_actor": fa, "fwd_critic": fp,
             "bwd_critic": bp, "bwd_actor": ba, "xspi": xspi.v}
+
+
+# ---------------------------------------------------------------------------------------------------------------- exact arithmetic
+def lsb_exp(x):
+    """exponent of the lowest set bit of every element (+inf for 0)"""
+    x = np.asarray(x, np.float64)
+    m, e = np.frexp(x)
+    mi = np.abs(m * 2.0 ** 53).astype(np.int64)
+    low = mi & -mi
+    ctz = np.log2(np.where(low > 0, low, 1)).astype(np.int64)
+    return np.where(x != 0, (e - 53 + ctz).astype(np.float64), np.inf)
+
+
+def sig_bits(x):
+    """significant bits of every nonzero element"""
+    x = np.asarray(x, np.float64)
+    _, e = np.frexp(x)
+    return np.where(x != 0, e - lsb_exp(x), 0)
+
+
+def tf32_exact(x):
+    x = np.asarray(x, np.float64)
+    f = x.astype(np.float32)
+    return bool(np.all(f.astype(np.float64) == x) and np.all((f.view(np.uint32) & 0x1FFF) == 0))
+
+
+def grid_units(A, Bm, bias=None, where=None):
+    """max over the outputs of A @ Bm (+ bias) of sum |terms| / the grid every term lies on.
+
+    The grid of output (m, n) is 2^g with g = min over k of lsb(A[m, k]) + lsb(Bm[k, n]) over nonzero terms.  It comes from one
+    product: max_k 2^-(ga + gb) <= (sum_k 2^-p(ga + gb))^(1/p) <= K^(1/p) max_k, so floor(-log2(...)/p) is never above the true g."""
+    A, Bm = np.asarray(A, np.float64), np.asarray(Bm, np.float64)
+    ga, gb = lsb_exp(A), lsb_exp(Bm)
+    oa = ga[np.isfinite(ga)].min() if np.isfinite(ga).any() else 0.0
+    ob = gb[np.isfinite(gb)].min() if np.isfinite(gb).any() else 0.0
+    rng = max(1.0, (ga[np.isfinite(ga)] - oa).max(initial=0), (gb[np.isfinite(gb)] - ob).max(initial=0))
+    p = float(min(32, int(480 // rng)))
+    a = np.where(np.isfinite(ga), np.exp2(p * (oa - np.where(np.isfinite(ga), ga, oa))), 0.0)
+    b = np.where(np.isfinite(gb), np.exp2(p * (ob - np.where(np.isfinite(gb), gb, ob))), 0.0)
+    P = a @ b
+    with np.errstate(divide="ignore"):
+        g = np.where(P > 0, np.floor(oa + ob - np.log2(np.where(P > 0, P, 1.0)) / p), np.inf)
+    tot = np.abs(A) @ np.abs(Bm)
+    if bias is not None:
+        bias = np.asarray(bias, np.float64)
+        g = np.minimum(g, lsb_exp(bias)[None, :])
+        tot = tot + np.abs(bias)[None, :]
+    assert np.all(np.isfinite(g) | (tot == 0))
+    u = np.where(np.isfinite(g), tot * np.exp2(-np.where(np.isfinite(g), g, 0.0)), 0.0)
+    if where is not None:
+        u = u * where
+    return float(u.max(initial=0.0))

@@ -28,62 +28,11 @@ import pytest
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import ddpg_f64 as R  # noqa: E402
+from ddpg_f64 import grid_units, lsb_exp, sig_bits, tf32_exact  # noqa: E402,F401
 
 ACTOR, CRITIC, ACTOR_T, CRITIC_T = 0, 1, 2, 3
 GRID_LIMIT = 2.0 ** 22
 C_BOUND = 2.0
-
-
-# ---------------------------------------------------------------------------------------------------------------- exact arithmetic
-def lsb_exp(x):
-    """exponent of the lowest set bit of every element (+inf for 0)"""
-    x = np.asarray(x, np.float64)
-    m, e = np.frexp(x)
-    mi = np.abs(m * 2.0 ** 53).astype(np.int64)
-    low = mi & -mi
-    ctz = np.log2(np.where(low > 0, low, 1)).astype(np.int64)
-    return np.where(x != 0, (e - 53 + ctz).astype(np.float64), np.inf)
-
-
-def sig_bits(x):
-    """significant bits of every nonzero element"""
-    x = np.asarray(x, np.float64)
-    _, e = np.frexp(x)
-    return np.where(x != 0, e - lsb_exp(x), 0)
-
-
-def tf32_exact(x):
-    x = np.asarray(x, np.float64)
-    f = x.astype(np.float32)
-    return bool(np.all(f.astype(np.float64) == x) and np.all((f.view(np.uint32) & 0x1FFF) == 0))
-
-
-def grid_units(A, Bm, bias=None, where=None):
-    """max over the outputs of A @ Bm (+ bias) of sum |terms| / the grid every term lies on.
-
-    The grid of output (m, n) is 2^g with g = min over k of lsb(A[m, k]) + lsb(Bm[k, n]) over nonzero terms.  It comes from one
-    product: max_k 2^-(ga + gb) <= (sum_k 2^-p(ga + gb))^(1/p) <= K^(1/p) max_k, so floor(-log2(...)/p) is never above the true g."""
-    A, Bm = np.asarray(A, np.float64), np.asarray(Bm, np.float64)
-    ga, gb = lsb_exp(A), lsb_exp(Bm)
-    oa = ga[np.isfinite(ga)].min() if np.isfinite(ga).any() else 0.0
-    ob = gb[np.isfinite(gb)].min() if np.isfinite(gb).any() else 0.0
-    rng = max(1.0, (ga[np.isfinite(ga)] - oa).max(initial=0), (gb[np.isfinite(gb)] - ob).max(initial=0))
-    p = float(min(32, int(480 // rng)))
-    a = np.where(np.isfinite(ga), np.exp2(p * (oa - np.where(np.isfinite(ga), ga, oa))), 0.0)
-    b = np.where(np.isfinite(gb), np.exp2(p * (ob - np.where(np.isfinite(gb), gb, ob))), 0.0)
-    P = a @ b
-    with np.errstate(divide="ignore"):
-        g = np.where(P > 0, np.floor(oa + ob - np.log2(np.where(P > 0, P, 1.0)) / p), np.inf)
-    tot = np.abs(A) @ np.abs(Bm)
-    if bias is not None:
-        bias = np.asarray(bias, np.float64)
-        g = np.minimum(g, lsb_exp(bias)[None, :])
-        tot = tot + np.abs(bias)[None, :]
-    assert np.all(np.isfinite(g) | (tot == 0))
-    u = np.where(np.isfinite(g), tot * np.exp2(-np.where(np.isfinite(g), g, 0.0)), 0.0)
-    if where is not None:
-        u = u * where
-    return float(u.max(initial=0.0))
 
 
 # ------------------------------------------------------------------------------------------------------------ Part A data
