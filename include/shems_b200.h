@@ -262,6 +262,27 @@ SHEMS_API int32_t replay_set_priorities(ShemsReplay* rp, const float* prio_host 
  * x_j = leaf_j len / root in Float64.  batch <= the memory's length is not required (draws are with replacement). */
 SHEMS_API int32_t replay_sample_prioritized(ShemsReplay* rp, int32_t batch, uint64_t seed, float beta, int32_t* idx_dev /*[batch]*/,
                                             float* w_dev /*[batch]*/);
+/* n-step returns (no reference counterpart).  replay_enable_successors gives the memory a successor link per slot, and every
+ * existing record starts with none.  After every write (replay_push: one step of n instances; replay_push_groups: n_per; shems_rollout
+ * with this replay: n_envs; ddpg_episode: the instances of its learner), in stream order, each new record i gets no successor, and the
+ * record W before it (W the write's instances per step), if it has done == 0 and its s' equals s(i) in all 9 fields bit for bit, gets
+ * i as its successor.  Episode boundaries end a chain by themselves (a reset breaks the equality).  A memory without links pays
+ * nothing. */
+SHEMS_API int32_t replay_enable_successors(ShemsReplay* rp);
+/* successor of each of the len records in logical order (0 = oldest): a logical index, or -1; synchronises the memory's stream.
+ * SHEMS_ERR_STATE without links. */
+SHEMS_API int32_t replay_get_successors(ShemsReplay* rp, int32_t* next_host /*[len]*/);
+/* checkpoint restore: the len successors in logical order; each must be -1 or in (i, len), else SHEMS_ERR_INVALID and nothing
+ * changes.  SHEMS_ERR_STATE without links. */
+SHEMS_API int32_t replay_set_successors(ShemsReplay* rp, const int32_t* next_host /*[len]*/);
+/* what update 0 of ddpg_update(seed) trains on for an n-step learner with discount gamma, enqueued on the memory's stream: row j
+ * starts at the record ring_draw(seed, j) picks (or idx_host[j], a logical index) and walks its successors in Float64 with explicit
+ * roundings: gp = 1, R = r_0, k = 1; while k < n, done_{k-1} == 0 and the record has a successor: gp = RN64(gp gamma),
+ * R = RN64(R + RN64(gp r_k)), k += 1.  s, a: the first record's; s2: the last record's s'; r = RN32(R);
+ * done = RN32(1 - RN64(gp RN64(1 - done_{k-1}))), so the 1-step target r + gamma (1 - done) q' bootstraps with gamma^k; k_dev[j] = k
+ * (k_dev may be NULL).  1 <= n <= 16, gamma in [0, 1]; n > 1 needs links (SHEMS_ERR_STATE). */
+SHEMS_API int32_t replay_sample_nstep(ShemsReplay* rp, int32_t batch, const int32_t* idx_host, uint64_t seed, int32_t n, float gamma,
+                                      float* s_dev, float* a_dev, float* r_dev, float* s2_dev, float* done_dev, int32_t* k_dev);
 /* min_max_buffer(n) (memory_plotting_saving.jl:50-53): min/max of s over a with-replacement
  * sample of size n_samples -> s_min_host[9], s_max_host[9]. */
 SHEMS_API int32_t replay_minmax(ShemsReplay* rp, int64_t n_samples, const int32_t* idx_host, uint64_t seed,
@@ -321,6 +342,16 @@ SHEMS_API int32_t ddpg_set_fused(Ddpg* h, int32_t on);
  * ddpg_update_phase, ddpg_dp_connect and ddpg_update_dp return SHEMS_ERR_STATE on a prioritized handle. */
 SHEMS_API int32_t ddpg_set_prioritized(Ddpg* h, int32_t on, float alpha, float beta, float eps);
 SHEMS_API int32_t ddpg_get_prioritized(Ddpg* h, int32_t* on, float* alpha, float* beta, float* eps);
+/* n-step returns for every learner of the handle (1 <= n <= 16; n = 1, the default, is the 1-step update).  With n > 1 each row of
+ * an update from the replay memories is the walk replay_sample_nstep describes, with the learner's own gamma, and the unchanged TD
+ * target r + gamma (1 - done) q' then is the n-step target.  The fused, tiled, tensor-core, chain and population paths all take it,
+ * with uniform and with prioritized draws (a prioritized learner's priorities go back to the rows' first records).  n is handle-wide
+ * and written in stream order (n > 1 to another n > 1 needs no re-capture).  Every update and training episode then needs memories
+ * with links (replay_enable_successors, else SHEMS_ERR_STATE, nothing launched); ddpg_update_phase, ddpg_dp_connect and
+ * ddpg_update_dp return SHEMS_ERR_STATE on an n-step handle, and so does n > 1 on a connected data-parallel learner.
+ * ddpg_update_batch trains on the caller's minibatch as it is. */
+SHEMS_API int32_t ddpg_set_nstep(Ddpg* h, int32_t n);
+SHEMS_API int32_t ddpg_get_nstep(const Ddpg* h);
 /* glorot_uniform hidden layers, U(-3e-3,3e-3) last layers, zero biases, targets = copies
  * (DDPG.jl:21-22, 30-46) from Philox(seed) (Julia's MersenneTwister stream is not reproduced); fresh optimisers
  * (ADAM moments zero, βp = β, update counter 0: input.jl:126-127). */

@@ -114,6 +114,10 @@ SIGNATURES = {
     "replay_get_priorities": (I32, [VP, PF, PF]),
     "replay_set_priorities": (I32, [VP, PF, F32]),
     "replay_sample_prioritized": (I32, [VP, I32, U64, F32, VP, VP]),
+    "replay_enable_successors": (I32, [VP]),
+    "replay_get_successors": (I32, [VP, PI]),
+    "replay_set_successors": (I32, [VP, PI]),
+    "replay_sample_nstep": (I32, [VP, I32, PI, U64, I32, F32, VP, VP, VP, VP, VP, VP]),
     "ddpg_default_params": (I32, [C.POINTER(DdpgParams)]),
     "ddpg_create": (I32, [C.POINTER(DdpgParams), I32, C.POINTER(VP)]),
     "ddpg_destroy": (I32, [VP]),
@@ -122,6 +126,8 @@ SIGNATURES = {
     "ddpg_set_fused": (I32, [VP, I32]),
     "ddpg_set_prioritized": (I32, [VP, I32, F32, F32, F32]),
     "ddpg_get_prioritized": (I32, [VP, PI, PF, PF, PF]),
+    "ddpg_set_nstep": (I32, [VP, I32]),
+    "ddpg_get_nstep": (I32, [VP]),
     "ddpg_init": (I32, [VP, U64]),
     "ddpg_set_layer": (I32, [VP, I32, I32, PF, PF]),
     "ddpg_get_layer": (I32, [VP, I32, I32, PF, PF]),

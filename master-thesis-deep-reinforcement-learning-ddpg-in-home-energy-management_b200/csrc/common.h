@@ -95,6 +95,7 @@ struct ShemsReplay {
   float* prio_alloc;  // replay_enable_priorities: header + sum tree of the slots' priorities (ring.cuh), else NULL
   float* prio;        // node 0 of the tree (prio_alloc + PRIO_HEADER_FLOATS)
   int64_t prio_p2;    // prio_p2(capacity)
+  int32_t* next;      // replay_enable_successors: next[cap], the successor link of every slot (ring.cuh), else NULL
 };
 
 struct ShemsEnv {
@@ -125,9 +126,11 @@ struct ShemsEnv {
   long long gstart[SHEMS_MAX_GROUPS + 1];
 };
 
-// a writer has stored n_written transitions from slot head on: advances head and length, and for a memory with priorities enqueues on
-// `st` (the writer's stream) the refresh that gives the surviving min(n_written, cap) slots the priority p_max
-int replay_after_rollout(ShemsReplay* rp, int64_t n_written, cudaStream_t st);
+// a writer has stored n_written transitions from slot head on, `width` instances per step (slot head + t*width + i holds step t of
+// instance i): advances head and length, and enqueues on `st` (the writer's stream, after the records are written) the refresh that
+// gives the surviving min(n_written, cap) slots the priority p_max (a memory with priorities) and the successor-link pass over them
+// (a memory with links)
+int replay_after_rollout(ShemsReplay* rp, int64_t n_written, int64_t width, cudaStream_t st);
 // entry of rp's series table holding series `series` of env `serial` (nrows rows at rows_dev), copied on first use; -1 when the table
 // is full.  The copy is enqueued on rp->stream and `user` (the stream of the writer) waits for it.
 int replay_series_entry(ShemsReplay* rp, unsigned long long serial, int series, const float4* rows_dev, int nrows, cudaStream_t user,

@@ -553,6 +553,9 @@ struct Ddpg {
   // weigh the critic's dq and write the rows' priorities back.  per_knobs: α, β, ε on the device (handle-wide, written in stream order);
   // per_slot / per_leaf [pop][B]: the slot each row of the current update drew and its priority at the draw
   bool per; float per_host[3]; float* per_knobs; float** trees_dev; int32_t* per_slot; float* per_leaf;
+  // n-step returns (ddpg_set_nstep): nstep > 1 gathers every row by walking its memory's successor links (links_dev, staged beside
+  // rings_dev); nstep_knob: n on the device (handle-wide, written in stream order), so only a switch between 1 and > 1 re-captures
+  int nstep; int* nstep_knob; const int32_t** links_dev;
 };
 static inline int round_ld(int x) { return (x + 31) & ~31; }  // activation rows start on 128-byte lines: one L2 request per TMA box row
 #ifndef TC_MIN_ROWS
@@ -674,6 +677,8 @@ extern "C" int32_t ddpg_create(const DdpgParams* p, int32_t device, Ddpg** out) 
   DMALLOC(h->rings_dev, pop);
   DMALLOC(h->trees_dev, pop);
   DMALLOC(h->per_knobs, 3);
+  DMALLOC(h->links_dev, pop);
+  DMALLOC(h->nstep_knob, 1);
   DMALLOC(h->per_slot, (long long)pop * B);
   DMALLOC(h->per_leaf, (long long)pop * B);
   h->best_stride = (na + 63) & ~63ll;   // every copy starts on a 256-byte boundary (float4 copies)
@@ -706,6 +711,11 @@ extern "C" int32_t ddpg_create(const DdpgParams* p, int32_t device, Ddpg** out) 
     cudaMemcpy(h->ctrl, ctl.data(), sizeof(DdpgCtrl) * (size_t)pop, cudaMemcpyHostToDevice);
   }
   for (int n = 0; n < 2; ++n) { h->beta_pow[n][0] = p->adam_beta1; h->beta_pow[n][1] = p->adam_beta2; }
+  h->nstep = 1;
+  {
+    const cudaError_t e_ = cudaMemcpy(h->nstep_knob, &h->nstep, sizeof(int), cudaMemcpyHostToDevice);
+    if (e_ != cudaSuccess) { shems_set_error("ddpg_create: nstep -> %s", cudaGetErrorString(e_)); ddpg_destroy(h); return SHEMS_ERR_CUDA; }
+  }
   *out = h;
   return SHEMS_OK;
 }
@@ -727,6 +737,7 @@ extern "C" int32_t ddpg_destroy(Ddpg* h) {
   cudaFree(h->ctrl); cudaFree(h->idx_dev); cudaFree(h->ws); cudaFree((void*)h->rings_dev); cudaFree(h->trees_dev); cudaFree(h->dp_box); cudaFree(h->counters);
   cudaFree(h->ws_side); cudaFree(h->counters_side);
   cudaFree(h->per_knobs); cudaFree(h->per_slot); cudaFree(h->per_leaf);
+  cudaFree(h->nstep_knob); cudaFree((void*)h->links_dev);
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
   if (h->ev_mid) cudaEventDestroy(h->ev_mid);
   if (h->ev_join) cudaEventDestroy(h->ev_join);
@@ -834,6 +845,22 @@ extern "C" int32_t ddpg_get_prioritized(Ddpg* h, int32_t* on, float* alpha, floa
   return SHEMS_OK;
 }
 
+extern "C" int32_t ddpg_set_nstep(Ddpg* h, int32_t n) {
+  REQUIRE(h, SHEMS_ERR_INVALID, "ddpg_set_nstep: NULL handle");
+  REQUIRE(n >= 1 && n <= NSTEP_MAX, SHEMS_ERR_INVALID, "ddpg_set_nstep: n=%d outside 1..%d", n, NSTEP_MAX);
+  REQUIRE(n == 1 || !h->dp_on, SHEMS_ERR_STATE, "ddpg_set_nstep: not available for a data-parallel learner");
+  GUARD(h->device);
+  // pageable source: staged before the call returns; ordered like ddpg_set_hparams, so a captured update reads the new n
+  CUDA_TRY(cudaMemcpyAsync(h->nstep_knob, &n, sizeof(int), cudaMemcpyHostToDevice, h->stream));
+  if ((n > 1) != (h->nstep > 1)) {   // the update's graph gains or loses the walking gather: re-captured by the next update
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }
+  }
+  h->nstep = n;
+  return SHEMS_OK;
+}
+extern "C" int32_t ddpg_get_nstep(const Ddpg* h) { return h ? h->nstep : 0; }
+
 extern "C" int64_t ddpg_num_params(const Ddpg* h, int32_t net) {
   return (h && net >= 0 && net <= DDPG_NET_ACTOR_BEST) ? dims_of(h, net).n_params : 0;   // ACTOR_BEST has the actor's shape
 }
@@ -931,13 +958,16 @@ extern "C" int32_t ddpg_init(Ddpg* h, uint64_t seed) {
 // One thread per (sample j, state field k): thread k == 0 also moves a, r, done.
 // PER: the ring rows come from the learner's sum tree (trees[blockIdx.y], ring_draw_prioritized; caller-supplied indices as they are),
 // and thread k == 0 of row j records its slot and priority in per_slot / per_leaf [pop][B] for ddpg_per_kernel.
-template <bool PER>
+// NSTEP: every thread of row j walks the chain from the drawn record (ring_nstep over links[blockIdx.y], n = *nstep, the learner's γ):
+// s and a stay the drawn record's, s' is the last record's, and thread k == 0 sums r and folds γ^{k-1} into done.
+template <bool PER, bool NSTEP = false>
 __device__ __forceinline__ void gather_body(const float* const* __restrict__ rings, const float* __restrict__ rs, const float* __restrict__ ra,
                                             const float* __restrict__ rr, const float* __restrict__ rs2, const float* __restrict__ rd, long long ld,
                                             DdpgCtrl* __restrict__ ctrl, const int32_t* __restrict__ idx, long long idx_stride,
                                             const float* __restrict__ norm, int B, float* __restrict__ xs, float* __restrict__ xs2,
                                             float* __restrict__ xspi, float* __restrict__ r, float* __restrict__ done, long long pop_stride,
-                                            const float* const* __restrict__ trees, int32_t* __restrict__ per_slot, float* __restrict__ per_leaf) {
+                                            const float* const* __restrict__ trees, int32_t* __restrict__ per_slot, float* __restrict__ per_leaf,
+                                            const int32_t* const* __restrict__ links = nullptr, const int* __restrict__ nstep = nullptr) {
   asm volatile("griddepcontrol.launch_dependents;\n" ::: "memory");   // the forward-chain launch after it stages its weights under this kernel
   const unsigned g = blockIdx.x * blockDim.x + threadIdx.x;
   const int j = g / 9, k = g % 9;  // unsigned: k is known to be < 9, which folds ring_field's field-range tests
@@ -973,6 +1003,12 @@ __device__ __forceinline__ void gather_body(const float* const* __restrict__ rin
     if (k == 0) {
       a0 = ring_field(q, row, RING_A); a1 = ring_field(q, row, RING_A + 1); rv = ring_field(q, row, RING_R); dv = ring_field(q, row, RING_DONE);
     }
+    if (NSTEP) {
+      const RingNstep w = ring_nstep(ring, ring_table(ring), links[blockIdx.y], slot, *nstep, ctrl->hp.gamma, k == 0);
+      const float* q2 = ring + ring_base(w.last);
+      s2v = ring_field(q2, ring_row(ring_table(ring), q2), RING_S2 + k);
+      if (k == 0) { rv = w.r; dv = w.done; }
+    }
   } else {
     sv = rs[k * ld + j]; s2v = rs2[k * ld + j];
     if (k == 0) { a0 = ra[j]; a1 = ra[ld + j]; rv = rr[j]; dv = rd ? rd[j] : 0.0f; }
@@ -997,6 +1033,24 @@ ddpg_gather_per_kernel(const float* const* __restrict__ rings, DdpgCtrl* __restr
                        int32_t* __restrict__ per_slot, float* __restrict__ per_leaf) {
   gather_body<true>(rings, nullptr, nullptr, nullptr, nullptr, nullptr, 0, ctrl, idx, idx_stride, norm, B, xs, xs2, xspi, r, done, pop_stride, trees,
                     per_slot, per_leaf);
+}
+// n-step instantiations: uniform draws and PER draws, each row walked over its memory's successor links
+__global__ void __launch_bounds__(128)
+ddpg_gather_nstep_kernel(const float* const* __restrict__ rings, DdpgCtrl* __restrict__ ctrl, const int32_t* __restrict__ idx, long long idx_stride,
+                         const float* __restrict__ norm, int B, float* __restrict__ xs, float* __restrict__ xs2, float* __restrict__ xspi,
+                         float* __restrict__ r, float* __restrict__ done, long long pop_stride, const int32_t* const* __restrict__ links,
+                         const int* __restrict__ nstep) {
+  gather_body<false, true>(rings, nullptr, nullptr, nullptr, nullptr, nullptr, 0, ctrl, idx, idx_stride, norm, B, xs, xs2, xspi, r, done, pop_stride,
+                           nullptr, nullptr, nullptr, links, nstep);
+}
+__global__ void __launch_bounds__(128)
+ddpg_gather_per_nstep_kernel(const float* const* __restrict__ rings, DdpgCtrl* __restrict__ ctrl, const int32_t* __restrict__ idx, long long idx_stride,
+                             const float* __restrict__ norm, int B, float* __restrict__ xs, float* __restrict__ xs2, float* __restrict__ xspi,
+                             float* __restrict__ r, float* __restrict__ done, long long pop_stride, const float* const* __restrict__ trees,
+                             int32_t* __restrict__ per_slot, float* __restrict__ per_leaf, const int32_t* const* __restrict__ links,
+                             const int* __restrict__ nstep) {
+  gather_body<true, true>(rings, nullptr, nullptr, nullptr, nullptr, nullptr, 0, ctrl, idx, idx_stride, norm, B, xs, xs2, xspi, r, done, pop_stride,
+                          trees, per_slot, per_leaf, links, nstep);
 }
 
 // Prioritized replay between the TD target and the critic's backward pass, one block per learner (blockIdx.y):
@@ -1816,6 +1870,7 @@ static int enqueue_update_fused(Ddpg* h, cudaStream_t st, bool dp, const GatherS
   a.src_s = src.s; a.src_a = src.a; a.src_r = src.r; a.src_s2 = src.s2; a.src_d = src.done; a.src_ld = src.ld;
   a.ctrl = h->ctrl; a.idx = h->idx_dev; a.norm = h->norm; a.xs_w = h->xs;
   a.vec16 = w2_vec16(h) ? 1 : 0;
+  if (src.from_rings && h->nstep > 1) { a.links = h->links_dev; a.nstep = h->nstep_knob; }
   // each pass is followed by the reduction of its partial sums and the optimiser step (dp: with the gradient exchange) in ONE kernel
   a.part = h->parts[1]; a.part_stride = h->dims[1].n_params;
   TRY(ddpg_fused_critic(st, a));
@@ -1836,6 +1891,18 @@ static int enqueue_update_body(Ddpg* h, cudaStream_t st, bool dp = false) {
 static int enqueue_gather(Ddpg* h, cudaStream_t st, bool from_rings, const float* s, const float* a, const float* r, const float* s2,
                           const float* done, long long ld) {
   const int B = h->p.batch;
+  if (from_rings && h->nstep > 1) {
+    if (h->per)
+      ddpg_gather_per_nstep_kernel<<<dim3((B * 9 + 127) / 128, h->pop), 128, 0, st>>>(h->rings_dev, h->ctrl, h->idx_dev, h->idx_stride, h->norm, B,
+                                                                                     h->xs, h->xs2, h->xspi, h->r, h->done, h->pop_stride, h->trees_dev,
+                                                                                     h->per_slot, h->per_leaf, h->links_dev, h->nstep_knob);
+    else
+      ddpg_gather_nstep_kernel<<<dim3((B * 9 + 127) / 128, h->pop), 128, 0, st>>>(h->rings_dev, h->ctrl, h->idx_dev, h->idx_stride, h->norm, B, h->xs,
+                                                                                 h->xs2, h->xspi, h->r, h->done, h->pop_stride, h->links_dev,
+                                                                                 h->nstep_knob);
+    CUDA_TRY(cudaGetLastError());
+    return SHEMS_OK;
+  }
   if (h->per && from_rings) {
     ddpg_gather_per_kernel<<<dim3((B * 9 + 127) / 128, h->pop), 128, 0, st>>>(h->rings_dev, h->ctrl, h->idx_dev, h->idx_stride, h->norm, B, h->xs,
                                                                              h->xs2, h->xspi, h->r, h->done, h->pop_stride, h->trees_dev,
@@ -1890,6 +1957,17 @@ static int per_memories_ok(const Ddpg* h, ShemsReplay* const* rps, const char* w
   return SHEMS_OK;
 }
 
+// an n-step learner walks its memory's successor links: every learner needs a memory with links
+static int nstep_memories_ok(const Ddpg* h, ShemsReplay* const* rps, const char* who) {
+  if (h->nstep == 1) return SHEMS_OK;
+  for (int l = 0; l < h->pop; ++l) {
+    REQUIRE(rps[l], SHEMS_ERR_INVALID, "%s: learner %d has no replay memory", who, l);
+    REQUIRE(rps[l]->next, SHEMS_ERR_STATE, "%s: n-step learner (n = %d), but the memory of learner %d has no successor links (replay_enable_successors)",
+            who, h->nstep, l);
+  }
+  return SHEMS_OK;
+}
+
 struct CtrlHostPart { unsigned long long seed; unsigned update; int use_idx; long long len, head, cap; int idx_cursor; unsigned blocks_done; };
 static_assert(sizeof(CtrlHostPart) == offsetof(DdpgCtrl, bp), "control block layout");
 
@@ -1900,13 +1978,16 @@ static int stage_update_inputs(Ddpg* h, ShemsReplay* const* rps, const uint64_t*
   std::vector<CtrlHostPart> hp((size_t)pop);
   std::vector<const float*> rings((size_t)pop);
   std::vector<float*> trees((size_t)pop);
+  std::vector<const int32_t*> links((size_t)pop);
   TRY(per_memories_ok(h, rps, "ddpg_update"));
+  TRY(nstep_memories_ok(h, rps, "ddpg_update"));
   for (int l = 0; l < pop; ++l) {
     ShemsReplay* rp = rps[l];
     REQUIRE(rp, SHEMS_ERR_INVALID, "ddpg_update: learner %d has no replay memory", l);
     REQUIRE(rp->device == h->device, SHEMS_ERR_INVALID, "ddpg_update: replay on device %d, learner on %d", rp->device, h->device);
     REQUIRE(rp->length > 0, SHEMS_ERR_STATE, "ddpg_update: memory is empty");
     trees[l] = rp->prio;
+    links[l] = rp->next;
     if (idx_host)
       for (long long j = 0; j < per_learner; ++j) {
         const int32_t v = idx_host[(long long)l * per_learner + j];
@@ -1939,6 +2020,7 @@ static int stage_update_inputs(Ddpg* h, ShemsReplay* const* rps, const uint64_t*
   CUDA_TRY(cudaMemcpy2DAsync(h->ctrl, sizeof(DdpgCtrl), hp.data(), sizeof(CtrlHostPart), sizeof(CtrlHostPart), (size_t)pop, cudaMemcpyHostToDevice, h->stream));
   CUDA_TRY(cudaMemcpyAsync((void*)h->rings_dev, rings.data(), sizeof(const float*) * (size_t)pop, cudaMemcpyHostToDevice, h->stream));
   if (h->per) CUDA_TRY(cudaMemcpyAsync(h->trees_dev, trees.data(), sizeof(float*) * (size_t)pop, cudaMemcpyHostToDevice, h->stream));
+  if (h->nstep > 1) CUDA_TRY(cudaMemcpyAsync((void*)h->links_dev, links.data(), sizeof(const int32_t*) * (size_t)pop, cudaMemcpyHostToDevice, h->stream));
   return SHEMS_OK;
 }
 
@@ -1966,6 +2048,7 @@ extern "C" int32_t ddpg_update_phase(Ddpg* h, ShemsReplay* rp, int32_t phase, co
   REQUIRE(phase >= 0 && phase <= 2, SHEMS_ERR_INVALID, "ddpg_update_phase: phase=%d", phase);
   REQUIRE(h->pop == 1, SHEMS_ERR_INVALID, "ddpg_update_phase: not available for a population handle");
   REQUIRE(!h->per, SHEMS_ERR_STATE, "ddpg_update_phase: not available for a prioritized learner");
+  REQUIRE(h->nstep == 1, SHEMS_ERR_STATE, "ddpg_update_phase: not available for an n-step learner");
   GUARD(h->device);
   if (phase == 0) {
     REQUIRE(rp, SHEMS_ERR_STATE, "ddpg_update_phase: replay missing");
@@ -2014,6 +2097,7 @@ extern "C" int32_t ddpg_dp_connect(Ddpg* h, int32_t rank, int32_t world, const v
   REQUIRE(world >= 1 && world <= DP_MAX_WORLD && rank >= 0 && rank < world, SHEMS_ERR_INVALID, "ddpg_dp_connect: rank=%d world=%d (max %d)", rank, world, DP_MAX_WORLD);
   REQUIRE(h->pop == 1 && !h->dp_on, SHEMS_ERR_STATE, "ddpg_dp_connect: population handle, or already connected");
   REQUIRE(!h->per, SHEMS_ERR_STATE, "ddpg_dp_connect: not available for a prioritized learner");
+  REQUIRE(h->nstep == 1, SHEMS_ERR_STATE, "ddpg_dp_connect: not available for an n-step learner");
   REQUIRE(h->dp_box, SHEMS_ERR_STATE, "ddpg_dp_connect: call ddpg_dp_export on this handle first");
   GUARD(h->device);
   memset(&h->dp, 0, sizeof(h->dp));
@@ -2076,6 +2160,7 @@ extern "C" int32_t ddpg_update_dp(Ddpg* h, ShemsReplay* rp, int32_t n_updates, c
   REQUIRE(h && rp, SHEMS_ERR_INVALID, "ddpg_update_dp: NULL argument");
   REQUIRE(h->dp_on, SHEMS_ERR_STATE, "ddpg_update_dp: call ddpg_dp_connect first");
   REQUIRE(!h->per, SHEMS_ERR_STATE, "ddpg_update_dp: not available for a prioritized learner");
+  REQUIRE(h->nstep == 1, SHEMS_ERR_STATE, "ddpg_update_dp: not available for an n-step learner");
   REQUIRE(n_updates >= 1, SHEMS_ERR_INVALID, "ddpg_update_dp: n_updates=%d", n_updates);
   GUARD(h->device);
   TRY(stage_update_inputs(h, &rp, &seed, idx_host, (long long)n_updates * h->p.batch));
@@ -2367,6 +2452,7 @@ extern "C" int32_t ddpg_episode(Ddpg* h, ShemsEnv* env, ShemsReplay* const* rps,
           "ddpg_episode: bind the environment, the learner and the replay memories to one CUDA stream");
   REQUIRE(env->was_reset, SHEMS_ERR_STATE, "ddpg_episode: reset! must come first");
   if (train) TRY(per_memories_ok(h, rps, "ddpg_episode"));
+  if (train) TRY(nstep_memories_ok(h, rps, "ddpg_episode"));
   if (ensure_rows(env, n_steps)) {  // nothing is enqueued for an episode that would leave the series
     shems_set_error("BoundsError: episode of %d steps from row %d leaves the %d-row series (next_state!, shems_LU1.jl:266-268)", n_steps, env->max_idx,
                     env->nrows);
@@ -2392,6 +2478,8 @@ extern "C" int32_t ddpg_episode(Ddpg* h, ShemsEnv* env, ShemsReplay* const* rps,
   std::vector<uint64_t> seeds((size_t)h->pop);
   if (train && h->per && h->pop == 1 && updates_per_step > 0)   // the post-step kernel below stages the ring, not the tree
     CUDA_TRY(cudaMemcpyAsync(h->trees_dev, &rps[0]->prio, sizeof(float*), cudaMemcpyHostToDevice, h->stream));
+  if (train && h->nstep > 1 && h->pop == 1 && updates_per_step > 0)   // and not the links either
+    CUDA_TRY(cudaMemcpyAsync((void*)h->links_dev, &rps[0]->next, sizeof(const int32_t*), cudaMemcpyHostToDevice, h->stream));
   for (int step = 1; step <= n_steps; ++step) {
     const uint64_t rng_step = (seed * 1000003ull + (uint64_t)step) & 0x7fffffffffffffffull;
     if (train && h->noise_kind == 1) {
@@ -2407,15 +2495,15 @@ extern "C" int32_t ddpg_episode(Ddpg* h, ShemsEnv* env, ShemsReplay* const* rps,
       ShemsReplay* rp = rps[0];
       REQUIRE(rp && rp->device == h->device, SHEMS_ERR_INVALID, "ddpg_episode: replay memory missing or on another device");
       REQUIRE(N <= rp->capacity, SHEMS_ERR_INVALID, "ddpg_episode: %lld instances exceed the memory's capacity %lld", N, (long long)rp->capacity);
-      const long long head = rp->head;
-      TRY(replay_after_rollout(rp, N, h->stream));
+      const long long head = rp->head, cap = rp->capacity;
       CtrlHostPart hp; memset(&hp, 0, sizeof(hp));
       hp.seed = rng_step; hp.update = 0u; hp.use_idx = 0;
-      hp.len = rp->length; hp.head = rp->head; hp.cap = rp->capacity;
+      hp.len = rp->length + N > cap ? cap : rp->length + N; hp.head = (head + N) % cap; hp.cap = cap;   // the ring after this step's push
       ddpg_episode_post_step_kernel<<<(unsigned)((N + 255) / 256), 256, 0, h->stream>>>(rp->ring, rp->capacity, head, h->ep_sprev, h->ep_a, h->ep_r,
                                                                                        h->ep_r64, env->obs, N, ep_return_dev, step == 1,
                                                                                        updates_per_step > 0 ? h->ctrl : nullptr, hp, h->rings_dev);
       CUDA_TRY(cudaGetLastError());
+      TRY(replay_after_rollout(rp, N, N, h->stream));   // after the kernel: the link pass reads the records it wrote
       if (updates_per_step > 0) {
         TRY(ensure_graph(h));
         for (int u = 0; u < updates_per_step; ++u) CUDA_TRY(cudaGraphLaunch(h->graph_exec, h->stream));

@@ -55,6 +55,9 @@ struct FusedArgs {
   const float *src_s, *src_a, *src_r, *src_s2, *src_d; long long src_ld;   // [9][ld], [2][ld], [ld], [9][ld], [ld] or NULL (done = 0)
   DdpgCtrl* ctrl; const int32_t* idx; const float* norm;
   float* xs_w;               // = xs, written by the critic pass
+  // n-step returns (ddpg_set_nstep > 1, rows from the ring): the critic pass walks each row's chain over links[0] with n = *nstep
+  // (ring.cuh ring_nstep) and takes s', r and done from the walk; NULL for 1-step updates
+  const int32_t* const* links; const int* nstep;
 };
 // may this shape run fused?  (widths within the shared-memory plan, whole clusters of 8 rows)
 static inline bool ddpg_fused_shape_ok(int B, int l1, int l2) {

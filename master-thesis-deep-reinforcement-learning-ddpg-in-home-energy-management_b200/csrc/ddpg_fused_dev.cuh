@@ -37,6 +37,9 @@ struct FusedSmem {
   float qv[8], rr[8], dd[8];
   unsigned long long src_row[8];   // where the cluster's 8 sampled transitions live (ring offset or column of the caller's arrays)
   const float* src_ser[8];         // a compact ring record's series row (ring.cuh ring_row), else NULL
+  unsigned long long ns_row[8];    // n-step rows: ring offset of the walk's last record (s' comes from there) ...
+  const float* ns_ser[8];          // ... its series row ...
+  float ns_r[8], ns_d[8];          // ... and the walk's r and done
 };
 
 __device__ __forceinline__ void cp_async4z(float* smem_dst, const float* gsrc, bool valid) {

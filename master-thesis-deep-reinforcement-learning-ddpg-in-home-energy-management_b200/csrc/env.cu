@@ -972,6 +972,6 @@ extern "C" int32_t shems_rollout(ShemsEnv* e, const ShemsRolloutArgs* a) {
   e->max_idx += a->n_steps;
   e->step += a->n_steps;
   e->consistent = true;
-  if (a->replay) return replay_after_rollout(a->replay, total, e->stream);
+  if (a->replay) return replay_after_rollout(a->replay, total, e->n, e->stream);   // step t of instance i went to slot head + t*n + i
   return SHEMS_OK;
 }

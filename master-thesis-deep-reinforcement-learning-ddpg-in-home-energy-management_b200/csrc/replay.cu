@@ -38,6 +38,7 @@ extern "C" int32_t replay_destroy(ShemsReplay* rp) {
   GUARD(rp->device);
   for (int i = 0; i < rp->n_src; ++i) cudaFree(rp->src[i].rows);
   cudaFree(rp->alloc); cudaFree(rp->prio_alloc); cudaFree(rp->idx_scratch); cudaFree(rp->minmax_scratch); cudaFree(rp->group_refs);
+  cudaFree(rp->next);
   delete rp;
   return SHEMS_OK;
 }
@@ -106,13 +107,113 @@ static int prio_refresh(ShemsReplay* rp, long long s0, long long m, cudaStream_t
   return SHEMS_OK;
 }
 
-int replay_after_rollout(ShemsReplay* rp, int64_t n_written, cudaStream_t st) {
+// ---- successor links (ring.cuh: n-step returns)
+// does the record at logical index i continue the one at p?  done(p) == 0 and s(i) == s'(p) in all 9 logical fields, bit for bit
+__device__ __forceinline__ bool ring_continues(const float* ring, long long p, long long i, long long head, long long len, long long cap) {
+  const float* qp = ring + ring_base(ring_slot(p, head, len, cap));
+  const float* qi = ring + ring_base(ring_slot(i, head, len, cap));
+  const float* const* table = ring_table(ring);
+  const float* rowp = ring_row(table, qp);
+  const float* rowi = ring_row(table, qi);
+  if (ring_field(qp, rowp, RING_DONE) != 0.0f) return false;
+  bool same = true;
+#pragma unroll
+  for (int k = 0; k < 9; ++k) same = same && __float_as_uint(ring_field(qi, rowi, RING_S + k)) == __float_as_uint(ring_field(qp, rowp, RING_S2 + k));
+  return same;
+}
+// the link rule after a write whose m surviving records are the logical indices len - m .. len - 1 (len, head: after the write).  One
+// thread per new record i sets next[i] (a link to i + W when that record is new too, else -1) and, when p = i - W is an older record,
+// next[p]; so every slot is written by one thread.
+__global__ void __launch_bounds__(256)
+replay_link_kernel(const float* __restrict__ ring, int32_t* __restrict__ next, long long cap, long long head, long long len, long long m,
+                   long long W) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= m) return;
+  const long long i = len - m + t;
+  const long long j = i + W, p = i - W;
+  next[ring_slot(i, head, len, cap)] = (j < len && ring_continues(ring, i, j, head, len, cap)) ? (int32_t)ring_slot(j, head, len, cap) : -1;
+  if (p >= 0 && p < len - m && ring_continues(ring, p, i, head, len, cap)) next[ring_slot(p, head, len, cap)] = (int32_t)ring_slot(i, head, len, cap);
+}
+
+int replay_after_rollout(ShemsReplay* rp, int64_t n_written, int64_t width, cudaStream_t st) {
   const int64_t m = n_written < rp->capacity ? n_written : rp->capacity;   // the slots that survive the push
   const int64_t s0 = (rp->head + n_written - m) % rp->capacity;
   rp->head = (rp->head + n_written) % rp->capacity;
   rp->length = rp->length + n_written > rp->capacity ? rp->capacity : rp->length + n_written;
-  if (rp->prio && m > 0) return prio_refresh(rp, s0, m, st);
+  if (m <= 0) return SHEMS_OK;
+  if (rp->prio) TRY_PRIO(prio_refresh(rp, s0, m, st));
+  if (rp->next) {
+    replay_link_kernel<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(rp->ring, rp->next, rp->capacity, rp->head, rp->length, m, width);
+    CUDA_TRY(cudaGetLastError());
+  }
   return SHEMS_OK;
+}
+
+extern "C" int32_t replay_enable_successors(ShemsReplay* rp) {
+  REQUIRE(rp, SHEMS_ERR_INVALID, "replay_enable_successors: NULL handle");
+  if (rp->next) return SHEMS_OK;
+  GUARD(rp->device);
+  CUDA_TRY(cudaStreamSynchronize(rp->stream));
+  CUDA_TRY(cudaMalloc(&rp->next, sizeof(int32_t) * (size_t)rp->capacity));
+  CUDA_TRY(cudaMemsetAsync(rp->next, 0xff, sizeof(int32_t) * (size_t)rp->capacity, rp->stream));   // every record: no successor (-1)
+  CUDA_TRY(cudaStreamSynchronize(rp->stream));
+  return SHEMS_OK;
+}
+
+extern "C" int32_t replay_get_successors(ShemsReplay* rp, int32_t* next_host) {
+  REQUIRE(rp && next_host, SHEMS_ERR_INVALID, "replay_get_successors: NULL argument");
+  REQUIRE(rp->next, SHEMS_ERR_STATE, "replay_get_successors: the memory has no successor links (replay_enable_successors)");
+  GUARD(rp->device);
+  const int64_t cap = rp->capacity, len = rp->length;
+  std::vector<int32_t> slots((size_t)cap);
+  CUDA_TRY(cudaStreamSynchronize(rp->stream));
+  CUDA_TRY(cudaMemcpy(slots.data(), rp->next, sizeof(int32_t) * (size_t)cap, cudaMemcpyDeviceToHost));
+  for (int64_t i = 0; i < len; ++i) {
+    const int32_t nx = slots[(size_t)ring_slot(i, rp->head, len, cap)];
+    next_host[i] = nx < 0 ? -1 : (int32_t)ring_logical(nx, rp->head, len, cap);
+  }
+  return SHEMS_OK;
+}
+
+extern "C" int32_t replay_set_successors(ShemsReplay* rp, const int32_t* next_host) {
+  REQUIRE(rp && next_host, SHEMS_ERR_INVALID, "replay_set_successors: NULL argument");
+  REQUIRE(rp->next, SHEMS_ERR_STATE, "replay_set_successors: the memory has no successor links (replay_enable_successors)");
+  const int64_t cap = rp->capacity, len = rp->length;
+  for (int64_t i = 0; i < len; ++i)
+    REQUIRE(next_host[i] == -1 || (next_host[i] > i && next_host[i] < len), SHEMS_ERR_INVALID,
+            "replay_set_successors: next[%lld]=%d must be -1 or a newer record (%lld < next < %lld)", (long long)i, next_host[i], (long long)i,
+            (long long)len);
+  GUARD(rp->device);
+  std::vector<int32_t> slots((size_t)cap, -1);
+  for (int64_t i = 0; i < len; ++i)
+    if (next_host[i] >= 0) slots[(size_t)ring_slot(i, rp->head, len, cap)] = (int32_t)ring_slot(next_host[i], rp->head, len, cap);
+  CUDA_TRY(cudaMemcpyAsync(rp->next, slots.data(), sizeof(int32_t) * (size_t)cap, cudaMemcpyHostToDevice, rp->stream));
+  CUDA_TRY(cudaStreamSynchronize(rp->stream));   // the host source lives on this stack frame
+  return SHEMS_OK;
+}
+
+// the n-step minibatch of update 0 of ddpg_update(seed) (or of the caller's logical indices): row j starts at the drawn record and
+// walks its chain (ring_nstep); s, a from rec_0, s' from rec_{k-1}, r and done the walk's; k [B] the records walked
+__global__ void __launch_bounds__(128)
+replay_sample_nstep_kernel(const float* __restrict__ ring, const int32_t* __restrict__ next, long long cap, long long head, long long len,
+                           const int32_t* __restrict__ idx, unsigned long long seed, int B, int n, float gamma, float* __restrict__ s,
+                           float* __restrict__ a, float* __restrict__ r, float* __restrict__ s2, float* __restrict__ done, int32_t* __restrict__ k_out) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= B) return;
+  const long long li = idx ? idx[j] : ring_draw(seed, j, 0u, len);
+  const long long slot = ring_slot(li, head, len, cap);
+  const float* q = ring + ring_base(slot);
+  const float* row = ring_row(ring_table(ring), q);
+  const RingNstep w = ring_nstep(ring, ring_table(ring), next, slot, n, gamma, true);
+  const float* q2 = ring + ring_base(w.last);
+  const float* row2 = ring_row(ring_table(ring), q2);
+#pragma unroll
+  for (int k = 0; k < 9; ++k) { s[k * B + j] = ring_field(q, row, RING_S + k); s2[k * B + j] = ring_field(q2, row2, RING_S2 + k); }
+  a[j] = ring_field(q, row, RING_A);
+  a[B + j] = ring_field(q, row, RING_A + 1);
+  r[j] = w.r;
+  done[j] = w.done;
+  if (k_out) k_out[j] = w.k;
 }
 
 extern "C" int32_t replay_enable_priorities(ShemsReplay* rp) {
@@ -255,7 +356,7 @@ extern "C" int32_t replay_push(ShemsReplay* rp, const float* s_dev, const float*
   replay_push_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, rp->stream>>>(rp->ring, rp->capacity, rp->head, s_dev, a_dev, r_dev, s2_dev,
                                                                            done_dev, n, first);
   CUDA_TRY(cudaGetLastError());
-  return replay_after_rollout(rp, n, rp->stream);
+  return replay_after_rollout(rp, n, n, rp->stream);   // one step of n instances
 }
 
 // remember() for a population: arrays are SoA over all N = P*n_per instances, learner l = instances l*n_per .. l*n_per+n_per-1
@@ -301,7 +402,7 @@ extern "C" int32_t replay_push_groups(ShemsReplay* const* rps, int32_t n_groups,
                                                                                                 r_dev, s2_dev, done_dev, n_per,
                                                                                                 n_per * n_groups);
   CUDA_TRY(cudaGetLastError());
-  for (int g = 0; g < n_groups; ++g) TRY_PRIO(replay_after_rollout(rps[g], n_per, r0->stream));
+  for (int g = 0; g < n_groups; ++g) TRY_PRIO(replay_after_rollout(rps[g], n_per, n_per, r0->stream));
   return SHEMS_OK;
 }
 
@@ -351,6 +452,32 @@ extern "C" int32_t replay_sample(ShemsReplay* rp, int32_t batch, const int32_t* 
   }
   replay_sample_kernel<<<(batch + 127) / 128, 128, 0, rp->stream>>>(rp->ring, rp->capacity, rp->head, rp->length, didx, seed, 0u, batch,
                                                                    s_dev, a_dev, r_dev, s2_dev, done_dev);
+  CUDA_TRY(cudaGetLastError());
+  if (idx_host) CUDA_TRY(cudaStreamSynchronize(rp->stream));  // idx_host was staged asynchronously
+  return SHEMS_OK;
+}
+
+extern "C" int32_t replay_sample_nstep(ShemsReplay* rp, int32_t batch, const int32_t* idx_host, uint64_t seed, int32_t n, float gamma, float* s_dev,
+                                       float* a_dev, float* r_dev, float* s2_dev, float* done_dev, int32_t* k_dev) {
+  REQUIRE(rp && s_dev && a_dev && r_dev && s2_dev && done_dev, SHEMS_ERR_INVALID, "replay_sample_nstep: NULL argument");
+  REQUIRE(batch >= 1, SHEMS_ERR_INVALID, "replay_sample_nstep: batch=%d", batch);
+  REQUIRE(n >= 1 && n <= NSTEP_MAX, SHEMS_ERR_INVALID, "replay_sample_nstep: n=%d outside 1..%d", n, NSTEP_MAX);
+  REQUIRE(isfinite(gamma) && gamma >= 0.0f && gamma <= 1.0f, SHEMS_ERR_INVALID, "replay_sample_nstep: gamma=%g outside [0, 1]", (double)gamma);
+  REQUIRE(rp->next || n == 1, SHEMS_ERR_STATE, "replay_sample_nstep: n=%d needs successor links (replay_enable_successors)", n);
+  REQUIRE(rp->length > 0, SHEMS_ERR_STATE, "replay_sample_nstep: memory is empty");
+  GUARD(rp->device);
+  const int32_t* didx = nullptr;
+  if (idx_host) {
+    for (int j = 0; j < batch; ++j)
+      REQUIRE(idx_host[j] >= 0 && idx_host[j] < rp->length, SHEMS_ERR_INVALID, "replay_sample_nstep: idx[%d]=%d outside 0..%lld", j, idx_host[j],
+              (long long)rp->length - 1);
+    int st = ensure_idx_scratch(rp, batch);
+    if (st) return st;
+    CUDA_TRY(cudaMemcpyAsync(rp->idx_scratch, idx_host, sizeof(int32_t) * batch, cudaMemcpyHostToDevice, rp->stream));
+    didx = rp->idx_scratch;
+  }
+  replay_sample_nstep_kernel<<<(batch + 127) / 128, 128, 0, rp->stream>>>(rp->ring, rp->next, rp->capacity, rp->head, rp->length, didx, seed, batch,
+                                                                         n, gamma, s_dev, a_dev, r_dev, s2_dev, done_dev, k_dev);
   CUDA_TRY(cudaGetLastError());
   if (idx_host) CUDA_TRY(cudaStreamSynchronize(rp->stream));  // idx_host was staged asynchronously
   return SHEMS_OK;

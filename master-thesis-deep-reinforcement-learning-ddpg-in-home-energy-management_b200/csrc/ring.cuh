@@ -162,6 +162,45 @@ __host__ __device__ __forceinline__ float ring_priority(float y, float q, float 
   return (float)pow((double)fabsf(d) + (double)eps, (double)alpha);
 }
 
+// ---- n-step returns (replay_enable_successors)
+// A memory with successor links keeps int32 next[cap] beside the ring: next[slot] = the physical slot of the record that continues
+// the one in `slot`, or -1.  After a write of per-step width W (replay_after_rollout), every surviving new record i (logical index)
+// gets next[i] = -1, and the record p = i - W, when it exists, has done == 0 and its s' equals s(i) in all 9 logical fields bit for
+// bit, gets next[p] = i.  A reset breaks the state equality, so episode boundaries end a chain; a link always points to a newer
+// record, and the ring overwrites oldest first, so no link outlives its target.
+#define NSTEP_MAX 16
+struct RingNstep {
+  long long last;   // slot of rec_{k-1}: s' comes from here
+  float r, done;    // RN32(R) and RN32(1 - RN64(γ^{k-1} RN64(1 - done(rec_{k-1})))): the 1-step TD epilogue then bootstraps with ~γ^k
+  int k;            // records walked, 1 .. n
+};
+// the walk from the record in slot0 over at most n records with the learner's γ, in Float64 with explicit roundings (no contraction):
+//   gp = 1, R = r(rec_0);  while k < n, done(rec_{k-1}) == 0 and next[rec_{k-1}] >= 0:  gp = RN64(gp γ), R = RN64(R + RN64(gp r(rec_k)))
+// sum = false skips R (the s' fields of the last record are all such a thread needs).  table: ring_table(ring).
+__device__ __forceinline__ RingNstep ring_nstep(const float* ring, const float* const* table, const int32_t* next, long long slot0, int n,
+                                                float gamma, bool sum) {
+  const float* q = ring + ring_base(slot0);
+  const float* row = ring_row(table, q);
+  double gp = 1.0, R = sum ? (double)ring_field(q, row, RING_R) : 0.0;
+  float d = ring_field(q, row, RING_DONE);
+  RingNstep w;
+  w.last = slot0; w.k = 1;
+  while (w.k < n && d == 0.0f) {
+    const int32_t nx = next[w.last];
+    if (nx < 0) break;
+    w.last = nx;
+    q = ring + ring_base(nx);
+    row = ring_row(table, q);
+    gp = __dmul_rn(gp, (double)gamma);
+    if (sum) R = __dadd_rn(R, __dmul_rn(gp, (double)ring_field(q, row, RING_R)));
+    d = ring_field(q, row, RING_DONE);
+    ++w.k;
+  }
+  w.r = (float)R;
+  w.done = (float)__dsub_rn(1.0, __dmul_rn(gp, __dsub_rn(1.0, (double)d)));
+  return w;
+}
+
 // the words both record forms store; a compact record adds its tag, a full one the other 14 fields
 __device__ __forceinline__ void ring_store_own(float* q, float sb, float sev, float a0, float a1, float r, float sb2, float sev2) {
   q[(RING_S + 0) * 32] = sb; q[(RING_S + 1) * 32] = sev;

@@ -130,6 +130,46 @@ class Replay:
         L.check(self.lib.replay_sample_prioritized(self._h, int(batch), int(seed) & (2**64 - 1), float(beta), _ptr(idx), _ptr(w)))
         return idx, w
 
+    # ---- n-step returns (replay_enable_successors): a successor link per slot, kept by every writer
+    def enable_successors(self):
+        """every record starts with no successor; every write from now on links a new record to the one it continues"""
+        L.check(self.lib.replay_enable_successors(self._h))
+        self.has_successors = True
+        return self
+
+    has_successors = False
+
+    def successors(self):
+        """successor of every record in logical order (oldest first): a logical index or -1, [len] int32"""
+        nx = np.empty(len(self), np.int32)
+        L.check(self.lib.replay_get_successors(self._h, nx.ctypes.data_as(L.PI)))
+        return nx
+
+    def set_successors(self, nx):
+        """checkpoint restore: nx [len] in logical order, each -1 or in (i, len)"""
+        nx = np.ascontiguousarray(nx, np.int32)
+        assert nx.size == len(self)
+        L.check(self.lib.replay_set_successors(self._h, nx.ctypes.data_as(L.PI)))
+
+    def sample_nstep(self, batch, seed=0, n=3, gamma=0.99, idx=None):
+        """what update 0 of an n-step Learner.replay(rng_rpl=seed) trains on (or the rows starting at the logical indices idx):
+        (s [9][B], a [2][B], r [B], s' [9][B], done [B], k [B] int32) device tensors; r is the n-step return and done folds
+        gamma^(k-1) in, so that gamma (1 - done) is the bootstrap factor gamma^k"""
+        d = self._dev
+        s = torch.empty((9, batch), dtype=torch.float32, device=d)
+        a = torch.empty((2, batch), dtype=torch.float32, device=d)
+        r = torch.empty(batch, dtype=torch.float32, device=d)
+        s2 = torch.empty((9, batch), dtype=torch.float32, device=d)
+        dn = torch.empty(batch, dtype=torch.float32, device=d)
+        k = torch.empty(batch, dtype=torch.int32, device=d)
+        ip = None
+        if idx is not None:
+            idx = np.ascontiguousarray(idx, np.int32)
+            ip = idx.ctypes.data_as(L.PI)
+        L.check(self.lib.replay_sample_nstep(self._h, int(batch), ip, int(seed) & (2**64 - 1), int(n), float(gamma), _ptr(s), _ptr(a), _ptr(r),
+                                             _ptr(s2), _ptr(dn), _ptr(k)))
+        return s, a, r, s2, dn, k
+
     def get(self):
         n = len(self)
         s, a, r, s2, d = (np.empty((9, n), np.float32), np.empty((2, n), np.float32), np.empty(n, np.float32),
@@ -196,6 +236,15 @@ class Learner:
         on, a, b, e = C.c_int32(), C.c_float(), C.c_float(), C.c_float()
         L.check(self.lib.ddpg_get_prioritized(self._h, C.byref(on), C.byref(a), C.byref(b), C.byref(e)))
         return dict(alpha=a.value, beta=b.value, eps=e.value) if on.value else None
+
+    def set_nstep(self, n):
+        """ddpg_set_nstep: n-step returns (1 <= n <= 16) for every learner of the handle; n > 1 needs memories with successor links
+        (Replay.enable_successors), one per learner"""
+        L.check(self.lib.ddpg_set_nstep(self._h, int(n)))
+        return self
+
+    def get_nstep(self):
+        return int(self.lib.ddpg_get_nstep(self._h))
 
     def select(self, learner):
         """ddpg_select_learner: the learner of a population that set/get_layer, get_grad, set_norm and losses address."""
@@ -509,9 +558,10 @@ class Driver:
     (Julia's string-concatenated MersenneTwister seeds cannot be reproduced)."""
 
     def __init__(self, env_train, env_eval=None, learner=None, mem_size=24_000, ep_length=72, sigma=0.1, updates_per_step=1,
-                 rng_run=1231, noise_type="gn", theta=0.15, ou_dt=1e-2, native=True, per=None):
+                 rng_run=1231, noise_type="gn", theta=0.15, ou_dt=1e-2, native=True, per=None, nstep=1):
         """per = (alpha, beta0[, eps]) or a dict of them: proportional prioritized replay, β annealed linearly from beta0 to 1
-        over the episodes of run_episodes (per_beta)"""
+        over the episodes of run_episodes (per_beta).  nstep > 1: n-step returns (the memory keeps successor links from its first
+        write on)"""
         self.env_train, self.env_eval = env_train, env_eval
         self.learner = learner if learner is not None else Learner(device=env_train.device)
         self.memory = Replay(mem_size, device=env_train.device)
@@ -529,6 +579,10 @@ class Driver:
         if self.per is not None:
             self.memory.enable_priorities()
             self.learner.set_prioritized(self.per["alpha"], self.per["beta0"], self.per["eps"])
+        self.nstep = int(nstep)
+        if self.nstep > 1:
+            self.memory.enable_successors()
+            self.learner.set_nstep(self.nstep)
 
     def set_beta(self, episode, num_ep):
         """prioritized replay: β of training episode `episode` of num_ep (per_beta); run_episodes calls it before every episode"""
@@ -671,7 +725,8 @@ class PopulationDriver:
     hparams: per-learner hyper-parameters, a dict of lists of length P with keys from Learner.HPARAMS (lr_actor, lr_critic, gamma,
     tau, noise_scale); missing keys keep the DdpgParams values (noise_scale: 1).  Learner l explores with σ_eff = sigma × noise_scale[l],
     so a σ grid is sigma=1.0 with the grid values as noise_scale.  per = (alpha, beta0[, eps]): prioritized replay for every learner,
-    β annealed from beta0 to 1 over the episodes of run_episodes, as Driver(per=...).
+    β annealed from beta0 to 1 over the episodes of run_episodes, as Driver(per=...).  nstep > 1: n-step returns for every learner,
+    as Driver(nstep=...).
 
     eval_series ([8][nrows], or [G][8][nrows] with one series per run of equal chargers) adds the reference's evaluation protocol
     (run_episodes / inference): an evaluation handle of test_runs instances per learner, one group per charger run, with
@@ -680,7 +735,7 @@ class PopulationDriver:
     instances of its charger, env_id_base 0), as every run of the reference evaluates with the same rng."""
 
     def __init__(self, series, chargers, seeds, n_envs=64, mem_size=24_000, ep_length=72, sigma=0.1, device=0, use_tensor_cores=1, native=True,
-                 hparams=None, eval_series=None, test_runs=100, per=None, **ddpg_kw):
+                 hparams=None, eval_series=None, test_runs=100, per=None, nstep=1, **ddpg_kw):
         from .env import Shems
         assert len(chargers) == len(seeds)
         self.native = bool(native)
@@ -710,6 +765,11 @@ class PopulationDriver:
             for m in self.mems:
                 m.enable_priorities()
             self.learner.set_prioritized(self.per["alpha"], self.per["beta0"], self.per["eps"])
+        self.nstep = int(nstep)     # n-step returns for every learner, as Driver(nstep=...)
+        if self.nstep > 1:
+            for m in self.mems:
+                m.enable_successors()
+            self.learner.set_nstep(self.nstep)
         self._dev = torch.device("cuda", int(device))
         self._s_prev = torch.empty((9, self.N), dtype=torch.float32, device=self._dev)
         self.n_env_steps = 0

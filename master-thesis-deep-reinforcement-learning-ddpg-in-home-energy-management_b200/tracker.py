@@ -63,7 +63,7 @@ def save_checkpoint(path, learner, s_min=None, s_max=None, memories=None, **scor
     the hyper-parameters (`l{l}_hparams` = [lr_actor, lr_critic, gamma, tau, noise_scale] float32: ddpg_get_hparams), the best
     actors (`l{l}_actor_best_W1` ...) with `best_score` [P] / `best_run` [P] (ddpg_get_best; a score keyword of the same name
     replaces them), OUNoise.X when OU episodes ran, and — with `memories` (one Replay per learner) — the replay memories in logical order,
-    with their priorities and p_max when they have them."""
+    with their priorities and p_max, and their successor links, when they have them."""
     out = {}
     P = learner.population
     keep = getattr(learner, "_sel", 0)
@@ -103,6 +103,8 @@ def save_checkpoint(path, learner, s_min=None, s_max=None, memories=None, **scor
                 out[f"mem{l}_prio"], pm = m.priorities()
                 out[f"mem{l}_pmax"] = np.float32(pm)
                 out[f"mem{l}_head"] = np.int64(m.head)
+            if m.has_successors:   # n-step returns: the links, in logical indices
+                out[f"mem{l}_next"] = m.successors()
     if s_min is not None:
         out["s_min"], out["s_max"] = np.asarray(s_min, np.float32), np.asarray(s_max, np.float32)
     for k, v in scores.items():
@@ -160,4 +162,7 @@ def load_checkpoint(path, learner, memories=None):
             if f"mem{l}_prio" in z:
                 m.enable_priorities()
                 m.set_priorities(z[f"mem{l}_prio"], float(z[f"mem{l}_pmax"]))
+            if f"mem{l}_next" in z:   # after the pushes, which link by their own rule
+                m.enable_successors()
+                m.set_successors(z[f"mem{l}_next"])
     return z

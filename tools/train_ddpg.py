@@ -26,6 +26,7 @@ ap.add_argument("--sigma", type=float, default=0.1)
 ap.add_argument("--tc", type=int, default=1, help="TF32 tensor cores for the 250x500 products")
 ap.add_argument("--noise", default="gn", choices=["gn", "ou"])
 ap.add_argument("--per", default=None, metavar="ALPHA,BETA0", help="prioritized replay, beta annealed from BETA0 to 1 over the episodes")
+ap.add_argument("--nstep", type=int, default=1, help="n-step returns (1: the 1-step TD target)")
 args = ap.parse_args()
 
 train = sb.series.synth_charger98(4320, seed=98)
@@ -35,7 +36,8 @@ ev = sb.Shems(72, evals, n_envs=1024)          # evaluation: 1024 random 72-step
 le = sb.Learner(params=sb.default_ddpg_params(batch=args.batch, use_tensor_cores=args.tc))   # γ=0.99, τ=1e-3, η=1e-4/1e-3, 250/500 (README.md:68-86)
 le.init(args.seed)
 drv = sb.Driver(env, ev, learner=le, mem_size=args.mem, ep_length=72, sigma=args.sigma, updates_per_step=args.updates_per_step,
-                rng_run=args.seed, noise_type=args.noise, per=tuple(float(x) for x in args.per.split(",")) if args.per else None)
+                rng_run=args.seed, noise_type=args.noise, per=tuple(float(x) for x in args.per.split(",")) if args.per else None,
+                nstep=args.nstep)
 t0 = time.time()
 drv.populate_memory()
 drv.min_max_buffer()

@@ -39,6 +39,7 @@ ap.add_argument("--test-runs", type=int, default=100, help="evaluation episodes 
 ap.add_argument("--inference-dir", default=None, help="write the test-set inference CSVs of the best actors here (needs --test-every)")
 ap.add_argument("--pbt", default=None, metavar="EVERY,FRAC", help="population-based training every EVERY evaluation rounds, share FRAC (needs --test-every)")
 ap.add_argument("--per", default=None, metavar="ALPHA,BETA0", help="prioritized replay for every learner, beta annealed from BETA0 to 1")
+ap.add_argument("--nstep", type=int, default=1, help="n-step returns for every learner (1: the 1-step TD target)")
 ap.add_argument("--pbt-factors", default="0.8,1.25", metavar="LO,HI", help="perturbation factors of --pbt")
 ap.add_argument("--pbt-keys", default=",".join(sb.Learner.HPARAMS), metavar="NAME,...", help="hyper-parameters --pbt perturbs")
 args = ap.parse_args()
@@ -80,6 +81,7 @@ if protocol:
     drv_kw.update(eval_series=sb.series.synth_charger98(1440, seed=1440), test_runs=args.test_runs)
 if args.per:
     drv_kw["per"] = tuple(float(x) for x in args.per.split(","))
+drv_kw["nstep"] = args.nstep
 drv = sb.PopulationDriver(ser, chargers=chargers, seeds=seeds, n_envs=args.envs, device=local, use_tensor_cores=args.tc, hparams=hparams, **drv_kw)
 t0 = time.time()
 drv.populate_memory()
